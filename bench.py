@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's B200 path
     python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs
 
 A "step" is one training step (Diffusion.loss forward + backward, gradient all-reduce when N > 1,
 global-norm clip, AdamW) on one synthetic batch.  Workload (BASELINE.json configs[1]): the
@@ -67,7 +68,32 @@ def parse_args():
     ap.add_argument("--no-gpu-comparator", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the ensemble-generation and more_blocks side measurements")
     ap.add_argument("--kernel-table", default="", help="write the per-kernel breakdown to this file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32, "
+                         "64 MB at most); the inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
+    return args
+
+
+DUMP_BUDGET = 63_000_000  # bytes of array data over all files: the .npy headers keep the total under 64 MB
+
+
+def dump_outputs(out_dir, outputs):
+    """Write every tensor of `outputs` as out_dir/<name>.npy in float32, smallest first.  One larger than its share of
+    what is left of DUMP_BUDGET is written flattened, as the elements at a fixed sample of positions (sorted, drawn
+    by a generator seeded with 0: the same positions in every run and every build)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = sorted(((k, v.detach().float().cpu().numpy()) for k, v in outputs.items()), key=lambda kv: kv[1].size)
+    left = DUMP_BUDGET
+    for i, (name, a) in enumerate(arrays):
+        share = left // (len(arrays) - i) // a.itemsize
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def load_peaks():
@@ -312,6 +338,8 @@ def run_b200(args, H, W, arch_kw):
     diff = Diffusion(UNet(**arch_kw), timesteps=1000).to(dev)
     diff.train()
     eng = TrainEngine(diff, (B, 1, H, W), (B, 1, Kf, H, W), use_graph=not args.no_graph)
+    # the seeded starting state (weights, AdamW moments, step count and loss scale) for --dump-outputs
+    start = [t.clone() for t in (eng.opt.p, eng.opt.m, eng.opt.v, eng.opt.state)] if args.dump_outputs else None
 
     # synthetic (member, time, lat, lon, channel) ensemble; a small pool of pinned host batches
     ds = SyntheticEnsemble(members=4, times=max(8, Kf + 5), lat=H, lon=W, seed=1234 + rank, K=Kf)
@@ -365,6 +393,33 @@ def run_b200(args, H, W, arch_kw):
     losses.clear()
     ms_e2e, _ = timed(e2e_step)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # What is written is the last timed step (the e2e pass's last TrainEngine.step: same graph, same batch, the
+        # RNG where the timed steps left it) repeated once, untimed, from the seeded starting state.  The timed step
+        # itself starts from weights that differ from run to run by more than rounding: fp32 atomics add in a
+        # different order each time, and AdamW's normalised update turns a last-bit difference in a near-zero
+        # gradient into a full step of either sign, so the weights drift apart over the timed steps.  From the seeded
+        # state, two runs and two builds start from the same inputs.  The weights the repeated step leaves are not
+        # written: its update already flips sign where the gradient is near zero (1e-4 of max|w| between two runs, 10x
+        # the gradient's difference; profiles/r03_dump_reproducibility.txt), and they follow elementwise from the
+        # gradient and the seeded state.  The state the timed run reached and the RNG are put back afterwards, so
+        # every reported field still describes the timed run.
+        live = (eng.opt.p, eng.opt.m, eng.opt.v, eng.opt.state)
+        reached, rng = [t.clone() for t in live], torch.cuda.get_rng_state(dev)
+        for dst, src in zip(live, start):
+            dst.copy_(src)
+        scale = eng.opt.loss_scale.clone()
+        cond, x0 = pool[(args.steps - 1) % len(pool)]
+        eng.step(x0, cond)
+        # p.grad views the flat gradient buffer, which holds the loss-scaled gradient before clipping (module order)
+        outputs = {"loss": eng.loss, "grad_norm": eng.grad_norm, "loss_scale": eng.opt.loss_scale,
+                   "gradient": torch.cat([p.grad.reshape(-1) for p in diff.parameters() if p.requires_grad]) / scale}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
+        del outputs
+        for dst, src in zip(live, reached):
+            dst.copy_(src)
+        torch.cuda.set_rng_state(rng, dev)
 
     in_sync = None
     if world > 1:
@@ -479,7 +534,7 @@ def run_b200(args, H, W, arch_kw):
         os._exit(0)
 
 
-def measure_sampling(args, H, W, arch_kw, dev, rank, world, steps, warmup, B=16):
+def measure_sampling(args, H, W, arch_kw, dev, rank, world, steps, warmup, B=16, dump_dir=""):
     """BASELINE.json's second metric, "ensemble-gen fields/s": reverse-diffusion steps for a batch of independent
     fields (inference.py:217-232 -> model.py:186-194), one CUDA-graph replay per step, fields sharded over ranks
     (each rank its own batch, no collective inside the chain).  A step = one UNet call (F = 1) + fused p_sample
@@ -516,6 +571,8 @@ def measure_sampling(args, H, W, arch_kw, dev, rank, world, steps, warmup, B=16)
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"x": eng.x})   # the fields after the last timed reverse step
     finite = bool(torch.isfinite(eng.x).all())
     gflop = 178.5 * (H * W) / (192 * 288) if arch_kw is BASELINE_KW else None  # SURVEY 8(d): per UNet call per field
     peaks = load_peaks()
@@ -654,7 +711,8 @@ def run_sample(args, H, W, arch_kw):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     B = args.batch if args.batch != 2 else 16  # inference.py:180 default batch_size 16
-    out = measure_sampling(args, H, W, arch_kw, dev, rank, world, steps=args.steps, warmup=args.warmup, B=B)
+    out = measure_sampling(args, H, W, arch_kw, dev, rank, world, steps=args.steps, warmup=args.warmup, B=B,
+                           dump_dir=args.dump_outputs)
     if rank == 0 and args.kernel_table:
         # untimed instrumented reverse step: per-C-ABI-call device time
         from cesm_emulator_b200 import _lib

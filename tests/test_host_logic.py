@@ -79,8 +79,9 @@ def _bucket_worker(rank, world, port, q):
         assert buckets._pending == [0] * buckets.n_buckets, buckets._pending
         buckets.finish_step()
         norm = buckets.clip_(1e9)
-        # the flat buffer pads every tensor to a 64-byte boundary: compare the per-parameter views
-        q.put((rank, torch.cat([p.grad.reshape(-1) for p in buckets.params]), x, float(norm)))
+        # the flat buffer pads every tensor to a 64-byte boundary: compare the per-parameter views.  numpy copies:
+        # a tensor is passed as a file descriptor that the parent fetches from this process, which may have exited
+        q.put((rank, torch.cat([p.grad.reshape(-1) for p in buckets.params]).numpy(), x.numpy(), float(norm)))
     finally:
         dist.destroy_process_group()
 
@@ -98,6 +99,7 @@ def test_grad_buckets_allreduce_world2_gloo():
         p.join(timeout=60)
         assert p.exitcode == 0
     (_, g0, x0, n0), (_, g1, x1, n1) = res
+    g0, x0, g1, x1 = (torch.from_numpy(a) for a in (g0, x0, g1, x1))
     assert torch.equal(g0, g1)  # every rank holds the same averaged gradient
     # single-process run over the concatenated batch gives the same gradient (mean over both halves)
     from cesm_emulator_b200.engine import _ready_order

@@ -128,6 +128,8 @@ _SIGNATURES: dict[str, list] = {
     "cesm_tattn_proj_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_long_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_long_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
+    "cesm_mattn_fwd": [_P, _P, _P, _I, _I, _I, _I, _F, _P],
+    "cesm_mattn_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P],
     "cesm_linattn_fwd": [_P, _P, _P, _I, _I, _I, _I, _F, _P],
     "cesm_linattn_fwd_out": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_linattn_bwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P],

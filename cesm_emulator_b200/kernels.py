@@ -450,6 +450,32 @@ def tattn_proj_bwd(xn, wqkv_packed, bias, cs, sn, dout, B: int, F: int, HW: int,
     return dqkv, dbias
 
 
+def mattn_fwd(qkv, NI: int, n: int, H: int, D: int, scale: float):
+    """Full softmax attention over the n pixels of each of NI images (use_mid_attn's bottleneck block).
+    qkv: fp16 [NI*n, 3*H*D] -> (out fp16 [NI*n, H*D], lse fp32 [NI*n, H])."""
+    _req_cuda(qkv)
+    assert qkv.dtype == H16 and qkv.shape == (NI * n, 3 * H * D), (tuple(qkv.shape), NI, n, H, D)
+    out = torch.empty((NI * n, H * D), dtype=H16, device=qkv.device)
+    lse = torch.empty((NI * n, H), dtype=torch.float32, device=qkv.device)
+    _lib.call("cesm_mattn_fwd", _ptr(qkv), _ptr(out), _ptr(lse), NI, n, H, D, scale, _stream(),
+              _meta={"kind": "fwd", "flops": 4.0 * NI * H * n * n * D, "bytes": float(qkv.numel() * 2 + out.numel() * 2)})
+    return out, lse
+
+
+def mattn_bwd(qkv, out, lse, dout, NI: int, n: int, H: int, D: int, scale: float):
+    """-> dqkv fp16 [NI*n, 3*H*D] (q, k and v gradients; no accumulation, deterministic)."""
+    _req_cuda(qkv, out, lse, dout)
+    assert qkv.dtype == H16 and out.dtype == H16 and dout.dtype == H16 and lse.dtype == torch.float32
+    assert qkv.shape == (NI * n, 3 * H * D) and out.shape == dout.shape == (NI * n, H * D) and lse.numel() == NI * n * H
+    dqkv = torch.empty_like(qkv)
+    delta = torch.empty((NI * n, H), dtype=torch.float32, device=qkv.device)
+    # S and P recomputed twice (dQ pass, dK/dV pass), dP twice, dQ, dK, dV once: 4 + 4 + 2 + 2 + 2 = 14 n^2 D per head
+    _lib.call("cesm_mattn_bwd", _ptr(qkv), _ptr(out), _ptr(lse), _ptr(dout), _ptr(dqkv), _ptr(delta), NI, n, H, D, scale,
+              _stream(), _meta={"kind": "bwd", "flops": 14.0 * NI * H * n * n * D,
+                                "bytes": float(qkv.numel() * 4 + out.numel() * 2 + dout.numel() * 2)})
+    return dqkv
+
+
 def linattn_fwd(qkv, NI: int, n: int, H: int, D: int, scale: float):
     """-> (out fp16 [NI*n, H*D], ws fp32 workspace kept for the backward)."""
     _req_cuda(qkv)

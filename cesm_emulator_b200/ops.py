@@ -6,7 +6,7 @@ reference's layouts; the fp16 GEMM operand copies (forward layout and data-gradi
 a registry (`PackCache`) and are refreshed by ONE batched kernel per optimizer step.
 
 Two granularities are offered:
-  * block level (`ResnetBlockFn`, `TemporalAttnBlockFn`, `SpatialAttnBlockFn`): one autograd node
+  * block level (`ResnetBlockFn`, `TemporalAttnBlockFn`, `SpatialAttnBlockFn`, `MidAttnBlockFn`): one autograd node
     per reference block (video_net.py ResnetBlock / Residual(PreNorm(attention))), with a
     hand-ordered backward in which residual-gradient adds live in GEMM / LayerNorm epilogues and
     conv-bias gradients come out of the GroupNorm backward's per-channel sums.  `UNetModel3D` uses these.
@@ -544,6 +544,25 @@ class TemporalAttnCoreFn(_Fn):
         return dqkv, dbias, None, None, None, None, None, None, None
 
 
+class MidAttnCoreFn(_Fn):
+    """softmax((q * scale) k^T) v over all n pixels of each image, no mask / bias / rotary (video_net.py:413-453 as the
+    use_mid_attn block calls it).  qkv: [NI*n, 3*H*D] -> [NI*n, H*D]."""
+
+    @staticmethod
+    def forward(ctx, qkv, NI: int, n: int, H: int, D: int):
+        qkv = qkv.contiguous()
+        out, lse = K.mattn_fwd(qkv, NI, n, H, D, D ** -0.5)
+        ctx.save_for_backward(qkv, out, lse)
+        ctx.dims = (NI, n, H, D)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        qkv, out, lse = ctx.saved_tensors
+        NI, n, H, D = ctx.dims
+        return K.mattn_bwd(qkv, out, lse, dout.contiguous(), NI, n, H, D, D ** -0.5), None, None, None, None
+
+
 class RelPosBiasFn(_Fn):
     """Embedding gather of the T5 bucket table -> [heads, n, n] (video_net.py:302-310).  The
     table has 32 x heads entries; gather and scatter-add are index ops on a few hundred floats."""
@@ -774,6 +793,54 @@ class TemporalAttnBlockFn(_Fn):
             dx, dg = K.ln_bwd(x, g, dxn, dy, eps)
             dgamma = dg.view(ctx.gshape)
         return dx, dgamma, dwqkv, dwout, dbias, None, None, None, None, None
+
+
+class MidAttnBlockFn(_Fn):
+    """Residual(PreNorm(EinopsToAndFrom('b c f h w' -> 'b f (h w) c', Attention))) (use_mid_attn=True,
+    video_net.py:713-719) as one node: y = x + to_out(softmax attention over the h*w pixels of each frame of
+    to_qkv(LN(x))).  No rotary embedding, no position bias; every frame (also F = 1) runs the full attention.
+    args: x, gamma [1,C,1,1,1], wqkv [3*hidden, C], wout [C, hidden], meta(heads, dim_head, eps, cq, co)."""
+
+    @staticmethod
+    def forward(ctx, x, gamma, wqkv, wout, meta):
+        x = x.contiguous()
+        NI, H_, W_, C = x.shape
+        heads, D, eps = meta.heads, meta.dim_head, meta.eps
+        hidden, n = heads * D, H_ * W_
+        g = gamma.reshape(-1)
+        train = _train(ctx)
+        xn = K.ln_fwd(x, g, eps)
+        qkv = K.igemm(xn, _conv_fwd_weight(meta.cq, wqkv, 3 * hidden, C, 1, train))
+        o, lse = K.mattn_fwd(qkv.view(-1, 3 * hidden), NI, n, heads, D, D ** -0.5)
+        y = K.igemm(o.view(NI, H_, W_, hidden), _conv_fwd_weight(meta.co, wout, C, hidden, 1, train), residual=x)
+        if train:
+            ctx.wdq = _conv_dgrad_weights(meta.cq, wqkv, 3 * hidden, C, 0, 1, train)[0]
+            ctx.wdo = _conv_dgrad_weights(meta.co, wout, C, hidden, 0, 1, train)[0]
+            ctx.save_for_backward(x, g, xn, qkv, o, lse, wqkv, wout, gamma)
+            ctx.cfg, ctx.gshape = (heads, D, eps), gamma.shape
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, g, xn, qkv, o, lse, wqkv, wout, gamma = ctx.saved_tensors
+        heads, D, eps = ctx.cfg
+        hidden = heads * D
+        NI, H_, W_, C = x.shape
+        dy = dy.contiguous()
+        do = K.igemm(dy, ctx.wdo)
+        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1)
+        dqkv = K.mattn_bwd(qkv.view(-1, 3 * hidden), o.view(-1, hidden), lse, do.view(-1, hidden), NI, H_ * W_, heads, D,
+                           D ** -0.5)
+        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv.view(NI, H_, W_, 3 * hidden))
+        # + dy: the residual branch, added in the LN-backward epilogue
+        if _direct_all(gamma):
+            dx, _ = K.ln_bwd(x, g, dxn, dy, eps, into=gamma.grad.view(-1))
+            _ready(gamma)
+            dgamma = None
+        else:
+            dx, dg = K.ln_bwd(x, g, dxn, dy, eps)
+            dgamma = dg.view(ctx.gshape)
+        return dx, dgamma, dwqkv, dwout, None
 
 
 class SpatialAttnBlockFn(_Fn):

@@ -131,9 +131,10 @@ class Residual(nn.Module):
 
 
 def _fused_attention_block(res: "Residual", x, B, F, pos_bias=None, focus_present_mask=None):
-    """Residual(PreNorm(SpatialLinearAttention)) and Residual(PreNorm(EinopsToAndFrom(Attention)))
-    with the default all-False focus mask run as ONE autograd node (ops.*AttnBlockFn); anything
-    else returns None and takes the generic op-by-op path."""
+    """Residual(PreNorm(SpatialLinearAttention)), Residual(PreNorm(EinopsToAndFrom(Attention))) over frames
+    with the default all-False focus mask, and the use_mid_attn block Residual(PreNorm(EinopsToAndFrom(Attention)))
+    over pixels run as ONE autograd node (ops.*AttnBlockFn); anything else returns None and takes the generic
+    op-by-op path."""
     pre = res.fn
     if not isinstance(pre, PreNorm):
         return None
@@ -157,6 +158,14 @@ def _fused_attention_block(res: "Residual", x, B, F, pos_bias=None, focus_presen
             pos_bias = torch.zeros((att.heads, F, F), dtype=torch.float32, device=x.device)
         return ops.TemporalAttnBlockFn.apply(x, pre.norm.gamma, att.to_qkv.weight, att.to_out.weight, pos_bias, cs, sn,
                                              B, F, meta)
+    if (isinstance(inner, EinopsToAndFrom) and inner.to_einops == "b f (h w) c" and isinstance(inner.fn, Attention)
+            and focus_present_mask is None):
+        att = inner.fn
+        meta = att.__dict__.get("_bmeta")
+        if meta is None:
+            meta = att.__dict__["_bmeta"] = ops.BlockMeta(heads=att.heads, dim_head=att.dim_head, eps=pre.norm.eps,
+                                                          cq=ops.PackCache(), co=ops.PackCache())
+        return ops.MidAttnBlockFn.apply(x, pre.norm.gamma, att.to_qkv.weight, att.to_out.weight, meta)
     return None
 
 
@@ -332,9 +341,10 @@ class SpatialLinearAttention(nn.Module):
 
 
 class EinopsToAndFrom(nn.Module):
-    """video_net.py:350-365.  The reference materialises "b c f h w" <-> "b (h w) f c" copies
-    around the wrapped attention; with the channels-last internal layout the attention kernel
-    indexes frames directly, so this wrapper only records which axis is the sequence."""
+    """video_net.py:350-365.  The reference materialises "b c f h w" <-> "b (h w) f c" (temporal) or
+    "b f (h w) c" (use_mid_attn's spatial block) copies around the wrapped attention; with the channels-last
+    internal layout the attention kernels index frames or pixels directly, so this wrapper only records which
+    axis is the sequence -- and tells a wrapped Attention (`Attention.seq`)."""
 
     def __init__(self, from_einops, to_einops, fn):
         super().__init__()
@@ -343,12 +353,10 @@ class EinopsToAndFrom(nn.Module):
         self.fn = fn
         if from_einops != "b c f h w" or to_einops not in ("b (h w) f c", "b f (h w) c"):
             raise NotImplementedError(f"unsupported rearrangement {from_einops} -> {to_einops}")
+        if isinstance(fn, Attention):
+            fn.seq = "pixels" if to_einops == "b f (h w) c" else "frames"
 
     def forward_cl(self, x, B, F, **kwargs):
-        if self.to_einops == "b f (h w) c":
-            raise NotImplementedError(
-                "use_mid_attn=True (full softmax attention over pixels, video_net.py:713-719) is not "
-                "configured by config/baseline or config/more_blocks and has no B200 kernel yet")
         return self.fn.forward_cl(x, B, F, **kwargs)
 
     def forward(self, x, **kwargs):
@@ -357,7 +365,9 @@ class EinopsToAndFrom(nn.Module):
 
 
 class Attention(nn.Module):
-    """video_net.py:368-454, temporal use: sequences are the F frames of each pixel column."""
+    """video_net.py:368-454.  `seq` (set by the EinopsToAndFrom wrapper) names the sequence axis: "frames" (temporal
+    use, the default: the F frames of each pixel column) or "pixels" (use_mid_attn: the h*w pixels of each frame,
+    no rotary embedding, no position bias)."""
 
     def __init__(self, dim, heads=4, dim_head=32, rotary_emb=None, use_checkpoint=False):
         super().__init__()
@@ -371,6 +381,7 @@ class Attention(nn.Module):
         self.to_out = nn.Linear(hidden_dim, dim, bias=False)
         self._cache = ops.PackCache()
         self._cache_out = ops.PackCache()
+        self.seq = "frames"
 
     def forward_cl(self, x, B, F, pos_bias=None, focus_present_mask=None, residual=None):
         NI, H, W, _ = x.shape
@@ -383,6 +394,10 @@ class Attention(nn.Module):
                 return ops.ConvFn.apply(v, None, self.to_out.weight, None, residual, 1, self._cache_out)
             if bool(focus_present_mask.any()):
                 raise NotImplementedError("per-sample focus_present_mask is not supported by the fused kernel")
+        if self.seq == "pixels":
+            out = ops.MidAttnCoreFn.apply(qkv.view(NI * H * W, 3 * hidden), NI, H * W, self.heads, self.dim_head)
+            return ops.ConvFn.apply(out.view(NI, H, W, hidden), None, self.to_out.weight, None, residual, 1,
+                                    self._cache_out)
         if not exists(self.rotary_emb):
             raise NotImplementedError("temporal attention without rotary embedding has no B200 kernel")
         cs, sn = self.rotary_emb.tables(F)
@@ -394,9 +409,15 @@ class Attention(nn.Module):
         return ops.ConvFn.apply(out, None, self.to_out.weight, None, residual, 1, self._cache_out)
 
     def forward(self, x, pos_bias=None, focus_present_mask=None):
-        """x: [b, (h w), f, c] as the reference's EinopsToAndFrom hands it over."""
+        """x: [b, (h w), f, c] (temporal) or [b, f, (h w), c] (seq == "pixels") as the reference's EinopsToAndFrom
+        hands it over; attention runs over dim -2 either way."""
         if x.dim() != 4:
-            raise ValueError(f"expected [b, n_seq, f, c], got {tuple(x.shape)}")
+            raise ValueError(f"expected a 4-D [b, ., n_seq, c] tensor, got {tuple(x.shape)}")
+        if self.seq == "pixels":
+            b, f, n, c = x.shape
+            xc = x.reshape(b * f, n, 1, c).to(torch.float16).contiguous()
+            y = self.forward_cl(xc, b, f, pos_bias=pos_bias, focus_present_mask=focus_present_mask)
+            return y.view(b, f, n, c).to(x.dtype)
         b, n, f, c = x.shape
         xc = x.permute(0, 2, 1, 3).reshape(b * f, n, 1, c).to(torch.float16).contiguous()
         y = self.forward_cl(xc, b, f, pos_bias=pos_bias, focus_present_mask=focus_present_mask)

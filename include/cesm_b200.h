@@ -260,6 +260,18 @@ int cesm_tattn_long_bwd(const void* qkv, const float* bias_diag, const float* cs
                         const float* lse, const void* dout, void* dqkv, float* dbias_diag, int B, int F, int HW, int H,
                         int dim_head, float scale, void* stream);
 
+/* Bottleneck spatial attention (use_mid_attn=True, video_net.py:713-719): per image of n pixels and per head,
+ * out = softmax((q * scale) k^T) v over all n pixels, no mask, no bias, no rotary embedding; flash style on the
+ * tensor cores (csrc/mid_attn.cu).  dim_head must be 32.
+ *   qkv : fp16 [NI*n][3*H*32] (q | k | v, each (head, d));  out / dout: fp16 [NI*n][H*32]
+ *   lse : fp32 [NI*n][H], log sum_j exp(scale q.k_j), written by fwd and read by bwd
+ *   delta: fp32 [NI*n][H] scratch of the backward (rowsum(dout * out), overwritten)
+ *   dqkv: fp16 [NI*n][3*H*32], every element written; no atomics, so the backward is bitwise deterministic.
+ * fp16 pointers must be 16-byte aligned.  1 <= NI <= 65535, n >= 1. */
+int cesm_mattn_fwd(const void* qkv, void* out, float* lse, int NI, int n, int H, int dim_head, float scale, void* stream);
+int cesm_mattn_bwd(const void* qkv, const void* out, const float* lse, const void* dout, void* dqkv, float* delta, int NI,
+                   int n, int H, int dim_head, float scale, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Spatial linear attention core, video_net.py:338-344, per image (frame) of n pixels and head:
  * qs = scale*softmax(q) over d, kh = softmax(k) over the n pixels, ctx = kh^T v, out = qs ctx.

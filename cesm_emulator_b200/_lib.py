@@ -29,11 +29,11 @@ class IgemmArgs(Structure):
         ("tap_dh", c_int32 * CESM_MAX_TAPS), ("tap_dw", c_int32 * CESM_MAX_TAPS),
         ("wt", c_void_p), ("cout", c_int32),
         ("oh", c_int32), ("ow", c_int32),
-        ("out", c_void_p), ("out_fp32", c_int32), ("ldo", c_int32),
+        ("out", c_void_p), ("ldo", c_int32),
         ("out_h", c_int32), ("out_w", c_int32),
         ("o_sh", c_int32), ("o_sw", c_int32), ("o_h0", c_int32), ("o_w0", c_int32),
         ("bias", c_void_p), ("residual", c_void_p), ("ldr", c_int32),
-        ("gn_sums", c_void_p), ("gn_groups", c_int32), ("gn_frames", c_int32), ("wt_stable", c_int32),
+        ("gn_sums", c_void_p), ("gn_groups", c_int32), ("gn_frames", c_int32),
         ("ln_colsum", c_void_p), ("ln_eps", ctypes.c_float), ("reserved_", c_int32),
     ]
 
@@ -125,13 +125,11 @@ _SIGNATURES: dict[str, list] = {
     "cesm_tattn_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_proj_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],
-    "cesm_tattn_proj_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_long_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_tattn_long_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_mattn_fwd": [_P, _P, _P, _I, _I, _I, _I, _F, _P],
     "cesm_mattn_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P],
     "cesm_linattn_fwd": [_P, _P, _P, _I, _I, _I, _I, _F, _P],
-    "cesm_linattn_fwd_out": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
     "cesm_linattn_bwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P],
     "cesm_film_fwd": [_P, _P, _P, _I, _I, _I, _I, _P],
     "cesm_film_bwd": [_P, _P, _P, _I, _I, _P, _I, _I, _I, _P],

@@ -1,5 +1,5 @@
-// C-ABI core: error reporting, TMA descriptor cache, and the cesm_igemm entry point
-// (tile-shape selection + tensor-map construction for igemm.cu).
+// C-ABI core: error reporting, TMA descriptor cache, and the cesm_igemm / cesm_wgrad entry points
+// (tile-shape selection + tensor-map construction for igemm2.cu, wgrad.cu and wgrad3.cu).
 #include <stdlib.h>
 
 #include <atomic>
@@ -176,13 +176,12 @@ static int sm_count() {
     return n;
 }
 
-// tuning / bisection knobs (read once): CESM_IGEMM_V1=1 routes everything to the first-generation
-// kernel, CESM_IGEMM_NO_HALO=1 disables the halo-reuse mode, CESM_IGEMM_NO_BRES=1 streams weights.
+// tuning / bisection knobs (read once): CESM_IGEMM_NO_HALO=1 disables the halo-reuse mode,
+// CESM_IGEMM_NO_BRES=1 streams weights.
 static int env_flag(const char* name) {
     const char* v = getenv(name);
     return (v && v[0] && v[0] != '0') ? 1 : 0;
 }
-static int knob_v1() { static int v = env_flag("CESM_IGEMM_V1"); return v; }
 static int knob_no_halo() { static int v = env_flag("CESM_IGEMM_NO_HALO"); return v; }
 static int knob_no_bres() { static int v = env_flag("CESM_IGEMM_NO_BRES"); return v; }
 static int knob_int(const char* name) {
@@ -348,7 +347,7 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
     p.dbg = knob_dbg();
     if (a->ln_colsum) {
         CESM_REQUIRE(a->cout == 64 && a->c0 == 64 && a->c1 == 0 && a->num_taps == 1 && a->stride == 1 && !a->gn_sums &&
-                         a->residual == a->a0 && a->ldr == 64 && !a->out_fp32,
+                         a->residual == a->a0 && a->ldr == 64,
                      "the LayerNorm fold needs a 64 -> 64 one-tap projection whose residual is its own input");
         p.ln_colsum = a->ln_colsum;
         p.ln_eps = a->ln_eps;
@@ -427,7 +426,6 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
     // 64->768 projection at 192x288: 131.5 us n-major, 106.6 us m-major (the output rows are completed in one
     // go instead of in three passes over the 510 MB tensor; tools/bench_igemm.py)
     p.m_major = ((knob_mmajor == 1 && p.b_resident) || knob_mmajor == 2) && p.n_tiles > 1 ? 1 : 0;
-    p.wt_stable = a->wt_stable ? 1 : 0;
     int grid;
     if (pair) {
         const int units = ((p.m_tiles + 1) / 2) * p.n_tiles, clusters = sm_count() / 2;
@@ -453,86 +451,7 @@ extern "C" int cesm_igemm(const cesm_igemm_args* a, void* stream) {
     CESM_REQUIRE(a->n > 0 && a->h > 0 && a->w > 0 && a->oh > 0 && a->ow > 0, "empty geometry");
     CESM_REQUIRE((a->c1 == 0) == (a->a1 == nullptr), "a1 / c1 mismatch");
     CESM_REQUIRE(a->ldo % 8 == 0 && (a->residual == nullptr || a->ldr % 8 == 0), "row pitches must be multiples of 8");
-    if (!a->out_fp32 && !(knob_v1() && a->gn_sums == nullptr && a->ln_colsum == nullptr))
-        return igemm2_run(a, as_stream(stream));  // persistent kernel (igemm2.cu)
-    CESM_REQUIRE(a->ln_colsum == nullptr, "the LayerNorm fold exists in the fp16 persistent kernel only");
-    CESM_REQUIRE(a->gn_sums == nullptr, "fused GroupNorm statistics need fp16 output");
-
-    IgemmParams p{};
-    p.c0 = a->c0;
-    p.c1 = a->c1;
-    p.num_taps = a->num_taps;
-    p.n = a->n;
-    p.oh = a->oh;
-    p.ow = a->ow;
-    choose_tile(a->n, a->oh, a->ow, &p.bw, &p.bh, &p.bn);
-    p.a_box_bytes = 64u * 2u * p.bw * p.bh * p.bn;
-    p.cout = a->cout;
-    p.out = a->out;
-    p.out_fp32 = a->out_fp32;
-    p.ldo = a->ldo;
-    p.out_h = a->out_h;
-    p.out_w = a->out_w;
-    p.o_sh = a->o_sh;
-    p.o_sw = a->o_sw;
-    p.o_h0 = a->o_h0;
-    p.o_w0 = a->o_w0;
-    p.bias = a->bias;
-    p.residual = a->residual;
-    p.ldr = a->ldr;
-
-    CUtensorMap amaps[4];
-    int n_amaps = 0;
-    const uint32_t box[4] = {64u, (uint32_t)p.bw, (uint32_t)p.bh, (uint32_t)p.bn};
-    if (a->stride == 1) {
-        const void* src[2] = {a->a0, a->a1};
-        const int cs[2] = {a->c0, a->c1};
-        for (int s = 0; s < 2; ++s) {
-            if (!src[s]) continue;
-            const uint64_t dims[4] = {(uint64_t)cs[s], (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-            const uint64_t str[3] = {(uint64_t)cs[s] * 2, (uint64_t)a->w * cs[s] * 2, (uint64_t)a->h * a->w * cs[s] * 2};
-            int rc = get_tensor_map_h16(&amaps[s], src[s], 4, dims, str, box);
-            if (rc) return rc;
-            n_amaps = s + 1;
-        }
-        for (int t = 0; t < a->num_taps; ++t) {
-            p.tap_map[t] = 0;
-            p.tap_dh[t] = a->tap_dh[t];
-            p.tap_dw[t] = a->tap_dw[t];
-        }
-    } else {
-        // stride 2: four parity sub-images of the source, each a unit-stride [n, h/2, w/2, c] view
-        const int c = a->c0;
-        for (int ph = 0; ph < 2; ++ph)
-            for (int pw = 0; pw < 2; ++pw) {
-                const char* base = static_cast<const char*>(a->a0) + (size_t)(ph * a->w + pw) * c * 2;
-                const uint64_t dims[4] = {(uint64_t)c, (uint64_t)a->w / 2, (uint64_t)a->h / 2, (uint64_t)a->n};
-                const uint64_t str[3] = {(uint64_t)c * 4, (uint64_t)a->w * c * 4, (uint64_t)a->h * a->w * c * 2};
-                int rc = get_tensor_map_h16(&amaps[ph * 2 + pw], base, 4, dims, str, box);
-                if (rc) return rc;
-            }
-        n_amaps = 4;
-        for (int t = 0; t < a->num_taps; ++t) {
-            const int ph = a->tap_dh[t] & 1, pw = a->tap_dw[t] & 1;
-            p.tap_map[t] = ph * 2 + pw;
-            p.tap_dh[t] = (a->tap_dh[t] - ph) / 2;
-            p.tap_dw[t] = (a->tap_dw[t] - pw) / 2;
-        }
-    }
-
-    const int ktot = a->num_taps * (a->c0 + a->c1);
-    const int block_n = (a->cout % 256 == 0) ? 256 : (a->cout % 128 == 0 ? 128 : 64);
-    CUtensorMap bmap;
-    {
-        const uint64_t dims[2] = {(uint64_t)ktot, (uint64_t)a->cout};
-        const uint64_t str[1] = {(uint64_t)ktot * 2};
-        const uint32_t bbox[2] = {64u, (uint32_t)block_n};
-        int rc = get_tensor_map_h16(&bmap, a->wt, 2, dims, str, bbox);
-        if (rc) return rc;
-    }
-    note_launch();
-    CESM_CHECK_CUDA(igemm_launch(amaps, n_amaps, bmap, p, block_n, as_stream(stream)));
-    return CESM_OK;
+    return igemm2_run(a, as_stream(stream));
 }
 
 // 64-pixel K tile for the weight gradient: powers of two with bw*bh*bn == 64, fewest tiles

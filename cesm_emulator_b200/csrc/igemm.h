@@ -1,33 +1,10 @@
-// Internal launch interface of the tcgen05 implicit-GEMM kernels (igemm.cu, wgrad.cu).
+// Internal launch interface of the tcgen05 implicit-GEMM kernels (igemm2.cu, wgrad.cu, wgrad3.cu).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 namespace cesm {
-
-struct IgemmParams {
-    // K loop: num_taps taps x (c0 + c1)/64 channel blocks.  Tap t reads TMA map tap_map[t] (+1 for
-    // the second concat source) at pixel offset (tap_dh[t], tap_dw[t]) from the output pixel.
-    int32_t c0, c1;
-    int32_t num_taps;
-    int32_t tap_map[16];
-    int32_t tap_dh[16];
-    int32_t tap_dw[16];
-    // pixel space iterated by the M tiles and the tile box (bw*bh*bn <= 128)
-    int32_t n, oh, ow;
-    int32_t bw, bh, bn;
-    uint32_t a_box_bytes;
-    // output: pixel (n, oh, ow) -> row ((n*out_h + oh*o_sh + o_h0)*out_w + ow*o_sw + o_w0)
-    int32_t cout;
-    void* out;
-    int32_t out_fp32;
-    int32_t ldo;
-    int32_t out_h, out_w, o_sh, o_sw, o_h0, o_w0;
-    const float* bias;     // [cout] or null
-    const void* residual;  // fp16, same pixel addressing as out, row pitch ldr; or null
-    int32_t ldr;
-};
 
 struct WgradParams {
     int32_t c0, c1;
@@ -94,7 +71,6 @@ struct Igemm2Params {
     int32_t gn_groups, gn_cpg, gn_frames;
     int32_t epi_warp;                  // 1: every epilogue warp stores its own 32-row slab (see igemm2.cu)
     int32_t m_major;                   // 1: consecutive tiles are the column tiles of ONE row tile (resident weights)
-    int32_t wt_stable;                 // 1: weights predate the preceding kernel: their loads need not wait for it
     int32_t dbg;                       // CESM_IGEMM_DBG bisection bits (0 in production)
     const float* ln_colsum;            // LayerNorm folded into a 64 -> 64 projection (see cesm_igemm_args) or null
     float ln_eps;
@@ -107,8 +83,5 @@ cudaError_t igemm2_launch(const Igemm2Maps& maps, const Igemm2Params& p, int blo
 // pair: clusters of two CTAs along the (tap, ci) blocks working as one cta_group::2 unit (block_n >= 128)
 cudaError_t wgrad_launch(const CUtensorMap* xmaps, int n_xmaps, const CUtensorMap& ymap, const WgradParams& p,
                          int block_n, int ksplit, bool pair, cudaStream_t stream);
-
-cudaError_t igemm_launch(const CUtensorMap* amaps, int n_amaps, const CUtensorMap& bmap, const IgemmParams& p,
-                         int block_n, cudaStream_t stream);
 
 }  // namespace cesm

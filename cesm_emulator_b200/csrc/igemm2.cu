@@ -1,4 +1,4 @@
-// Persistent tcgen05 / TMEM / TMA implicit GEMM for sm_100a (second generation of igemm.cu).
+// Persistent tcgen05 / TMEM / TMA implicit GEMM for sm_100a: every forward and data-gradient contraction.
 //
 //     out[pixel, co] = sum_{tap, ci} A[pixel + tap, ci] * Wt[co, tap, ci]   (+ bias) (+ residual)
 //
@@ -267,8 +267,7 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
         }
     } else if (warp == 1 && lane == 0) {
         // ===== weight producer =====
-        // weights re-packed at the top of the step are fetched while the preceding kernel still drains
-        if (!p.wt_stable) pdl_wait();
+        pdl_wait();
         const int row_off = (int)cta_rank * kBRows;   // PAIR: this CTA's half of a block's weight rows
         if (p.b_resident) {
             const uint32_t total_bytes = (uint32_t)p.n_tiles * p.num_kb * b_blk_bytes;

@@ -396,13 +396,6 @@ __device__ __forceinline__ void row_softmax(float (&f)[8]) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) f[i] *= inv;
 }
-__device__ __forceinline__ uint4 ldg_stream16(const void* p) {  // read-once data: do not pollute L1
-    uint4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.b32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                 : "l"(p));
-    return v;
-}
 
 // ------------------------------------------------------------------------------------------------
 // apply (forward): out[p][e] = sum_d qs[p][d] ctx[d][e]; warp = head; APPLY_MT 16-pixel tiles per
@@ -487,161 +480,6 @@ la_apply_kernel(const h16* __restrict__ qkv, float* __restrict__ ws, h16* __rest
                 if (row < p1) *reinterpret_cast<uint4*>(obase + (size_t)row * HD) = pack8(o[h2]);
             }
         }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// apply + output projection + residual (no-grad forward, round 2):
-//     y[p] = x[p] + b + W_out * concat_h( ctx_h^T qs_h[p] )                 (video_net.py:344-347 + Residual :69)
-// The attention output [pixels, H*32] never reaches HBM: a warp owns 16-pixel tiles and ALL heads; per head the
-// 16 x 32 result of the first MMA is already in A-fragment layout (see above) and feeds a second MMA with that
-// head's 32 x C slice of W_out, accumulating the C output channels across heads in registers.  The small B
-// operands (ctx, W_out) are turned into fragments once per block and read back from shared memory.
-// Traffic per pixel: q (1/3 of the q|k|v row) + x in, y out, instead of + 2 x the H*32-wide attention output.
-// ------------------------------------------------------------------------------------------------
-// B fragments of a 32x32 block of a row-major fp32 matrix with row stride `ld`: Bm[k][n] = M[n*ld + k] (k, n via phi32)
-__device__ __forceinline__ void load_bfrag32_t_strided(const float* __restrict__ M, int ld, int g, int t,
-                                                       uint32_t (&b)[2][4][2]) {
-#pragma unroll
-    for (int ks = 0; ks < 2; ++ks)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int nn = phi32(8 * j + g);
-#pragma unroll
-            for (int hi = 0; hi < 2; ++hi) {
-                const int k0 = phi32(16 * ks + 8 * hi + 2 * t);
-                b[ks][j][hi] = pack_h2(M[(size_t)nn * ld + k0], M[(size_t)nn * ld + k0 + 1]);
-            }
-        }
-}
-// fragment store / load in shared memory: word (4*q + i) of lane l at [(q*32 + l)*4 + i] (16-byte accesses, conflict-free)
-__device__ __forceinline__ void frag_to_smem(uint32_t* dst, int lane, const uint32_t (&b)[2][4][2]) {
-    const uint32_t* w = &b[0][0][0];
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-        *reinterpret_cast<uint4*>(dst + (q * 32 + lane) * 4) = make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
-}
-__device__ __forceinline__ void frag_from_smem(const uint32_t* src, int lane, uint32_t (&b)[2][4][2]) {
-    uint32_t* w = &b[0][0][0];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        const uint4 u = *reinterpret_cast<const uint4*>(src + (q * 32 + lane) * 4);
-        w[4 * q] = u.x; w[4 * q + 1] = u.y; w[4 * q + 2] = u.z; w[4 * q + 3] = u.w;
-    }
-}
-template <int NB, int HH>   // NB = output channels / 32, HH = heads (a multiple of 4: processed in groups of 4)
-__global__ void __launch_bounds__(256, NB <= 2 ? 2 : 1)
-la_apply_out_kernel(const h16* __restrict__ qkv, float* __restrict__ ws, const float* __restrict__ wout,
-                    const float* __restrict__ bias, const h16* __restrict__ x, h16* __restrict__ y, int n, int chunk,
-                    float scale) {
-    pdl_trigger();
-    pdl_wait();
-    extern __shared__ __align__(16) uint8_t la_smem[];
-    constexpr int HD = HH * LD, ld = 3 * HD, C = NB * 32, G = HH / 4;
-    static_assert(HH % 4 == 0, "heads are processed four at a time");
-    const int ni = blockIdx.y, w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int g = lane >> 2, t = lane & 3;
-    uint32_t* s_ctx = reinterpret_cast<uint32_t*>(la_smem);   // [HH][512] words
-    uint32_t* s_w = s_ctx + HH * 512;                         // [HH][NB][512] words
-    float* s_bias = reinterpret_cast<float*>(s_w + HH * NB * 512);   // [C]
-    const LaWs W = la_ws(ws, ni, HD, HH);
-    for (int i = w; i < HH * (1 + NB); i += 8) {
-        uint32_t b[2][4][2];
-        if (i < HH) {
-            load_bfrag32<false>(W.ctx + (size_t)i * LD * LD, g, t, b);
-            frag_to_smem(s_ctx + i * 512, lane, b);
-        } else {
-            const int h = (i - HH) / NB, nb = (i - HH) % NB;
-            load_bfrag32_t_strided(wout + (size_t)(nb * 32) * HD + h * LD, HD, g, t, b);
-            frag_to_smem(s_w + (h * NB + nb) * 512, lane, b);
-        }
-    }
-    if ((int)threadIdx.x < C) s_bias[threadIdx.x] = bias ? bias[threadIdx.x] : 0.f;
-    __syncthreads();
-
-    const size_t row0 = (size_t)ni * n;
-    const int pstart = blockIdx.x * chunk, p1 = min(n, pstart + chunk);
-    const h16* qbase = qkv + row0 * ld + t * 8;
-    auto load_q = [&](int p, int grp, uint4 (&q)[4][2]) {
-#pragma unroll
-        for (int hh = 0; hh < 4; ++hh)
-#pragma unroll
-            for (int h2 = 0; h2 < 2; ++h2) {
-                const int row = min(p + g + 8 * h2, p1 - 1);
-                q[hh][h2] = ldg_stream16(qbase + (size_t)row * ld + (grp * 4 + hh) * LD);
-            }
-    };
-    // no software prefetch: registers buy occupancy here (two blocks = 16 warps per SM hide the load latency of
-    // one another; with a register-resident next tile the kernel sat at 158 registers, one block per SM, and was
-    // slower than the two kernels it replaces)
-    int p = pstart + 16 * w, grp = 0;
-    float yc[NB][4][4];
-    while (p < p1) {
-        uint4 cq[4][2];
-        load_q(p, grp, cq);
-        int np = p, ng = grp + 1;
-        if (ng == G) {
-            ng = 0;
-            np = p + 16 * 8;
-        }
-        if (grp == 0) {
-#pragma unroll
-            for (int nb = 0; nb < NB; ++nb)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) yc[nb][j][0] = yc[nb][j][1] = yc[nb][j][2] = yc[nb][j][3] = 0.f;
-        }
-#pragma unroll
-        for (int hh = 0; hh < 4; ++hh) {
-            const int h = grp * 4 + hh;
-            uint4 pk[2];
-#pragma unroll
-            for (int h2 = 0; h2 < 2; ++h2) {
-                float f[8];
-                unpack8(cq[hh][h2], f);
-                row_softmax(f);
-#pragma unroll
-                for (int i = 0; i < 8; ++i) f[i] *= scale;
-                pk[h2] = pack8(f);
-            }
-            uint32_t a[2][4], bfr[2][4][2];
-            rows_to_afrag(pk[0], pk[1], a);
-            frag_from_smem(s_ctx + h * 512, lane, bfr);
-            float cfr[4][4], o[2][8];
-            frag_gemm(a, bfr, cfr);
-            c_to_rows(cfr, o);
-            rows_to_afrag(pack8(o[0]), pack8(o[1]), a);   // the head's 16 x 32 output as the next A operand
-#pragma unroll
-            for (int nb = 0; nb < NB; ++nb) {
-                frag_from_smem(s_w + (h * NB + nb) * 512, lane, bfr);
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-#pragma unroll
-                    for (int ks = 0; ks < 2; ++ks) mma_16816(yc[nb][j], a[ks], bfr[ks][j][0], bfr[ks][j][1]);
-            }
-        }
-        if (grp == G - 1) {
-#pragma unroll
-            for (int nb = 0; nb < NB; ++nb) {
-                float o[2][8];
-                c_to_rows(yc[nb], o);
-                const float4 b0 = *reinterpret_cast<const float4*>(s_bias + nb * 32 + 8 * t),
-                             b1 = *reinterpret_cast<const float4*>(s_bias + nb * 32 + 8 * t + 4);
-                const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-                for (int h2 = 0; h2 < 2; ++h2) {
-                    const int row = p + g + 8 * h2;
-                    if (row < p1) {
-                        float r[8];   // residual row, same lane layout as the output
-                        unpack8(ldg_stream16(x + (row0 + row) * C + nb * 32 + t * 8), r);
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) o[h2][i] += bv[i] + r[i];
-                        *reinterpret_cast<uint4*>(y + (row0 + row) * C + nb * 32 + t * 8) = pack8(o[h2]);
-                    }
-                }
-            }
-        }
-        p = np;
-        grp = ng;
     }
 }
 
@@ -824,38 +662,6 @@ extern "C" int cesm_linattn_fwd(const void* qkv, float* ws, void* out, int NI, i
                                                     scale);
     CESM_CHECK_LAUNCH();
     (void)HD;
-    return CESM_OK;
-}
-
-// colmax -> context -> finalize as in cesm_linattn_fwd, then ONE kernel for apply + to_out + bias + residual
-extern "C" int cesm_linattn_fwd_out(const void* qkv, float* ws, const float* wout, const float* bias, const void* x,
-                                    void* y, int NI, int n, int H, int dim_head, int C, float scale, void* stream) {
-    CESM_REQUIRE(dim_head == LD, "linear attention kernel needs dim_head == 32 (got %d)", dim_head);
-    CESM_REQUIRE((H == 4 || H == 8) && (C == 64 || C == 128),
-                 "fused apply + projection: 4 or 8 heads, 64 or 128 output channels (H=%d C=%d)", H, C);
-    cudaStream_t st = as_stream(stream);
-    CESM_ZERO_SCRATCH(ws, sizeof(float) * cesm_linattn_ws_floats(NI, H), st);
-    const int chunk = la_chunk(n, NI);
-    dim3 grid(ceil_div(n, chunk), NI);
-    launch_pdl(la_colmax_kernel, grid, 256, 0, st, (const h16*)qkv, ws, n, H, chunk);
-    CESM_CHECK_LAUNCH();
-    const size_t sh = la_context_smem(H, 0);
-    launch_pdl(la_context_kernel<0>, grid, 32 * H, sh, st, (const h16*)qkv, nullptr, ws, nullptr, n, H, chunk, scale);
-    CESM_CHECK_LAUNCH();
-    launch_pdl(la_finalize_kernel, ceil_div(NI * H * LD * LD, 256), 256, 0, st, ws, H, NI);
-    CESM_CHECK_LAUNCH();
-    const size_t sh_out = (size_t)H * (1 + C / 32) * 512 * 4 + (size_t)C * 4;
-    auto go = [&](auto kern) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh_out);
-        if (e != cudaSuccess) return e;
-        return launch_pdl(kern, grid, 256, sh_out, st, (const h16*)qkv, ws, wout, bias, (const h16*)x, (h16*)y, n, chunk,
-                          scale);
-    };
-    if (H == 4 && C == 64) CESM_CHECK_CUDA(go(la_apply_out_kernel<2, 4>));
-    else if (H == 4) CESM_CHECK_CUDA(go(la_apply_out_kernel<4, 4>));
-    else if (C == 64) CESM_CHECK_CUDA(go(la_apply_out_kernel<2, 8>));
-    else CESM_CHECK_CUDA(go(la_apply_out_kernel<4, 8>));
-    CESM_CHECK_LAUNCH();
     return CESM_OK;
 }
 

@@ -1,22 +1,15 @@
-// Temporal attention for short windows (F <= 3: the training window K = 3) FUSED WITH ITS q/k/v PROJECTION, for
-// 64 input channels (the three full-resolution blocks and the level-1 up block of config/baseline):
+// Temporal attention for short windows (F <= 3) FUSED WITH ITS q/k/v PROJECTION, for 64 input channels (the three
+// full-resolution blocks and the level-1 up block of config/baseline), forward only -- calls without gradients:
 //
 //     o = attention(LN(x) Wq^T, LN(x) Wk^T, LN(x) Wv^T)            video_net.py:403-453, rotary_embedding.py:29-48
 //
-// Unfused, the projection writes a 768-wide q|k|v tensor (510 MB per block at 192x288, B = 2), the attention core
-// reads it back, and the backward reads it a third time: 1.5 GB of HBM traffic per block for 43 GFLOP.  Here q, k and
-// v never reach HBM in the forward pass, and the backward recomputes them from LN(x) (42 MB) instead of re-reading
-// them:
+// Unfused, the projection writes a 768-wide q|k|v tensor (510 MB per block at 192x288, B = 2) and the attention core
+// reads it back.  Here q, k and v never reach HBM: a warp owns 16 pixel columns (all F frames): LN(x) rows -> mma.sync
+// A fragments (registers, loaded once); per head, q|k (then v) = A * W_h^T with W resident in shared memory; RoPE,
+// scores, softmax and P.V run on the accumulator fragments (a pixel row's 32 head features live in one quad: dot
+// products are quad shuffles); o leaves through a warp-private staging tile as 64-byte row segments.
 //
-//   forward  : a warp owns 16 pixel columns (all F frames): LN(x) rows -> mma.sync A fragments (registers, loaded
-//              once); per head, q|k (then v) = A * W_h^T with W resident in shared memory; RoPE, scores, softmax and
-//              P.V run on the accumulator fragments (a pixel row's 32 head features live in one quad: dot products
-//              are quad shuffles); o leaves through a warp-private staging tile as 64-byte row segments.
-//   backward : the same recomputation, then the attention backward on the fragments with dout staged per head;
-//              dq|dk|dv are written for the fused projection backward (qkvbwd.cu), d(bias) is reduced per CTA.
-//              W_h is streamed per head (double buffered): the CTA's warps walk the heads in lock step.
-//
-// Roofline: HBM for the backward (dq|dk|dv written: 1.5 KB per row), tensor / issue for the forward.
+// Roofline: tensor / issue.
 #include "api_common.h"
 #include "common.cuh"
 
@@ -45,19 +38,12 @@ __device__ __forceinline__ void cp16(uint32_t dst, const void* src) {
 }
 __device__ __forceinline__ void cp_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ float quad_sum(float v) {
     v += __shfl_xor_sync(0xffffffffu, v, 1);
     return v + __shfl_xor_sync(0xffffffffu, v, 2);
 }
 __device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
     asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t lds32(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
 }
 
 // acc[f][nt] (16 pixels x 8 output channels, F frames) for NTILES consecutive 8-row blocks of W starting at `wrow`
@@ -246,264 +232,9 @@ tattn_proj_fwd_kernel(const h16* __restrict__ xn, const h16* __restrict__ wqkv /
     }
 }
 
-// ------------------------------------------------------------------------------------------------
-// backward: W streamed per head (q, k, v rows of head h: 96 x 64), double buffered, CTA in lock step
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void unpack_frag(float (&x)[4][4], const uint32_t (&pk)[4][2]) {
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-        const float2 lo = unpack_h2(pk[nt][0]), hi = unpack_h2(pk[nt][1]);
-        x[nt][0] = lo.x; x[nt][1] = lo.y; x[nt][2] = hi.x; x[nt][3] = hi.y;
-    }
-}
-
-template <int F>
-__global__ void __launch_bounds__(32 * WARPS, 1)
-tattn_proj_bwd_kernel(const h16* __restrict__ xn, const h16* __restrict__ wqkv, const float* __restrict__ bias,
-                      const float* __restrict__ cs, const float* __restrict__ sn, const h16* __restrict__ dout,
-                      h16* __restrict__ dqkv, float* __restrict__ dbias, long long groups, int HW, float scale) {
-    pdl_trigger();
-    extern __shared__ __align__(16) uint8_t smem[];
-    const uint32_t sbase = smem_u32(smem);
-    constexpr uint32_t kWBuf = 3 * D * WP * 2;                        // one head's q|k|v rows
-    constexpr uint32_t kXs = F * 16 * WP * 2;                          // staged LN(x) rows, then dout of the current head
-    constexpr uint32_t kOs = 3 * F * 16 * OP * 2;                      // staged dq | dk | dv tiles
-    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, t = lane & 3, g = lane >> 2;
-    const uint32_t xs = sbase + 2 * kWBuf + (uint32_t)w * (kXs + kOs);
-    const uint32_t os = xs + kXs;
-    float* sb = reinterpret_cast<float*>(smem + 2 * kWBuf + (size_t)WARPS * (kXs + kOs));   // bias [H][F][F]
-    float* sdb = sb + HEADS * F * F;                                                          // d(bias) [WARPS][H][F][F]
-    auto fetch_w = [&](int h, int buf) {   // 3 x 32 rows x 8 chunks = 768 chunks of 16 bytes
-        for (int c = threadIdx.x; c < 3 * D * 8; c += blockDim.x) {
-            const int row = c >> 3, part = row >> 5, r = row & 31;
-            cp16(sbase + buf * kWBuf + (uint32_t)(row * WP + (c & 7) * 8) * 2u, wqkv + ((size_t)(part * HID + h * D + r) * C + (c & 7) * 8));
-        }
-        cp_commit();
-    };
-    fetch_w(0, 0);
-    pdl_wait();
-    for (int i = threadIdx.x; i < HEADS * F * F; i += blockDim.x) sb[i] = bias[i];
-    for (int i = threadIdx.x; i < WARPS * HEADS * F * F; i += blockDim.x) sdb[i] = 0.f;
-    float cf[F][4], sf[F][4];
-#pragma unroll
-    for (int f = 0; f < F; ++f)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-            cf[f][nt] = __ldg(cs + f * 16 + nt * 4 + t);
-            sf[f][nt] = __ldg(sn + f * 16 + nt * 4 + t);
-        }
-    const int gpp = HW / 16;
-    const long long stride = (long long)gridDim.x * WARPS;
-    const long long iters = (groups + stride - 1) / stride;   // the same trip count for every warp of every CTA
-    int buf = 0;
-    for (long long it = 0; it < iters; ++it) {
-        const long long grp = it * stride + (long long)blockIdx.x * WARPS + w;
-        const bool valid = grp < groups;
-        const long long b = valid ? grp / gpp : 0, p0 = valid ? (grp - b * gpp) * 16 : 0;
-        uint32_t a[F][4][4];
-        load_group<F>(a, xs, xn, b, p0, HW, lane);
-#pragma unroll 1
-        for (int h = 0; h < HEADS; ++h) {
-            // this head's dout rows -> xs (the LN(x) rows are in registers by now)
-#pragma unroll
-            for (int i = 0; i < (F * 64 + 31) / 32; ++i) {
-                const int c = lane + 32 * i;
-                if (c < F * 64) {
-                    const int row = c >> 2, ch = c & 3, f = row >> 4, px = row & 15;
-                    cp16(xs + (uint32_t)(row * OP + ch * 8) * 2u, dout + ((b * F + f) * HW + p0 + px) * HID + h * D + ch * 8);
-                }
-            }
-            cp_commit();
-            // W of head h has landed for everybody, and everybody is done with the other buffer: prefetch into it
-            cp_wait<1>();
-            __syncthreads();
-            {
-                const int hn = h + 1 < HEADS ? h + 1 : 0;
-                if (h + 1 < HEADS || it + 1 < iters) fetch_w(hn, buf ^ 1);
-                else cp_commit();
-            }
-            const uint32_t wb = sbase + buf * kWBuf;
-            uint32_t qh[F][4][2], kh[F][4][2];   // rotated q (scaled) and rotated k as packed fp16 fragments
-            float p[2][F][F];
-            {
-                float q[F][4][4], k[F][4][4];
-                project<F, 4>(q, a, wb, lane);
-                project<F, 4>(k, a, wb + (uint32_t)(D * WP) * 2u, lane);
-                rotate<F>(q, cf, sf, scale);
-                rotate<F>(k, cf, sf, 1.f);
-                scores_softmax<F>(p, q, k, sb + h * F * F);
-#pragma unroll
-                for (int f = 0; f < F; ++f)
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt) {
-                        qh[f][nt][0] = pack_h2(q[f][nt][0], q[f][nt][1]);
-                        qh[f][nt][1] = pack_h2(q[f][nt][2], q[f][nt][3]);
-                        kh[f][nt][0] = pack_h2(k[f][nt][0], k[f][nt][1]);
-                        kh[f][nt][1] = pack_h2(k[f][nt][2], k[f][nt][3]);
-                    }
-            }
-            // dout fragments of frame f straight from the staging tile (same layout as the accumulators: rows g / g+8,
-            // columns nt*8 + 2t, +1); read twice (dP, dV) instead of being held in registers
-            auto load_do = [&](float (&d)[4][4], int f) {
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) {
-                    const uint32_t ad = xs + (uint32_t)((f * 16 + g) * OP + nt * 8 + 2 * t) * 2u;
-                    const float2 lo = unpack_h2(lds32(ad)), hi = unpack_h2(lds32(ad + (uint32_t)(8 * OP) * 2u));
-                    d[nt][0] = lo.x; d[nt][1] = lo.y; d[nt][2] = hi.x; d[nt][3] = hi.y;
-                }
-            };
-            // dP_ij = dout_i . v_j (v of this head is recomputed and dies here);  dS = P (dP - sum_j P dP)
-            float ds[2][F][F];
-            {
-                float v[F][4][4];
-                project<F, 4>(v, a, wb + (uint32_t)(2 * D * WP) * 2u, lane);
-                cp_wait<1>();   // dout of this head (the W prefetch may still be in flight)
-                __syncwarp();
-#pragma unroll
-                for (int i = 0; i < F; ++i) {
-                    float di[4][4];
-                    load_do(di, i);
-#pragma unroll
-                    for (int j = 0; j < F; ++j)
-#pragma unroll
-                        for (int r = 0; r < 2; ++r) {
-                            float sacc = 0.f;
-#pragma unroll
-                            for (int nt = 0; nt < 4; ++nt)
-                                sacc = fmaf(di[nt][2 * r], v[j][nt][2 * r], fmaf(di[nt][2 * r + 1], v[j][nt][2 * r + 1], sacc));
-                            ds[r][i][j] = quad_sum(sacc);
-                        }
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 2; ++r)
-#pragma unroll
-                for (int i = 0; i < F; ++i) {
-                    float dl = 0.f;
-#pragma unroll
-                    for (int j = 0; j < F; ++j) dl = fmaf(p[r][i][j], ds[r][i][j], dl);
-#pragma unroll
-                    for (int j = 0; j < F; ++j) ds[r][i][j] = valid ? p[r][i][j] * (ds[r][i][j] - dl) : 0.f;
-                }
-            // d(bias)[h][i][j]: sum over this warp's 16 pixel rows (every lane of a quad holds the same value)
-            {
-                float* dst = sdb + (w * HEADS + h) * F * F;
-#pragma unroll
-                for (int i = 0; i < F; ++i)
-#pragma unroll
-                    for (int j = 0; j < F; ++j) {
-                        float sacc = ds[0][i][j] + ds[1][i][j];
-                        sacc += __shfl_xor_sync(0xffffffffu, sacc, 4);
-                        sacc += __shfl_xor_sync(0xffffffffu, sacc, 8);
-                        sacc += __shfl_xor_sync(0xffffffffu, sacc, 16);
-                        if (lane == 0) dst[i * F + j] += sacc;
-                    }
-            }
-            __syncwarp();   // the staged gradients of the previous head have been copied out
-            const uint32_t tile_b = (uint32_t)(F * 16 * OP) * 2u;   // one staged [F][16][32] tile
-            auto stage_one = [&](const float (&x)[4][4], uint32_t base, int f) {
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) {
-                    const uint32_t ad = base + (uint32_t)((f * 16 + g) * OP + nt * 8 + 2 * t) * 2u;
-                    sts32(ad, pack_h2(x[nt][0], x[nt][1]));
-                    sts32(ad + (uint32_t)(8 * OP) * 2u, pack_h2(x[nt][2], x[nt][3]));
-                }
-            };
-            // dv_j = sum_i P_ij dout_i
-#pragma unroll
-            for (int j = 0; j < F; ++j) {
-                float x[4][4];
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) x[nt][0] = x[nt][1] = x[nt][2] = x[nt][3] = 0.f;
-#pragma unroll
-                for (int i = 0; i < F; ++i) {
-                    float di[4][4];
-                    load_do(di, i);
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) x[nt][e] = fmaf(p[e >> 1][i][j], di[nt][e], x[nt][e]);
-                }
-                stage_one(x, os + 2 * tile_b, j);
-            }
-            // dq_i = R_i^T (sum_j dS_ij k_j) * scale
-#pragma unroll
-            for (int i = 0; i < F; ++i) {
-                float x[4][4];
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) x[nt][0] = x[nt][1] = x[nt][2] = x[nt][3] = 0.f;
-#pragma unroll
-                for (int j = 0; j < F; ++j) {
-                    float kj[4][4];
-                    unpack_frag(kj, kh[j]);
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) x[nt][e] = fmaf(ds[e >> 1][i][j], kj[nt][e], x[nt][e]);
-                }
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-                    for (int r = 0; r < 2; ++r) {
-                        const float g0 = x[nt][2 * r], g1 = x[nt][2 * r + 1];
-                        x[nt][2 * r] = (g0 * cf[i][nt] + g1 * sf[i][nt]) * scale;
-                        x[nt][2 * r + 1] = (g1 * cf[i][nt] - g0 * sf[i][nt]) * scale;
-                    }
-                stage_one(x, os, i);
-            }
-            // dk_j = R_j^T (sum_i dS_ij q_i)
-#pragma unroll
-            for (int j = 0; j < F; ++j) {
-                float x[4][4];
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) x[nt][0] = x[nt][1] = x[nt][2] = x[nt][3] = 0.f;
-#pragma unroll
-                for (int i = 0; i < F; ++i) {
-                    float qi[4][4];
-                    unpack_frag(qi, qh[i]);
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) x[nt][e] = fmaf(ds[e >> 1][i][j], qi[nt][e], x[nt][e]);
-                }
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-                    for (int r = 0; r < 2; ++r) {
-                        const float g0 = x[nt][2 * r], g1 = x[nt][2 * r + 1];
-                        x[nt][2 * r] = g0 * cf[j][nt] + g1 * sf[j][nt];
-                        x[nt][2 * r + 1] = g1 * cf[j][nt] - g0 * sf[j][nt];
-                    }
-                stage_one(x, os + tile_b, j);
-            }
-            __syncwarp();
-            if (valid) {
-#pragma unroll
-                for (int part = 0; part < 3; ++part)
-                    flush_tile<F>(os + part * tile_b, dqkv + part * HID + h * D, b, p0, HW, 3 * HID, lane);
-            }
-            buf ^= 1;
-        }
-        __syncwarp();
-    }
-    cp_wait_all();
-    __syncthreads();
-    for (int i = threadIdx.x; i < HEADS * F * F; i += blockDim.x) {
-        float s = 0.f;
-#pragma unroll
-        for (int ww = 0; ww < WARPS; ++ww) s += sdb[ww * HEADS * F * F + i];
-        if (s != 0.f) atomicAdd(dbias + i, s);
-    }
-}
-
 template <int F>
 static constexpr size_t fwd_smem() {
     return (size_t)3 * HID * WP * 2 + (size_t)WARPS * F * 16 * WP * 2 + (size_t)HEADS * F * F * 4;
-}
-template <int F>
-static constexpr size_t bwd_smem() {
-    return (size_t)2 * 3 * D * WP * 2 + (size_t)WARPS * ((size_t)F * 16 * WP * 2 + (size_t)3 * F * 16 * OP * 2) +
-           (size_t)HEADS * F * F * 4 * (1 + WARPS);
 }
 
 }  // namespace tp
@@ -545,38 +276,6 @@ extern "C" int cesm_tattn_proj_fwd(const void* xn, const void* wqkv, const float
         default: TP_FWD(3) break;
     }
 #undef TP_FWD
-    CESM_CHECK_LAUNCH();
-    return CESM_OK;
-}
-
-extern "C" int cesm_tattn_proj_bwd(const void* xn, const void* wqkv, const float* bias, const float* cs, const float* sn,
-                                   const void* dout, void* dqkv, float* dbias, int B, int F, int HW, int H, int dim_head, int cin,
-                                   float scale, void* stream) {
-    if (int rc = tp_check(B, F, HW, H, dim_head, cin)) return rc;
-    const long long groups = (long long)B * HW / 16;
-    int sms = 148, dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const long long want = (groups + tp::WARPS - 1) / tp::WARPS;
-    const int grid = (int)(want < sms ? want : sms);
-    cudaStream_t st = as_stream(stream);
-    CESM_ZERO_SCRATCH(dbias, sizeof(float) * H * F * F, st);
-#define TP_BWD(FF)                                                                                                         \
-    {                                                                                                                      \
-        static bool cfg = false;                                                                                           \
-        if (!cfg) {                                                                                                        \
-            CESM_CHECK_CUDA(cudaFuncSetAttribute(tp::tattn_proj_bwd_kernel<FF>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                                 (int)tp::bwd_smem<FF>()));                                                \
-            cfg = true;                                                                                                    \
-        }                                                                                                                  \
-        launch_pdl(tp::tattn_proj_bwd_kernel<FF>, grid, 32 * tp::WARPS, tp::bwd_smem<FF>(), st, (const h16*)xn, (const h16*)wqkv, \
-                   bias, cs, sn, (const h16*)dout, (h16*)dqkv, dbias, groups, HW, scale);                                  \
-    }
-    switch (F) {
-        case 1: TP_BWD(1) break;
-        case 2: TP_BWD(2) break;
-        default: TP_BWD(3) break;
-    }
-#undef TP_BWD
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

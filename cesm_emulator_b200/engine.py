@@ -358,14 +358,12 @@ class TrainEngine:
             self._step_body_inner()
         finally:
             self.arena.end()
-            K.STABLE_WEIGHT_PTRS = set()
             ops.set_side_stream(None)
 
     def _step_body_inner(self):
         ops.set_grad_sink(self.buckets)
         ops.set_side_stream(self.side_stream)
         ops.prepack_all()  # one kernel refreshes every fp16 operand copy of the (just updated) weights
-        K.STABLE_WEIGHT_PTRS = ops.packed_ptrs()  # nothing rewrites them until the next step
         self.buckets.begin_step()
         loss = self.diffusion.loss(self.x0, self.cond)
         if isinstance(self.opt, FusedAdamW):

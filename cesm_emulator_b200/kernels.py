@@ -96,27 +96,16 @@ def zero_scratch(shape, device) -> torch.Tensor:
     return torch.empty(tuple(shape), dtype=torch.float32, device=device)
 
 
-# Packed weight copies known to predate the current stream position by more than one kernel (the training
-# engine fills this after its once-per-step re-pack, the sampling engine after its warm-up step): igemm may
-# then fetch them before the preceding kernel has finished (cesm_igemm_args.wt_stable).
-STABLE_WEIGHT_PTRS: set = set()
-# linattn_fwd_out (apply + to_out + residual in one mma.sync kernel) is correct and removes ~1 GB of traffic per
-# full-resolution block of the sampling step, but it is issue-bound (softmax + 192 MMAs per 16 pixels on CUDA-core
-# rates): 6.19 ms per reverse step against 6.10 ms with the split kernels on B200.  Opt-in: CESM_LINATTN_OUT=1.
-_NO_LINATTN_OUT = not bool(int(__import__("os").environ.get("CESM_LINATTN_OUT", "0")))
-_NO_WT_STABLE = not bool(int(__import__("os").environ.get("CESM_WT_STABLE", "0")))  # opt-in (CESM_WT_STABLE=1): -0.03 ms per step
-
-
 def igemm(a0: torch.Tensor, wt: torch.Tensor, *, taps: Sequence[Tuple[int, int]] = TAPS_1x1,
           a1: Optional[torch.Tensor] = None, stride: int = 1,
           out: Optional[torch.Tensor] = None, out_hw: Optional[Tuple[int, int]] = None,
           out_place: Tuple[int, int, int, int] = (1, 1, 0, 0),
           bias: Optional[torch.Tensor] = None, residual: Optional[torch.Tensor] = None,
-          out_dtype: torch.dtype = H16, gn_sums: Optional[torch.Tensor] = None, gn_frames: int = 1,
+          gn_sums: Optional[torch.Tensor] = None, gn_frames: int = 1,
           ln_fold: Optional[Tuple[torch.Tensor, float]] = None):
     """out[n,oh,ow,:] = sum_t A[n, oh*stride+dh_t, ow*stride+dw_t, :] @ wt[:, t, :]^T (+bias)(+residual).
 
-    a0/a1: fp16 [N,H,W,C]; wt: fp16 [cout, len(taps)*(C0+C1)].  `out_hw` is the iterated output
+    a0/a1: fp16 [N,H,W,C]; wt: fp16 [cout, len(taps)*(C0+C1)]; out: fp16.  `out_hw` is the iterated output
     grid (defaults to H//stride, W//stride); `out_place` = (o_sh, o_sw, o_h0, o_w0) scatters the
     grid into a larger `out` tensor (transposed-conv phases).
 
@@ -134,7 +123,8 @@ def igemm(a0: torch.Tensor, wt: torch.Tensor, *, taps: Sequence[Tuple[int, int]]
     o_sh, o_sw, o_h0, o_w0 = out_place
     if out is None:
         assert out_place == (1, 1, 0, 0)
-        out = torch.empty((n, oh, ow, cout), dtype=out_dtype, device=a0.device)
+        out = torch.empty((n, oh, ow, cout), dtype=H16, device=a0.device)
+    assert out.dtype == H16, out.dtype
     args = IgemmArgs()
     args.a0, args.a1, args.c0, args.c1 = _ptr(a0), _ptr(a1), c0, c1
     args.n, args.h, args.w, args.stride = n, h, w, stride
@@ -142,9 +132,8 @@ def igemm(a0: torch.Tensor, wt: torch.Tensor, *, taps: Sequence[Tuple[int, int]]
     for i, (dh, dw) in enumerate(taps):
         args.tap_dh[i], args.tap_dw[i] = dh, dw
     args.wt, args.cout = _ptr(wt), cout
-    args.wt_stable = 1 if (wt.data_ptr() in STABLE_WEIGHT_PTRS and not _NO_WT_STABLE) else 0
     args.oh, args.ow = oh, ow
-    args.out, args.out_fp32, args.ldo = _ptr(out), int(out.dtype == torch.float32), out.shape[-1]
+    args.out, args.ldo = _ptr(out), out.shape[-1]
     args.out_h, args.out_w = out.shape[1], out.shape[2]
     args.o_sh, args.o_sw, args.o_h0, args.o_w0 = o_sh, o_sw, o_h0, o_w0
     args.bias = _ptr(bias)
@@ -412,17 +401,9 @@ def tattn_bwd(qkv, bias, cs, sn, out, lse, dout, B: int, F: int, HW: int, H: int
     return dqkv, dbias
 
 
-# Measured on B200 at the bench workload (profiles/r02_fused_tattn_ab.txt): the fused forward beats projection +
-# attention core (-0.26 ms per step: 510 MB per block never written or re-read), but its recomputing backward is
-# issue-bound at 8 warps per SM (255 registers) and loses more than that (+0.56 ms) against the HBM-bound stream
-# kernel it replaces.  So the fused kernels serve forward-only calls (evaluation with K > 1 frames); a training step
-# takes them only with CESM_FUSED_TATTN_TRAIN=1.
-_FUSED_TATTN_TRAIN = bool(int(__import__("os").environ.get("CESM_FUSED_TATTN_TRAIN", "0")))
-
-
-def tattn_proj_ok(C: int, F: int, HW: int, H: int, D: int, train: bool = False) -> bool:
-    """Shapes / modes the fused projection + attention kernels (csrc/tattn_proj.cu) take."""
-    return C == 64 and 1 <= F <= 3 and HW % 16 == 0 and H == 8 and D == 32 and (_FUSED_TATTN_TRAIN or not train)
+def tattn_proj_ok(C: int, F: int, HW: int, H: int, D: int) -> bool:
+    """Shapes the fused projection + attention forward (csrc/tattn_proj.cu) takes."""
+    return C == 64 and 1 <= F <= 3 and HW % 16 == 0 and H == 8 and D == 32
 
 
 def tattn_proj_fwd(xn, wqkv_packed, bias, cs, sn, B: int, F: int, HW: int, H: int, D: int, scale: float):
@@ -436,18 +417,6 @@ def tattn_proj_fwd(xn, wqkv_packed, bias, cs, sn, B: int, F: int, HW: int, H: in
               64, scale, _stream(),
               _meta={"kind": "fused", "flops": 2.0 * rows * 64 * 3 * H * D, "bytes": float(rows * (64 + H * D) * 2)})
     return out
-
-
-def tattn_proj_bwd(xn, wqkv_packed, bias, cs, sn, dout, B: int, F: int, HW: int, H: int, D: int, scale: float):
-    """-> (dqkv fp16 [B*F*HW, 768], dbias fp32 [H, F, F]); q, k, v are recomputed from xn."""
-    _req_cuda(xn, wqkv_packed, bias, cs, sn, dout)
-    rows = B * F * HW
-    dqkv = torch.empty((rows, 3 * H * D), dtype=H16, device=xn.device)
-    dbias = zero_scratch((H, F, F), xn.device)
-    _lib.call("cesm_tattn_proj_bwd", _ptr(xn), _ptr(wqkv_packed), _ptr(bias), _ptr(cs), _ptr(sn), _ptr(dout), _ptr(dqkv),
-              _ptr(dbias), B, F, HW, H, D, 64, scale, _stream(),
-              _meta={"kind": "fused", "flops": 2.0 * rows * 64 * 3 * H * D, "bytes": float(rows * (64 + H * D + 3 * H * D) * 2)})
-    return dqkv, dbias
 
 
 def mattn_fwd(qkv, NI: int, n: int, H: int, D: int, scale: float):
@@ -485,26 +454,6 @@ def linattn_fwd(qkv, NI: int, n: int, H: int, D: int, scale: float):
     _lib.call("cesm_linattn_fwd", _ptr(qkv), _ptr(ws), _ptr(out), NI, n, H, D, scale, _stream(),
               _meta=_bytes_meta(qkv, out))
     return out, ws
-
-
-def linattn_out_ok(H: int, D: int, C: int) -> bool:
-    """Shapes the fused apply + to_out + residual kernel covers (csrc/linattn.cu la_apply_out_kernel)."""
-    return H in (4, 8) and D == 32 and C in (64, 128) and not _NO_LINATTN_OUT
-
-
-def linattn_fwd_out(qkv, wout, bout, x, NI: int, n: int, H: int, D: int, scale: float):
-    """No-grad forward of the whole tail of the block: y = x + bout + W_out * linear_attention(qkv), fp16 [NI*n, C];
-    the H*D-wide attention output stays in registers.  wout: fp32 [C, H*D] (Conv2d weight), bout: fp32 [C] or None."""
-    _req_cuda(qkv, wout, bout, x)
-    C = x.shape[-1]
-    assert wout.dtype == torch.float32 and wout.numel() == C * H * D and wout.is_contiguous()
-    assert x.dtype == H16 and x.is_contiguous() and x.numel() == NI * n * C
-    dev = qkv.device
-    ws = zero_scratch((_lib.load().cesm_linattn_ws_floats(NI, H),), dev)
-    y = torch.empty_like(x)
-    _lib.call("cesm_linattn_fwd_out", _ptr(qkv), _ptr(ws), _ptr(wout), _ptr(bout), _ptr(x), _ptr(y), NI, n, H, D, C,
-              scale, _stream(), _meta=_bytes_meta(qkv, x, y))
-    return y
 
 
 def linattn_bwd(qkv, ws, dout, NI: int, n: int, H: int, D: int, scale: float):

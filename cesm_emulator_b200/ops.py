@@ -206,11 +206,6 @@ def refresh_folds() -> None:
             e[0] = key
 
 
-def packed_ptrs() -> set:
-    """Addresses of every registered packed weight copy (full tensors; slices are not included)."""
-    return {e.out.data_ptr() for e in _ENTRIES if e.wref() is not None}
-
-
 # ------------------------------------------------------------------------------------------------
 # gradient delivery
 # ------------------------------------------------------------------------------------------------
@@ -742,24 +737,20 @@ class TemporalAttnBlockFn(_Fn):
             # into ONE C x C matrix W_out W_v, folded once per weight version: y = x + LN(x) (W_out W_v)^T.
             return K.igemm(xn, _fold_f1(meta, wqkv, wout, hidden, C), residual=x)
         wq = _conv_fwd_weight(meta.cq, wqkv, 3 * hidden, C, 1, train)
-        fused = K.tattn_proj_ok(C, F, H_ * W_, heads, D, train)
-        if fused:
-            # 64 input channels, F <= 3, forward-only by default (see kernels.tattn_proj_ok): q|k|v never reach HBM
-            # (csrc/tattn_proj.cu); when used in a training step the backward recomputes them from xn
-            qkv, lse = None, None
+        if not train and K.tattn_proj_ok(C, F, H_ * W_, heads, D):
+            # 64 input channels, F <= 3, no gradients: q|k|v never reach HBM (csrc/tattn_proj.cu).  A training step
+            # keeps the unfused path: a backward that recomputes q|k|v from xn was slower than streaming them back
+            # (profiles/r02_fused_tattn_ab.txt).
             o = K.tattn_proj_fwd(xn.view(-1, C), wq, pos_bias, cs, sn, B, F, H_ * W_, heads, D, D ** -0.5)
-        else:
-            qkv = K.igemm(xn, wq)
-            o, lse = K.tattn_fwd(qkv.view(-1, 3 * hidden), pos_bias, cs, sn, B, F, H_ * W_, heads, D, D ** -0.5)
+            return K.igemm(o.view(NI, H_, W_, hidden), _conv_fwd_weight(meta.co, wout, C, hidden, 1, train), residual=x)
+        qkv = K.igemm(xn, wq)
+        o, lse = K.tattn_fwd(qkv.view(-1, 3 * hidden), pos_bias, cs, sn, B, F, H_ * W_, heads, D, D ** -0.5)
         y = K.igemm(o.view(NI, H_, W_, hidden), _conv_fwd_weight(meta.co, wout, C, hidden, 1, train), residual=x)
         ctx.wdq = _conv_dgrad_weights(meta.cq, wqkv, 3 * hidden, C, 0, 1, train)[0]
         ctx.wdo = _conv_dgrad_weights(meta.co, wout, C, hidden, 0, 1, train)[0]
-        ctx.wq_fwd = wq if fused else None   # the packed operand (a cache buffer, valid until the next optimizer step)
-        saved = [x, g, xn, o, pos_bias, cs, sn, wqkv, wout, gamma]
-        if not fused:
-            saved.append(qkv)
-            if F > 4:
-                saved.append(lse)
+        saved = [x, g, xn, o, pos_bias, cs, sn, wqkv, wout, gamma, qkv]
+        if F > 4:
+            saved.append(lse)
         ctx.save_for_backward(*saved)
         ctx.cfg, ctx.gshape = (B, F, heads, D, eps), gamma.shape
         return y
@@ -767,8 +758,7 @@ class TemporalAttnBlockFn(_Fn):
     @staticmethod
     def backward(ctx, dy):
         saved = ctx.saved_tensors
-        x, g, xn, o, pos_bias, cs, sn, wqkv, wout, gamma = saved[:10]
-        qkv = saved[10] if len(saved) > 10 else None
+        x, g, xn, o, pos_bias, cs, sn, wqkv, wout, gamma, qkv = saved[:11]
         lse = saved[11] if len(saved) > 11 else None
         B, F, heads, D, eps = ctx.cfg
         hidden = heads * D
@@ -776,12 +766,8 @@ class TemporalAttnBlockFn(_Fn):
         dy = dy.contiguous()
         do = K.igemm(dy, ctx.wdo)
         dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1)
-        if ctx.wq_fwd is not None:
-            dqkv, dbias = K.tattn_proj_bwd(xn.view(-1, C), ctx.wq_fwd, pos_bias, cs, sn, do.view(-1, hidden), B, F, H_ * W_,
-                                           heads, D, D ** -0.5)
-        else:
-            dqkv, dbias = K.tattn_bwd(qkv.view(-1, 3 * hidden), pos_bias, cs, sn, o if F > 4 else None, lse,
-                                      do.view(-1, hidden), B, F, H_ * W_, heads, D, D ** -0.5)
+        dqkv, dbias = K.tattn_bwd(qkv.view(-1, 3 * hidden), pos_bias, cs, sn, o if F > 4 else None, lse,
+                                  do.view(-1, hidden), B, F, H_ * W_, heads, D, D ** -0.5)
         dqkv4 = dqkv.view(NI, H_, W_, 3 * hidden)
         dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv4)
         # + dy: the residual branch, added in the LN-backward epilogue
@@ -857,12 +843,6 @@ class SpatialAttnBlockFn(_Fn):
         train = _train(ctx)
         xn = K.ln_fwd(x, g, eps)
         qkv = K.igemm(xn, _conv_fwd_weight(meta.cq, wqkv, 3 * hidden, C, 1, train))
-        if not train and K.linattn_out_ok(heads, D, C):
-            # no gradients (sampling): apply + to_out + bias + residual in one kernel; the hidden-wide attention
-            # output is never written (kernels.linattn_fwd_out).  to_out's fp32 weight is read directly.
-            y = K.linattn_fwd_out(qkv.view(-1, 3 * hidden), wout.detach().reshape(C, hidden), bout.detach(),
-                                  x.view(-1, C), NI, H_ * W_, heads, D, D ** -0.5)
-            return y.view(NI, H_, W_, C)
         o, ws = K.linattn_fwd(qkv.view(-1, 3 * hidden), NI, H_ * W_, heads, D, D ** -0.5)
         y = K.igemm(o.view(NI, H_, W_, hidden), _conv_fwd_weight(meta.co, wout, C, hidden, 1, train), bias=bout,
                     residual=x)

@@ -73,8 +73,7 @@ typedef struct cesm_igemm_args {
     const void* wt; /* fp16 [cout, num_taps*(c0+c1)] */
     int32_t cout;
     int32_t oh, ow; /* output pixels iterated per image */
-    void* out;      /* fp16 (or fp32 if out_fp32) */
-    int32_t out_fp32;
+    void* out;      /* fp16 */
     int32_t ldo;
     int32_t out_h, out_w, o_sh, o_sw, o_h0, o_w0;
     const float* bias;    /* fp32 [cout] or NULL */
@@ -86,10 +85,6 @@ typedef struct cesm_igemm_args {
     float* gn_sums;
     int32_t gn_groups;
     int32_t gn_frames;
-    /* != 0: `wt` was written well before the kernel that precedes this call in the stream (the training
-     * engine re-packs every weight once at the top of a step), so the weight tiles may be fetched while
-     * that kernel is still draining (programmatic dependent launch).  0 is always safe. */
-    int32_t wt_stable;
     /* Optional channel-LayerNorm folded into a 64 -> 64 projection with a residual -- the whole temporal-attention
      * block at ONE frame without gradients (video_net.py:78-87 + :380-453: the softmax over a single key is 1, so
      * y = x + LN(x) (W_out W_v)^T).  If ln_colsum != NULL, `a0` and `residual` must both be the [rows, 64] tensor x,
@@ -235,17 +230,13 @@ int cesm_tattn_bwd(const void* qkv, const float* bias, const float* cs, const fl
                    const float* lse, const void* dout, void* dqkv, float* dbias, int B, int F, int HW, int H,
                    int dim_head, float scale, void* stream);
 
-/* Short windows (F <= 3: the training window) FUSED WITH THE q/k/v PROJECTION, 64 input channels, 8 heads of 32
- * (csrc/tattn_proj.cu): out = attention(xn Wq^T, xn Wk^T, xn Wv^T) with q, k, v never written to memory; the backward
- * recomputes them from xn and writes dq|dk|dv for cesm_qkv_bwd.
+/* Forward only, without gradients: short windows (F <= 3) FUSED WITH THE q/k/v PROJECTION, 64 input channels,
+ * 8 heads of 32 (csrc/tattn_proj.cu): out = attention(xn Wq^T, xn Wk^T, xn Wv^T) with q, k, v never written to
+ * memory.  A training step projects q/k/v with cesm_igemm and runs cesm_tattn_fwd / cesm_tattn_bwd instead.
  *   xn  : fp16 [B*F*HW][64] = LayerNorm(x);  wqkv: fp16 [768][64] (to_qkv.weight as cesm_pack_weight lays it out)
- *   bias: fp32 [8][F][F];  cs, sn: fp32 [F][16];  out / dout: fp16 [B*F*HW][256];  dqkv: fp16 [B*F*HW][768]
- *   dbias: fp32 [8][F][F], zeroed by the call.  HW must be a multiple of 16. */
+ *   bias: fp32 [8][F][F];  cs, sn: fp32 [F][16];  out: fp16 [B*F*HW][256].  HW must be a multiple of 16. */
 int cesm_tattn_proj_fwd(const void* xn, const void* wqkv, const float* bias, const float* cs, const float* sn, void* out,
                         int B, int F, int HW, int H, int dim_head, int cin, float scale, void* stream);
-int cesm_tattn_proj_bwd(const void* xn, const void* wqkv, const float* bias, const float* cs, const float* sn,
-                        const void* dout, void* dqkv, float* dbias, int B, int F, int HW, int H, int dim_head, int cin,
-                        float scale, void* stream);
 
 /* Long windows (F > 4, up to 128 frames; BASELINE.json configs[4]): the same computation, flash style.  A CTA
  * stages every frame of one pixel column in shared memory once and one warp per head runs the F x F attention on
@@ -285,12 +276,6 @@ int cesm_mattn_bwd(const void* qkv, const void* out, const float* lse, const voi
 size_t cesm_linattn_ws_floats(int NI, int H);
 int cesm_linattn_fwd(const void* qkv, float* ws, void* out, int NI, int n, int H, int dim_head, float scale,
                      void* stream);
-/* Forward without gradients: the same core followed, in the SAME kernel, by to_out (1x1 conv with bias,
- * video_net.py:323/347) and the block's residual add (:69): y = x + bias + W_out * out.  The H*32-wide attention
- * output never reaches HBM.  wout: fp32 [C][H*32] (the Conv2d weight), bias: fp32 [C] or NULL, x / y: fp16
- * [NI*n][C].  H in {4, 8}, dim_head == 32, C in {64, 128}. */
-int cesm_linattn_fwd_out(const void* qkv, float* ws, const float* wout, const float* bias, const void* x, void* y, int NI,
-                         int n, int H, int dim_head, int C, float scale, void* stream);
 int cesm_linattn_bwd(const void* qkv, float* ws, const void* dout, float* scratch, void* dqkv, int NI, int n, int H,
                      int dim_head, float scale, void* stream);
 

@@ -1,4 +1,4 @@
-"""GPU parity of the tcgen05 implicit-GEMM kernel (csrc/igemm.cu) through the C ABI.
+"""GPU parity of the tcgen05 implicit-GEMM kernel (csrc/igemm2.cu) through the C ABI.
 
 Reference = torch fp32 conv / matmul on the SAME fp16-rounded inputs, so the only differences
 are accumulation order and the final fp16 rounding of the output: tolerance 2e-3 * max|ref|
@@ -20,7 +20,7 @@ def _rand(shape, dev, scale=1.0):
 
 
 @pytest.mark.parametrize("m,k,n", [(128, 64, 64), (1000, 128, 128), (4096, 256, 768), (300, 512, 256), (77, 64, 64)])
-def test_plain_gemm(cuda, m, k, n):
+def test_plain_gemm_with_bias_and_residual(cuda, m, k, n):
     from cesm_emulator_b200 import kernels as K
     torch.manual_seed(0)
     a = _rand((1, 1, m, k), cuda)
@@ -30,9 +30,6 @@ def test_plain_gemm(cuda, m, k, n):
     out = K.igemm(a, w, bias=bias, residual=res)
     ref = a.float().view(m, k) @ w.float().t() + bias + res.float().view(m, n)
     assert _err(out.view(m, n), ref) < 2e-3
-    out32 = K.igemm(a, w, out_dtype=torch.float32)
-    ref32 = a.float().view(m, k) @ w.float().t()
-    assert _err(out32.view(m, n), ref32) < 1e-4
 
 
 @pytest.mark.parametrize("n,h,w,cin,cout", [(2, 128, 128, 64, 64), (3, 64, 64, 128, 128), (2, 32, 32, 256, 256),

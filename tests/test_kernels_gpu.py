@@ -240,10 +240,10 @@ def test_temporal_attention_core(cuda, B, Fr, HW, H):
 
 
 @pytest.mark.parametrize("B,Fr,HW", [(2, 3, 64), (1, 3, 48 * 72), (1, 2, 160), (3, 1, 32), (2, 3, 16)])
-def test_temporal_attention_fused_with_projection(cuda, B, Fr, HW):
-    """csrc/tattn_proj.cu: o = attention(xn Wq^T, xn Wk^T, xn Wv^T) without materialising q|k|v, and its recomputing
-    backward (-> dq|dk|dv, d bias), against the fp32 torch restatement of projection + attention on the same
-    fp16-rounded xn / W (video_net.py:403-453)."""
+def test_temporal_attention_fused_with_projection_forward(cuda, B, Fr, HW):
+    """csrc/tattn_proj.cu: o = attention(xn Wq^T, xn Wk^T, xn Wv^T) without materialising q|k|v (the no-grad
+    forward), against the fp32 torch restatement of projection + attention on the same fp16-rounded xn / W
+    (video_net.py:403-453)."""
     from cesm_emulator_b200 import kernels as K
     torch.manual_seed(7)
     H, D, C = 8, 32, 64
@@ -254,17 +254,9 @@ def test_temporal_attention_fused_with_projection(cuda, B, Fr, HW):
     freqs = (1.0 / (10000 ** (torch.arange(0, D, 2).float() / D))).to(cuda)
     ang = torch.arange(Fr, device=cuda, dtype=torch.float32)[:, None] * freqs[None]
     cs, sn = ang.cos().contiguous(), ang.sin().contiguous()
-    dout = rnd((rows, H * D), cuda)
     out = K.tattn_proj_fwd(xn, w, bias, cs, sn, B, Fr, HW, H, D, D ** -0.5)
-    dqkv, dbias = K.tattn_proj_bwd(xn, w, bias, cs, sn, dout, B, Fr, HW, H, D, D ** -0.5)
-    xr, wr, br = xn.float().requires_grad_(True), w.float().requires_grad_(True), bias.clone().requires_grad_(True)
-    qkv_ref = xr @ wr.t()
-    qkv_ref.retain_grad()
-    ref = _tattn_ref(qkv_ref, br, freqs, B, Fr, HW, H, D)
+    ref = _tattn_ref(xn.float() @ w.float().t(), bias, freqs, B, Fr, HW, H, D)
     assert err(out, ref) < 2e-3
-    ref.backward(dout.float())
-    assert err(dqkv, qkv_ref.grad) < 3e-3
-    assert err(dbias, br.grad) < 3e-3
     # and the unfused kernels on the materialised projection agree (same arithmetic, q|k|v rounded to fp16 in between)
     qkv = K.igemm(xn.view(1, 1, rows, C), w).view(rows, 3 * H * D)
     out2, _ = K.tattn_fwd(qkv, bias, cs, sn, B, Fr, HW, H, D, D ** -0.5)
@@ -656,9 +648,9 @@ def test_layernorm_folded_into_projection(cuda, rows_shape):
 
 @pytest.mark.parametrize("NI,n,C,H", [(2, 16 * 24, 64, 8), (3, 100, 64, 4), (2, 36 * 18, 128, 8), (1, 17, 128, 4),
                                       (16, 48 * 72, 64, 8)])
-def test_linear_attention_apply_fused_with_output_projection(cuda, NI, n, C, H):
-    """cesm_linattn_fwd_out (apply + to_out + bias + residual in one kernel, no-grad forward) against the two-step
-    path it replaces (cesm_linattn_fwd, then the 1x1 projection GEMM with bias and residual) and fp32 torch."""
+def test_linear_attention_with_output_projection(cuda, NI, n, C, H):
+    """The tail of the spatial-attention block as sampling runs it: cesm_linattn_fwd, then the 1x1 projection GEMM
+    with bias and residual (y = x + bout + W_out * attention), against fp32 torch."""
     from cesm_emulator_b200 import kernels as K
     torch.manual_seed(13)
     D = 32
@@ -667,10 +659,8 @@ def test_linear_attention_apply_fused_with_output_projection(cuda, NI, n, C, H):
     x = rnd((NI * n, C), cuda)
     wout = torch.randn(C, hid, device=cuda) * 0.1
     bout = torch.randn(C, device=cuda)
-    y = K.linattn_fwd_out(qkv, wout, bout, x, NI, n, H, D, D ** -0.5)
     o, _ = K.linattn_fwd(qkv, NI, n, H, D, D ** -0.5)
-    two = K.igemm(o.view(NI, 1, n, hid), wout.to(K.H16), bias=bout, residual=x.view(NI, 1, n, C)).view(-1, C)
-    assert err(y, two) < 3e-3
+    y = K.igemm(o.view(NI, 1, n, hid), wout.to(K.H16), bias=bout, residual=x.view(NI, 1, n, C)).view(-1, C)
     # fp32 restatement (video_net.py:338-347)
     q, k, v = qkv.float().view(NI, n, 3, H, D).unbind(2)
     qs = q.softmax(-1) * D ** -0.5

@@ -147,18 +147,6 @@ def _fresh(cuda, unet_kw):
     return diff
 
 
-def test_training_step_through_the_fused_projection_attention_kernels(cuda, baseline):
-    """csrc/tattn_proj.cu in the training step (off by default: slower than the unfused backward, see
-    profiles/r02_fused_tattn_ab.txt): forward without q|k|v in HBM, backward recomputing them -- same parity bars."""
-    from cesm_emulator_b200 import kernels as K
-    K._FUSED_TATTN_TRAIN = True
-    try:
-        for seed in (5, 6):
-            _check_against_oracle(baseline, BASELINE_KW, 2, 3, 64, 64, seed, cuda)
-    finally:
-        K._FUSED_TATTN_TRAIN = False
-
-
 def test_more_blocks_architecture_against_oracle(cuda):
     """config/more_blocks: ch_mults [1,2,4,8] -> a fourth level with 512 channels (and the level-0
     temporal attention going through `temporal_op`, video_net.py:701), at its configured 64x64 crop."""

@@ -1,6 +1,6 @@
 """Time the implicit-GEMM kernel on the shapes of the baseline model (run on the GPU box).
 
-    python tools/bench_igemm.py            # env knobs: CESM_IGEMM_V1, CESM_IGEMM_NO_HALO, CESM_IGEMM_NO_BRES
+    python tools/bench_igemm.py            # env knobs: CESM_IGEMM_NO_HALO, CESM_IGEMM_NO_BRES
 """
 import os
 import sys

@@ -34,8 +34,6 @@ for rep in range(2):
     w = (torch.randn(3 * H * D, 64, device="cuda") * 0.1).half()
     bias3 = torch.randn(H, F, F, device="cuda")
     cs, sn = tables(F)
-    do = (torch.randn(B * F * HW, H * D, device="cuda") * 0.1).half()
-    o = K.tattn_proj_fwd(xn, w, bias3, cs, sn, B, F, HW, H, D, D ** -0.5)
-    K.tattn_proj_bwd(xn, w, bias3, cs, sn, do, B, F, HW, H, D, D ** -0.5)
+    K.tattn_proj_fwd(xn, w, bias3, cs, sn, B, F, HW, H, D, D ** -0.5)
     torch.cuda.synchronize()
 print("ok")

@@ -3,7 +3,7 @@
 //   7x7 input conv with fused concat / frame broadcast (video_net.py:808-815, model.py:110-121)
 //   1x1x1 output conv fused with centre-frame selection (video_net.py:763, model.py:129-130)
 //   time embedding + small fp32 linears (video_net.py:101-113, 651-656, 238-241)
-//   DDPM q_sample / MSE / p_sample update (model.py:168-208)
+//   DDPM q_sample / MSE / p_sample update (model.py:168-208), strided DDIM update
 //   column sums (bias gradients)
 #include "api_common.h"
 #include "common.cuh"
@@ -577,6 +577,33 @@ __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __res
     const float mean = sqrt_recip_a[tb] * (xt[idx] - betas[tb] / sqrt_1mac[tb] * eps[idx]);
     out[idx] = mean + sqrtf(post_var[tb]) * z[idx];
 }
+// Strided DDIM step (Song et al.): x_prev = A[t] * x_t + B[t] * eps + S[t] * z, with the three coefficients of each
+// schedule timestep precomputed on the host in float64 (model.ddim_schedule) and stored as coef[T][3] fp32.
+// `out` may alias `xt` (each thread reads its element before writing it), so no __restrict__ on either.
+// z == nullptr drops the noise term (valid when every S is 0, i.e. eta = 0).  A timestep outside [0, T) writes
+// NaN instead of reading outside the table.  t_out (optional, never aliasing t) receives next_t[t] per sample;
+// an out-of-range t is passed through unchanged, so a chain that overruns its schedule keeps producing NaN.
+__global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps, const float* __restrict__ z,
+                                 const long long* __restrict__ t, const float* __restrict__ coef,
+                                 const long long* __restrict__ next_t, long long* __restrict__ t_out, float* out,
+                                 int T, long long per, long long total) {
+    pdl_trigger();
+    pdl_wait();
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= total) return;
+    const long long b = idx / per;
+    const long long tb = t[b];
+    const bool valid = tb >= 0 && tb < T;
+    if (t_out && idx == b * per) t_out[b] = valid ? next_t[tb] : tb;
+    if (!valid) {
+        out[idx] = __int_as_float(0x7fc00000);
+        return;
+    }
+    const float* c = coef + 3 * tb;
+    float v = fmaf(c[0], xt[idx], c[1] * eps[idx]);
+    if (z) v = fmaf(c[2], z[idx], v);
+    out[idx] = v;
+}
 
 // ------------------------------------------------------------------------------------------------
 // On-device data path (dataset_single_member.py:168-196): the whole (T, M, H, W) condition and target
@@ -810,6 +837,20 @@ extern "C" int cesm_p_sample(const float* xt, const float* eps, const float* z, 
     const long long total = (long long)B * per_sample;
     launch_pdl(p_sample_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a,
                                                                     post_var, out, per_sample, total);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_ddim_step(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
+                              const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                              void* stream) {
+    CESM_REQUIRE(T > 0 && B > 0 && per_sample > 0, "bad DDIM step sizes (T=%d B=%d per_sample=%lld)", T, B, per_sample);
+    CESM_REQUIRE(xt && eps && t && coef && out, "DDIM step needs xt, eps, t, coef and out");
+    CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
+    CESM_REQUIRE(!t_out || (const void*)t_out != (const void*)t, "t_out must not alias t");
+    const long long total = (long long)B * per_sample;
+    launch_pdl(ddim_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, coef, next_t, t_out, out, T,
+               per_sample, total);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

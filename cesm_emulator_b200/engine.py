@@ -432,9 +432,16 @@ class TrainEngine:
 class SampleEngine:
     """Ensemble generation (inference.py:217-232 + model.py:186-194): the reverse chain for a batch
     of independent fields, one UNet call + fused p_sample update per step, replayed as a CUDA graph
-    whose only per-step inputs are the timestep vector and the fresh noise (device RNG)."""
+    whose only per-step inputs are the timestep vector and the fresh noise (device RNG).
 
-    def __init__(self, diffusion, shape, use_graph: bool = True):
+    With `ddim_steps=N` the engine runs the strided DDIM chain of `model.ddim_schedule` instead (N UNet calls per
+    field; `eta` scales its noise).  The mode is fixed per engine, so there is still one graph: a replay is one UNet
+    call, a noise draw only if eta > 0, and one `ddim_step` launch that updates `x` in place and writes the next
+    timestep to `t_next`, copied into `t`.  The coefficient and next-timestep tables live in static device buffers,
+    which the graph captures by address."""
+
+    def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0):
+        from .model import ddim_schedule
         self.diffusion = diffusion
         dev = next(diffusion.parameters()).device
         self.device = dev
@@ -447,6 +454,12 @@ class SampleEngine:
         self.use_graph = use_graph
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self.launches_per_step = 0
+        self.ddim_steps, self.eta = ddim_steps, float(eta)
+        if ddim_steps is not None:
+            self.ddim_taus, coef, next_t = ddim_schedule(diffusion.alphas_cumprod, ddim_steps, eta)
+            self.ddim_coef = coef.to(dev)
+            self.ddim_next_t = next_t.to(dev)
+            self.t_next = torch.zeros_like(self.t)
 
     def _body(self):
         if self.arena is None:
@@ -461,6 +474,15 @@ class SampleEngine:
         d = self.diffusion
         with torch.no_grad():
             eps = d.model(self.x, self.cond, self.t)
+            if self.ddim_steps is not None:
+                z = None
+                if self.eta > 0:
+                    self.z.normal_()
+                    z = self.z
+                K.ddim_step(self.x, eps, z, self.t, self.ddim_coef, d.T, out=self.x, next_t=self.ddim_next_t,
+                            t_out=self.t_next)
+                self.t.copy_(self.t_next)
+                return
             self.z.normal_()  # model.py:181 randn_like; kept in a static buffer so that a caller can read the draw
             self.x.copy_(K.p_sample(self.x, eps, self.z, self.t, d.betas, d.sqrt_one_minus_alphas_cumprod,
                                     d.sqrt_recip_alphas, d.posterior_variance))
@@ -496,8 +518,13 @@ class SampleEngine:
 
     @torch.no_grad()
     def sample(self, cond: torch.Tensor, steps: Optional[int] = None) -> torch.Tensor:
-        """cond: [B,1,H,W] -> generated field [B,1,H,W] after `steps` (default T) reverse steps."""
+        """cond: [B,1,H,W] -> generated field [B,1,H,W] after `steps` (default T) reverse steps.  In DDIM mode
+        the chain is always the engine's N strided steps, and `steps` must be None."""
         T = self.diffusion.T
+        if self.ddim_steps is not None:
+            if steps is not None:
+                raise ValueError("steps does not apply to a DDIM-mode SampleEngine (its chain is ddim_steps long)")
+            steps = len(self.ddim_taus)
         steps = T if steps is None else steps
         self.refresh_operands()
         self.cond.copy_(cond, non_blocking=True)

@@ -648,3 +648,21 @@ def p_sample(xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a, post_var):
     _lib.call("cesm_p_sample", _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(betas), _ptr(sqrt_1mac), _ptr(sqrt_recip_a),
               _ptr(post_var), _ptr(out), B, xt.numel() // B, _stream())
     return out
+
+
+def ddim_step(xt, eps, z, t, coef, T: int, out=None, next_t=None, t_out=None):
+    """out = A[t]*xt + B[t]*eps + S[t]*z per sample from the fp32 [T, 3] table of `model.ddim_schedule`.
+    `out` may be `xt` (in place); `z` may be None when every S is 0.  With `t_out`, next_t[t] is written there
+    (a buffer other than `t`)."""
+    _req_cuda(xt, eps, z, t, coef, out, next_t, t_out)
+    assert coef.dtype == torch.float32 and coef.shape == (T, 3), (coef.dtype, tuple(coef.shape), T)
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert z is None or (z.dtype == torch.float32 and z.shape == xt.shape)
+    assert (t_out is None) == (next_t is None), "next_t and t_out go together"
+    assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
+    out = torch.empty_like(xt) if out is None else out
+    assert out.dtype == torch.float32 and out.shape == xt.shape
+    B = xt.shape[0]
+    _lib.call("cesm_ddim_step", _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out), _ptr(out),
+              T, B, xt.numel() // B, _stream())
+    return out

@@ -8,6 +8,8 @@ kernels of libcesm_b200.so; there is no CPU path.
 """
 from __future__ import annotations
 
+import numbers
+
 import torch
 from torch import nn
 
@@ -57,6 +59,47 @@ class UNet(nn.Module):
         return out.squeeze(2)
 
 
+def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
+    """Strided DDIM reverse chain (Song et al., "Denoising Diffusion Implicit Models") over the trained DDPM schedule.
+
+    Timesteps use "trailing" spacing, tau_i = floor(T (N - i) / N) - 1 for i = 0..N-1: the chain starts at T - 1,
+    where x ~ N(0, I) is valid, its last step goes to alpha_bar = 1, and N = T gives T-1, ..., 0.  One step from
+    tau to p (the next tau, alpha_bar_p = 1 after the last one) is, in the x0-prediction form rewritten as three
+    coefficients (no x0 clipping, as in p_sample):
+        sigma = eta sqrt((1 - ab_p) / (1 - ab_tau)) sqrt(1 - ab_tau / ab_p)
+        x_p = A x + B eps + S z,  A = sqrt(ab_p / ab_tau),  S = sigma,
+        B = sqrt(max(0, 1 - ab_p - sigma^2)) - sqrt(ab_p) sqrt(1 - ab_tau) / sqrt(ab_tau)
+    eta = 0 is deterministic; eta = 1 with N = T is the DDPM posterior step.  The coefficients are computed in float64
+    from the fp32 alphas_cumprod (1 - ab cancels at small tau in fp32) and stored as fp32.
+
+    Returns (taus: list of N ints, coef: fp32 [T, 3] rows (A, B, S), next_t: int64 [T]), both tables on the CPU.
+    Rows off the schedule hold NaN coefficients and next_t = -1; next_t of the last step is -1."""
+    T = int(alphas_cumprod.shape[0])
+    if isinstance(steps, bool) or not isinstance(steps, numbers.Integral):
+        raise ValueError(f"DDIM steps must be an integer, got {steps!r}")
+    steps = int(steps)
+    if not 1 <= steps <= T:
+        raise ValueError(f"DDIM steps must be in [1, {T}], got {steps}")
+    eta = float(eta)
+    if not eta >= 0.0:  # also rejects NaN
+        raise ValueError(f"DDIM eta must be >= 0, got {eta}")
+    ac = alphas_cumprod.detach().to("cpu", torch.float64)
+    taus = [T * (steps - i) // steps - 1 for i in range(steps)]
+    coef = torch.full((T, 3), float("nan"), dtype=torch.float64)
+    next_t = torch.full((T,), -1, dtype=torch.int64)
+    one = torch.ones((), dtype=torch.float64)
+    for i, tau in enumerate(taus):
+        a_t = ac[tau]
+        a_p = ac[taus[i + 1]] if i + 1 < steps else one
+        sigma = eta * torch.sqrt((1 - a_p) / (1 - a_t)) * torch.sqrt(1 - a_t / a_p)
+        coef[tau, 0] = torch.sqrt(a_p / a_t)
+        coef[tau, 1] = torch.sqrt(torch.clamp(1 - a_p - sigma * sigma, min=0)) - torch.sqrt(a_p) * torch.sqrt(1 - a_t) / torch.sqrt(a_t)
+        coef[tau, 2] = sigma
+        if i + 1 < steps:
+            next_t[tau] = taus[i + 1]
+    return taus, coef.float(), next_t
+
+
 class Diffusion(nn.Module):
     """model.py:141-208."""
 
@@ -103,6 +146,21 @@ class Diffusion(nn.Module):
             for tt in reversed(range(self.T)):
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
                 x = self.p_sample(x, cond, t_tensor)
+            return x
+
+    def ddim_sample(self, cond, shape, device, steps=50, eta=0.0):
+        """Strided DDIM chain of `steps` UNet calls (ddim_schedule), eager; an addition beyond the reference.
+        Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T."""
+        taus, coef, _ = ddim_schedule(self.alphas_cumprod, steps, eta)
+        coef = coef.to(device)
+        with torch.no_grad():
+            B = shape[0]
+            x = torch.randn(shape, device=device)
+            for tt in taus:
+                t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
+                eps_theta = self.model(x, cond, t_tensor)
+                z = torch.randn_like(x) if eta > 0 else None
+                x = K.ddim_step(x, eps_theta, z, t_tensor, coef, self.T)
             return x
 
     # -- training ------------------------------------------------------------------------------

@@ -353,6 +353,13 @@ int cesm_scale_by_scalar(const float* in, const float* gscale, float factor, flo
 int cesm_p_sample(const float* xt, const float* eps, const float* z, const long long* t, const float* betas,
                   const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out, int B,
                   long long per_sample, void* stream);
+/* Strided DDIM step: out = A[t]*xt + B[t]*eps + S[t]*z per sample, coef = fp32 [T][3] rows (A, B, S) computed on the
+ * host in float64.  out may equal xt.  z may be NULL when every S is 0.  t_out (optional, must not alias t) receives
+ * next_t[t] from the int64 [T] table.  A t outside [0, T) writes NaN.  Rejects T, B, per_sample <= 0 and NULL xt,
+ * eps, t, coef or out with CESM_ERR_INVALID. */
+int cesm_ddim_step(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
+                   const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                   void* stream);
 
 #ifdef __cplusplus
 }

@@ -3,7 +3,7 @@
 //   7x7 input conv with fused concat / frame broadcast (video_net.py:808-815, model.py:110-121)
 //   1x1x1 output conv fused with centre-frame selection (video_net.py:763, model.py:129-130)
 //   time embedding + small fp32 linears (video_net.py:101-113, 651-656, 238-241)
-//   DDPM q_sample / MSE / p_sample update (model.py:168-208), strided DDIM update
+//   DDPM q_sample / MSE / p_sample update (model.py:168-208), strided DDIM and DPM-Solver++(2M) updates
 //   column sums (bias gradients)
 #include "api_common.h"
 #include "common.cuh"
@@ -604,6 +604,38 @@ __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps,
     if (z) v = fmaf(c[2], z[idx], v);
     out[idx] = v;
 }
+// DPM-Solver++(2M) step (Lu et al.), data-prediction form, from the fp32 coef[T][5] rows (P, Q, R, K0, K1) that
+// model.dpm_schedule computes on the host in float64:
+//     x0 = P x + Q eps,   out = R x + K0 x0 + K1 hist,   hist <- x0
+// hist is the previous step's x0 prediction.  Where K1 == 0 (the first-order first and last steps) hist is not read,
+// so a stale or NaN history cannot reach the output and a new chain needs no reset.  `out` may alias `xt`; hist
+// aliases nothing.  An out-of-range t writes NaN to out and hist and passes t through to t_out, as ddim_step does.
+__global__ void dpm_step_kernel(const float* xt, const float* __restrict__ eps, float* __restrict__ hist,
+                                const long long* __restrict__ t, const float* __restrict__ coef,
+                                const long long* __restrict__ next_t, long long* __restrict__ t_out, float* out,
+                                int T, long long per, long long total) {
+    pdl_trigger();
+    pdl_wait();
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= total) return;
+    const long long b = idx / per;
+    const long long tb = t[b];
+    const bool valid = tb >= 0 && tb < T;
+    if (t_out && idx == b * per) t_out[b] = valid ? next_t[tb] : tb;
+    if (!valid) {
+        out[idx] = __int_as_float(0x7fc00000);
+        hist[idx] = __int_as_float(0x7fc00000);
+        return;
+    }
+    const float* c = coef + 5 * tb;
+    const float x = xt[idx];
+    const float x0 = fmaf(c[0], x, c[1] * eps[idx]);
+    float v = fmaf(c[2], x, c[3] * x0);
+    const float k1 = c[4];
+    if (k1 != 0.0f) v = fmaf(k1, hist[idx], v);
+    hist[idx] = x0;
+    out[idx] = v;
+}
 
 // ------------------------------------------------------------------------------------------------
 // On-device data path (dataset_single_member.py:168-196): the whole (T, M, H, W) condition and target
@@ -851,6 +883,33 @@ extern "C" int cesm_ddim_step(const float* xt, const float* eps, const float* z,
     const long long total = (long long)B * per_sample;
     launch_pdl(ddim_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, coef, next_t, t_out, out, T,
                per_sample, total);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+// True when the byte ranges [a, a + na) and [b, b + nb) share a byte (a null b shares none).
+static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+    const char *pa = (const char*)a, *pb = (const char*)b;
+    return pb && pa < pb + nb && pb < pa + na;
+}
+
+extern "C" int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
+                             const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                             void* stream) {
+    CESM_REQUIRE(T > 0 && B > 0 && per_sample > 0, "bad DPM step sizes (T=%d B=%d per_sample=%lld)", T, B, per_sample);
+    CESM_REQUIRE(xt && eps && hist && t && coef && out, "DPM step needs xt, eps, hist, t, coef and out");
+    CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
+    CESM_REQUIRE(!t_out || (const void*)t_out != (const void*)t, "t_out must not alias t");
+    const long long total = (long long)B * per_sample;
+    const size_t field = (size_t)total * sizeof(float), tb = (size_t)B * sizeof(long long);
+    CESM_REQUIRE(!ranges_overlap(hist, field, xt, field) && !ranges_overlap(hist, field, eps, field) &&
+                     !ranges_overlap(hist, field, out, field) && !ranges_overlap(hist, field, t, tb) &&
+                     !ranges_overlap(hist, field, t_out, tb) &&
+                     !ranges_overlap(hist, field, coef, (size_t)T * 5 * sizeof(float)) &&
+                     !ranges_overlap(hist, field, next_t, (size_t)T * sizeof(long long)),
+                 "hist must not overlap xt, eps, out, t, t_out, coef or next_t");
+    launch_pdl(dpm_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, hist, t, coef, next_t, t_out, out,
+               T, per_sample, total);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

@@ -438,10 +438,20 @@ class SampleEngine:
     field; `eta` scales its noise).  The mode is fixed per engine, so there is still one graph: a replay is one UNet
     call, a noise draw only if eta > 0, and one `ddim_step` launch that updates `x` in place and writes the next
     timestep to `t_next`, copied into `t`.  The coefficient and next-timestep tables live in static device buffers,
-    which the graph captures by address."""
+    which the graph captures by address.
 
-    def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0):
-        from .model import ddim_schedule
+    With `dpm_steps=N` it runs the deterministic DPM-Solver++(2M) chain of `model.dpm_schedule` (N UNet calls per
+    field).  A replay is one UNet call and one `dpm_step` launch that updates `x` and the previous-x0 buffer `hist`
+    in place and writes `t_next`, copied into `t`: no noise draw, and the same library launches per step as DDIM with
+    eta = 0.  The first step does not read `hist`, so a new chain needs no reset of it."""
+
+    def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0,
+                 dpm_steps: Optional[int] = None):
+        from .model import ddim_schedule, dpm_schedule
+        if dpm_steps is not None and ddim_steps is not None:
+            raise ValueError("ddim_steps and dpm_steps are mutually exclusive")
+        if dpm_steps is not None and float(eta) != 0.0:
+            raise ValueError(f"eta applies to DDIM only; the DPM-Solver++(2M) chain is deterministic (got eta={eta})")
         self.diffusion = diffusion
         dev = next(diffusion.parameters()).device
         self.device = dev
@@ -460,6 +470,13 @@ class SampleEngine:
             self.ddim_coef = coef.to(dev)
             self.ddim_next_t = next_t.to(dev)
             self.t_next = torch.zeros_like(self.t)
+        self.dpm_steps = dpm_steps
+        if dpm_steps is not None:
+            self.dpm_taus, coef, next_t = dpm_schedule(diffusion.alphas_cumprod, dpm_steps)
+            self.dpm_coef = coef.to(dev)
+            self.dpm_next_t = next_t.to(dev)
+            self.t_next = torch.zeros_like(self.t)
+            self.hist = torch.zeros(self.shape, dtype=torch.float32, device=dev)
 
     def _body(self):
         if self.arena is None:
@@ -483,6 +500,11 @@ class SampleEngine:
                             t_out=self.t_next)
                 self.t.copy_(self.t_next)
                 return
+            if self.dpm_steps is not None:
+                K.dpm_step(self.x, eps, self.hist, self.t, self.dpm_coef, d.T, out=self.x, next_t=self.dpm_next_t,
+                           t_out=self.t_next)
+                self.t.copy_(self.t_next)
+                return
             self.z.normal_()  # model.py:181 randn_like; kept in a static buffer so that a caller can read the draw
             self.x.copy_(K.p_sample(self.x, eps, self.z, self.t, d.betas, d.sqrt_one_minus_alphas_cumprod,
                                     d.sqrt_recip_alphas, d.posterior_variance))
@@ -497,10 +519,13 @@ class SampleEngine:
             return
         if self.graph is None:
             x_keep, t_keep = self.x.clone(), self.t.clone()
+            h_keep = self.hist.clone() if self.dpm_steps is not None else None  # a mid-chain step reads hist
             self._body()  # eager warm-up
             torch.cuda.synchronize()
             self.x.copy_(x_keep)
             self.t.copy_(t_keep)
+            if h_keep is not None:
+                self.hist.copy_(h_keep)
             self.graph = torch.cuda.CUDAGraph()
             n0 = _lib.launch_count()
             with torch.cuda.graph(self.graph):
@@ -518,13 +543,17 @@ class SampleEngine:
 
     @torch.no_grad()
     def sample(self, cond: torch.Tensor, steps: Optional[int] = None) -> torch.Tensor:
-        """cond: [B,1,H,W] -> generated field [B,1,H,W] after `steps` (default T) reverse steps.  In DDIM mode
-        the chain is always the engine's N strided steps, and `steps` must be None."""
+        """cond: [B,1,H,W] -> generated field [B,1,H,W] after `steps` (default T) reverse steps.  In DDIM and DPM
+        mode the chain is always the engine's N steps, and `steps` must be None."""
         T = self.diffusion.T
         if self.ddim_steps is not None:
             if steps is not None:
                 raise ValueError("steps does not apply to a DDIM-mode SampleEngine (its chain is ddim_steps long)")
             steps = len(self.ddim_taus)
+        if self.dpm_steps is not None:
+            if steps is not None:
+                raise ValueError("steps does not apply to a DPM-mode SampleEngine (its chain is dpm_steps long)")
+            steps = len(self.dpm_taus)
         steps = T if steps is None else steps
         self.refresh_operands()
         self.cond.copy_(cond, non_blocking=True)

@@ -666,3 +666,22 @@ def ddim_step(xt, eps, z, t, coef, T: int, out=None, next_t=None, t_out=None):
     _lib.call("cesm_ddim_step", _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out), _ptr(out),
               T, B, xt.numel() // B, _stream())
     return out
+
+
+def dpm_step(xt, eps, hist, t, coef, T: int, out=None, next_t=None, t_out=None):
+    """DPM-Solver++(2M) step per sample from the fp32 [T, 5] table (P, Q, R, K0, K1) of `model.dpm_schedule`:
+    x0 = P*xt + Q*eps, out = R*xt + K0*x0 + K1*hist, then hist = x0.  `hist` is read only where K1 != 0 and must
+    be a buffer of its own; `out` may be `xt` (in place).  With `t_out`, next_t[t] is written there (a buffer other
+    than `t`)."""
+    _req_cuda(xt, eps, hist, t, coef, out, next_t, t_out)
+    assert coef.dtype == torch.float32 and coef.shape == (T, 5), (coef.dtype, tuple(coef.shape), T)
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert hist.dtype == torch.float32 and hist.shape == xt.shape
+    assert (t_out is None) == (next_t is None), "next_t and t_out go together"
+    assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
+    out = torch.empty_like(xt) if out is None else out
+    assert out.dtype == torch.float32 and out.shape == xt.shape
+    B = xt.shape[0]
+    _lib.call("cesm_dpm_step", _ptr(xt), _ptr(eps), _ptr(hist), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out),
+              _ptr(out), T, B, xt.numel() // B, _stream())
+    return out

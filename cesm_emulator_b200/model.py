@@ -8,6 +8,7 @@ kernels of libcesm_b200.so; there is no CPU path.
 """
 from __future__ import annotations
 
+import math
 import numbers
 
 import torch
@@ -100,6 +101,54 @@ def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
     return taus, coef.float(), next_t
 
 
+def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
+    """DPM-Solver++(2M) reverse chain (Lu et al., "DPM-Solver++: Fast Solver for Guided Sampling of Diffusion
+    Probabilistic Models"), multistep second order in the data-prediction form, over the trained DDPM schedule.
+
+    The timesteps and the next_t chain are ddim_schedule's (trailing spacing), so the two samplers compare at equal N.
+    With alpha = sqrt(ab), sigma = sqrt(1 - ab), lambda = log(alpha / sigma), step i goes from s = tau_i to p =
+    tau_{i+1} (ab_p = 1 after the last step), h_i = lambda_p - lambda_s and phi = -alpha_p expm1(-h_i).  The row of
+    tau_i holds (P, Q, R, K0, K1) for
+        x0 = P x + Q eps,   x_p = R x + K0 x0 + K1 x0_prev,   P = 1 / alpha_s,  Q = -sigma_s / alpha_s,
+        R = sigma_p / sigma_s,   and with r = h_{i-1} / h_i:  K0 = phi (1 + 1 / (2r)),  K1 = -phi / (2r),
+    where x0_prev is the previous step's x0.  The first and the last step are first order (the usual lower order at
+    the ends): the first has K0 = phi, K1 = 0; the last lands on ab = 1 with R = 0, K0 = 1, K1 = 0, i.e. x_0 is the
+    x0 prediction.  Both are DDIM eta = 0 steps, so N <= 2 is exactly the DDIM eta = 0 chain.  The chain is
+    deterministic after x_T.  The coefficients are computed in float64 from the fp32 alphas_cumprod and stored as fp32.
+
+    Returns (taus: list of N ints, coef: fp32 [T, 5] rows (P, Q, R, K0, K1), next_t: int64 [T]), both tables on the
+    CPU.  Rows off the schedule hold NaN coefficients and next_t = -1; next_t of the last step is -1."""
+    T = int(alphas_cumprod.shape[0])
+    if isinstance(steps, bool) or not isinstance(steps, numbers.Integral):
+        raise ValueError(f"DPM-Solver steps must be an integer, got {steps!r}")
+    steps = int(steps)
+    if not 1 <= steps <= T:
+        raise ValueError(f"DPM-Solver steps must be in [1, {T}], got {steps}")
+    taus, _, next_t = ddim_schedule(alphas_cumprod, steps)
+    ac = alphas_cumprod.detach().to("cpu", torch.float64).tolist()
+    lam = lambda a: 0.5 * math.log(a / (1.0 - a))  # noqa: E731  log(alpha / sigma)
+    coef = torch.full((T, 5), float("nan"), dtype=torch.float64)
+    h_prev = None
+    for i, s in enumerate(taus):
+        a_s = ac[s]
+        P, Q = 1.0 / math.sqrt(a_s), -math.sqrt(1.0 - a_s) / math.sqrt(a_s)
+        if i + 1 == steps:
+            coef[s] = torch.tensor([P, Q, 0.0, 1.0, 0.0], dtype=torch.float64)
+            break
+        a_p = ac[taus[i + 1]]
+        h = lam(a_p) - lam(a_s)
+        phi = -math.sqrt(a_p) * math.expm1(-h)
+        R = math.sqrt(1.0 - a_p) / math.sqrt(1.0 - a_s)
+        if h_prev is None:
+            K0, K1 = phi, 0.0
+        else:
+            r = h_prev / h
+            K0, K1 = phi * (1.0 + 0.5 / r), -phi * 0.5 / r
+        coef[s] = torch.tensor([P, Q, R, K0, K1], dtype=torch.float64)
+        h_prev = h
+    return taus, coef.float(), next_t
+
+
 class Diffusion(nn.Module):
     """model.py:141-208."""
 
@@ -161,6 +210,21 @@ class Diffusion(nn.Module):
                 eps_theta = self.model(x, cond, t_tensor)
                 z = torch.randn_like(x) if eta > 0 else None
                 x = K.ddim_step(x, eps_theta, z, t_tensor, coef, self.T)
+            return x
+
+    def dpm_sample(self, cond, shape, device, steps=20):
+        """DPM-Solver++(2M) chain of `steps` UNet calls (dpm_schedule), eager; an addition beyond the reference.
+        Deterministic after x_T.  `hist` carries the previous step's x0 prediction; the first step does not read it."""
+        taus, coef, _ = dpm_schedule(self.alphas_cumprod, steps)
+        coef = coef.to(device)
+        with torch.no_grad():
+            B = shape[0]
+            x = torch.randn(shape, device=device)
+            hist = torch.empty_like(x)
+            for tt in taus:
+                t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
+                eps_theta = self.model(x, cond, t_tensor)
+                x = K.dpm_step(x, eps_theta, hist, t_tensor, coef, self.T)
             return x
 
     # -- training ------------------------------------------------------------------------------

@@ -360,6 +360,14 @@ int cesm_p_sample(const float* xt, const float* eps, const float* z, const long 
 int cesm_ddim_step(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
                    const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
                    void* stream);
+/* DPM-Solver++(2M) step: x0 = P[t]*xt + Q[t]*eps, out = R[t]*xt + K0[t]*x0 + K1[t]*hist, then hist = x0, from the
+ * fp32 [T][5] rows (P, Q, R, K0, K1) computed on the host in float64.  hist (B*per_sample floats) is read only where
+ * K1 != 0.  out may equal xt.  t_out (optional, must not alias t) receives next_t[t] from the int64 [T] table.  A t
+ * outside [0, T) writes NaN to out and hist.  Rejects T, B, per_sample <= 0, NULL xt, eps, hist, t, coef or out, and
+ * a hist that overlaps any other buffer with CESM_ERR_INVALID. */
+int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
+                  const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                  void* stream);
 
 #ifdef __cplusplus
 }

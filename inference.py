@@ -3,6 +3,7 @@
 
     python inference.py --ckpt runs/exp/checkpoints/final.pt [--batch_size 16] [--steps 1000] [--out pred.npy | pred.nc]
     python inference.py --ckpt ... --ddim_steps 50 [--eta 0.0]     # strided DDIM chain: 50 UNet calls per field
+    python inference.py --ckpt ... --dpm_steps 15                  # DPM-Solver++(2M) chain: 15 UNet calls per field
     torchrun --standalone --nproc_per_node=8 inference.py --ckpt ...
 
 `predict_temperature_from_emissions` keeps the reference's flow: rebuild UNet/Diffusion from
@@ -43,12 +44,17 @@ def load_diffusion_from_checkpoint(path, device):
 
 @torch.no_grad()
 def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_size=16, steps=None, rank=0, world=1,
-                                       device="cuda", ddim_steps=None, eta=0.0):
+                                       device="cuda", ddim_steps=None, eta=0.0, dpm_steps=None):
     """cond (T, M, 1, H, W) -> prediction (T, M, H, W); fields are independent and sharded over ranks.
     `ddim_steps=N` generates with the strided DDIM chain (N UNet calls per field, noise scaled by `eta`) instead of
-    the full DDPM chain; it cannot be combined with `steps`."""
+    the full DDPM chain; it cannot be combined with `steps`.  `dpm_steps=N` generates with the deterministic
+    DPM-Solver++(2M) chain (N UNet calls per field); it cannot be combined with `steps`, `ddim_steps` or eta != 0."""
     if ddim_steps is not None and steps is not None:
         raise ValueError("steps and ddim_steps are mutually exclusive")
+    if dpm_steps is not None and (steps is not None or ddim_steps is not None):
+        raise ValueError("dpm_steps cannot be combined with steps or ddim_steps")
+    if dpm_steps is not None and eta != 0:
+        raise ValueError(f"eta applies to DDIM only; dpm_steps is deterministic (got eta={eta})")
     T, M, _, H, W = cond_tm1hw.shape
     flat = torch.from_numpy(cond_tm1hw.reshape(T * M, 1, H, W))
     mine = list(range(rank, T * M, world))
@@ -60,7 +66,7 @@ def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_
         if c.shape[0] < batch_size:  # keep the captured graph's static shape
             c = torch.cat([c, c[-1:].expand(batch_size - c.shape[0], -1, -1, -1)], 0)
         if eng is None:
-            eng = SampleEngine(diffusion, (batch_size, 1, H, W), ddim_steps=ddim_steps, eta=eta)
+            eng = SampleEngine(diffusion, (batch_size, 1, H, W), ddim_steps=ddim_steps, eta=eta, dpm_steps=dpm_steps)
         y = eng.sample(c.to(device), steps=steps)
         out[sel] = y[: len(sel)].cpu()
     if world > 1:
@@ -107,12 +113,18 @@ def _cli():
     ap.add_argument("--ddim_steps", type=int, default=None,
                     help="generate with a strided DDIM chain of this many UNet calls instead of the T-step DDPM chain")
     ap.add_argument("--eta", type=float, default=0.0, help="DDIM noise scale (0 = deterministic, 1 = DDPM-like)")
+    ap.add_argument("--dpm_steps", type=int, default=None,
+                    help="generate with a deterministic DPM-Solver++(2M) chain of this many UNet calls")
     ap.add_argument("--members", type=int, default=2)
     ap.add_argument("--times", type=int, default=4)
     ap.add_argument("--out", default="pred.npy")
     a = ap.parse_args()
     if a.steps is not None and a.ddim_steps is not None:
         ap.error("--steps and --ddim_steps are mutually exclusive")
+    if a.dpm_steps is not None and (a.steps is not None or a.ddim_steps is not None):
+        ap.error("--dpm_steps cannot be combined with --steps or --ddim_steps")
+    if a.dpm_steps is not None and a.eta != 0:
+        ap.error("--eta applies to --ddim_steps only; --dpm_steps is deterministic")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
@@ -125,7 +137,7 @@ def _cli():
     ds = SyntheticEnsemble(members=a.members, times=a.times, lat=syn.get("lat", 192), lon=syn.get("lon", 288),
                            seed=syn.get("seed", 1234))
     pred = predict_temperature_from_emissions(diffusion, ds.cond, a.batch_size, a.steps, rank, world, dev,
-                                              ddim_steps=a.ddim_steps, eta=a.eta)
+                                              ddim_steps=a.ddim_steps, eta=a.eta, dpm_steps=a.dpm_steps)
     if rank == 0:
         if a.out.endswith(".nc"):
             write_prediction_netcdf(a.out, pred, attrs={"checkpoint": os.path.abspath(a.ckpt), "cond_var": "synthetic"})

@@ -11,8 +11,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int32, c_int64, c_vo
 from pathlib import Path
 
 _PKG = Path(__file__).resolve().parent
-_VARIANT = __import__("os").environ.get("CESM_LIB_VARIANT", "")   # ablation builds only (see build.py)
-LIB_PATH = _PKG / (f"libcesm_b200_{_VARIANT}.so" if _VARIANT else "libcesm_b200.so")
+LIB_PATH = _PKG / "libcesm_b200.so"
 
 CESM_MAX_TAPS = 16
 

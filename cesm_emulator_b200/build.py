@@ -14,12 +14,7 @@ from pathlib import Path
 PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 BUILD_DIR = PKG_DIR / "csrc" / "build"
-# CESM_LIB_VARIANT=name builds / loads libcesm_b200_<name>.so from the same sources with CESM_NVCC_EXTRA appended to the
-# flags (ablation builds only, e.g. CESM_LIB_VARIANT=fastsig CESM_NVCC_EXTRA=-DCESM_FAST_SIGMOID); unset = the product.
-_VARIANT = os.environ.get("CESM_LIB_VARIANT", "")
-LIB_PATH = PKG_DIR / (f"libcesm_b200_{_VARIANT}.so" if _VARIANT else "libcesm_b200.so")
-if _VARIANT:
-    BUILD_DIR = PKG_DIR / "csrc" / f"build_{_VARIANT}"
+LIB_PATH = PKG_DIR / "libcesm_b200.so"
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -55,7 +50,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
         if (not force and obj.exists() and obj.stat().st_mtime >= src.stat().st_mtime
                 and obj.stat().st_mtime >= hdr_mtime):
             return obj, None
-        cmd = [nvcc, *NVCC_FLAGS, *os.environ.get("CESM_NVCC_EXTRA", "").split(), "-c", str(src), "-o", str(obj)]
+        cmd = [nvcc, *NVCC_FLAGS, "-c", str(src), "-o", str(obj)]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError(f"nvcc failed for {src.name}:\n{r.stdout}\n{r.stderr}")

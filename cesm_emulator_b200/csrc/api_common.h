@@ -42,8 +42,6 @@ bool scratch_prezeroed();
 // Every kernel is launched with the programmatic-stream-serialization attribute: its CTAs may be scheduled
 // while the preceding kernel of the stream drains (they park in griddepcontrol.wait, see pdl_wait() in
 // common.cuh), which hides launch latency and the CTA ramp between the ~480 back-to-back kernels of a step.
-// CESM_NO_PDL=1 turns the attribute off (plain stream order).
-bool pdl_enabled();
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -55,7 +53,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
@@ -69,12 +67,9 @@ inline cudaError_t launch_pdl_cluster(void (*kern)(KArgs...), dim3 grid, dim3 bl
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[2];
-    int n = 0;
-    if (pdl_enabled()) {
-        attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    int n = 1;
     if (cluster_x > 1) {
         attr[n].id = cudaLaunchAttributeClusterDimension;
         attr[n].val.clusterDim.x = (unsigned)cluster_x;

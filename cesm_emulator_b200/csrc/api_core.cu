@@ -1,7 +1,5 @@
 // C-ABI core: error reporting, TMA descriptor cache, and the cesm_igemm / cesm_wgrad entry points
 // (tile-shape selection + tensor-map construction for igemm2.cu, wgrad.cu and wgrad3.cu).
-#include <stdlib.h>
-
 #include <atomic>
 #include <mutex>
 #include <string>
@@ -15,10 +13,6 @@ namespace cesm {
 static thread_local std::string g_last_error;
 static std::atomic<long long> g_launches{0};
 void note_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("CESM_NO_PDL"); return !(e && atoi(e)); }();
-    return on;
-}
 static std::atomic<int> g_prezeroed{0};
 bool scratch_prezeroed() { return g_prezeroed.load(std::memory_order_relaxed) != 0; }
 
@@ -176,27 +170,6 @@ static int sm_count() {
     return n;
 }
 
-// tuning / bisection knobs (read once): CESM_IGEMM_NO_HALO=1 disables the halo-reuse mode,
-// CESM_IGEMM_NO_BRES=1 streams weights.
-static int env_flag(const char* name) {
-    const char* v = getenv(name);
-    return (v && v[0] && v[0] != '0') ? 1 : 0;
-}
-static int knob_no_halo() { static int v = env_flag("CESM_IGEMM_NO_HALO"); return v; }
-static int knob_no_bres() { static int v = env_flag("CESM_IGEMM_NO_BRES"); return v; }
-static int knob_int(const char* name) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : 0;
-}
-static int knob_pw() { static int v = knob_int("CESM_IGEMM_PW"); return v; }            // force halo row width
-static int knob_bn() { static int v = knob_int("CESM_IGEMM_BN"); return v; }            // force the column-tile width
-static int knob_no_pair() { static int v = env_flag("CESM_IGEMM_NO_PAIR"); return v; }
-static int knob_astages() { static int v = knob_int("CESM_IGEMM_ASTAGES"); return v; }  // force A stages
-static int knob_dbg() {
-    static int v = [] { const char* e = getenv("CESM_IGEMM_DBG"); return e ? atoi(e) : 0; }();
-    return v;
-}
-
 static bool is_3x3_unit_taps(const cesm_igemm_args* a) {
     if (a->num_taps != 9 || a->stride != 1) return false;
     bool seen[9] = {false};
@@ -225,11 +198,10 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
 
     // ---- HALO candidates: padded row width pw in {16, 32, 64, 128}, bw = pw - 2, bh = 128 / pw ----
     bool halo = false;
-    if (is_3x3_unit_taps(a) && !knob_no_halo()) {
+    if (is_3x3_unit_taps(a)) {
         double best = 0.0;
         int best_pw = 0;
         for (int pw = 16; pw <= 128; pw <<= 1) {
-            if (knob_pw() && pw != knob_pw()) continue;
             const int bw = pw - 2, bh = 128 / pw;
             const double tiles = (double)ceil_div(a->ow, bw) * ceil_div(a->oh, bh);
             const double useful = ((double)a->ow * a->oh) / (tiles * 128.0);
@@ -257,8 +229,8 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
     // ~75 / 90 / 165 clocks at N = 64 / 128 / 256 (tools/bench_igemm.py).  With few row tiles (48x72 x 6 frames = 216
     // tiles on 148 SMs) a narrower N fills the last wave: 3 waves of N=128 tiles beat 2 waves of N=256 tiles.
     // CTA pairs (cta_group::2, igemm2.cu): two row tiles per cluster share the weight rows, so a CTA reads
-    // N*16 B instead of N*32 B of B per MMA (measured ~62 / 84 / 135 clocks).  CESM_IGEMM_NO_PAIR=1 keeps single CTAs.
-    const bool pair = halo && !knob_no_pair() && p.m_tiles >= 2 && sm_count() >= 2;
+    // N*16 B instead of N*32 B of B per MMA (measured ~62 / 84 / 135 clocks).
+    const bool pair = halo && p.m_tiles >= 2 && sm_count() >= 2;
     if (halo) {
         static const double clk1[3] = {75.0, 90.0, 165.0}, clk2[3] = {62.0, 84.0, 135.0};
         const double* clk = pair ? clk2 : clk1;
@@ -275,7 +247,6 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
             }
         }
     }
-    if (knob_bn() && a->cout % knob_bn() == 0) block_n = knob_bn();
     p.n_tiles = a->cout / block_n;
 
     // ---- GroupNorm statistics: every tile must lie within one sample ----
@@ -312,7 +283,7 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
     const long long b_total = (long long)a->cout * p.num_kb * 128 / (pair ? 2 : 1);   // per CTA
     const long long b_blk = (long long)block_n * 128 / (pair ? 2 : 1);
     const int a_min = 2;
-    if (b_total + a_min * (long long)p.a_stage_bytes <= budget && !knob_no_bres()) {
+    if (b_total + a_min * (long long)p.a_stage_bytes <= budget) {
         p.b_resident = 1;
         p.b_stages = 1;
         long long as = (budget - b_total) / p.a_stage_bytes;
@@ -330,7 +301,6 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
         CESM_REQUIRE(bs >= 2, "igemm2: no shared-memory plan for cout=%d K=%d", a->cout, p.num_kb * 64);
         p.b_stages = (int)bs;
     }
-    if (knob_astages() > 0 && knob_astages() <= p.a_stages) p.a_stages = knob_astages();
     const long long b_bytes = p.b_resident ? b_total : (long long)p.b_stages * b_blk;
     const size_t smem = 1024 + (size_t)p.a_stages * p.a_stage_bytes + (size_t)b_bytes + 2 * 16384 + 1024;
     CESM_REQUIRE(smem <= kIgemm2MaxSmem, "igemm2: shared-memory plan of %zu B exceeds the limit", smem);
@@ -344,7 +314,6 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
     p.bias = a->bias;
     p.residual = a->residual;
     p.ldr = a->ldr;
-    p.dbg = knob_dbg();
     if (a->ln_colsum) {
         CESM_REQUIRE(a->cout == 64 && a->c0 == 64 && a->c1 == 0 && a->num_taps == 1 && a->stride == 1 && !a->gn_sums &&
                          a->residual == a->a0 && a->ldr == 64,
@@ -412,7 +381,6 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
             p.epi_warp = (pw == 32);
         else
             p.epi_warp = (p.bw % 32 == 0);
-        if (knob_dbg() & 8) p.epi_warp = 0;  // bisection: force the block-staged epilogue
         uint32_t obox[4] = {64u, (uint32_t)p.bw, (uint32_t)(halo ? 1 : p.bh), (uint32_t)(halo ? 1 : p.bn)};
         if (p.epi_warp && !halo) {
             obox[1] = 32u;
@@ -422,10 +390,9 @@ static int igemm2_run(const cesm_igemm_args* a, cudaStream_t st) {
         int rc = get_tensor_map_h16(&maps.out, base, 4, dims, str, obox);
         if (rc) return rc;
     }
-    static const int knob_mmajor = [] { const char* e = getenv("CESM_IGEMM_MMAJOR"); return e ? atoi(e) : 1; }();
     // 64->768 projection at 192x288: 131.5 us n-major, 106.6 us m-major (the output rows are completed in one
     // go instead of in three passes over the 510 MB tensor; tools/bench_igemm.py)
-    p.m_major = ((knob_mmajor == 1 && p.b_resident) || knob_mmajor == 2) && p.n_tiles > 1 ? 1 : 0;
+    p.m_major = p.b_resident && p.n_tiles > 1 ? 1 : 0;
     int grid;
     if (pair) {
         const int units = ((p.m_tiles + 1) / 2) * p.n_tiles, clusters = sm_count() / 2;
@@ -473,11 +440,9 @@ static void choose_tile64(int n, int oh, int ow, int* bw, int* bh, int* bn) {
 // 3x3 stride-1 weight gradients with <= 128 output channels go to wgrad3.cu (one halo fetch serves all nine taps).
 // Its accumulators are 64 columns wide, so at 256+ output channels the wider MMAs of wgrad.cu win again
 // (tools/bench_wgrad.py on B200: 64->64 38.8 -> 32.2 us, 128->64 66.6 -> 53.4, 128->128 43.1 -> 33.9, 256->256 33.5 -> 36.1).
-// Returns true when it handled the call (*rc = status).  CESM_WGRAD3=0 disables it, CESM_WGRAD3_MAXCOUT moves the bar.
+// Returns true when it handled the call (*rc = status).
 static bool wgrad3_try(const cesm_wgrad_args* a, cudaStream_t st, int* rc) {
-    static const int enabled = [] { const char* e = getenv("CESM_WGRAD3"); return e ? atoi(e) : 1; }();
-    static const int max_cout = [] { const char* e = getenv("CESM_WGRAD3_MAXCOUT"); return e ? atoi(e) : 128; }();
-    if (!enabled || a->stride != 1 || a->num_taps != 9 || a->cout > max_cout) return false;
+    if (a->stride != 1 || a->num_taps != 9 || a->cout > 128) return false;
     if (a->oh != a->h || a->ow != a->w || a->y_h != a->oh || a->y_w != a->ow || a->y_sh != 1 || a->y_sw != 1 ||
         a->y_h0 != 0 || a->y_w0 != 0)
         return false;
@@ -655,18 +620,14 @@ extern "C" int cesm_wgrad(const cesm_wgrad_args* a, void* stream) {
     }
     const int block_n = (a->cout % 256 == 0) ? 256 : (a->cout % 128 == 0 ? 128 : 64);
     const int units = a->num_taps * (ctot / 64);
-    // CTA pairs where a launch has at least two 128-row blocks and is fed through L2 (multi-tap, or many input
-    // channels): CESM_WGRAD_PAIR=0 turns them off, =2 forces them wherever block_n >= 128
-    static const int wg_pair = [] { const char* e = getenv("CESM_WGRAD_PAIR"); return e ? atoi(e) : 1; }();
+    // CTA pairs where a launch has at least two 128-row blocks and is fed through L2 (multi-tap)
     const int m_tiles = (units + 1) / 2;
-    const bool pair = block_n >= 128 && m_tiles >= 2 && (wg_pair == 2 || (wg_pair == 1 && a->num_taps > 1));
+    const bool pair = block_n >= 128 && m_tiles >= 2 && a->num_taps > 1;
     const int base_ctas = (pair ? (m_tiles + 1) / 2 * 2 : m_tiles) * (a->cout / block_n);
     const int tiles = ceil_div(a->ow, p.bw) * ceil_div(a->oh, p.bh) * ceil_div(a->n, p.bn);
     // split-K so that the grid is ONE resident wave (two CTAs per SM; rounding up would leave a second
     // wave of a few CTAs that costs as much as the first)
-    static const int wg_ctas = [] { const char* e = getenv("CESM_WGRAD_CTAS"); return e ? atoi(e) : 2; }();
-    static const int wg_ceil = [] { const char* e = getenv("CESM_WGRAD_CEIL"); return e ? atoi(e) : 0; }();
-    int ksplit = wg_ceil ? ceil_div(148 * wg_ctas, base_ctas) : (148 * wg_ctas) / base_ctas;
+    int ksplit = (148 * 2) / base_ctas;
     if (ksplit > tiles) ksplit = tiles;
     if (ksplit < 1) ksplit = 1;
     note_launch();

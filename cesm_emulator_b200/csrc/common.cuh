@@ -78,27 +78,20 @@ __device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
         : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
     return d;
 }
-// tanh / sigmoid.  Default: ONE MUFU op, tanh.approx.f32 (~2^-11 relative error).  -DCESM_PRECISE_SIGMOID selects
-// (1 - e) / (1 + e), e = 2^(-2 h log2 e) through ex2.approx + rcp.approx (two MUFU ops, ~2^-22; the exponent is
-// clamped so that e stays finite and the quotient tends to -1).  Measured on B200 (profiles/r02_ablation_sigmoid.txt,
-// 3 input seeds at the config/baseline training shape): forward error 1.0-1.2e-3 and worst gradient tensor 2.1-2.9e-3
-// with EITHER form -- the approximation error is the size of one fp16 rounding of the value it feeds -- while the
-// two-MUFU form costs 0.16 ms per training step (the GroupNorm kernels are MUFU / issue limited).
+// tanh / sigmoid: ONE MUFU op, tanh.approx.f32 (~2^-11 relative error).  Measured on B200 against the two-MUFU
+// form (1 - e) / (1 + e), e = 2^(-2 h log2 e) through ex2.approx + rcp.approx (~2^-22;
+// profiles/r02_ablation_sigmoid.txt, 3 input seeds at the config/baseline training shape): forward error 1.0-1.2e-3
+// and worst gradient tensor 2.1-2.9e-3 with EITHER form -- the approximation error is the size of one fp16 rounding of
+// the value it feeds -- while the two-MUFU form costs 0.16 ms per training step (the GroupNorm kernels are MUFU /
+// issue limited).
 __device__ __forceinline__ float tanh_f(float h) {
     float t;
-#ifndef CESM_PRECISE_SIGMOID
     asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
-#else
-    float e, r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(fminf(-2.f * 1.4426950408889634f * h, 126.f)));
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.f + e));
-    t = (1.f - e) * r;
-#endif
     return t;
 }
 __device__ __forceinline__ float2 tanh2(float2 h) { return make_float2(tanh_f(h.x), tanh_f(h.y)); }
 
-// sigmoid(x) = 0.5 * tanh(x / 2) + 0.5 (see tanh_f for the two forms and their measured effect)
+// sigmoid(x) = 0.5 * tanh(x / 2) + 0.5 (see tanh_f for the measured effect of the one-MUFU form)
 __device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(0.5f, tanh_f(0.5f * x), 0.5f); }
 __device__ __forceinline__ float silu_f(float x) { return x * sigmoid_fast(x); }
 // d/dx silu(x) = s + x*s*(1-s)

@@ -71,7 +71,6 @@ struct Igemm2Params {
     int32_t gn_groups, gn_cpg, gn_frames;
     int32_t epi_warp;                  // 1: every epilogue warp stores its own 32-row slab (see igemm2.cu)
     int32_t m_major;                   // 1: consecutive tiles are the column tiles of ONE row tile (resident weights)
-    int32_t dbg;                       // CESM_IGEMM_DBG bisection bits (0 in production)
     const float* ln_colsum;            // LayerNorm folded into a 64 -> 64 projection (see cesm_igemm_args) or null
     float ln_eps;
 };

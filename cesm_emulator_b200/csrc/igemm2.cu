@@ -22,8 +22,7 @@
 //     per-group sum / sum-of-squares of the fp16-rounded outputs (video_net.py:216), kept in registers
 //     across tiles and reduced once per (sample, column tile).
 //   * (round 2) ONE elected thread runs the MMA issue loop: its instruction stream is the critical path
-//     (a 128x64x16 MMA is 32 tensor clocks), so the loop carries no per-MMA predicate, no per-tap branch
-//     and no debug knob (those exist only under -DCESM_IGEMM_DEBUG).
+//     (a 128x64x16 MMA is 32 tensor clocks), so the loop carries no per-MMA predicate and no per-tap branch.
 //   * (round 2) PAIR mode for the 3x3 convolutions: the two CTAs of a cluster work as one cta_group::2
 //     unit on two row tiles of the same column tile (M = 256).  What bounds a 128 x N x 16 SS-mode MMA is
 //     the shared-memory operand feed (~77-90 B/clk measured: 4 KB of A + N*32 B of B per MMA); in a pair
@@ -40,14 +39,6 @@
 #include "igemm.h"
 
 #include <type_traits>
-
-// Bisection knobs (CESM_IGEMM_DBG bits: 2 = no epilogue, 4 = no MMAs, 16 = no accumulator hand-over, 32 = no
-// activation loads) exist only in builds with -DCESM_IGEMM_DEBUG (CESM_NVCC_EXTRA); production code carries none.
-#ifdef CESM_IGEMM_DEBUG
-#define IGEMM2_DBG(x) (x)
-#else
-#define IGEMM2_DBG(x) 0
-#endif
 
 namespace cesm {
 
@@ -222,14 +213,6 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                     }
                     continue;
                 }
-                if (IGEMM2_DBG(p.dbg) & 32) {  // bisection: no activation traffic at all
-                    mbar_arrive(a_full(stage));
-                    if (++stage == p.a_stages) {
-                        stage = 0;
-                        phase ^= 1u;
-                    }
-                    continue;
-                }
                 mbar_arrive_expect_tx(a_full(stage), p.a_box_bytes);
                 if (HALO) {
                     int midx = 0, c = ai << 6;
@@ -338,18 +321,12 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
             const uint32_t tile_b16 = p.num_kb * b_blk16;   // resident: stride between n tiles
             const int n_a_stages = p.a_stages, n_b_stages = p.b_stages, n_tiles = p.n_tiles;
             const bool m_major = p.m_major != 0;
-            const int dbg = IGEMM2_DBG(p.dbg);
             auto mma4 = [&](uint32_t d_tmem, uint32_t a16, uint32_t b16, uint32_t first_accum) {
-                if (dbg & 4) return;  // bisection knob (debug builds only): no MMAs
-                // timing-only probes (results wrong): 64 = alternate between the two accumulator stages per MMA
-                // (is the chain of dependent accumulations the limit?), 128 = half-width MMAs (N/2: the operand
-                // bytes per MMA a CTA pair would read)
-                const uint32_t id = (dbg & 128) ? make_idesc_f16(kTileM, BLOCK_N / 2, 0, 0) : idesc;
 #pragma unroll
                 for (int k = 0; k < kKBlk / 16; ++k) {
                     const uint64_t da = desc_hi | (uint64_t)(a16 + 2 * k), db = desc_hi | (uint64_t)(b16 + 2 * k);
                     if (PAIR) umma_f16_pair(d_tmem, da, db, idesc, k == 0 ? first_accum : 1u);
-                    else umma_f16((dbg & 64) ? (tmem_base + (k & 1) * BLOCK_N) : d_tmem, da, db, id, k == 0 ? first_accum : 1u);
+                    else umma_f16(d_tmem, da, db, idesc, k == 0 ? first_accum : 1u);
                 }
             };
             auto commit = [&](uint32_t bar) {
@@ -363,7 +340,7 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                 if (RES) mbar_wait(b_all_bar, 0, 13);
                 for (int tile = work_id; tile < total_tiles; tile += work_stride) {
                     const int n_tile = m_major ? tile % n_tiles : tile / m_units;
-                    if (!(dbg & 16)) mbar_wait(t_empty(acc), acc_phase ^ 1u, 14);
+                    mbar_wait(t_empty(acc), acc_phase ^ 1u, 14);
                     tc_fence_after();
                     const uint32_t d_tmem = tmem_base + acc * BLOCK_N;
                     uint32_t b_kb16 = b_base16 + n_tile * tile_b16;   // resident: weight block (n_tile, kb = ai)
@@ -400,7 +377,7 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                             a_phase ^= 1u;
                         }
                     }
-                    if (!(dbg & 16)) commit(t_full(acc));
+                    commit(t_full(acc));
                     if (++acc == 2) {
                         acc = 0;
                         acc_phase ^= 1u;
@@ -545,13 +522,13 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                     cur_b = b;
                 }
             }
-            if (!(IGEMM2_DBG(p.dbg) & 16)) mbar_wait(t_full(acc), acc_phase, 17);
+            mbar_wait(t_full(acc), acc_phase, 17);
             tc_fence_after();
             const uint32_t taddr = tmem_base + acc * BLOCK_N + (static_cast<uint32_t>(q * 32) << 16);
             const int last_cc = BLOCK_N == 64 ? 0 : group * 64 + (BLOCK_N > 128 ? 128 : 0);   // this group's last chunk
             bool released = false;
 #pragma unroll 1
-            for (int cc = (BLOCK_N == 64 ? 0 : group * 64); cc < ((IGEMM2_DBG(p.dbg) & 2) ? 0 : BLOCK_N); cc += 128) {  // dbg 2: no epilogue
+            for (int cc = (BLOCK_N == 64 ? 0 : group * 64); cc < BLOCK_N; cc += 128) {
                 uint32_t v[64];
                 tmem_ld_32x64(taddr + cc, v);
                 // the store that last read this group's staging buffer must have drained
@@ -573,7 +550,7 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                     // store of this chunk, so the MMAs of the tile after next never wait for the epilogue's tail
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0 && !(IGEMM2_DBG(p.dbg) & 16)) {
+                    if (lane == 0) {
                         if (PAIR) mbar_arrive_leader(t_empty(acc));   // the leader's MMA warp waits for both epilogues
                         else mbar_arrive(t_empty(acc));
                     }
@@ -676,10 +653,11 @@ igemm2_kernel(const __grid_constant__ Igemm2Maps maps, const Igemm2Params p) {
                     }
                 }
             }
-            if (!released) {   // debug builds without an epilogue loop
+            if (!released) {   // not reached (every group's loop ends at last_cc); dropping it reschedules the
+                               // kernel and moves its spills (profiles/r07_env_switch_removal.txt)
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0 && !(IGEMM2_DBG(p.dbg) & 16)) {
+                if (lane == 0) {
                     if (PAIR) mbar_arrive_leader(t_empty(acc));
                     else mbar_arrive(t_empty(acc));
                 }

@@ -17,7 +17,6 @@
 //   backward: context (qs & dout -> dctx) -> delta = rowsum(ctx * dctx) -> bwd_apply (dq, dk, dv)
 //
 // Workspace `ws` (fp32, per image): [HD] encoded column max | [HD] Z | [H][32][32] ctx.
-#include <cstdlib>
 #include "api_common.h"
 #include "common.cuh"
 
@@ -622,9 +621,8 @@ static int la_chunk(int n, int NI) {
     // more blocks than SMs (>= ~4 per SM: 8 measured 6 % slower forward at 192x288, 2 measured 13 % slower)
     // so that the tail wave is a small fraction, while a block still amortises its per-head fragment
     // preloads and atomics over >= 128 pixels
-    static const int per_sm = [] { const char* e = getenv("CESM_LA_BLOCKS_PER_SM"); return e ? atoi(e) : 4; }();
     int chunk = 2048;
-    while (chunk > 128 && (long long)NI * ((n + chunk - 1) / chunk) < 148 * per_sm) chunk >>= 1;
+    while (chunk > 128 && (long long)NI * ((n + chunk - 1) / chunk) < 148 * 4) chunk >>= 1;
     return chunk;
 }
 

@@ -16,8 +16,6 @@
 // TMEM: D1 double-buffered (2 x 64 columns) + D2 (6 x 64 columns) = 512 columns exactly.
 // Warps: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocation, 4..7 = epilogue (D1 -> fp16 dX rows per
 // tile; D2 -> red.add into dW once at the end).
-#include <cstdlib>
-
 #include "api_common.h"
 #include "common.cuh"
 
@@ -39,19 +37,12 @@ struct QkvBwdMaps {
     CUtensorMap x;    // [rows][64],   box {64 ci, 128 px}
     CUtensorMap w;    // [64 ci][cout] (W^T, K-major for the data gradient), box {64 co, 64 ci}
 };
-// bisection knobs only in -DCESM_QKVBWD_DEBUG builds (CESM_NVCC_EXTRA)
-#ifdef CESM_QKVBWD_DEBUG
-#define QKVBWD_DBG(x) (x)
-#else
-#define QKVBWD_DBG(x) 0
-#endif
 struct QkvBwdParams {
     long long rows;
     int tiles, chunks;          // row tiles; cout / 128
     h16* dx;          // [rows][64]
     float* dw;                  // dW[co * so + ci] (+=)
     long long so;
-    int dbg;   // CESM_QKVBWD_DBG bisection bits (debug builds only): 1 = no data-gradient MMAs, 2 = no weight-gradient MMAs
 };
 
 __global__ void __launch_bounds__(QB_THREADS, 1)
@@ -133,7 +124,6 @@ qkv_bwd_kernel(const __grid_constant__ QkvBwdMaps maps, const QkvBwdParams p) {
         if (elect_one()) {
             const uint64_t dk = make_smem_desc_sw128(0, 0, 1024);              // K-major SW128
             const uint64_t dmn = make_smem_desc_sw128(0, QB_SUB, 1024);        // MN-major: 64-channel atoms QB_SUB apart
-            const int dbg = QKVBWD_DBG(p.dbg);
             const int chunks = p.chunks;
             int st = 0, xs = 0, acc = 0, it = 0;
             uint32_t ph = 0, xph = 0, accph = 0;
@@ -149,22 +139,18 @@ qkv_bwd_kernel(const __grid_constant__ QkvBwdMaps maps, const QkvBwdParams p) {
                     const uint32_t a16 = (smem_base + st * QB_STAGE) >> 4;
                     const uint32_t w16 = a16 + ((2 * QB_SUB) >> 4);
                     // data gradient: K = 128 co = 8 steps of 16 (32 B inside a 128-byte row; second sub-tile after 4)
-                    if (!(dbg & 1)) {
 #pragma unroll
-                        for (int k = 0; k < 8; ++k) {
-                            const uint32_t ao = a16 + (k >> 2) * (QB_SUB >> 4) + (k & 3) * 2;
-                            const uint32_t bo = w16 + (k >> 2) * (QB_WSUB >> 4) + (k & 3) * 2;
-                            umma_f16(d1, dk | (uint64_t)ao, dk | (uint64_t)bo, idesc_dg, k == 0 ? (uint32_t)(c != 0) : 1u);
-                        }
+                    for (int k = 0; k < 8; ++k) {
+                        const uint32_t ao = a16 + (k >> 2) * (QB_SUB >> 4) + (k & 3) * 2;
+                        const uint32_t bo = w16 + (k >> 2) * (QB_WSUB >> 4) + (k & 3) * 2;
+                        umma_f16(d1, dk | (uint64_t)ao, dk | (uint64_t)bo, idesc_dg, k == 0 ? (uint32_t)(c != 0) : 1u);
                     }
                     // weight gradient: K = 128 pixels = 8 steps of 16 pixels (2048 B)
                     const uint32_t d2 = tmem_d2 + c * 64;
-                    if (!(dbg & 2)) {
 #pragma unroll
-                        for (int k = 0; k < 8; ++k)
-                            umma_f16(d2, dmn | (uint64_t)(a16 + k * 128), dmn | (uint64_t)(x16 + k * 128), idesc_wg,
-                                     k == 0 ? (uint32_t)(it != 0) : 1u);
-                    }
+                    for (int k = 0; k < 8; ++k)
+                        umma_f16(d2, dmn | (uint64_t)(a16 + k * 128), dmn | (uint64_t)(x16 + k * 128), idesc_wg,
+                                 k == 0 ? (uint32_t)(it != 0) : 1u);
                     umma_commit(s_empty(st));
                     if (++st == QB_STAGES) {
                         st = 0;
@@ -290,8 +276,6 @@ extern "C" int cesm_qkv_bwd(const void* dy, const void* x, const void* wt, void*
     p.dx = (h16*)dx;
     p.dw = dw;
     p.so = dw_so;
-    static const int dbg = [] { const char* e = getenv("CESM_QKVBWD_DBG"); return e ? atoi(e) : 0; }();
-    p.dbg = dbg;
     static bool cfg = false;
     if (!cfg) {
         CESM_CHECK_CUDA(cudaFuncSetAttribute(qkv_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, QB_SMEM));

@@ -345,9 +345,8 @@ class TrainEngine:
         self.launches_per_step = 0
         self._warm = 0
         self.arena = K.ZeroArena(dev) if dev.type == "cuda" else None
-        # weight gradients on a second stream (ops._on_side); CESM_NO_SIDE_STREAM=1 keeps everything on one stream
-        self.side_stream = (torch.cuda.Stream(device=dev)
-                            if dev.type == "cuda" and not int(__import__("os").environ.get("CESM_NO_SIDE_STREAM", "0")) else None)
+        # weight gradients on a second stream (ops._on_side)
+        self.side_stream = torch.cuda.Stream(device=dev) if dev.type == "cuda" else None
 
     # the captured region ----------------------------------------------------------------------
     def _step_body(self):

@@ -1,6 +1,6 @@
 """Time the implicit-GEMM kernel on the shapes of the baseline model (run on the GPU box).
 
-    python tools/bench_igemm.py            # env knobs: CESM_IGEMM_NO_HALO, CESM_IGEMM_NO_BRES
+    python tools/bench_igemm.py            # CASE=substring: only the matching shapes; PLAIN=1: 3 ungraphed calls each
 """
 import os
 import sys

@@ -1,5 +1,7 @@
 """Time the tcgen05 weight-gradient kernel on the shapes of the baseline model (run on the GPU box).
-Env knobs: CESM_WGRAD_DEEP=1 (one CTA/SM, deep TMA ring), CESM_WGRAD_CTAS=n (split-K target CTAs per SM)."""
+
+    python tools/bench_wgrad.py            # CASE=substring times only the matching shapes
+"""
 import os
 import sys
 

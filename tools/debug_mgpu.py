@@ -44,5 +44,5 @@ for tag, kw in [("default", {}), ("sync", {"sync": True}), ("1bucket", {"n_bucke
     bad = [k for k in errs if errs[k] > 1e-2]
     zero = [k for k in bad if float(gd[k].norm()) == 0.0]
     if rank == 0:
-        print(tag, "PDL" if not os.environ.get("CESM_NO_PDL") else "noPDL", "bad", len(bad), "zero", len(zero), info, flush=True)
+        print(tag, "bad", len(bad), "zero", len(zero), info, flush=True)
 torch.cuda.synchronize(); dist.barrier(); os._exit(0)

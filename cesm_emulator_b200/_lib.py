@@ -115,6 +115,7 @@ _SIGNATURES: dict[str, list] = {
     "cesm_unpack_wgrads_batched": [_P, _I, _P],
     "cesm_unpack_wgrad": [_P, _P, _I, _I, _I, _L, _L, POINTER(c_int32), _I, _P],
     "cesm_adamw_step": [_P, _P, _P, _P, _L, _P, _P, _F, _F, _F, _F, _P],
+    "cesm_adamw_ema_step": [_P, _P, _P, _P, _P, _L, _P, _P, _F, _F, _F, _F, ctypes.c_double, _L, _P],
     "cesm_colsum": [_P, _P, _L, _I, _I, _P],
     "cesm_gn_stats": [_P, _P, _I, _L, _I, _I, _P],
     "cesm_gn_apply_fwd": [_P, _P, _P, _P, _P, _P, _P, _I, _L, _I, _I, _F, _P],

@@ -145,10 +145,18 @@ grad_sumsq_kernel(const float* __restrict__ g, long long n, float* __restrict__ 
 // min(1, max_norm / (|g| + 1e-6)) (torch.nn.utils.clip_grad_norm_, train.py:865) folded in: the gradients in
 // `g` are S times the true ones; a non-finite sum of squares means some gradient overflowed fp16 -> the step
 // is skipped (parameters and moments untouched) and scaler_update_kernel backs S off.
-__global__ void __launch_bounds__(kOptThreads)
+// kEma: also the exponential moving average `ema` of the updated parameters, in the same pass -- a copy e = p while
+// the step count after this step is <= ema_start, else e += ema_w (p - e) with ema_w = 1 - decay.  A skipped step
+// returns before it.  The EMA arguments come last so that the kEma = false instance keeps the parameter layout (and
+// the code) of the kernel without them.  Left alone, ptxas gives the kEma = true instance 52 registers (4 blocks of
+// 256 per SM); the minimum of 5 blocks holds it at the 48 registers and 5 blocks of the false instance, without
+// spills.  0 leaves the false instance unconstrained, as it was.
+template <bool kEma>
+__global__ void __launch_bounds__(kOptThreads, kEma ? 5 : 0)
 adamw_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                   long long n, const float* __restrict__ partials, int n_partials, float* __restrict__ state,
-                  float beta1, float beta2, float eps, float max_norm) {
+                  float beta1, float beta2, float eps, float max_norm, float* __restrict__ ema, float ema_w,
+                  long long ema_start) {
     pdl_trigger();
     pdl_wait();
     __shared__ float s_coef;
@@ -184,9 +192,14 @@ adamw_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __r
         vv = fmaf(vv, beta2, (1.f - beta2) * gg * gg);
         pp -= step_size * mm / (sqrtf(vv) * inv_bc2_sqrt + eps);
     };
+    const bool ema_copy = (long long)step <= ema_start;
+    float4* e4 = reinterpret_cast<float4*>(ema);
+    auto ema_upd = [&](float& ee, float pp) { ee = ema_copy ? pp : fmaf(ema_w, pp - ee, ee); };
     for (long long i = (long long)blockIdx.x * kOptThreads + threadIdx.x; i < n4; i += (long long)gridDim.x * kOptThreads) {
         float4 pp = p4[i], mm = m4[i], vv = v4[i];
         const float4 gg = g4[i];
+        float4 ee;
+        if constexpr (kEma) ee = e4[i];
         upd(pp.x, gg.x, mm.x, vv.x);
         upd(pp.y, gg.y, mm.y, vv.y);
         upd(pp.z, gg.z, mm.z, vv.z);
@@ -194,10 +207,18 @@ adamw_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __r
         p4[i] = pp;
         m4[i] = mm;
         v4[i] = vv;
+        if constexpr (kEma) {
+            ema_upd(ee.x, pp.x);
+            ema_upd(ee.y, pp.y);
+            ema_upd(ee.z, pp.z);
+            ema_upd(ee.w, pp.w);
+            e4[i] = ee;
+        }
     }
     if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
         const long long i = (n4 << 2) + threadIdx.x;
         upd(p[i], g[i], m[i], v[i]);
+        if constexpr (kEma) ema_upd(ema[i], p[i]);
     }
 }
 
@@ -265,8 +286,11 @@ extern "C" int cesm_unpack_wgrads_batched(const cesm_pack_desc* descs_device, in
 
 extern "C" int cesm_adamw_partials(void) { return 148 * 4; }
 
-extern "C" int cesm_adamw_step(float* p, const float* g, float* m, float* v, long long n, float* partials,
-                               float* state, float beta1, float beta2, float eps, float max_norm, void* stream) {
+// grad_sumsq -> adamw_clip<kEma> -> scaler_update: the whole optimizer step, with or without the EMA.
+template <bool kEma>
+static int adamw_launch(float* p, const float* g, float* m, float* v, float* ema, long long n, float* partials,
+                        float* state, float beta1, float beta2, float eps, float max_norm, float ema_w,
+                        long long ema_start, void* stream) {
     CESM_REQUIRE(n > 0 && (reinterpret_cast<uintptr_t>(p) & 15) == 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0 &&
                      (reinterpret_cast<uintptr_t>(m) & 15) == 0 && (reinterpret_cast<uintptr_t>(v) & 15) == 0,
                  "adamw_step needs n > 0 and 16-byte aligned flat buffers (n=%lld)", n);
@@ -274,10 +298,27 @@ extern "C" int cesm_adamw_step(float* p, const float* g, float* m, float* v, lon
     const int nb = cesm_adamw_partials();
     launch_pdl(grad_sumsq_kernel, nb, kOptThreads, 0, st, g, n, partials, state);
     CESM_CHECK_LAUNCH();
-    launch_pdl(adamw_clip_kernel, nb * 2, kOptThreads, 0, st, p, g, m, v, n, partials, nb, state, beta1, beta2, eps,
-                                                     max_norm);
+    launch_pdl(adamw_clip_kernel<kEma>, nb * 2, kOptThreads, 0, st, p, g, m, v, n, partials, nb, state, beta1, beta2,
+               eps, max_norm, ema, ema_w, ema_start);
     CESM_CHECK_LAUNCH();
     launch_pdl(scaler_update_kernel, 1, 32, 0, st, (const float*)partials, nb, state);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
+}
+
+extern "C" int cesm_adamw_step(float* p, const float* g, float* m, float* v, long long n, float* partials,
+                               float* state, float beta1, float beta2, float eps, float max_norm, void* stream) {
+    return adamw_launch<false>(p, g, m, v, nullptr, n, partials, state, beta1, beta2, eps, max_norm, 0.f, 0, stream);
+}
+
+extern "C" int cesm_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema, long long n,
+                                   float* partials, float* state, float beta1, float beta2, float eps, float max_norm,
+                                   double ema_decay, long long ema_start, void* stream) {
+    CESM_REQUIRE(ema != nullptr && (reinterpret_cast<uintptr_t>(ema) & 15) == 0,
+                 "adamw_ema_step needs a 16-byte aligned EMA buffer");
+    CESM_REQUIRE(ema_decay >= 0.0 && ema_decay < 1.0, "adamw_ema_step needs 0 <= ema_decay < 1 (got %g)", ema_decay);
+    CESM_REQUIRE(ema_start >= 0, "adamw_ema_step needs ema_start >= 0 (got %lld)", ema_start);
+    // 1 - decay rounded once, as torch's lerp weight in AveragedModel(get_ema_multi_avg_fn(decay))
+    return adamw_launch<true>(p, g, m, v, ema, n, partials, state, beta1, beta2, eps, max_norm,
+                              (float)(1.0 - ema_decay), ema_start, stream);
 }

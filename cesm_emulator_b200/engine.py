@@ -14,6 +14,8 @@ AdamW, scaler update -- with two differences that are deliberate and documented 
 """
 from __future__ import annotations
 
+import math
+import numbers
 from typing import List, Optional
 
 import torch
@@ -204,22 +206,45 @@ class GradBuckets:
         return total
 
 
+def check_ema_args(ema_decay, ema_start):
+    """Validated (decay, start) of a weight EMA: decay None (no EMA) or a real number in [0, 1), start an integer >= 0."""
+    if ema_decay is not None:
+        if isinstance(ema_decay, bool) or not isinstance(ema_decay, numbers.Real):
+            raise ValueError(f"ema_decay must be a number in [0, 1) or None, got {ema_decay!r}")
+        ema_decay = float(ema_decay)
+        if not (math.isfinite(ema_decay) and 0.0 <= ema_decay < 1.0):
+            raise ValueError(f"ema_decay must be in [0, 1), got {ema_decay}")
+    if isinstance(ema_start, bool) or not isinstance(ema_start, numbers.Integral):
+        raise ValueError(f"ema_start must be an integer, got {ema_start!r}")
+    if ema_start < 0:
+        raise ValueError(f"ema_start must be >= 0, got {ema_start}")
+    return ema_decay, int(ema_start)
+
+
 class FusedAdamW:
     """torch.optim.AdamW (train.py:1078-1083) + torch.amp.GradScaler (train.py:862-867, 1084) + clip_grad_norm_
     (train.py:865) as three launches of the library's own kernels over flat buffers (`cesm_adamw_step`).  Step
     counter, loss scale, growth tracker, learning rate and weight decay live in a small device vector (`state`,
     layout in include/cesm_b200.h) so that a replayed CUDA graph advances / honours them.  Drop-in for what the
     engine and train.py use of an optimizer: `step()`, `state_dict()`, `load_state_dict()`,
-    `param_groups[0]["lr"]` (picked up by the next step through `sync_hparams`, also after graph capture)."""
+    `param_groups[0]["lr"]` (picked up by the next step through `sync_hparams`, also after graph capture).
+
+    With `ema_decay` set, `self.ema` is a flat fp32 exponential moving average of the parameters (same layout as
+    `self.p`, starting as a copy of it) that every step updates in the same kernel (`cesm_adamw_ema_step`): a copy
+    while the step count is <= `ema_start`, then ema += (1 - ema_decay) (p - ema).  Both are fixed per optimizer.
+    The EMA is not optimizer state: `state_dict()` stays torch AdamW's format."""
 
     def __init__(self, buckets: "GradBuckets", lr, betas, weight_decay, eps, max_grad_norm,
-                 init_scale: float = 65536.0, growth_interval: int = 2000):
+                 init_scale: float = 65536.0, growth_interval: int = 2000, ema_decay: Optional[float] = None,
+                 ema_start: int = 0):
         from . import _lib
+        self.ema_decay, self.ema_start = check_ema_args(ema_decay, ema_start)
         self._buckets = buckets
         self.g = buckets.flat
         self.p = buckets.flatten_params_()
         self.m = torch.zeros_like(self.p)
         self.v = torch.zeros_like(self.p)
+        self.ema = self.p.clone() if self.ema_decay is not None else None
         st = torch.zeros(K.OPT_STATE_FLOATS, dtype=torch.float32)
         st[K.OPT_SCALE], st[K.OPT_INTERVAL] = init_scale, growth_interval  # GradScaler() defaults
         self.state = st.to(self.p.device)
@@ -259,8 +284,12 @@ class FusedAdamW:
         if not (self.p.is_cuda and torch.cuda.is_current_stream_capturing()):
             self.sync_hparams()
         self._frozen = (tuple(hp["betas"]), float(hp["eps"]), self.max_grad_norm)
-        K.adamw_step(self.p, self.g, self.m, self.v, self.partials, self.state, hp["betas"][0], hp["betas"][1],
-                     hp["eps"], self.max_grad_norm)
+        if self.ema is None:
+            K.adamw_step(self.p, self.g, self.m, self.v, self.partials, self.state, hp["betas"][0], hp["betas"][1],
+                         hp["eps"], self.max_grad_norm)
+        else:
+            K.adamw_ema_step(self.p, self.g, self.m, self.v, self.ema, self.partials, self.state, hp["betas"][0],
+                             hp["betas"][1], hp["eps"], self.max_grad_norm, self.ema_decay, self.ema_start)
         ops.invalidate_weight_cache()  # the fp16 operand copies are stale now
 
     def _slices(self):
@@ -316,13 +345,22 @@ class FusedAdamW:
 
 
 class TrainEngine:
-    """One data-parallel training step of `Diffusion.loss` as a replayable CUDA graph."""
+    """One data-parallel training step of `Diffusion.loss` as a replayable CUDA graph.
+
+    `ema_decay` / `ema_start` (CUDA only) keep an exponential moving average of the weights inside the captured
+    optimizer step (FusedAdamW).  It starts as a copy of the weights when the engine is built; loading weights into
+    the module afterwards does not touch it -- call `reset_ema()` or `load_ema_state_dict()`.  `ema_state_dict()`
+    has the layout of `diffusion.model.state_dict()`."""
 
     def __init__(self, diffusion, batch_shape, cond_shape, lr: float = 2e-4, betas=(0.9, 0.999),
                  weight_decay: float = 1e-4, eps: float = 1e-8, max_grad_norm: Optional[float] = 1.0,
-                 n_buckets: int = 4, use_graph: bool = True, process_group=None):
+                 n_buckets: int = 4, use_graph: bool = True, process_group=None, ema_decay: Optional[float] = None,
+                 ema_start: int = 0):
+        ema_decay, ema_start = check_ema_args(ema_decay, ema_start)
         self.diffusion = diffusion
         dev = next(diffusion.parameters()).device
+        if ema_decay is not None and dev.type != "cuda":
+            raise RuntimeError("the weight EMA is updated by the CUDA optimizer step; there is none on host tensors")
         self.device = dev
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.pg = process_group
@@ -333,7 +371,8 @@ class TrainEngine:
         self.max_grad_norm = max_grad_norm
         # AdamW as train.py:1078-1083 with the clip of train.py:865 folded in; the step lives inside the graph
         if self.buckets.on_cuda:
-            self.opt = FusedAdamW(self.buckets, lr, betas, weight_decay, eps, max_grad_norm)
+            self.opt = FusedAdamW(self.buckets, lr, betas, weight_decay, eps, max_grad_norm, ema_decay=ema_decay,
+                                  ema_start=ema_start)
         else:  # host tensors: only the gloo tests of the bucket logic come through here
             self.opt = torch.optim.AdamW(self.buckets.params, lr=lr, betas=betas, weight_decay=weight_decay, eps=eps)
         self.x0 = torch.zeros(batch_shape, dtype=torch.float32, device=dev)
@@ -408,6 +447,49 @@ class TrainEngine:
         ops.invalidate_weight_cache()
 
     # public -----------------------------------------------------------------------------------
+    @property
+    def has_ema(self) -> bool:
+        return isinstance(self.opt, FusedAdamW) and self.opt.ema is not None
+
+    def _require_ema(self) -> None:
+        if not self.has_ema:
+            raise RuntimeError("this TrainEngine keeps no weight EMA (build it with ema_decay=...)")
+
+    def _ema_entries(self):
+        """(name, module tensor, flat EMA slice or None for a frozen tensor) in diffusion.model.state_dict() order."""
+        self._require_ema()
+        offsets, e = self.buckets.offsets, self.opt.ema
+        out = []
+        for name, t in self.diffusion.model.state_dict(keep_vars=True).items():
+            o = offsets.get(id(t))
+            out.append((name, t, None if o is None else e[o:o + t.numel()].view(t.shape)))
+        return out
+
+    def ema_state_dict(self) -> dict:
+        """The EMA weights in the layout of `diffusion.model.state_dict()` (a checkpoint's "model"): trainable tensors
+        from the EMA, frozen ones (the rotary `freqs`) and buffers copied from the module."""
+        return {name: (t if e is None else e).detach().clone() for name, t, e in self._ema_entries()}
+
+    def load_ema_state_dict(self, sd: dict) -> None:
+        """Load an `ema_state_dict()`; keys and shapes must match exactly.  Frozen entries are checked, not loaded."""
+        entries = self._ema_entries()
+        names = [n for n, _, _ in entries]
+        missing, unexpected = [n for n in names if n not in sd], [k for k in sd if k not in set(names)]
+        if missing or unexpected:
+            raise RuntimeError(f"EMA state dict: missing keys {missing}, unexpected keys {unexpected}")
+        bad = [n for n, t, _ in entries if tuple(sd[n].shape) != tuple(t.shape)]
+        if bad:
+            raise RuntimeError(f"EMA state dict: shape mismatch for {bad}")
+        with torch.no_grad():
+            for n, _, e in entries:
+                if e is not None:
+                    e.copy_(sd[n])
+
+    def reset_ema(self) -> None:
+        """Restart the EMA from the current weights (e.g. after loading weights into the module)."""
+        self._require_ema()
+        self.opt.ema.copy_(self.opt.p)
+
     def step_resident(self) -> torch.Tensor:
         """One step on whatever is in the static device buffers `x0` / `cond`."""
         self._run()

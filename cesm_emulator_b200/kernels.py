@@ -269,6 +269,22 @@ def adamw_step(p: torch.Tensor, g: torch.Tensor, m: torch.Tensor, v: torch.Tenso
               _meta={"bytes": 28.0 * p.numel()})
 
 
+def adamw_ema_step(p: torch.Tensor, g: torch.Tensor, m: torch.Tensor, v: torch.Tensor, ema: torch.Tensor,
+                   partials: torch.Tensor, state: torch.Tensor, beta1: float, beta2: float, eps: float,
+                   max_norm: Optional[float], ema_decay: float, ema_start: int) -> None:
+    """adamw_step plus the exponential moving average `ema` of the updated parameters in the same pass (see
+    cesm_adamw_ema_step in include/cesm_b200.h): a copy while the step count is <= ema_start, then
+    ema += (1 - ema_decay) (p - ema)."""
+    _req_cuda(p, g, m, v, ema, partials, state)
+    for t in (p, g, m, v, ema, partials, state):
+        assert t.dtype == torch.float32 and t.is_contiguous()
+    assert p.numel() == g.numel() == m.numel() == v.numel() == ema.numel() and state.numel() >= OPT_STATE_FLOATS
+    assert partials.numel() >= _lib.load().cesm_adamw_partials()
+    _lib.call("cesm_adamw_ema_step", _ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(ema), p.numel(), _ptr(partials),
+              _ptr(state), float(beta1), float(beta2), float(eps), float(max_norm) if max_norm is not None else 0.0,
+              float(ema_decay), int(ema_start), _stream(), _meta={"bytes": 36.0 * p.numel()})
+
+
 def colsum(x: torch.Tensor, into: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Column sums of fp16 x[..., C]; with `into` (fp32 [C]) the sums are ADDED to it."""
     _req_cuda(x, into)

@@ -184,6 +184,17 @@ void cesm_set_prezeroed_scratch(int on);
 int cesm_adamw_partials(void);
 int cesm_adamw_step(float* p, const float* g, float* m, float* v, long long n, float* partials, float* state,
                     float beta1, float beta2, float eps, float max_norm, void* stream);
+/* cesm_adamw_step plus an exponential moving average of the parameters, updated in the same pass and the same
+ * three launches.  `ema`: fp32[n], 16-byte aligned, laid out like `p`.  With k = the step count after this step
+ * (state[0] + 1), every non-skipped call does, after the AdamW update of p:
+ *   k <= ema_start:  ema = p                                   (exact copy)
+ *   otherwise:       ema = fmaf(1 - ema_decay, p - ema, ema)   (1 - ema_decay rounded once to fp32)
+ * ema_start = 1 is torch.optim.swa_utils.AveragedModel(multi_avg_fn=get_ema_multi_avg_fn(ema_decay)) updated after
+ * every optimizer step.  A skipped step (non-finite gradient) leaves `ema` unchanged.  Requires 0 <= ema_decay < 1
+ * and ema_start >= 0. */
+int cesm_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema, long long n, float* partials,
+                        float* state, float beta1, float beta2, float eps, float max_norm, double ema_decay,
+                        long long ema_start, void* stream);
 int cesm_unpack_wgrad(const float* src, float* dst, int O, int T, int I, long long so, long long si,
                       const int32_t* tap_off, int accumulate, void* stream);
 /* out[c] (+)= sum over rows of fp16 x[M][C] (bias gradients).  `accumulate` != 0 here and in the other

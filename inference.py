@@ -4,6 +4,7 @@
     python inference.py --ckpt runs/exp/checkpoints/final.pt [--batch_size 16] [--steps 1000] [--out pred.npy | pred.nc]
     python inference.py --ckpt ... --ddim_steps 50 [--eta 0.0]     # strided DDIM chain: 50 UNet calls per field
     python inference.py --ckpt ... --dpm_steps 15                  # DPM-Solver++(2M) chain: 15 UNet calls per field
+    python inference.py --ckpt ... --ema [--dpm_steps 15]          # sample from the weight EMA (ckpt["ema"])
     torchrun --standalone --nproc_per_node=8 inference.py --ckpt ...
 
 `predict_temperature_from_emissions` keeps the reference's flow: rebuild UNet/Diffusion from
@@ -27,13 +28,17 @@ from cesm_emulator_b200.synthetic import SyntheticEnsemble
 from train import build_model_from_config
 
 
-def load_diffusion_from_checkpoint(path, device):
-    """inference.py:47-75."""
+def load_diffusion_from_checkpoint(path, device, ema=False):
+    """inference.py:47-75.  With `ema=True` the UNet gets the checkpoint's weight EMA (ckpt["ema"], written by a run
+    with train.ema_decay set) instead of its raw weights (ckpt["model"]); a checkpoint without one is an error."""
     ckpt = torch.load(path, map_location=device)
+    if ema and "ema" not in ckpt:
+        raise KeyError(f'{path} has no "ema" entry: it was not trained with train.ema_decay set '
+                       f'(load it without ema=True / --ema to sample from its raw weights)')
     cfg = ckpt["config"]
     diffusion = Diffusion(build_model_from_config(cfg.get("unet", {})),
                           timesteps=cfg.get("diffusion", {}).get("timesteps", 1000)).to(device)
-    missing, unexpected = diffusion.model.load_state_dict(ckpt["model"], strict=False)
+    missing, unexpected = diffusion.model.load_state_dict(ckpt["ema" if ema else "model"], strict=False)
     if missing or unexpected:
         print(f"[load] missing={list(missing)} unexpected={list(unexpected)}")
     diffusion.eval()
@@ -115,6 +120,8 @@ def _cli():
     ap.add_argument("--eta", type=float, default=0.0, help="DDIM noise scale (0 = deterministic, 1 = DDPM-like)")
     ap.add_argument("--dpm_steps", type=int, default=None,
                     help="generate with a deterministic DPM-Solver++(2M) chain of this many UNet calls")
+    ap.add_argument("--ema", action="store_true",
+                    help='generate from the weight EMA stored in the checkpoint ("ema") instead of its raw weights')
     ap.add_argument("--members", type=int, default=2)
     ap.add_argument("--times", type=int, default=4)
     ap.add_argument("--out", default="pred.npy")
@@ -132,7 +139,10 @@ def _cli():
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
-    diffusion, cfg = load_diffusion_from_checkpoint(a.ckpt, dev)
+    try:
+        diffusion, cfg = load_diffusion_from_checkpoint(a.ckpt, dev, ema=a.ema)
+    except KeyError as e:
+        raise SystemExit(f"inference.py: error: {e.args[0]}")
     syn = cfg.get("data", {}).get("synthetic", {})
     ds = SyntheticEnsemble(members=a.members, times=a.times, lat=syn.get("lat", 192), lon=syn.get("lon", 288),
                            seed=syn.get("seed", 1234))

@@ -55,6 +55,8 @@ def save_checkpoint(path, epoch, diffusion, engine, cfg):
         "optimizer": engine.opt.state_dict(),
         "config": cfg,
     }
+    if engine.has_ema:
+        ckpt["ema"] = engine.ema_state_dict()  # UNet state-dict layout, like "model"
     if "grad_scaler" in ckpt["optimizer"]:  # GradScaler.state_dict() layout; the reference loads "scaler" if present (train.py:940-944)
         ckpt["scaler"] = dict(ckpt["optimizer"]["grad_scaler"])
     os.makedirs(os.path.dirname(path), exist_ok=True)
@@ -62,7 +64,8 @@ def save_checkpoint(path, epoch, diffusion, engine, cfg):
 
 
 def load_checkpoint(path, diffusion, engine=None, device="cuda"):
-    """train.py:915-946 semantics: strict=False on the UNet, buffers merged, start_epoch = epoch + 1."""
+    """train.py:915-946 semantics: strict=False on the UNet, buffers merged, start_epoch = epoch + 1.  An engine with a
+    weight EMA loads the checkpoint's "ema", or restarts the EMA from the loaded weights if it has none."""
     ckpt = torch.load(path, map_location=device)
     missing, unexpected = diffusion.model.load_state_dict(ckpt["model"], strict=False)
     if missing or unexpected:
@@ -72,6 +75,12 @@ def load_checkpoint(path, diffusion, engine=None, device="cuda"):
             getattr(diffusion, k).copy_(v.to(device))
     if engine is not None and "optimizer" in ckpt:
         engine.opt.load_state_dict(ckpt["optimizer"])
+    if engine is not None and engine.has_ema:
+        if "ema" in ckpt:
+            engine.load_ema_state_dict(ckpt["ema"])
+        else:
+            engine.reset_ema()
+            print(f"[resume] {path} has no \"ema\": the weight EMA starts from the loaded weights")
     return int(ckpt.get("epoch", 0)) + 1
 
 
@@ -94,7 +103,8 @@ def main(cfg):
     opt = tcfg.get("optimizer", {})
     engine = TrainEngine(diffusion, (B, 1, h, w), (B, 1, K, h, w), lr=opt.get("lr", 2e-4),
                          betas=tuple(opt.get("betas", (0.9, 0.999))), weight_decay=opt.get("weight_decay", 1e-4),
-                         max_grad_norm=tcfg.get("max_grad_norm", 1.0))
+                         max_grad_norm=tcfg.get("max_grad_norm", 1.0), ema_decay=tcfg.get("ema_decay"),
+                         ema_start=tcfg.get("ema_start", 0))
     start = 1
     if tcfg.get("resume") and os.path.exists(tcfg["resume"]):
         start = load_checkpoint(tcfg["resume"], diffusion, engine, dev)

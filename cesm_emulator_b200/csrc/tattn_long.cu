@@ -8,7 +8,8 @@
 // contiguous run of the q, k and v slices of those heads -- and one WARP per head does the whole
 // (F x F) attention on the tensor cores with mma.sync.m16n8k16 (fp16 in, fp32 accumulate):
 //
-//   forward : RoPE(q * scale), RoPE(k) in place;  per 16-query tile  S = Q K^T (+ bias) -> softmax in the
+//   forward : RoPE(q * scale), RoPE(k) in place as fp16 hi + lo pairs (rotate_qk);  per 16-query tile
+//             S = Q K^T (+ bias) from the pairs -> softmax in the
 //             accumulator registers -> O = P V;  O overwrites the dead q rows and leaves with 16-byte stores.
 //   backward: recomputes S from q, k and the saved log-sum-exp.  Pass B (per query tile): dP = dO V^T,
 //             dS = P (dP - delta), dQ = dS K.  Pass A (per key tile, everything transposed so that no
@@ -67,7 +68,7 @@ __device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
 
 struct Geo {
     int F, Fp, HW, H, HG;      // frames, frames padded to 16, pixels per frame, heads, heads per CTA
-    int pq;                    // row pitch of the staged q|k|v tile in halfs: 3*HG*32 + 8
+    int pq;                    // row pitch of the staged q|k|v|q_lo|k_lo tile in halfs: 5*HG*32 + 8
     int po;                    // row pitch of a staged [Fp][HG*32] tile (dout, dq) in halfs: HG*32 + 8
 };
 
@@ -93,19 +94,34 @@ __device__ __forceinline__ void stage_rows(uint32_t dst, int pitch_h, const h16*
     }
 }
 
-// In-place RoPE of this warp's q (times `scale`) and k columns: (x0, x1) -> (x0 c - x1 s, x1 c + x0 s).
+// In-place RoPE of this warp's q (times `scale`) and k columns: (x0, x1) -> (x0 c - x1 s, x1 c + x0 s).  The rotated
+// values are stored as fp16 hi + lo pairs (lo = fp32 value - hi, in the q_lo / k_lo parts of the tile): logits are
+// formed as Q_hi K_hi^T + Q_lo K_hi^T + Q_hi K_lo^T, to fp32 accuracy.  With hi alone, a logit carries an absolute
+// error of ~2^-12 |logit|, which at sharp (trained) logits of standard deviation 10 moved the output by 3.5e-3.
+// Padded rows get zero lo parts (their hi parts are zeroed by stage_rows).
 __device__ __forceinline__ void rotate_qk(uint32_t tile, const Geo& g, int w, int lane, const float* __restrict__ cs,
                                           const float* __restrict__ sn, float scale) {
-    for (int idx = lane; idx < g.F * 16; idx += 32) {
+    for (int idx = lane; idx < g.Fp * 16; idx += 32) {
         const int r = idx >> 4, m = idx & 15;
-        const float c = __ldg(cs + idx), s = __ldg(sn + idx);
         const uint32_t aq = tile + (uint32_t)(r * g.pq + w * D + 2 * m) * 2u;
         const uint32_t ak = aq + (uint32_t)(g.HG * D) * 2u;
+        const uint32_t aql = aq + (uint32_t)(3 * g.HG * D) * 2u, akl = aq + (uint32_t)(4 * g.HG * D) * 2u;
+        if (r >= g.F) {
+            sts32(aql, 0u);
+            sts32(akl, 0u);
+            continue;
+        }
+        const float c = __ldg(cs + idx), s = __ldg(sn + idx);
         float2 q = unpack_h2(lds32(aq)), k = unpack_h2(lds32(ak));
         q.x *= scale;
         q.y *= scale;
-        sts32(aq, pack_h2(q.x * c - q.y * s, q.y * c + q.x * s));
-        sts32(ak, pack_h2(k.x * c - k.y * s, k.y * c + k.x * s));
+        const float2 qr = make_float2(q.x * c - q.y * s, q.y * c + q.x * s), kr = make_float2(k.x * c - k.y * s, k.y * c + k.x * s);
+        const uint32_t qh = pack_h2(qr.x, qr.y), kh = pack_h2(kr.x, kr.y);
+        const float2 qhf = unpack_h2(qh), khf = unpack_h2(kh);
+        sts32(aq, qh);
+        sts32(ak, kh);
+        sts32(aql, pack_h2(qr.x - qhf.x, qr.y - qhf.y));
+        sts32(akl, pack_h2(kr.x - khf.x, kr.y - khf.y));
     }
 }
 
@@ -125,6 +141,26 @@ __device__ __forceinline__ void gemm_nt(float (&acc)[NT][4], const uint32_t (&a)
         uint32_t b[4];
         ldsm4(b, base + (uint32_t)((nt * 8 + (lane & 7)) * pitch_h + col0 + (lane >> 3) * 8) * 2u);
         acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+        mma(acc[nt], a[0], b[0], b[1]);
+        mma(acc[nt], a[1], b[2], b[3]);
+    }
+}
+
+// the same for logits from hi / lo pairs: acc = A_hi M_hi^T + A_lo M_hi^T + A_hi M_lo^T (small terms first)
+template <int NT>
+__device__ __forceinline__ void gemm_nt_split(float (&acc)[NT][4], const uint32_t (&a)[2][4], const uint32_t (&al)[2][4],
+                                              uint32_t base, int pitch_h, int col0, int col0_lo, int lane) {
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt) {
+        const uint32_t row = base + (uint32_t)((nt * 8 + (lane & 7)) * pitch_h + (lane >> 3) * 8) * 2u;
+        uint32_t b[4], bl[4];
+        ldsm4(b, row + (uint32_t)col0 * 2u);
+        ldsm4(bl, row + (uint32_t)col0_lo * 2u);
+        acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+        mma(acc[nt], al[0], b[0], b[1]);
+        mma(acc[nt], al[1], b[2], b[3]);
+        mma(acc[nt], a[0], bl[0], bl[1]);
+        mma(acc[nt], a[1], bl[2], bl[3]);
         mma(acc[nt], a[0], b[0], b[1]);
         mma(acc[nt], a[1], b[2], b[3]);
     }
@@ -200,10 +236,11 @@ tattn_long_fwd_kernel(const h16* __restrict__ qkv, const float* __restrict__ bia
         const float* bw = bd + w * 2 * g.Fp + (g.Fp - 1);
 #pragma unroll 1
         for (int mt = 0; mt < NT / 2; ++mt) {
-            uint32_t a[2][4];
+            uint32_t a[2][4], al[2][4];
             load_a(a, tile, g.pq, mt * 16, w * D, lane);
+            load_a(al, tile, g.pq, mt * 16, 3 * g.HG * D + w * D, lane);
             float s[NT][4];
-            gemm_nt<NT>(s, a, tile, g.pq, g.HG * D + w * D, lane);
+            gemm_nt_split<NT>(s, a, al, tile, g.pq, g.HG * D + w * D, 4 * g.HG * D + w * D, lane);
             const int i0 = mt * 16 + gq, i1 = i0 + 8;
             float m0 = -INFINITY, m1 = -INFINITY;
 #pragma unroll
@@ -329,8 +366,12 @@ tattn_long_bwd_kernel(const h16* __restrict__ qkv, const float* __restrict__ bia
         for (int mt = 0; mt < NT / 2; ++mt) {
             uint32_t a[2][4];
             float s[NT][4], dp[NT][4];
-            load_a(a, tile, g.pq, mt * 16, w * D, lane);
-            gemm_nt<NT>(s, a, tile, g.pq, g.HG * D + w * D, lane);                 // S = Q K^T
+            {
+                uint32_t al[2][4];
+                load_a(a, tile, g.pq, mt * 16, w * D, lane);
+                load_a(al, tile, g.pq, mt * 16, 3 * g.HG * D + w * D, lane);
+                gemm_nt_split<NT>(s, a, al, tile, g.pq, g.HG * D + w * D, 4 * g.HG * D + w * D, lane);   // S = Q K^T
+            }
             load_a(a, t_do, g.po, mt * 16, w * D, lane);
             gemm_nt<NT>(dp, a, tile, g.pq, 2 * g.HG * D + w * D, lane);            // dP = dO V^T
             const int i0 = mt * 16 + gq, i1 = i0 + 8;
@@ -392,8 +433,12 @@ tattn_long_bwd_kernel(const h16* __restrict__ qkv, const float* __restrict__ bia
         for (int jt = 0; jt < NT / 2; ++jt) {
             uint32_t a[2][4];
             float st[NT][4], dpt[NT][4];
-            load_a(a, tile, g.pq, jt * 16, g.HG * D + w * D, lane);
-            gemm_nt<NT>(st, a, tile, g.pq, w * D, lane);                           // S^T = K Q^T
+            {
+                uint32_t al[2][4];
+                load_a(a, tile, g.pq, jt * 16, g.HG * D + w * D, lane);
+                load_a(al, tile, g.pq, jt * 16, 4 * g.HG * D + w * D, lane);
+                gemm_nt_split<NT>(st, a, al, tile, g.pq, w * D, 3 * g.HG * D + w * D, lane);          // S^T = K Q^T
+            }
             load_a(a, tile, g.pq, jt * 16, 2 * g.HG * D + w * D, lane);
             gemm_nt<NT>(dpt, a, t_do, g.po, w * D, lane);                          // dP^T = V dO^T
             const int j0 = jt * 16 + gq, j1 = j0 + 8;
@@ -474,7 +519,7 @@ static Geo make_geo(int F, int HW, int H, int HG) {
     g.HW = HW;
     g.H = H;
     g.HG = HG;
-    g.pq = 3 * HG * D + 8;
+    g.pq = 5 * HG * D + 8;
     g.po = HG * D + 8;
     return g;
 }

@@ -106,7 +106,7 @@ def load() -> ctypes.CDLL:
 
 
 # name -> argtypes; every function returns int (cesm_status)
-_P, _I, _L, _F = c_void_p, ctypes.c_int, ctypes.c_longlong, c_float
+_P, _I, _L, _F, _U = c_void_p, ctypes.c_int, ctypes.c_longlong, c_float, ctypes.c_uint
 _SIGNATURES: dict[str, list] = {
     "cesm_igemm": [POINTER(IgemmArgs), _P],
     "cesm_wgrad": [POINTER(WgradArgs), _P],
@@ -150,6 +150,9 @@ _SIGNATURES: dict[str, list] = {
     "cesm_p_sample": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _P],
     "cesm_ddim_step": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
     "cesm_dpm_step": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
+    "cesm_field_normal": [_U, _U, _P, _U, _P, _I, _L, _P],
+    "cesm_p_sample_seeded": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
+    "cesm_ddim_step_seeded": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
 }
 
 

@@ -563,7 +563,14 @@ __global__ void scale_by_device_scalar_kernel(const float* __restrict__ in, cons
     out[idx] = in[idx] * factor * gscale[0];
 }
 // x_{t-1} = sqrt_recip_alpha[t] * (x_t - beta[t]/sqrt_1mac[t] * eps) + sqrt(post_var[t]) * z
-// (post_var[0] == 0, so t == 0 adds no noise: identical to model.py:178-183)
+// (post_var[0] == 0, so t == 0 adds no noise: identical to model.py:178-183).  Shared by the buffered-z and the
+// seeded kernel so that both round the same way.
+__device__ __forceinline__ float p_sample_update(float x, float e, float z, long long tb, const float* betas,
+                                                 const float* sqrt_1mac, const float* sqrt_recip_a,
+                                                 const float* post_var) {
+    const float mean = sqrt_recip_a[tb] * (x - betas[tb] / sqrt_1mac[tb] * e);
+    return mean + sqrtf(post_var[tb]) * z;
+}
 __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
                                 const float* __restrict__ z, const long long* __restrict__ t,
                                 const float* __restrict__ betas, const float* __restrict__ sqrt_1mac,
@@ -574,8 +581,7 @@ __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __res
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
     const long long tb = t[idx / per];
-    const float mean = sqrt_recip_a[tb] * (xt[idx] - betas[tb] / sqrt_1mac[tb] * eps[idx]);
-    out[idx] = mean + sqrtf(post_var[tb]) * z[idx];
+    out[idx] = p_sample_update(xt[idx], eps[idx], z[idx], tb, betas, sqrt_1mac, sqrt_recip_a, post_var);
 }
 // Strided DDIM step (Song et al.): x_prev = A[t] * x_t + B[t] * eps + S[t] * z, with the three coefficients of each
 // schedule timestep precomputed on the host in float64 (model.ddim_schedule) and stored as coef[T][3] fp32.
@@ -583,6 +589,8 @@ __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __res
 // z == nullptr drops the noise term (valid when every S is 0, i.e. eta = 0).  A timestep outside [0, T) writes
 // NaN instead of reading outside the table.  t_out (optional, never aliasing t) receives next_t[t] per sample;
 // an out-of-range t is passed through unchanged, so a chain that overruns its schedule keeps producing NaN.
+// The noise term is fmaf(S, z, ddim_mean(...)) in this kernel and in the seeded one.
+__device__ __forceinline__ float ddim_mean(const float* c, float x, float e) { return fmaf(c[0], x, c[1] * e); }
 __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps, const float* __restrict__ z,
                                  const long long* __restrict__ t, const float* __restrict__ coef,
                                  const long long* __restrict__ next_t, long long* __restrict__ t_out, float* out,
@@ -600,7 +608,7 @@ __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps,
         return;
     }
     const float* c = coef + 3 * tb;
-    float v = fmaf(c[0], xt[idx], c[1] * eps[idx]);
+    float v = ddim_mean(c, xt[idx], eps[idx]);
     if (z) v = fmaf(c[2], z[idx], v);
     out[idx] = v;
 }
@@ -635,6 +643,148 @@ __global__ void dpm_step_kernel(const float* xt, const float* __restrict__ eps, 
     if (k1 != 0.0f) v = fmaf(k1, hist[idx], v);
     hist[idx] = x0;
     out[idx] = v;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Counter-based noise of the seeded sampling chains.  Element e of field f in draw d is word e & 3 of
+//     Philox4x32-10(counter = (e >> 2, d, f_lo, f_hi), key = (seed_lo, seed_hi))      (Salmon et al. 2011)
+// turned into normals by Box-Muller on the word pairs (w0, w1) and (w2, w3): u = ((w >> 9) + 0.5) 2^-23 lies in
+// (0, 1) and is exact in fp32 (24 significant bits; (w >> 8) + 0.5 would need 25 and round, up to 1.0 for the largest
+// words), r = sqrt(-2 log u_a), normals (r cospi(2 u_b), r sinpi(2 u_b)).  A value depends on
+// (seed, field, draw, e) only, never on the row, the batch, the device or the launch shape.  x_T is draw 0xFFFFFFFF
+// and the step leaving timestep t draws with d = t.  logf and sincospif are the accurate ones (no fast math).
+// One thread makes one quad of one field (grid.y = field row), so a quad never crosses a field.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, unsigned k0, unsigned k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+        const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    return c;
+}
+__device__ __forceinline__ float philox_uniform(unsigned w) { return ((float)(w >> 9) + 0.5f) * 0x1p-23f; }
+__device__ __forceinline__ void box_muller(unsigned wa, unsigned wb, float& n0, float& n1) {
+    const float r = sqrtf(-2.0f * logf(philox_uniform(wa)));
+    float s, c;
+    sincospif(2.0f * philox_uniform(wb), &s, &c);
+    n0 = r * c;
+    n1 = r * s;
+}
+// The four normals of quad q (elements 4q .. 4q+3) of `field` in `draw`.
+__device__ __forceinline__ void field_normal4(unsigned seed_lo, unsigned seed_hi, long long field, unsigned draw,
+                                              long long q, float (&z)[4]) {
+    const unsigned long long f = (unsigned long long)field;
+    const uint4 w = philox4x32_10(make_uint4((unsigned)q, draw, (unsigned)f, (unsigned)(f >> 32)), seed_lo, seed_hi);
+    box_muller(w.x, w.y, z[0], z[1]);
+    box_muller(w.z, w.w, z[2], z[3]);
+}
+// n = valid elements of the quad (4 unless it is the tail of a field whose size is not a multiple of 4); kVec means
+// per % 4 == 0 with 16-byte aligned rows, so the quad is one float4.
+template <bool kVec>
+__device__ __forceinline__ void load_quad(const float* p, int n, float (&v)[4]) {
+    if (kVec) {
+        const float4 a = *reinterpret_cast<const float4*>(p);
+        v[0] = a.x, v[1] = a.y, v[2] = a.z, v[3] = a.w;
+        return;
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = j < n ? p[j] : 0.0f;
+}
+template <bool kVec>
+__device__ __forceinline__ void store_quad(float* p, int n, const float (&v)[4]) {
+    if (kVec) {
+        *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
+        return;
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        if (j < n) p[j] = v[j];
+}
+
+template <bool kVec>
+__global__ void __launch_bounds__(256)
+field_normal_kernel(unsigned seed_lo, unsigned seed_hi, const long long* __restrict__ field_ids, unsigned draw,
+                    float* __restrict__ out, long long per) {
+    pdl_trigger();
+    pdl_wait();
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (4 * q >= per) return;
+    const int b = blockIdx.y;
+    float z[4];
+    field_normal4(seed_lo, seed_hi, field_ids[b], draw, q, z);
+    store_quad<kVec>(out + (long long)b * per + 4 * q, (int)min(4LL, per - 4 * q), z);
+}
+
+// p_sample_kernel with z drawn in registers from (seed, field_ids[b], draw t[b]).  `out` may alias `xt` (a thread
+// reads its quad before writing it).  A t outside [0, T) writes NaN instead of reading outside the schedule.
+template <bool kVec>
+__global__ void __launch_bounds__(256)
+p_sample_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned seed_lo, unsigned seed_hi,
+                       const long long* __restrict__ field_ids, const long long* __restrict__ t,
+                       const float* __restrict__ betas, const float* __restrict__ sqrt_1mac,
+                       const float* __restrict__ sqrt_recip_a, const float* __restrict__ post_var, float* out, int T,
+                       long long per) {
+    pdl_trigger();
+    pdl_wait();
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (4 * q >= per) return;
+    const int b = blockIdx.y;
+    const int n = (int)min(4LL, per - 4 * q);
+    const long long off = (long long)b * per + 4 * q;
+    const long long tb = t[b];
+    float v[4];
+    if (tb < 0 || tb >= T) {
+        const float nan = __int_as_float(0x7fc00000);
+        v[0] = v[1] = v[2] = v[3] = nan;
+        store_quad<kVec>(out + off, n, v);
+        return;
+    }
+    float x[4], e[4], z[4];
+    field_normal4(seed_lo, seed_hi, field_ids[b], (unsigned)tb, q, z);
+    load_quad<kVec>(xt + off, n, x);
+    load_quad<kVec>(eps + off, n, e);
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        v[j] = p_sample_update(x[j], e[j], z[j], tb, betas, sqrt_1mac, sqrt_recip_a, post_var);
+    store_quad<kVec>(out + off, n, v);
+}
+
+// ddim_step_kernel with z drawn in registers from (seed, field_ids[b], draw t[b]); same t_out / NaN contract.
+template <bool kVec>
+__global__ void __launch_bounds__(256)
+ddim_step_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned seed_lo, unsigned seed_hi,
+                        const long long* __restrict__ field_ids, const long long* __restrict__ t,
+                        const float* __restrict__ coef, const long long* __restrict__ next_t,
+                        long long* __restrict__ t_out, float* out, int T, long long per) {
+    pdl_trigger();
+    pdl_wait();
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (4 * q >= per) return;
+    const int b = blockIdx.y;
+    const int n = (int)min(4LL, per - 4 * q);
+    const long long off = (long long)b * per + 4 * q;
+    const long long tb = t[b];
+    const bool valid = tb >= 0 && tb < T;
+    if (t_out && q == 0) t_out[b] = valid ? next_t[tb] : tb;
+    float v[4];
+    if (!valid) {
+        const float nan = __int_as_float(0x7fc00000);
+        v[0] = v[1] = v[2] = v[3] = nan;
+        store_quad<kVec>(out + off, n, v);
+        return;
+    }
+    float x[4], e[4], z[4];
+    field_normal4(seed_lo, seed_hi, field_ids[b], (unsigned)tb, q, z);
+    load_quad<kVec>(xt + off, n, x);
+    load_quad<kVec>(eps + off, n, e);
+    const float* c = coef + 3 * tb;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = fmaf(c[2], z[j], ddim_mean(c, x[j], e[j]));
+    store_quad<kVec>(out + off, n, v);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -910,6 +1060,72 @@ extern "C" int cesm_dpm_step(const float* xt, const float* eps, float* hist, con
                  "hist must not overlap xt, eps, out, t, t_out, coef or next_t");
     launch_pdl(dpm_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, hist, t, coef, next_t, t_out, out,
                T, per_sample, total);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+// Seeded sampling noise: one thread per quad of a field, grid.y = field row.  The element index inside a field is
+// the Philox counter's first word after >> 2, so a field may hold up to 2^34 elements.
+static bool quads_aligned(long long per, const void* a, const void* b = nullptr, const void* c = nullptr) {
+    const auto al = [](const void* p) { return ((uintptr_t)p & 15) == 0; };
+    return per % 4 == 0 && al(a) && al(b) && al(c);
+}
+static dim3 quad_grid(int B, long long per) { return dim3((unsigned)nblk((per + 3) / 4, 256), (unsigned)B); }
+#define CESM_REQUIRE_SEEDED_SIZES(what)                                                                          \
+    CESM_REQUIRE(B > 0 && B <= 65535 && per_sample > 0 && per_sample <= (1LL << 34),                             \
+                 what " needs 0 < B <= 65535 and 0 < per_sample <= 2^34 (B=%d per_sample=%lld)", B, per_sample)
+
+extern "C" int cesm_field_normal(unsigned seed_lo, unsigned seed_hi, const long long* field_ids, unsigned draw,
+                                 float* out, int B, long long per_sample, void* stream) {
+    CESM_REQUIRE_SEEDED_SIZES("field_normal");
+    CESM_REQUIRE(field_ids && out, "field_normal needs field_ids and out");
+    const dim3 grid = quad_grid(B, per_sample);
+    if (quads_aligned(per_sample, out))
+        launch_pdl(field_normal_kernel<true>, grid, 256, 0, as_stream(stream), seed_lo, seed_hi, field_ids, draw, out,
+                   per_sample);
+    else
+        launch_pdl(field_normal_kernel<false>, grid, 256, 0, as_stream(stream), seed_lo, seed_hi, field_ids, draw, out,
+                   per_sample);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                    const long long* field_ids, const long long* t, const float* betas,
+                                    const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var,
+                                    float* out, int T, int B, long long per_sample, void* stream) {
+    CESM_REQUIRE_SEEDED_SIZES("seeded p_sample");
+    CESM_REQUIRE(T > 0, "seeded p_sample needs T > 0 (T=%d)", T);
+    CESM_REQUIRE(xt && eps && field_ids && t && betas && sqrt_1mac && sqrt_recip_a && post_var && out,
+                 "seeded p_sample needs xt, eps, field_ids, t, the four schedule tables and out");
+    const dim3 grid = quad_grid(B, per_sample);
+    if (quads_aligned(per_sample, xt, eps, out))
+        launch_pdl(p_sample_seeded_kernel<true>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi, field_ids,
+                   t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample);
+    else
+        launch_pdl(p_sample_seeded_kernel<false>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                     const long long* field_ids, const long long* t, const float* coef,
+                                     const long long* next_t, long long* t_out, float* out, int T, int B,
+                                     long long per_sample, void* stream) {
+    CESM_REQUIRE_SEEDED_SIZES("seeded DDIM step");
+    CESM_REQUIRE(T > 0, "seeded DDIM step needs T > 0 (T=%d)", T);
+    CESM_REQUIRE(xt && eps && field_ids && t && coef && out, "seeded DDIM step needs xt, eps, field_ids, t, coef and out");
+    CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
+    CESM_REQUIRE(!t_out || ((const void*)t_out != (const void*)t && (const void*)t_out != (const void*)field_ids),
+                 "t_out must not alias t or field_ids");
+    const dim3 grid = quad_grid(B, per_sample);
+    if (quads_aligned(per_sample, xt, eps, out))
+        launch_pdl(ddim_step_seeded_kernel<true>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, coef, next_t, t_out, out, T, per_sample);
+    else
+        launch_pdl(ddim_step_seeded_kernel<false>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, coef, next_t, t_out, out, T, per_sample);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

@@ -524,11 +524,19 @@ class SampleEngine:
     With `dpm_steps=N` it runs the deterministic DPM-Solver++(2M) chain of `model.dpm_schedule` (N UNet calls per
     field).  A replay is one UNet call and one `dpm_step` launch that updates `x` and the previous-x0 buffer `hist`
     in place and writes `t_next`, copied into `t`: no noise draw, and the same library launches per step as DDIM with
-    eta = 0.  The first step does not read `hist`, so a new chain needs no reset of it."""
+    eta = 0.  The first step does not read `hist`, so a new chain needs no reset of it.
+
+    With `seed` (an int in [0, 2^64)) the noise is counter-based instead of torch's generator: x_T of the field in row
+    b is `kernels.field_normal(seed, field_ids[b], X_T_DRAW)` and the step leaving timestep t draws z with id t inside
+    the fused `p_sample_seeded` / `ddim_step_seeded` kernel.  A field's chain then depends on (seed, field id) only, not
+    on its row, its batch, `batch_size` or the rank it runs on.  The ids live in a static int64 buffer `field_ids`
+    that the graph captures by address; a replay has no noise draw and there is no z buffer."""
 
     def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0,
-                 dpm_steps: Optional[int] = None):
+                 dpm_steps: Optional[int] = None, seed: Optional[int] = None):
         from .model import ddim_schedule, dpm_schedule
+        if seed is not None:
+            K.split_seed(seed)
         if dpm_steps is not None and ddim_steps is not None:
             raise ValueError("ddim_steps and dpm_steps are mutually exclusive")
         if dpm_steps is not None and float(eta) != 0.0:
@@ -539,7 +547,11 @@ class SampleEngine:
         self.shape = tuple(shape)
         self.x = torch.zeros(self.shape, dtype=torch.float32, device=dev)
         self.cond = torch.zeros(self.shape, dtype=torch.float32, device=dev)
-        self.z = torch.zeros(self.shape, dtype=torch.float32, device=dev)
+        self.seed = None if seed is None else int(seed)
+        if seed is None:
+            self.z = torch.zeros(self.shape, dtype=torch.float32, device=dev)
+        else:
+            self.field_ids = torch.arange(self.shape[0], dtype=torch.int64, device=dev)
         self.t = torch.zeros((self.shape[0],), dtype=torch.long, device=dev)
         self.arena = K.ZeroArena(dev) if dev.type == "cuda" else None
         self.use_graph = use_graph
@@ -574,6 +586,11 @@ class SampleEngine:
             eps = d.model(self.x, self.cond, self.t)
             if self.ddim_steps is not None:
                 z = None
+                if self.seed is not None and self.eta > 0:
+                    K.ddim_step_seeded(self.x, eps, self.seed, self.field_ids, self.t, self.ddim_coef, d.T, out=self.x,
+                                       next_t=self.ddim_next_t, t_out=self.t_next)
+                    self.t.copy_(self.t_next)
+                    return
                 if self.eta > 0:
                     self.z.normal_()
                     z = self.z
@@ -585,6 +602,12 @@ class SampleEngine:
                 K.dpm_step(self.x, eps, self.hist, self.t, self.dpm_coef, d.T, out=self.x, next_t=self.dpm_next_t,
                            t_out=self.t_next)
                 self.t.copy_(self.t_next)
+                return
+            if self.seed is not None:
+                K.p_sample_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.betas,
+                                  d.sqrt_one_minus_alphas_cumprod, d.sqrt_recip_alphas, d.posterior_variance,
+                                  out=self.x)
+                self.t.sub_(1)
                 return
             self.z.normal_()  # model.py:181 randn_like; kept in a static buffer so that a caller can read the draw
             self.x.copy_(K.p_sample(self.x, eps, self.z, self.t, d.betas, d.sqrt_one_minus_alphas_cumprod,
@@ -623,10 +646,15 @@ class SampleEngine:
         ops.refresh_folds()
 
     @torch.no_grad()
-    def sample(self, cond: torch.Tensor, steps: Optional[int] = None) -> torch.Tensor:
+    def sample(self, cond: torch.Tensor, steps: Optional[int] = None, field_ids=None) -> torch.Tensor:
         """cond: [B,1,H,W] -> generated field [B,1,H,W] after `steps` (default T) reverse steps.  In DDIM and DPM
-        mode the chain is always the engine's N steps, and `steps` must be None."""
+        mode the chain is always the engine's N steps, and `steps` must be None.  `field_ids` (B integers >= 0,
+        default arange(B), repeats allowed) name the fields of a seeded engine; an unseeded one takes none."""
         T = self.diffusion.T
+        if self.seed is None and field_ids is not None:
+            raise ValueError("field_ids needs a seeded SampleEngine (SampleEngine(..., seed=...))")
+        if self.seed is not None:
+            ids = K.field_id_vector(field_ids, self.shape[0], self.device)
         if self.ddim_steps is not None:
             if steps is not None:
                 raise ValueError("steps does not apply to a DDIM-mode SampleEngine (its chain is ddim_steps long)")
@@ -638,7 +666,11 @@ class SampleEngine:
         steps = T if steps is None else steps
         self.refresh_operands()
         self.cond.copy_(cond, non_blocking=True)
-        self.x.normal_()
+        if self.seed is None:
+            self.x.normal_()
+        else:
+            self.field_ids.copy_(ids)
+            K.field_normal(self.seed, self.field_ids, K.X_T_DRAW, out=self.x)
         self.t.fill_(T - 1)
         for _ in range(steps):
             self.step()

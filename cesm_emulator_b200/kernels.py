@@ -5,6 +5,7 @@ Nothing here computes with PyTorch; torch only owns the memory and the stream.
 from __future__ import annotations
 
 import ctypes
+import numbers
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -700,4 +701,83 @@ def dpm_step(xt, eps, hist, t, coef, T: int, out=None, next_t=None, t_out=None):
     B = xt.shape[0]
     _lib.call("cesm_dpm_step", _ptr(xt), _ptr(eps), _ptr(hist), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out),
               _ptr(out), T, B, xt.numel() // B, _stream())
+    return out
+
+
+# ---- seeded sampling noise ------------------------------------------------------------------------
+X_T_DRAW = 0xFFFFFFFF  # draw id of the initial noise x_T; the step leaving timestep t draws with id t
+
+
+def split_seed(seed) -> Tuple[int, int]:
+    """A sampling seed (an int in [0, 2^64), not a bool) -> its (low, high) 32-bit words, the Philox key."""
+    if isinstance(seed, bool) or not isinstance(seed, numbers.Integral) or not 0 <= int(seed) < 1 << 64:
+        raise ValueError(f"seed must be an integer in [0, 2**64), got {seed!r}")
+    seed = int(seed)
+    return seed & 0xFFFFFFFF, seed >> 32
+
+
+def field_id_vector(field_ids, B: int, device) -> torch.Tensor:
+    """Validate the field ids of a seeded chain -> int64 [B] on `device`.  None means arange(B); ids must be integers
+    >= 0, and repeats are allowed (padding rows that regenerate a real field)."""
+    if field_ids is None:
+        return torch.arange(B, dtype=torch.int64, device=device)
+    ids = torch.as_tensor(field_ids)
+    if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+        raise ValueError(f"field_ids must be integers, got dtype {ids.dtype}")
+    if tuple(ids.shape) != (B,):
+        raise ValueError(f"field_ids must have shape ({B},), got {tuple(ids.shape)}")
+    ids = ids.to(torch.int64)
+    if bool((ids < 0).any()):
+        raise ValueError("field_ids must be >= 0")
+    return ids.to(device)
+
+
+def _seeded_ids(field_ids: torch.Tensor, B: int) -> None:
+    assert field_ids.dtype == torch.int64 and field_ids.shape == (B,), (field_ids.dtype, tuple(field_ids.shape), B)
+
+
+def field_normal(seed: int, field_ids: torch.Tensor, draw: int, shape=None, out: Optional[torch.Tensor] = None):
+    """out[b] = the standard normals of field `field_ids[b]` in draw `draw` under `seed` (counter-based Philox4x32-10,
+    see include/cesm_b200.h): the same values whatever the row, batch or device.  Give `out` or the [B, ...] `shape`."""
+    lo, hi = split_seed(seed)
+    out = torch.empty(shape, dtype=torch.float32, device=field_ids.device) if out is None else out
+    _req_cuda(field_ids, out)
+    assert out.dtype == torch.float32 and 0 <= int(draw) <= 0xFFFFFFFF
+    B = out.shape[0]
+    _seeded_ids(field_ids, B)
+    _lib.call("cesm_field_normal", lo, hi, _ptr(field_ids), int(draw), _ptr(out), B, out.numel() // B, _stream())
+    return out
+
+
+def p_sample_seeded(xt, eps, seed: int, field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out=None):
+    """p_sample with z = field_normal(seed, field_ids, draw=t[b]) drawn inside the kernel (no z buffer), bit-identical
+    to p_sample fed that draw.  `out` may be `xt` (in place).  A t outside [0, T) gives NaN."""
+    lo, hi = split_seed(seed)
+    _req_cuda(xt, eps, field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out)
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    out = torch.empty_like(xt) if out is None else out
+    assert out.dtype == torch.float32 and out.shape == xt.shape
+    B = xt.shape[0]
+    _seeded_ids(field_ids, B)
+    _lib.call("cesm_p_sample_seeded", _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(betas),
+              _ptr(sqrt_1mac), _ptr(sqrt_recip_a), _ptr(post_var), _ptr(out), betas.shape[0], B, xt.numel() // B,
+              _stream())
+    return out
+
+
+def ddim_step_seeded(xt, eps, seed: int, field_ids, t, coef, T: int, out=None, next_t=None, t_out=None):
+    """ddim_step with z = field_normal(seed, field_ids, draw=t[b]) drawn inside the kernel (no z buffer),
+    bit-identical to ddim_step fed that draw.  Same `out` / `next_t` / `t_out` contract as ddim_step."""
+    lo, hi = split_seed(seed)
+    _req_cuda(xt, eps, field_ids, t, coef, out, next_t, t_out)
+    assert coef.dtype == torch.float32 and coef.shape == (T, 3), (coef.dtype, tuple(coef.shape), T)
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert (t_out is None) == (next_t is None), "next_t and t_out go together"
+    assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
+    out = torch.empty_like(xt) if out is None else out
+    assert out.dtype == torch.float32 and out.shape == xt.shape
+    B = xt.shape[0]
+    _seeded_ids(field_ids, B)
+    _lib.call("cesm_ddim_step_seeded", _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(coef),
+              _ptr(next_t), _ptr(t_out), _ptr(out), T, B, xt.numel() // B, _stream())
     return out

@@ -187,39 +187,61 @@ class Diffusion(nn.Module):
                               self.betas, self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
                               self.posterior_variance)
 
-    def sample(self, cond, shape, device):
-        """model.py:186-194."""
+    def _x_T(self, shape, device, seed, field_ids):
+        """Initial noise: torch's CUDA generator without a seed; with one, the counter-based draw of each field id
+        (kernels.field_normal), which is what SampleEngine(seed=...) starts from too.  -> (x_T, ids or None)."""
+        if seed is None:
+            if field_ids is not None:
+                raise ValueError("field_ids needs a seed (they select counter-based noise)")
+            return torch.randn(shape, device=device), None
+        K.split_seed(seed)
+        ids = K.field_id_vector(field_ids, shape[0], device)
+        return K.field_normal(seed, ids, K.X_T_DRAW, shape), ids
+
+    def sample(self, cond, shape, device, *, seed=None, field_ids=None):
+        """model.py:186-194.  With `seed` (an int in [0, 2^64)) every field's noise is drawn from (seed, its id in
+        `field_ids`, default arange(B)) instead of torch's generator, so a field does not depend on its row or batch."""
         with torch.no_grad():
             B = shape[0]
-            x = torch.randn(shape, device=device)
+            x, ids = self._x_T(shape, device, seed, field_ids)
             for tt in reversed(range(self.T)):
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
-                x = self.p_sample(x, cond, t_tensor)
+                if ids is None:
+                    x = self.p_sample(x, cond, t_tensor)
+                    continue
+                eps_theta = self.model(x, cond, t_tensor)
+                x = K.p_sample_seeded(x.float().contiguous(), eps_theta, seed, ids, t_tensor, self.betas,
+                                      self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
+                                      self.posterior_variance)
             return x
 
-    def ddim_sample(self, cond, shape, device, steps=50, eta=0.0):
+    def ddim_sample(self, cond, shape, device, steps=50, eta=0.0, *, seed=None, field_ids=None):
         """Strided DDIM chain of `steps` UNet calls (ddim_schedule), eager; an addition beyond the reference.
-        Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T."""
+        Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T.  `seed` / `field_ids` as in `sample`."""
         taus, coef, _ = ddim_schedule(self.alphas_cumprod, steps, eta)
         coef = coef.to(device)
         with torch.no_grad():
             B = shape[0]
-            x = torch.randn(shape, device=device)
+            x, ids = self._x_T(shape, device, seed, field_ids)
             for tt in taus:
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
                 eps_theta = self.model(x, cond, t_tensor)
+                if ids is not None and eta > 0:
+                    x = K.ddim_step_seeded(x, eps_theta, seed, ids, t_tensor, coef, self.T)
+                    continue
                 z = torch.randn_like(x) if eta > 0 else None
                 x = K.ddim_step(x, eps_theta, z, t_tensor, coef, self.T)
             return x
 
-    def dpm_sample(self, cond, shape, device, steps=20):
+    def dpm_sample(self, cond, shape, device, steps=20, *, seed=None, field_ids=None):
         """DPM-Solver++(2M) chain of `steps` UNet calls (dpm_schedule), eager; an addition beyond the reference.
-        Deterministic after x_T.  `hist` carries the previous step's x0 prediction; the first step does not read it."""
+        Deterministic after x_T.  `hist` carries the previous step's x0 prediction; the first step does not read it.
+        `seed` / `field_ids` as in `sample` (only x_T is random)."""
         taus, coef, _ = dpm_schedule(self.alphas_cumprod, steps)
         coef = coef.to(device)
         with torch.no_grad():
             B = shape[0]
-            x = torch.randn(shape, device=device)
+            x, _ = self._x_T(shape, device, seed, field_ids)
             hist = torch.empty_like(x)
             for tt in taus:
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)

@@ -380,6 +380,30 @@ int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long lon
                   const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
                   void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Seeded sampling noise.  Element e of field f in draw d is word e & 3 of Philox4x32-10 with counter
+ * (e >> 2, d, f_lo, f_hi) and key (seed_lo, seed_hi), mapped to normals by Box-Muller on the word pairs (w0, w1) and
+ * (w2, w3): u = ((w >> 9) + 0.5) * 2^-23 (exact in fp32, inside (0, 1)), r = sqrtf(-2 logf(u_a)),
+ * (r cospi(2 u_b), r sinpi(2 u_b)).  A value depends
+ * on (seed, field id, draw, e) only.  x_T is draw 0xFFFFFFFF; the reverse step leaving timestep t draws with d = t.
+ * field_ids is an int64 [B] device vector (one id per row); rows are per_sample floats.  All three reject B outside
+ * [1, 65535], per_sample outside [1, 2^34] and NULL pointers with CESM_ERR_INVALID.
+ * ---------------------------------------------------------------------------------------------- */
+/* out[b] = the normals of field field_ids[b] in `draw`. */
+int cesm_field_normal(unsigned seed_lo, unsigned seed_hi, const long long* field_ids, unsigned draw, float* out,
+                      int B, long long per_sample, void* stream);
+/* cesm_p_sample with z = the field's draw t[b], made in registers: bit-identical to cesm_p_sample fed
+ * cesm_field_normal(draw = t[b]).  out may equal xt.  A t outside [0, T) writes NaN; rejects T <= 0. */
+int cesm_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                         const long long* field_ids, const long long* t, const float* betas, const float* sqrt_1mac,
+                         const float* sqrt_recip_a, const float* post_var, float* out, int T, int B,
+                         long long per_sample, void* stream);
+/* cesm_ddim_step with z = the field's draw t[b], made in registers: bit-identical to cesm_ddim_step fed
+ * cesm_field_normal(draw = t[b]).  Same out / t_out / NaN contract; t_out must not alias t or field_ids. */
+int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                          const long long* field_ids, const long long* t, const float* coef, const long long* next_t,
+                          long long* t_out, float* out, int T, int B, long long per_sample, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,6 +5,7 @@
     python inference.py --ckpt ... --ddim_steps 50 [--eta 0.0]     # strided DDIM chain: 50 UNet calls per field
     python inference.py --ckpt ... --dpm_steps 15                  # DPM-Solver++(2M) chain: 15 UNet calls per field
     python inference.py --ckpt ... --ema [--dpm_steps 15]          # sample from the weight EMA (ckpt["ema"])
+    python inference.py --ckpt ... --seed 7                        # counter-based noise: same fields on any world size
     torchrun --standalone --nproc_per_node=8 inference.py --ckpt ...
 
 `predict_temperature_from_emissions` keeps the reference's flow: rebuild UNet/Diffusion from
@@ -17,6 +18,7 @@ through scipy (xarray / netCDF4 are not in this image).
 """
 import argparse
 import os
+import sys
 
 import numpy as np
 import torch
@@ -49,11 +51,16 @@ def load_diffusion_from_checkpoint(path, device, ema=False):
 
 @torch.no_grad()
 def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_size=16, steps=None, rank=0, world=1,
-                                       device="cuda", ddim_steps=None, eta=0.0, dpm_steps=None):
+                                       device="cuda", ddim_steps=None, eta=0.0, dpm_steps=None, seed=None):
     """cond (T, M, 1, H, W) -> prediction (T, M, H, W); fields are independent and sharded over ranks.
     `ddim_steps=N` generates with the strided DDIM chain (N UNet calls per field, noise scaled by `eta`) instead of
     the full DDPM chain; it cannot be combined with `steps`.  `dpm_steps=N` generates with the deterministic
-    DPM-Solver++(2M) chain (N UNet calls per field); it cannot be combined with `steps`, `ddim_steps` or eta != 0."""
+    DPM-Solver++(2M) chain (N UNet calls per field); it cannot be combined with `steps`, `ddim_steps` or eta != 0.
+
+    With `seed` (an int in [0, 2^64)) the noise of (year index t, member m) is drawn from the field id (t << 32) | m,
+    so the prediction does not depend on `batch_size`, on the number of ranks or on --times / --members, up to
+    run-to-run rounding.  Without it every rank draws from torch's CUDA generator, whose default seed is the same on
+    every process."""
     if ddim_steps is not None and steps is not None:
         raise ValueError("steps and ddim_steps are mutually exclusive")
     if dpm_steps is not None and (steps is not None or ddim_steps is not None):
@@ -61,6 +68,9 @@ def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_
     if dpm_steps is not None and eta != 0:
         raise ValueError(f"eta applies to DDIM only; dpm_steps is deterministic (got eta={eta})")
     T, M, _, H, W = cond_tm1hw.shape
+    if seed is None and world > 1 and rank == 0:
+        print(f"inference: the {world} ranks share one noise stream, so members can coincide; --seed gives every "
+              "field its own noise", file=sys.stderr)
     flat = torch.from_numpy(cond_tm1hw.reshape(T * M, 1, H, W))
     mine = list(range(rank, T * M, world))
     out = torch.zeros((T * M, 1, H, W), dtype=torch.float32)
@@ -71,8 +81,13 @@ def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_
         if c.shape[0] < batch_size:  # keep the captured graph's static shape
             c = torch.cat([c, c[-1:].expand(batch_size - c.shape[0], -1, -1, -1)], 0)
         if eng is None:
-            eng = SampleEngine(diffusion, (batch_size, 1, H, W), ddim_steps=ddim_steps, eta=eta, dpm_steps=dpm_steps)
-        y = eng.sample(c.to(device), steps=steps)
+            eng = SampleEngine(diffusion, (batch_size, 1, H, W), ddim_steps=ddim_steps, eta=eta, dpm_steps=dpm_steps,
+                               seed=seed)
+        ids = None
+        if seed is not None:  # padding rows repeat the last real field
+            ids = [((k // M) << 32) | (k % M) for k in sel]
+            ids = torch.tensor(ids + ids[-1:] * (batch_size - len(sel)), dtype=torch.int64)
+        y = eng.sample(c.to(device), steps=steps, field_ids=ids)
         out[sel] = y[: len(sel)].cpu()
     if world > 1:
         out = out.to(device)
@@ -110,7 +125,7 @@ def write_prediction_netcdf(path, pred_tmhw: np.ndarray, stack_coord=None, membe
             setattr(v, k, val)
 
 
-def _cli():
+def _parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--ckpt", required=True)
     ap.add_argument("--batch_size", type=int, default=16)
@@ -122,16 +137,26 @@ def _cli():
                     help="generate with a deterministic DPM-Solver++(2M) chain of this many UNet calls")
     ap.add_argument("--ema", action="store_true",
                     help='generate from the weight EMA stored in the checkpoint ("ema") instead of its raw weights')
+    ap.add_argument("--seed", type=int, default=None,
+                    help="draw every field's noise from (seed, year, member), in [0, 2**64): the output then does not "
+                         "depend on --batch_size or the number of GPUs")
     ap.add_argument("--members", type=int, default=2)
     ap.add_argument("--times", type=int, default=4)
     ap.add_argument("--out", default="pred.npy")
-    a = ap.parse_args()
+    a = ap.parse_args(argv)
     if a.steps is not None and a.ddim_steps is not None:
         ap.error("--steps and --ddim_steps are mutually exclusive")
     if a.dpm_steps is not None and (a.steps is not None or a.ddim_steps is not None):
         ap.error("--dpm_steps cannot be combined with --steps or --ddim_steps")
     if a.dpm_steps is not None and a.eta != 0:
         ap.error("--eta applies to --ddim_steps only; --dpm_steps is deterministic")
+    if a.seed is not None and not 0 <= a.seed < 1 << 64:
+        ap.error(f"--seed must be in [0, 2**64), got {a.seed}")
+    return a
+
+
+def _cli():
+    a = _parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, local = int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
@@ -147,7 +172,7 @@ def _cli():
     ds = SyntheticEnsemble(members=a.members, times=a.times, lat=syn.get("lat", 192), lon=syn.get("lon", 288),
                            seed=syn.get("seed", 1234))
     pred = predict_temperature_from_emissions(diffusion, ds.cond, a.batch_size, a.steps, rank, world, dev,
-                                              ddim_steps=a.ddim_steps, eta=a.eta, dpm_steps=a.dpm_steps)
+                                              ddim_steps=a.ddim_steps, eta=a.eta, dpm_steps=a.dpm_steps, seed=a.seed)
     if rank == 0:
         if a.out.endswith(".nc"):
             write_prediction_netcdf(a.out, pred, attrs={"checkpoint": os.path.abspath(a.ckpt), "cond_var": "synthetic"})

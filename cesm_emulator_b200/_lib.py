@@ -139,12 +139,14 @@ _SIGNATURES: dict[str, list] = {
     "cesm_input_weight_pack": [_P, _P, _P, _I, _I, _I, _P],
     "cesm_input_conv_fwd": [_P, _P, _I, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     "cesm_input_conv_wgrad": [_P, _P, _I, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
+    "cesm_input_conv_dgrad": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _F, _I, _P],
     "cesm_out_conv_fwd": [_P, _P, _P, _P, _I, _I, _I, _L, _I, _P],
     "cesm_out_conv_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _L, _I, _P],
     "cesm_sinusoidal": [_P, _P, _I, _I, _P],
     "cesm_small_linear_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _P],
     "cesm_small_linear_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P],
     "cesm_q_sample": [_P, _P, _P, _P, _P, _P, _I, _L, _P],
+    "cesm_q_sample_bwd": [_P, _P, _P, _P, _P, _P, _I, _L, _P],
     "cesm_mse_fwd": [_P, _P, _P, _P, _L, _P],
     "cesm_scale_by_scalar": [_P, _P, _F, _P, _L, _P],
     "cesm_p_sample": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _P],

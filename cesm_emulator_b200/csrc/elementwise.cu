@@ -286,6 +286,87 @@ input_conv_wgrad_kernel(const float* __restrict__ in0, const float* __restrict__
     }
 }
 
+// d_in_p[b][fp][h][w] (+)= scale * sum_f sum_co sum_{kh,kw} dy[(b,f)][h-kh+PAD][w-kw+PAD][co] * W[co][p][kh][kw]:
+// the transposed convolution of the input conv (zero padding), fp32 accumulation.  A block owns a 16x16 pixel tile
+// of one batch element and walks its F frames: plane p is written after every frame when fp == F, and summed over
+// the frames (the forward's broadcast) when fp == 1 < F.  Thread = one pixel.  Dynamic shared memory: the weights
+// as float4 {W[co][0][t], W[co][1][t], W[co+1][0][t], W[co+1][1][t]} per (tap, channel pair), then the frame's dy
+// halo tile as half2 words with a pixel stride of COUT/2 + 1 words and a row stride = 16 (mod 32) words, so the 32
+// pixels (2 rows x 16) a warp reads per channel pair fall in 32 different banks.
+template <int KS, int COUT>
+struct InputDgradSmem {
+    static constexpr int T = 16, PAD = KS / 2, PW = T + KS - 1, CP = COUT / 2, PS = CP + 1;
+    static constexpr int RS = PW * PS + ((16 - (PW * PS) % 32) + 32) % 32;
+    static constexpr size_t W_BYTES = (size_t)KS * KS * CP * sizeof(float4);
+    static constexpr size_t BYTES = W_BYTES + (size_t)PW * RS * sizeof(uint32_t);
+};
+template <int KS, int COUT, bool DX, bool DC>
+__global__ void __launch_bounds__(256)
+input_conv_dgrad_kernel(const h16* __restrict__ dy, const float* __restrict__ w /* [COUT][2][KS][KS] */,
+                        float* __restrict__ dx, float* __restrict__ dc, int f0, int f1, int F, int H, int W,
+                        float scale, int accumulate) {
+    pdl_trigger();
+    pdl_wait();
+    using S = InputDgradSmem<KS, COUT>;
+    constexpr int T = S::T, PAD = S::PAD, PW = S::PW, CP = S::CP, PS = S::PS, RS = S::RS, KK = KS * KS;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float4* sw = reinterpret_cast<float4*>(smem_raw);                       // [KK][CP]
+    uint32_t* sdy = reinterpret_cast<uint32_t*>(smem_raw + S::W_BYTES);     // [PW][RS], half2 words
+    for (int x = threadIdx.x; x < KK * CP; x += 256) {
+        const int tap = x / CP, cp = x % CP;
+        const float* wa = w + (size_t)(2 * cp) * 2 * KK;
+        const float* wb = wa + 2 * KK;
+        sw[x] = make_float4(wa[tap], wa[KK + tap], wb[tap], wb[KK + tap]);
+    }
+    const int b = blockIdx.z, h0 = blockIdx.y * T, w0 = blockIdx.x * T;
+    const int ty = threadIdx.x / T, tx = threadIdx.x % T;
+    const int h = h0 + ty, ww = w0 + tx;
+    const bool inside = h < H && ww < W;
+    const size_t HW = (size_t)H * W, pix = (size_t)h * W + ww;
+    const auto put = [&](float* p, float v) { *p = accumulate ? fmaf(scale, v, *p) : scale * v; };
+    float a0 = 0.f, a1 = 0.f;
+    for (int f = 0; f < F; ++f) {
+        const size_t img = (size_t)b * F + f;
+        __syncthreads();  // the previous frame's tile has been read by every thread
+        for (int x = threadIdx.x; x < PW * PW * (COUT / 8); x += 256) {
+            const int px = x / (COUT / 8), v8 = x % (COUT / 8);
+            const int r = px / PW, c = px % PW;
+            const int hh = h0 - PAD + r, wq = w0 - PAD + c;
+            uint4 u = make_uint4(0, 0, 0, 0);
+            if (hh >= 0 && hh < H && wq >= 0 && wq < W)
+                u = *reinterpret_cast<const uint4*>(dy + ((img * H + hh) * W + wq) * COUT + v8 * 8);
+            uint32_t* d = sdy + r * RS + c * PS + v8 * 4;
+            d[0] = u.x; d[1] = u.y; d[2] = u.z; d[3] = u.w;
+        }
+        __syncthreads();
+        // dy row of tap kh is h - kh + PAD, i.e. halo row ty - kh + 2*PAD (the halo starts at h0 - PAD)
+        for (int kh = 0; kh < KS; ++kh) {
+#pragma unroll
+            for (int kw = 0; kw < KS; ++kw) {
+                const uint32_t* dp = sdy + (ty - kh + 2 * PAD) * RS + (tx - kw + 2 * PAD) * PS;
+                const float4* wp = sw + (kh * KS + kw) * CP;
+#pragma unroll 8
+                for (int cp = 0; cp < CP; ++cp) {
+                    const float2 g = unpack_h2(dp[cp]);
+                    const float4 q = wp[cp];
+                    if (DX) { a0 = fmaf(g.x, q.x, a0); a0 = fmaf(g.y, q.z, a0); }
+                    if (DC) { a1 = fmaf(g.x, q.y, a1); a1 = fmaf(g.y, q.w, a1); }
+                }
+            }
+        }
+        if (DX && f0 == F) {
+            if (inside) put(dx + ((size_t)b * F + f) * HW + pix, a0);
+            a0 = 0.f;
+        }
+        if (DC && f1 == F) {
+            if (inside) put(dc + ((size_t)b * F + f) * HW + pix, a1);
+            a1 = 0.f;
+        }
+    }
+    if (DX && f0 != F && inside) put(dx + (size_t)b * HW + pix, a0);
+    if (DC && f1 != F && inside) put(dc + (size_t)b * HW + pix, a1);
+}
+
 // eps[b][h][w] = bias + sum_c a[(b*F + mid)][h][w][c] * w[c]   ; 8 lanes per pixel (C == 64)
 __global__ void __launch_bounds__(256)
 out_conv_fwd_kernel(const h16* __restrict__ a, const float* __restrict__ w, const float* __restrict__ bias,
@@ -529,6 +610,19 @@ __global__ void q_sample_kernel(const float* __restrict__ x0, const float* __res
     if (idx >= total) return;
     const long long tb = t[idx / per];
     xt[idx] = sqrt_ac[tb] * x0[idx] + sqrt_1mac[tb] * noise[idx];
+}
+// dx0 = sqrt_ac[t] * g, dnoise = sqrt_1mac[t] * g (either may be null)
+__global__ void q_sample_bwd_kernel(const float* __restrict__ g, const long long* __restrict__ t,
+                                    const float* __restrict__ sqrt_ac, const float* __restrict__ sqrt_1mac,
+                                    float* __restrict__ dx0, float* __restrict__ dnoise, long long per, long long total) {
+    pdl_trigger();
+    pdl_wait();
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= total) return;
+    const long long tb = t[idx / per];
+    const float gv = g[idx];
+    if (dx0) dx0[idx] = sqrt_ac[tb] * gv;
+    if (dnoise) dnoise[idx] = sqrt_1mac[tb] * gv;
 }
 // loss += sum (eps-noise)^2 / total ; diff = eps - noise
 __global__ void __launch_bounds__(256)
@@ -913,6 +1007,35 @@ extern "C" int cesm_input_conv_wgrad(const float* in0, const float* in1, int f0,
     return CESM_OK;
 }
 
+template <bool DX, bool DC>
+static int launch_input_conv_dgrad(const void* dy, const float* w, float* dx, float* dc, int f0, int f1, int B, int F,
+                                   int H, int W, float scale, int accumulate, cudaStream_t st) {
+    auto kern = input_conv_dgrad_kernel<7, 64, DX, DC>;
+    constexpr size_t smem = InputDgradSmem<7, 64>::BYTES;
+    static bool attr_set = false;
+    if (!attr_set) {
+        CESM_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_set = true;
+    }
+    dim3 grid(ceil_div(W, 16), ceil_div(H, 16), B);
+    launch_pdl(kern, grid, 256, smem, st, (const h16*)dy, w, dx, dc, f0, f1, F, H, W, scale, accumulate);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_input_conv_dgrad(const void* dy, const float* w, float* d_in0, float* d_in1, int f0, int f1, int B,
+                                     int F, int H, int W, int ks, int cout, float scale, int accumulate, void* stream) {
+    CESM_REQUIRE(ks == 7 && cout == 64, "input conv kernel is specialised for 7x7, 64 channels (ks=%d cout=%d)", ks, cout);
+    CESM_REQUIRE(B > 0 && B <= 65535 && F > 0 && H > 0 && W > 0, "bad input conv dgrad shape (B=%d F=%d H=%d W=%d)", B, F,
+                 H, W);
+    CESM_REQUIRE((f0 == 1 || f0 == F) && (f1 == 1 || f1 == F), "frame counts must be 1 or F");
+    CESM_REQUIRE(dy && w && (d_in0 || d_in1), "input conv dgrad needs dy, w and at least one output");
+    cudaStream_t st = as_stream(stream);
+    if (d_in0 && d_in1) return launch_input_conv_dgrad<true, true>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
+    if (d_in0) return launch_input_conv_dgrad<true, false>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
+    return launch_input_conv_dgrad<false, true>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
+}
+
 extern "C" int cesm_out_conv_fwd(const void* a, const float* w, const float* bias, float* eps, int B, int F, int mid,
                                  long long HW, int C, void* stream) {
     CESM_REQUIRE(C == 64, "output conv kernel needs 64 input channels (C=%d)", C);
@@ -991,6 +1114,18 @@ extern "C" int cesm_q_sample(const float* x0, const float* noise, const long lon
                              const float* sqrt_1mac, float* xt, int B, long long per_sample, void* stream) {
     const long long total = (long long)B * per_sample;
     launch_pdl(q_sample_kernel, nblk(total, 256), 256, 0, as_stream(stream), x0, noise, t, sqrt_ac, sqrt_1mac, xt, per_sample, total);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_q_sample_bwd(const float* g, const long long* t, const float* sqrt_ac, const float* sqrt_1mac,
+                                 float* dx0, float* dnoise, int B, long long per_sample, void* stream) {
+    CESM_REQUIRE(B > 0 && per_sample > 0, "bad q_sample backward sizes (B=%d per_sample=%lld)", B, per_sample);
+    CESM_REQUIRE(g && t && sqrt_ac && sqrt_1mac && (dx0 || dnoise),
+                 "q_sample backward needs g, t, both schedule tables and at least one output");
+    const long long total = (long long)B * per_sample;
+    launch_pdl(q_sample_bwd_kernel, nblk(total, 256), 256, 0, as_stream(stream), g, t, sqrt_ac, sqrt_1mac, dx0, dnoise,
+               per_sample, total);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

@@ -675,3 +675,166 @@ class SampleEngine:
         for _ in range(steps):
             self.step()
         return self.x.clone()
+
+
+SALIENCY_LOSS_SCALE = 65536.0
+
+
+def saliency_timesteps(T: int, draws) -> torch.Tensor:
+    """Stratified saliency timesteps t_d = floor((d + 1/2) T / D), d = 0..D-1: the midpoint of each of D equal strata
+    of [0, T), deterministic and the same for every field.  D must be an integer in [1, T] (distinct timesteps).
+    -> int64 [D] on the CPU."""
+    if isinstance(draws, bool) or not isinstance(draws, numbers.Integral):
+        raise ValueError(f"draws must be an integer, got {draws!r}")
+    D = int(draws)
+    if not 1 <= D <= T:
+        raise ValueError(f"draws must be in [1, {T}], got {D}")
+    return torch.tensor([(2 * d + 1) * T // (2 * D) for d in range(D)], dtype=torch.int64)
+
+
+class SaliencyEngine:
+    """Emission saliency of a frozen model: how sensitive the denoising loss is to each pixel and frame of the
+    condition.  For field b (target x0_b, condition window cond_b),
+
+        S_b = (1/D) sum_d  d/d cond_b  MSE_b(eps_theta(q_sample(x0_b, t_d, eps_d), cond_b, t_d), eps_d),
+
+    where MSE_b is the mean over field b's own H*W pixels.  `Diffusion.loss` is the mean over the whole batch, so
+    its gradient is multiplied by B: a field's saliency does not depend on the batch it is computed in.
+
+    Timesteps: `saliency_timesteps(T, draws)` (stratified, no RNG), or an explicit int64 `timesteps` tensor of shape
+    [D] (the same for every field) or [D, B].  Noise: torch's CUDA generator; with `seed` (an int in [0, 2^64)) the
+    counter-based normals of `kernels.field_normal(seed, field_id, SALIENCY_DRAW_BASE + d)`, so a field's saliency
+    depends on (seed, field id) only -- not on its row, its batch or the rank it runs on.
+
+    One draw is a forward and a backward with frozen weights (no weight-gradient launch), captured once as a CUDA
+    graph and replayed D times; the condition gradient is added, scaled by B / D, straight into the output buffer by
+    the input convolution's data-gradient kernel.  Every parameter must have requires_grad False
+    (`inference.load_diffusion_from_checkpoint` freezes them); the training gradient sink is off while a draw runs,
+    so a TrainEngine in the same process never receives saliency gradients.  `launches_per_step` counts the library
+    launches of one draw."""
+
+    def __init__(self, diffusion, x0_shape, cond_shape, draws: int = 16, use_graph: bool = True,
+                 seed: Optional[int] = None, timesteps=None):
+        trainable = [n for n, p in diffusion.named_parameters() if p.requires_grad]
+        if trainable:
+            raise ValueError(f"SaliencyEngine needs a frozen model; {len(trainable)} parameters require grad "
+                             f"(e.g. {trainable[0]}): call requires_grad_(False) on the model")
+        if seed is not None:
+            K.split_seed(seed)
+        x0_shape, cond_shape = tuple(x0_shape), tuple(cond_shape)
+        if len(x0_shape) != 4 or x0_shape[1] != 1:
+            raise ValueError(f"x0_shape must be [B, 1, H, W], got {x0_shape}")
+        B, _, H, W = x0_shape
+        if len(cond_shape) == 4:
+            frames = 1
+        elif len(cond_shape) == 5:
+            frames = cond_shape[2]
+        else:
+            raise ValueError(f"cond_shape must be [B, 1, H, W] or [B, 1, K, H, W], got {cond_shape}")
+        if cond_shape[:2] != (B, 1) or cond_shape[-2:] != (H, W):
+            raise ValueError(f"cond_shape {cond_shape} does not match x0_shape {x0_shape}")
+        T = diffusion.T
+        if timesteps is None:
+            tab = saliency_timesteps(T, draws)
+        else:
+            tab = torch.as_tensor(timesteps)
+            if tab.dtype.is_floating_point or tab.dtype.is_complex or tab.dtype == torch.bool:
+                raise ValueError(f"timesteps must be integers, got dtype {tab.dtype}")
+            if tab.dim() not in (1, 2) or tab.shape[0] < 1 or (tab.dim() == 2 and tab.shape[1] != B):
+                raise ValueError(f"timesteps must have shape [D] or [D, {B}], got {tuple(tab.shape)}")
+            tab = tab.to("cpu", torch.int64)
+            if bool((tab < 0).any()) or bool((tab >= T).any()):
+                raise ValueError(f"timesteps must lie in [0, {T})")
+        if tab.shape[0] > K.SALIENCY_MAX_DRAWS:
+            raise ValueError(f"at most {K.SALIENCY_MAX_DRAWS} draws")
+        if tab.dim() == 1:
+            tab = tab[:, None].expand(-1, B)
+        self.diffusion = diffusion
+        dev = next(diffusion.parameters()).device
+        if dev.type != "cuda":
+            raise ValueError("SaliencyEngine runs on the CUDA kernels; the model is on " + str(dev))
+        self.device = dev
+        self.x0_shape, self.cond_shape = x0_shape, cond_shape
+        self.draws = int(tab.shape[0])
+        self.t_table = tab.contiguous().to(dev)
+        # the gradient stream is fp16: like the training step (GradScaler's initial scale), the backward starts
+        # from 2^16 instead of 1, and the sink's scale takes it out again
+        self.grad_seed = torch.full((), SALIENCY_LOSS_SCALE, dtype=torch.float32, device=dev)
+        self.scale = B / (self.draws * SALIENCY_LOSS_SCALE)
+        self.x0 = torch.zeros(x0_shape, dtype=torch.float32, device=dev)
+        self.cond = torch.zeros(cond_shape, dtype=torch.float32, device=dev, requires_grad=True)
+        self.noise = torch.zeros(x0_shape, dtype=torch.float32, device=dev)
+        self.t = torch.zeros((B,), dtype=torch.int64, device=dev)
+        self.out = torch.zeros((B, 1, frames, H, W), dtype=torch.float32, device=dev)
+        self.seed = None if seed is None else int(seed)
+        if seed is not None:
+            self.field_ids = torch.arange(B, dtype=torch.int64, device=dev)
+        self.arena = K.ZeroArena(dev)
+        self.use_graph = use_graph
+        self.graph: Optional[torch.cuda.CUDAGraph] = None
+        self.launches_per_step = 0
+
+    def _draw(self, d: int) -> None:
+        """Timesteps and noise of draw d into the static buffers the captured pass reads."""
+        self.t.copy_(self.t_table[d])
+        if self.seed is None:
+            self.noise.normal_()
+        else:
+            K.field_normal(self.seed, self.field_ids, K.SALIENCY_DRAW_BASE + d, out=self.noise)
+
+    def _body(self) -> None:
+        prev = ops._GRAD_SINK[0]
+        ops.set_grad_sink(None)
+        ops.set_cond_grad_sink(self.out, self.scale)
+        self.arena.begin()
+        try:
+            with torch.enable_grad():
+                self.diffusion.loss(self.x0, self.cond, self.t, self.noise).backward(self.grad_seed)
+        finally:
+            self.arena.end()
+            ops.set_cond_grad_sink(None)
+            ops.set_grad_sink(prev)
+
+    def refresh_operands(self) -> None:
+        """Packed fp16 weight copies are captured by address: bring them up to date with the module's weights."""
+        ops.prepack_all()
+        ops.refresh_folds()
+
+    def saliency(self, x0: torch.Tensor, cond: torch.Tensor, field_ids=None) -> torch.Tensor:
+        """x0: [B, 1, H, W] target fields, cond: their condition windows (cond_shape) -> fp32 [B, 1, K, H, W]
+        saliency (K = 1 for a 4-D cond).  `field_ids` (B integers >= 0, default arange(B)) name the fields of a
+        seeded engine; an unseeded one takes none."""
+        from . import _lib
+        if tuple(x0.shape) != self.x0_shape or tuple(cond.shape) != self.cond_shape:
+            raise ValueError(f"expected x0 {self.x0_shape} and cond {self.cond_shape}, got {tuple(x0.shape)} and "
+                             f"{tuple(cond.shape)}")
+        if self.seed is None and field_ids is not None:
+            raise ValueError("field_ids needs a seeded SaliencyEngine (SaliencyEngine(..., seed=...))")
+        ids = K.field_id_vector(field_ids, self.x0_shape[0], self.device) if self.seed is not None else None
+        self.refresh_operands()
+        with torch.no_grad():
+            self.x0.copy_(x0, non_blocking=True)
+            self.cond.copy_(cond, non_blocking=True)
+            if ids is not None:
+                self.field_ids.copy_(ids)
+        if self.use_graph and self.graph is None:
+            self.t.copy_(self.t_table[0])
+            self._body()  # eager warm-up on whatever noise the buffer holds; what it added to `out` is cleared below
+            torch.cuda.synchronize()
+            ops.prepack_all()  # every operand the warm-up registered is current: the capture re-packs none
+            self.graph = torch.cuda.CUDAGraph()
+            n0 = _lib.launch_count()
+            with torch.cuda.graph(self.graph):
+                self._body()
+            self._graph_launches = _lib.launch_count() - n0
+        self.out.zero_()
+        for d in range(self.draws):
+            n0 = _lib.launch_count()
+            self._draw(d)
+            if self.graph is not None:
+                self.graph.replay()
+                self.launches_per_step = _lib.launch_count() - n0 + self._graph_launches
+            else:
+                self._body()
+                self.launches_per_step = _lib.launch_count() - n0
+        return self.out.clone()

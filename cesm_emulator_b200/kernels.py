@@ -540,6 +540,37 @@ def input_conv_wgrad(in0, in1, dy, B: int, F: int, H: int, W: int, ks: int):
     return dw, db
 
 
+def input_conv_dgrad(dy, w, B: int, F: int, H: int, W: int, ks: int, f0: int, f1: int, *, need_x: bool = True,
+                     need_cond: bool = True, dx_out: Optional[torch.Tensor] = None,
+                     dcond_out: Optional[torch.Tensor] = None, scale: float = 1.0, accumulate: bool = False):
+    """Data gradient of the input convolution (cesm_input_conv_dgrad): dy fp16 [B*F, H, W, C] and the fp32 weight
+    [C, 2, 1, ks, ks] -> (d_x fp32 [B, 1, f0, H, W] or None, d_cond fp32 [B, 1, f1, H, W] or None).  A side with one
+    frame while F > 1 gets the sum over the F frames (the forward's broadcast).  Each result is scale * grad, written
+    into `dx_out` / `dcond_out` when given -- or, with `accumulate`, added to them."""
+    _req_cuda(dy, w, dx_out, dcond_out)
+    assert dy.dtype == H16 and tuple(dy.shape[:3]) == (B * F, H, W) and w.dtype == torch.float32
+    cout = dy.shape[-1]
+    assert tuple(w.shape) == (cout, 2, 1, ks, ks), tuple(w.shape)
+    assert need_x or need_cond
+    outs = []
+    for need, given, fp in ((need_x, dx_out, f0), (need_cond, dcond_out, f1)):
+        if not need:
+            outs.append(None)
+            continue
+        if given is None:
+            assert not accumulate, "accumulate needs the output buffers"
+            given = torch.empty((B, 1, fp, H, W), dtype=torch.float32, device=dy.device)
+        assert given.dtype == torch.float32 and given.numel() == B * fp * H * W, (given.dtype, tuple(given.shape))
+        outs.append(given)
+    meta = None
+    if _lib.PROFILER is not None:
+        meta = {"flops": 2.0 * B * F * H * W * cout * ks * ks * (int(need_x) + int(need_cond)),
+                "bytes": float(dy.numel() * 2 + sum(o.numel() * 4 for o in outs if o is not None))}
+    _lib.call("cesm_input_conv_dgrad", _ptr(dy), _ptr(w), _ptr(outs[0]), _ptr(outs[1]), f0, f1, B, F, H, W, ks, cout,
+              float(scale), int(accumulate), _stream(), _meta=meta)
+    return outs[0], outs[1]
+
+
 def out_conv_fwd(a, w, bias, B: int, F: int, H: int, W: int, mid: Optional[int] = None):
     _req_cuda(a, w, bias)
     mid = F // 2 if mid is None else mid
@@ -643,6 +674,19 @@ def q_sample(x0, noise, t, sqrt_ac, sqrt_1mac):
     return xt
 
 
+def q_sample_bwd(g, t, sqrt_ac, sqrt_1mac, need_x0: bool = True, need_noise: bool = True):
+    """Backward of q_sample: (dx0 = sqrt_ac[t] g or None, dnoise = sqrt_1mac[t] g or None) per sample."""
+    _req_cuda(g, t, sqrt_ac, sqrt_1mac)
+    assert g.dtype == torch.float32 and t.dtype == torch.int64 and (need_x0 or need_noise)
+    B = g.shape[0]
+    assert t.shape == (B,), (tuple(t.shape), B)
+    dx0 = torch.empty_like(g) if need_x0 else None
+    dnoise = torch.empty_like(g) if need_noise else None
+    _lib.call("cesm_q_sample_bwd", _ptr(g), _ptr(t), _ptr(sqrt_ac), _ptr(sqrt_1mac), _ptr(dx0), _ptr(dnoise), B,
+              g.numel() // B, _stream())
+    return dx0, dnoise
+
+
 def mse_fwd(eps, noise):
     _req_cuda(eps, noise)
     diff = torch.empty_like(eps)
@@ -706,6 +750,10 @@ def dpm_step(xt, eps, hist, t, coef, T: int, out=None, next_t=None, t_out=None):
 
 # ---- seeded sampling noise ------------------------------------------------------------------------
 X_T_DRAW = 0xFFFFFFFF  # draw id of the initial noise x_T; the step leaving timestep t draws with id t
+# Saliency draw d (engine.SaliencyEngine) uses draw id SALIENCY_DRAW_BASE + d, d < SALIENCY_MAX_DRAWS: above every
+# sampler timestep (T < 2^31) and below X_T_DRAW, so saliency noise never repeats a sampling draw of the same field.
+SALIENCY_DRAW_BASE = 0x80000000
+SALIENCY_MAX_DRAWS = X_T_DRAW - SALIENCY_DRAW_BASE
 
 
 def split_seed(seed) -> Tuple[int, int]:

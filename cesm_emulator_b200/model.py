@@ -251,11 +251,11 @@ class Diffusion(nn.Module):
 
     # -- training ------------------------------------------------------------------------------
     def q_sample(self, x0, t, noise=None):
-        """model.py:196-201."""
+        """model.py:196-201.  Differentiable in x0 and noise (ops.QSampleFn)."""
         if noise is None:
             noise = torch.randn_like(x0)
-        x_t = K.q_sample(x0.float().contiguous(), noise.float().contiguous(), t.contiguous(),
-                         self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod)
+        x_t = ops.QSampleFn.apply(x0.float().contiguous(), noise.float().contiguous(), t.contiguous(),
+                                  self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod)
         return x_t, noise
 
     def loss(self, x0, cond, t=None, noise=None):

@@ -233,6 +233,16 @@ def _ready(*params) -> None:
         _GRAD_SINK[0].ready(p)
 
 
+# Condition-gradient sink (engine.SaliencyEngine): (fp32 buffer, scale) or None.  While set, the input convolution's
+# backward adds scale * d cond straight into the buffer (the data-gradient kernel's accumulate mode) and hands
+# autograd no gradient for cond, so averaging over draws costs no extra launch.
+_COND_GRAD_SINK = [None]
+
+
+def set_cond_grad_sink(buf: Optional[torch.Tensor], scale: float = 1.0) -> None:
+    _COND_GRAD_SINK[0] = None if buf is None else (buf, float(scale))
+
+
 # Leaf-gradient side stream (engine mode only).  Weight gradients are not on the backward pass's critical chain: they
 # are launched on a second stream that forks from the main one where their inputs become available and joins before
 # the optimizer (TrainEngine).  At the coarse U-Net levels most kernels have a nearly empty last wave; work from the
@@ -651,6 +661,7 @@ class ResnetBlockFn(_Fn):
         B, G, eps = ctx.cfg
         dout = dout.contiguous()
         ntaps = [(-dh, -dw) for dh, dw in K.TAPS_3x3]
+        need = ctx.needs_input_grad  # a frozen weight (requires_grad False) gets no weight-gradient launch
         # GroupNorm / conv-bias gradients go straight into the parameters' .grad in engine mode
         # ---- block 2 ----
         if _direct_all(g2w, g2b, b2):
@@ -660,7 +671,7 @@ class ResnetBlockFn(_Fn):
             dg2w = dg2b = db2 = None
         else:
             dy2, dg2w, dg2b, _, db2 = K.gn_bwd(y2, dout, sums2, g2w, g2b, None, B, G, eps, conv_bias_grad=True)
-        dw2 = _conv_wgrad(w2, h1, None, dy2, 3)
+        dw2 = _conv_wgrad(w2, h1, None, dy2, 3) if need[7] else None
         dh1 = K.igemm(dy2, ctx.wd2[0], taps=ntaps)
         # ---- block 1 ----
         if _direct_all(g1w, g1b, b1):
@@ -670,34 +681,38 @@ class ResnetBlockFn(_Fn):
             dg1w = dg1b = db1 = None
         else:
             dy1, dg1w, dg1b, dfilm, db1 = K.gn_bwd(y1, dh1, sums1, g1w, g1b, film, B, G, eps, conv_bias_grad=True)
-        dw1 = _conv_wgrad(w1, x, x1, dy1, 3)
+        dw1 = _conv_wgrad(w1, x, x1, dy1, 3) if need[3] else None
         # ---- inputs: conv-1 data gradient with the residual-branch gradient added in its epilogue ----
         dx = dx1 = dwres = dbres = None
         if wres is None:
-            if ctx.needs_input_grad[0]:
+            if need[0]:
                 dx = K.igemm(dy1, ctx.wd1[0], taps=ntaps, residual=dout)
         else:
-            if ctx.needs_input_grad[0]:
+            if need[0]:
                 r0 = K.igemm(dout, ctx.wdres[0])
                 dx = K.igemm(dy1, ctx.wd1[0], taps=ntaps, residual=r0)
-            if x1 is not None and ctx.needs_input_grad[1]:
+            if x1 is not None and need[1]:
                 r1 = K.igemm(dout, ctx.wdres[1])
                 dx1 = K.igemm(dy1, ctx.wd1[1], taps=ntaps, residual=r1)
-            dwres = _conv_wgrad(wres, x, x1, dout, 1)
-            if _direct_all(bres):
+            if need[11]:
+                dwres = _conv_wgrad(wres, x, x1, dout, 1)
+            if need[12] and _direct_all(bres):
                 with _on_side(dout):
                     K.colsum(dout, into=bres.grad)
                 _ready(bres)
-            else:
+            elif need[12]:
                 dbres = K.colsum(dout)
         return dx, dx1, dfilm, dw1, db1, dg1w, dg1b, dw2, db2, dg2w, dg2b, dwres, dbres, None, None
 
 
-def _qkv_backward(wqkv, wdq, xn, dqkv4):
+def _qkv_backward(wqkv, wdq, xn, dqkv4, need_w: bool = True):
     """Data gradient (w.r.t. the projection's input xn) and weight gradient of the bias-free q/k/v projection.
     For 64 input channels both come from ONE pass over dqkv (cesm_qkv_bwd: 101 us instead of 83 + 84 us at
-    192x288); otherwise from the implicit-GEMM and weight-gradient kernels.  -> (dxn, dwqkv or None)."""
+    192x288); otherwise from the implicit-GEMM and weight-gradient kernels.  A frozen projection (`need_w` False)
+    takes the data-gradient GEMM alone.  -> (dxn, dwqkv or None)."""
     C, cout = xn.shape[-1], dqkv4.shape[-1]
+    if not need_w:
+        return K.igemm(dqkv4, wdq), None
     if C == 64 and cout % 128 == 0 and cout <= 768:
         if _direct(wqkv):
             dxn, _ = K.qkv_bwd(dqkv4, xn, wdq, dw_into=wqkv.grad)
@@ -765,11 +780,11 @@ class TemporalAttnBlockFn(_Fn):
         NI, H_, W_, C = x.shape
         dy = dy.contiguous()
         do = K.igemm(dy, ctx.wdo)
-        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1)
+        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1) if ctx.needs_input_grad[3] else None
         dqkv, dbias = K.tattn_bwd(qkv.view(-1, 3 * hidden), pos_bias, cs, sn, o if F > 4 else None, lse,
                                   do.view(-1, hidden), B, F, H_ * W_, heads, D, D ** -0.5)
         dqkv4 = dqkv.view(NI, H_, W_, 3 * hidden)
-        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv4)
+        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv4, ctx.needs_input_grad[2])
         # + dy: the residual branch, added in the LN-backward epilogue
         if _direct_all(gamma):
             dx, _ = K.ln_bwd(x, g, dxn, dy, eps, into=gamma.grad.view(-1))
@@ -814,10 +829,10 @@ class MidAttnBlockFn(_Fn):
         NI, H_, W_, C = x.shape
         dy = dy.contiguous()
         do = K.igemm(dy, ctx.wdo)
-        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1)
+        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1) if ctx.needs_input_grad[3] else None
         dqkv = K.mattn_bwd(qkv.view(-1, 3 * hidden), o.view(-1, hidden), lse, do.view(-1, hidden), NI, H_ * W_, heads, D,
                            D ** -0.5)
-        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv.view(NI, H_, W_, 3 * hidden))
+        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv.view(NI, H_, W_, 3 * hidden), ctx.needs_input_grad[2])
         # + dy: the residual branch, added in the LN-backward epilogue
         if _direct_all(gamma):
             dx, _ = K.ln_bwd(x, g, dxn, dy, eps, into=gamma.grad.view(-1))
@@ -860,17 +875,18 @@ class SpatialAttnBlockFn(_Fn):
         NI, H_, W_, C = x.shape
         dy = dy.contiguous()
         do = K.igemm(dy, ctx.wdo)
-        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1)
-        if _direct_all(bout):
+        need = ctx.needs_input_grad
+        dwout = _conv_wgrad(wout, o.view(NI, H_, W_, hidden), None, dy, 1) if need[3] else None
+        dbout = None
+        if need[4] and _direct_all(bout):
             with _on_side(dy):
                 K.colsum(dy, into=bout.grad)
             _ready(bout)
-            dbout = None
-        else:
+        elif need[4]:
             dbout = K.colsum(dy)
         dqkv = K.linattn_bwd(qkv.view(-1, 3 * hidden), ws, do.view(-1, hidden), NI, H_ * W_, heads, D, D ** -0.5)
         dqkv4 = dqkv.view(NI, H_, W_, 3 * hidden)
-        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv4)
+        dxn, dwqkv = _qkv_backward(wqkv, ctx.wdq, xn, dqkv4, need[2])
         if _direct_all(gamma):
             dx, _ = K.ln_bwd(x, g, dxn, dy, eps, into=gamma.grad.view(-1))
             _ready(gamma)
@@ -892,28 +908,48 @@ class InputConvFn(_Fn):
     def forward(ctx, x, cond, weight, bias, F: int):
         """Tensor-core path: fp16 (hi, lo) im2col patches x [w | w | bias] through the tcgen05 implicit GEMM
         (kernels.input_patches / input_weight_pack); the patches are kept for the weight gradient."""
+        shapes = (x.shape, cond.shape)
         x, cond = x.contiguous().float(), cond.contiguous().float()
         B, H, W = x.shape[0], x.shape[-2], x.shape[-1]
         ks = weight.shape[-1]
         patches = K.input_patches(x, cond, B, F, H, W, ks)
         out = K.igemm(patches, K.input_weight_pack(weight.detach(), bias.detach()))
         if _train(ctx):
-            ctx.save_for_backward(patches, weight, bias)
+            # the patches serve the weight gradient only
+            need_w = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+            ctx.save_for_backward(patches if need_w else None, weight, bias)
+            ctx.dims = (B, F, H, W, x.numel() // (B * H * W), cond.numel() // (B * H * W), shapes)
         return out
 
     @staticmethod
     def backward(ctx, dy):
         patches, weight, bias = ctx.saved_tensors
+        B, F, H, W, f0, f1, shapes = ctx.dims
+        ks = weight.shape[-1]
+        dy = dy.contiguous()
+        need_x, need_c = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        dx = dcond = None
+        sink = _COND_GRAD_SINK[0] if need_c else None
+        if sink is not None:  # scale * d cond added into the sink's buffer; autograd gets none
+            K.input_conv_dgrad(dy, weight.detach(), B, F, H, W, ks, f0, f1, need_x=False, dcond_out=sink[0],
+                               scale=sink[1], accumulate=True)
+            need_c = False
+        if need_x or need_c:
+            dx, dcond = K.input_conv_dgrad(dy, weight.detach(), B, F, H, W, ks, f0, f1, need_x=need_x, need_cond=need_c)
+            dx = None if dx is None else dx.view(shapes[0])
+            dcond = None if dcond is None else dcond.view(shapes[1])
+        if not (ctx.needs_input_grad[2] or ctx.needs_input_grad[3]):
+            return dx, dcond, None, None, None
         nt = weight[0].numel()  # 2 * ks * ks
-        full = K.wgrad(patches, dy.contiguous())[:, 0, :]          # fp32 [cout, KPAD]
+        full = K.wgrad(patches, dy)[:, 0, :]                       # fp32 [cout, KPAD]
         dw = (full[:, :nt] + full[:, nt:2 * nt]).view_as(weight)   # hi and lo column blocks see the same dy
         db = full[:, 2 * nt]                                       # the ones column: sum of dy
         if _direct_all(weight, bias):
             weight.grad.add_(dw)
             bias.grad.add_(db)
             _ready(weight, bias)
-            return None, None, None, None, None
-        return None, None, dw, db.contiguous(), None
+            return dx, dcond, None, None, None
+        return dx, dcond, dw, db.contiguous(), None
 
 
 class OutConvFn(_Fn):
@@ -1020,7 +1056,25 @@ class MseLossFn(_Fn):
     def backward(ctx, g):
         (diff,) = ctx.saved_tensors
         g = g.reshape(1).float().contiguous()
-        return K.scale_by_scalar(diff, g, 2.0 / diff.numel()), None
+        deps = K.scale_by_scalar(diff, g, 2.0 / diff.numel()) if ctx.needs_input_grad[0] else None
+        dnoise = K.scale_by_scalar(diff, g, -2.0 / diff.numel()) if ctx.needs_input_grad[1] else None
+        return deps, dnoise
+
+
+class QSampleFn(_Fn):
+    """x_t = sqrt_ac[t] x0 + sqrt_1mac[t] noise (model.py:196-201), differentiable in x0 and noise."""
+
+    @staticmethod
+    def forward(ctx, x0, noise, t, sqrt_ac, sqrt_1mac):
+        ctx.save_for_backward(t, sqrt_ac, sqrt_1mac)
+        return K.q_sample(x0, noise, t, sqrt_ac, sqrt_1mac)
+
+    @staticmethod
+    def backward(ctx, g):
+        t, sqrt_ac, sqrt_1mac = ctx.saved_tensors
+        dx0, dnoise = K.q_sample_bwd(g.contiguous().float(), t, sqrt_ac, sqrt_1mac, ctx.needs_input_grad[0],
+                                     ctx.needs_input_grad[1])
+        return dx0, dnoise, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------

@@ -338,6 +338,13 @@ int cesm_input_conv_fwd(const float* in0, const float* in1, int f0, int f1, cons
                         void* out, int B, int F, int H, int W, int ks, int cout, void* stream);
 int cesm_input_conv_wgrad(const float* in0, const float* in1, int f0, int f1, const void* dy, float* dw, float* db,
                           int B, int F, int H, int W, int ks, int cout, void* stream);
+/* Data gradient of the input convolution: the transposed 7x7 convolution (zero padding, fp32 accumulation) of
+ * dy fp16 [B*F][H][W][cout] with the fp32 weight [cout][2][ks][ks], giving d_in0 fp32 [B][f0][H][W] and
+ * d_in1 fp32 [B][f1][H][W].  A plane with one frame while F > 1 (the broadcast of cesm_input_conv_fwd) receives
+ * the sum over the F frames.  out = scale * grad, or out += scale * grad with `accumulate`.  Either output may be
+ * NULL (not requested), not both.  ks = 7, cout = 64, B <= 65535. */
+int cesm_input_conv_dgrad(const void* dy, const float* w, float* d_in0, float* d_in1, int f0, int f1, int B, int F,
+                          int H, int W, int ks, int cout, float scale, int accumulate, void* stream);
 int cesm_out_conv_fwd(const void* a, const float* w, const float* bias, float* eps, int B, int F, int mid,
                       long long HW, int C, void* stream);
 int cesm_out_conv_bwd(const void* a, const float* w, const float* deps, void* da, float* dw, float* db, int B, int F,
@@ -358,6 +365,10 @@ int cesm_small_linear_bwd(const float* x, const float* W, const float* dy, float
  * ---------------------------------------------------------------------------------------------- */
 int cesm_q_sample(const float* x0, const float* noise, const long long* t, const float* sqrt_ac,
                   const float* sqrt_1mac, float* xt, int B, long long per_sample, void* stream);
+/* Backward of cesm_q_sample: dx0 = sqrt_ac[t[b]] * g, dnoise = sqrt_1mac[t[b]] * g.  Either output may be NULL
+ * (not requested), not both. */
+int cesm_q_sample_bwd(const float* g, const long long* t, const float* sqrt_ac, const float* sqrt_1mac, float* dx0,
+                      float* dnoise, int B, long long per_sample, void* stream);
 int cesm_mse_fwd(const float* eps, const float* noise, float* diff, float* loss, long long total, void* stream);
 int cesm_scale_by_scalar(const float* in, const float* gscale, float factor, float* out, long long total,
                          void* stream);

@@ -102,26 +102,32 @@ def write_prediction_netcdf(path, pred_tmhw: np.ndarray, stack_coord=None, membe
     (year, member_id, lat, lon), coordinate variables and the description / units attributes.  xarray and
     netCDF4 are not in this image, so the file is written as classic NetCDF-3 by scipy
     (`xr.open_dataset` reads it with its scipy engine)."""
-    from scipy.io import netcdf_file
     T, M, H, W = pred_tmhw.shape
     coords = [(stack_dim, stack_coord, T), (member_dim, member_coord, M), (lat_name, lat, H), (lon_name, lon, W)]
+    write_netcdf_variable(path, "TREFHT_pred", pred_tmhw, coords, {
+        "description": "Predicted near-surface air temperature from emissions via diffusion model",
+        "units": "standardized", **(attrs or {})})
+
+
+def write_netcdf_variable(path, name, data, coords, attrs):
+    """One float32 variable `name` over the dimensions `coords` = [(dim name, coordinate values or None for
+    arange, length), ...] with its coordinate variables and attributes, as classic NetCDF-3 through scipy."""
+    from scipy.io import netcdf_file
     d = os.path.dirname(path)
     if d:
         os.makedirs(d, exist_ok=True)
     with netcdf_file(path, "w", version=2) as f:
-        for name, vals, n in coords:
-            f.createDimension(name, n)
+        for dim, vals, n in coords:
+            f.createDimension(dim, n)
             vals = np.arange(n) if vals is None else np.asarray(vals)
             if vals.shape != (n,):
-                raise ValueError(f"coordinate {name} has shape {vals.shape}, expected ({n},)")
+                raise ValueError(f"coordinate {dim} has shape {vals.shape}, expected ({n},)")
             vals = vals.astype(np.float64 if vals.dtype.kind == "f" else np.int32)
-            v = f.createVariable(name, vals.dtype, (name,))
+            v = f.createVariable(dim, vals.dtype, (dim,))
             v[:] = vals
-        v = f.createVariable("TREFHT_pred", np.float32, (stack_dim, member_dim, lat_name, lon_name))
-        v[:] = np.asarray(pred_tmhw, dtype=np.float32)
-        v.description = "Predicted near-surface air temperature from emissions via diffusion model"
-        v.units = "standardized"
-        for k, val in (attrs or {}).items():
+        v = f.createVariable(name, np.float32, tuple(dim for dim, _, _ in coords))
+        v[:] = np.asarray(data, dtype=np.float32)
+        for k, val in attrs.items():
             setattr(v, k, val)
 
 

@@ -149,6 +149,8 @@ _SIGNATURES: dict[str, list] = {
     "cesm_q_sample_bwd": [_P, _P, _P, _P, _P, _P, _I, _L, _P],
     "cesm_mse_fwd": [_P, _P, _P, _P, _L, _P],
     "cesm_scale_by_scalar": [_P, _P, _F, _P, _L, _P],
+    "cesm_diffusion_loss_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _I, _P],
+    "cesm_diffusion_loss_bwd": [_P, _P, _P, _P, _P, _F, _P, _P, _P, _I, _L, _I, _P],
     "cesm_p_sample": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _P],
     "cesm_ddim_step": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
     "cesm_dpm_step": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],

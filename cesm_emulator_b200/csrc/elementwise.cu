@@ -647,6 +647,70 @@ mse_fwd_kernel(const float* __restrict__ eps, const float* __restrict__ noise, f
         atomicAdd(loss, tot / (float)total);
     }
 }
+// Diffusion objective with a per-timestep target and weight.  Block (x, b) covers part of sample b, so t, the target
+// row and the weight are uniform in a block.  target = c_n[t] * noise + c_x[t] * x0 from coef[T][2] rows (c_n, c_x);
+// a null coef is the eps target (x0 not read).  A null weight is 1.  A t outside [0, T) yields NaN.
+struct LossRow {
+    float cn, cx, w;
+    bool valid;
+};
+__device__ __forceinline__ LossRow loss_row(const long long* __restrict__ t, const float* __restrict__ coef,
+                                            const float* __restrict__ weight, int T, int b) {
+    const long long tb = t[b];
+    LossRow r;
+    r.valid = tb >= 0 && tb < T;
+    r.cn = 1.f, r.cx = 0.f, r.w = 1.f;
+    if (r.valid && coef) r.cn = coef[2 * tb], r.cx = coef[2 * tb + 1];
+    if (r.valid && weight) r.w = weight[tb];
+    return r;
+}
+// diff = pred - target;  loss += w[t] * sum diff^2 / total
+__global__ void __launch_bounds__(256)
+diffusion_loss_fwd_kernel(const float* __restrict__ pred, const float* __restrict__ x0, const float* __restrict__ noise,
+                          const long long* __restrict__ t, const float* __restrict__ coef,
+                          const float* __restrict__ weight, float* __restrict__ diff, float* __restrict__ loss, int T,
+                          long long per, long long total) {
+    pdl_trigger();
+    pdl_wait();
+    const int b = blockIdx.y;
+    const LossRow r = loss_row(t, coef, weight, T, b);
+    const float qnan = __int_as_float(0x7fc00000);
+    const long long base = (long long)b * per;
+    float s = 0.f;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < per; i += (long long)gridDim.x * blockDim.x) {
+        const long long idx = base + i;
+        float d = qnan;
+        if (r.valid) d = pred[idx] - (coef ? fmaf(r.cn, noise[idx], r.cx * x0[idx]) : noise[idx]);
+        diff[idx] = d;
+        s = fmaf(d, d, s);
+    }
+    __shared__ float red[8];
+    s = warp_sum(s);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float tot = 0.f;
+        for (int i = 0; i < 8; ++i) tot += red[i];
+        atomicAdd(loss, r.valid ? tot * (r.w / (float)total) : qnan);
+    }
+}
+// dpred = factor * g * w[t] * diff;  dnoise = -c_n[t] * dpred;  dx0 = -c_x[t] * dpred  (each output may be null)
+__global__ void diffusion_loss_bwd_kernel(const float* __restrict__ diff, const long long* __restrict__ t,
+                                          const float* __restrict__ coef, const float* __restrict__ weight,
+                                          const float* __restrict__ gscale, float factor, float* __restrict__ dpred,
+                                          float* __restrict__ dnoise, float* __restrict__ dx0, int T, long long per) {
+    pdl_trigger();
+    pdl_wait();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= per) return;
+    const int b = blockIdx.y;
+    const LossRow r = loss_row(t, coef, weight, T, b);
+    const long long idx = (long long)b * per + i;
+    const float p = r.valid ? diff[idx] * (factor * gscale[0] * r.w) : __int_as_float(0x7fc00000);
+    if (dpred) dpred[idx] = p;
+    if (dnoise) dnoise[idx] = -r.cn * p;
+    if (dx0) dx0[idx] = -r.cx * p;
+}
 // out = in * factor * (*gscale)
 __global__ void scale_by_device_scalar_kernel(const float* __restrict__ in, const float* __restrict__ gscale,
                                               float factor, float* __restrict__ out, long long total) {
@@ -1137,6 +1201,37 @@ extern "C" int cesm_mse_fwd(const float* eps, const float* noise, float* diff, f
     long long blocks = (total + 255) / 256;
     if (blocks > 148 * 4) blocks = 148 * 4;
     launch_pdl(mse_fwd_kernel, (int)blocks, 256, 0, st, eps, noise, diff, loss, total);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_diffusion_loss_fwd(const float* pred, const float* x0, const float* noise, const long long* t,
+                                       const float* tgt_coef, const float* weight, float* diff, float* loss, int B,
+                                       long long per_sample, int T, void* stream) {
+    CESM_REQUIRE(T > 0 && B > 0 && B <= 65535 && per_sample > 0, "bad diffusion loss sizes (T=%d B=%d per_sample=%lld)",
+                 T, B, per_sample);
+    CESM_REQUIRE(pred && noise && t && diff && loss && (x0 || !tgt_coef),
+                 "diffusion loss needs pred, noise, t, diff, loss, and x0 with a target table");
+    cudaStream_t st = as_stream(stream);
+    CESM_CHECK_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), st));
+    long long bx = (per_sample + 255) / 256;
+    const long long cap = (148 * 4 + B - 1) / B;  // about as many blocks in all as cesm_mse_fwd
+    if (bx > cap) bx = cap;
+    launch_pdl(diffusion_loss_fwd_kernel, dim3((unsigned)bx, B), 256, 0, st, pred, x0, noise, t, tgt_coef, weight, diff,
+               loss, T, per_sample, (long long)B * per_sample);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_diffusion_loss_bwd(const float* diff, const long long* t, const float* tgt_coef, const float* weight,
+                                       const float* gscale, float factor, float* dpred, float* dnoise, float* dx0, int B,
+                                       long long per_sample, int T, void* stream) {
+    CESM_REQUIRE(T > 0 && B > 0 && B <= 65535 && per_sample > 0, "bad diffusion loss backward sizes (T=%d B=%d per_sample=%lld)",
+                 T, B, per_sample);
+    CESM_REQUIRE(diff && t && gscale && (dpred || dnoise || dx0),
+                 "diffusion loss backward needs diff, t, gscale and at least one output");
+    launch_pdl(diffusion_loss_bwd_kernel, dim3((unsigned)((per_sample + 255) / 256), B), 256, 0, as_stream(stream), diff, t,
+               tgt_coef, weight, gscale, factor, dpred, dnoise, dx0, T, per_sample);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

@@ -350,13 +350,20 @@ class TrainEngine:
     `ema_decay` / `ema_start` (CUDA only) keep an exponential moving average of the weights inside the captured
     optimizer step (FusedAdamW).  It starts as a copy of the weights when the engine is built; loading weights into
     the module afterwards does not touch it -- call `reset_ema()` or `load_ema_state_dict()`.  `ema_state_dict()`
-    has the layout of `diffusion.model.state_dict()`."""
+    has the layout of `diffusion.model.state_dict()`.
+
+    `min_snr_gamma` (a real number > 0, or None for uniform weights) trains with Min-SNR-gamma loss weights for the
+    diffusion's target (`Diffusion.min_snr_weights`), held in a device buffer the captured step reads.  The weights go
+    down to 4e-5 (v, t = 999) and scale a sample's whole backward, which runs in fp16: the step divides the loss
+    scale's seed by the batch's largest weight (over all ranks), so the fp16 gradient stream carries the magnitudes
+    of an unweighted step, and multiplies the fp32 gradients by it before the optimizer step."""
 
     def __init__(self, diffusion, batch_shape, cond_shape, lr: float = 2e-4, betas=(0.9, 0.999),
                  weight_decay: float = 1e-4, eps: float = 1e-8, max_grad_norm: Optional[float] = 1.0,
                  n_buckets: int = 4, use_graph: bool = True, process_group=None, ema_decay: Optional[float] = None,
-                 ema_start: int = 0):
+                 ema_start: int = 0, min_snr_gamma: Optional[float] = None):
         ema_decay, ema_start = check_ema_args(ema_decay, ema_start)
+        self.loss_weights = None if min_snr_gamma is None else diffusion.min_snr_weights(min_snr_gamma)
         self.diffusion = diffusion
         dev = next(diffusion.parameters()).device
         if ema_decay is not None and dev.type != "cuda":
@@ -403,13 +410,25 @@ class TrainEngine:
         ops.set_side_stream(self.side_stream)
         ops.prepack_all()  # one kernel refreshes every fp16 operand copy of the (just updated) weights
         self.buckets.begin_step()
-        loss = self.diffusion.loss(self.x0, self.cond)
+        if self.loss_weights is None:
+            loss, wmax = self.diffusion.loss(self.x0, self.cond), None
+        else:
+            # the reference's randint draw, made here so that the batch's largest weight is known
+            t = torch.randint(0, self.diffusion.T, (self.x0.shape[0],), device=self.x0.device)
+            loss = self.diffusion.loss(self.x0, self.cond, t, weights=self.loss_weights)
+            wmax = self.loss_weights[t].max()
+            if self.world > 1:
+                dist.all_reduce(wmax, op=dist.ReduceOp.MAX, group=self.pg)
         if isinstance(self.opt, FusedAdamW):
             # scaler.scale(loss).backward() (train.py:862); /world turns the bucket SUM into the mean
-            (loss * (self.opt.loss_scale * (1.0 / self.world))).backward()
+            seed = self.opt.loss_scale * (1.0 / self.world)
+            (loss * (seed if wmax is None else seed / wmax)).backward()
         else:
-            (loss / self.world if self.world > 1 else loss).backward()
+            scaled = loss / self.world if self.world > 1 else loss
+            (scaled if wmax is None else scaled / wmax).backward()
         self.buckets.finish_step()
+        if wmax is not None:
+            self.buckets.flat.mul_(wmax)
         if isinstance(self.opt, FusedAdamW):
             self.opt.step()
             self.grad_norm.copy_(self.opt.grad_norm)
@@ -530,7 +549,11 @@ class SampleEngine:
     b is `kernels.field_normal(seed, field_ids[b], X_T_DRAW)` and the step leaving timestep t draws z with id t inside
     the fused `p_sample_seeded` / `ddim_step_seeded` kernel.  A field's chain then depends on (seed, field id) only, not
     on its row, its batch, `batch_size` or the rank it runs on.  The ids live in a static int64 buffer `field_ids`
-    that the graph captures by address; a replay has no noise draw and there is no z buffer."""
+    that the graph captures by address; a replay has no noise draw and there is no z buffer.
+
+    A v-prediction diffusion (`diffusion.prediction_type == "v"`) runs every mode through tables with the conversion to
+    eps folded in; its DDPM chain is the `ddim_step` (or `ddim_step_seeded`) launch with `diffusion.ddpm_coef`, the
+    N = T, eta = 1 table, in place of `p_sample`."""
 
     def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0,
                  dpm_steps: Optional[int] = None, seed: Optional[int] = None):
@@ -559,13 +582,14 @@ class SampleEngine:
         self.launches_per_step = 0
         self.ddim_steps, self.eta = ddim_steps, float(eta)
         if ddim_steps is not None:
-            self.ddim_taus, coef, next_t = ddim_schedule(diffusion.alphas_cumprod, ddim_steps, eta)
+            self.ddim_taus, coef, next_t = ddim_schedule(diffusion.alphas_cumprod, ddim_steps, eta,
+                                                         diffusion.prediction_type)
             self.ddim_coef = coef.to(dev)
             self.ddim_next_t = next_t.to(dev)
             self.t_next = torch.zeros_like(self.t)
         self.dpm_steps = dpm_steps
         if dpm_steps is not None:
-            self.dpm_taus, coef, next_t = dpm_schedule(diffusion.alphas_cumprod, dpm_steps)
+            self.dpm_taus, coef, next_t = dpm_schedule(diffusion.alphas_cumprod, dpm_steps, diffusion.prediction_type)
             self.dpm_coef = coef.to(dev)
             self.dpm_next_t = next_t.to(dev)
             self.t_next = torch.zeros_like(self.t)
@@ -603,6 +627,10 @@ class SampleEngine:
                            t_out=self.t_next)
                 self.t.copy_(self.t_next)
                 return
+            if self.seed is not None and d.prediction_type == "v":
+                K.ddim_step_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.ddpm_coef, d.T, out=self.x)
+                self.t.sub_(1)
+                return
             if self.seed is not None:
                 K.p_sample_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.betas,
                                   d.sqrt_one_minus_alphas_cumprod, d.sqrt_recip_alphas, d.posterior_variance,
@@ -610,6 +638,10 @@ class SampleEngine:
                 self.t.sub_(1)
                 return
             self.z.normal_()  # model.py:181 randn_like; kept in a static buffer so that a caller can read the draw
+            if d.prediction_type == "v":
+                K.ddim_step(self.x, eps, self.z, self.t, d.ddpm_coef, d.T, out=self.x)
+                self.t.sub_(1)
+                return
             self.x.copy_(K.p_sample(self.x, eps, self.z, self.t, d.betas, d.sqrt_one_minus_alphas_cumprod,
                                     d.sqrt_recip_alphas, d.posterior_variance))
             self.t.sub_(1)
@@ -711,7 +743,10 @@ class SaliencyEngine:
     the input convolution's data-gradient kernel.  Every parameter must have requires_grad False
     (`inference.load_diffusion_from_checkpoint` freezes them); the training gradient sink is off while a draw runs,
     so a TrainEngine in the same process never receives saliency gradients.  `launches_per_step` counts the library
-    launches of one draw."""
+    launches of one draw.
+
+    The loss is the eps-MSE for either target.  For a v-model the per-timestep weights ab[t] turn its v-MSE into it:
+    at the same x_t, eps_hat - eps = sqrt(ab) (v_hat - v).  Training loss weights (Min-SNR) never enter."""
 
     def __init__(self, diffusion, x0_shape, cond_shape, draws: int = 16, use_graph: bool = True,
                  seed: Optional[int] = None, timesteps=None):
@@ -757,6 +792,7 @@ class SaliencyEngine:
         self.x0_shape, self.cond_shape = x0_shape, cond_shape
         self.draws = int(tab.shape[0])
         self.t_table = tab.contiguous().to(dev)
+        self.loss_weights = diffusion.alphas_cumprod.float() if diffusion.prediction_type == "v" else None
         # the gradient stream is fp16: like the training step (GradScaler's initial scale), the backward starts
         # from 2^16 instead of 1, and the sink's scale takes it out again
         self.grad_seed = torch.full((), SALIENCY_LOSS_SCALE, dtype=torch.float32, device=dev)
@@ -789,7 +825,7 @@ class SaliencyEngine:
         self.arena.begin()
         try:
             with torch.enable_grad():
-                self.diffusion.loss(self.x0, self.cond, self.t, self.noise).backward(self.grad_seed)
+                self.diffusion.loss(self.x0, self.cond, self.t, self.noise, self.loss_weights).backward(self.grad_seed)
         finally:
             self.arena.end()
             ops.set_cond_grad_sink(None)

@@ -695,6 +695,42 @@ def mse_fwd(eps, noise):
     return loss, diff
 
 
+def _loss_tables(t, tgt_coef, weight, T: int, B: int) -> None:
+    assert t.dtype == torch.int64 and t.shape == (B,), (t.dtype, tuple(t.shape), B)
+    assert tgt_coef is None or (tgt_coef.dtype == torch.float32 and tgt_coef.shape == (T, 2) and tgt_coef.is_contiguous())
+    assert weight is None or (weight.dtype == torch.float32 and weight.shape == (T,) and weight.is_contiguous())
+
+
+def diffusion_loss_fwd(pred, x0, noise, t, tgt_coef, weight, T: int):
+    """Per sample b: target = c_n[t_b] noise + c_x[t_b] x0 (rows of the fp32 [T, 2] `tgt_coef`; None is the eps target
+    and x0 is not read), diff = pred - target, loss = sum_b weight[t_b] sum diff^2 / numel (None weight: 1).
+    A t outside [0, T) gives NaN.  -> (0-dim loss, diff)."""
+    _req_cuda(pred, x0, noise, t, tgt_coef, weight)
+    B = pred.shape[0]
+    _loss_tables(t, tgt_coef, weight, T, B)
+    assert pred.dtype == noise.dtype == torch.float32 and noise.shape == pred.shape
+    assert tgt_coef is None or (x0.dtype == torch.float32 and x0.shape == pred.shape)
+    diff = torch.empty_like(pred)
+    loss = torch.empty((), dtype=torch.float32, device=pred.device)
+    _lib.call("cesm_diffusion_loss_fwd", _ptr(pred), _ptr(x0), _ptr(noise), _ptr(t), _ptr(tgt_coef), _ptr(weight),
+              _ptr(diff), _ptr(loss), B, pred.numel() // B, T, _stream())
+    return loss, diff
+
+
+def diffusion_loss_bwd(diff, t, tgt_coef, weight, gscale, factor: float, T: int, need_pred: bool = True,
+                       need_noise: bool = False, need_x0: bool = False):
+    """Backward of diffusion_loss_fwd in one pass: dpred = factor * gscale * weight[t] * diff, dnoise = -c_n[t] dpred,
+    dx0 = -c_x[t] dpred (the target's share).  -> (dpred, dnoise, dx0), None where not requested."""
+    _req_cuda(diff, t, tgt_coef, weight, gscale)
+    B = diff.shape[0]
+    _loss_tables(t, tgt_coef, weight, T, B)
+    assert diff.dtype == torch.float32 and (need_pred or need_noise or need_x0)
+    dpred, dnoise, dx0 = (torch.empty_like(diff) if n else None for n in (need_pred, need_noise, need_x0))
+    _lib.call("cesm_diffusion_loss_bwd", _ptr(diff), _ptr(t), _ptr(tgt_coef), _ptr(weight), _ptr(gscale), factor,
+              _ptr(dpred), _ptr(dnoise), _ptr(dx0), B, diff.numel() // B, T, _stream())
+    return dpred, dnoise, dx0
+
+
 def scale_by_scalar(x, gscale, factor: float):
     _req_cuda(x, gscale)
     out = torch.empty_like(x)

@@ -60,7 +60,18 @@ class UNet(nn.Module):
         return out.squeeze(2)
 
 
-def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
+PREDICTION_TYPES = ("eps", "v")
+
+
+def check_prediction_type(prediction_type) -> str:
+    """The network's output: "eps" (the noise, the reference's target) or "v" = sqrt(ab) eps - sqrt(1 - ab) x0
+    (Salimans & Ho, "Progressive Distillation for Fast Sampling of Diffusion Models")."""
+    if not isinstance(prediction_type, str) or prediction_type not in PREDICTION_TYPES:
+        raise ValueError(f"prediction_type must be one of {PREDICTION_TYPES}, got {prediction_type!r}")
+    return prediction_type
+
+
+def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0, prediction_type: str = "eps"):
     """Strided DDIM reverse chain (Song et al., "Denoising Diffusion Implicit Models") over the trained DDPM schedule.
 
     Timesteps use "trailing" spacing, tau_i = floor(T (N - i) / N) - 1 for i = 0..N-1: the chain starts at T - 1,
@@ -73,6 +84,11 @@ def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
     eta = 0 is deterministic; eta = 1 with N = T is the DDPM posterior step.  The coefficients are computed in float64
     from the fp32 alphas_cumprod (1 - ab cancels at small tau in fp32) and stored as fp32.
 
+    For prediction_type "v" the network output is v and eps = sqrt(ab_tau) v + sqrt(1 - ab_tau) x, so the rows become
+    (A + B sqrt(1 - ab_tau), B sqrt(ab_tau), S), written in the closed form
+        A_v = sqrt(ab_p) sqrt(ab_tau) + c sqrt(1 - ab_tau),   B_v = c sqrt(ab_tau) - sqrt(ab_p) sqrt(1 - ab_tau),
+    c = sqrt(max(0, 1 - ab_p - sigma^2)), which does not subtract two terms of size 1 / sqrt(ab_tau).
+
     Returns (taus: list of N ints, coef: fp32 [T, 3] rows (A, B, S), next_t: int64 [T]), both tables on the CPU.
     Rows off the schedule hold NaN coefficients and next_t = -1; next_t of the last step is -1."""
     T = int(alphas_cumprod.shape[0])
@@ -84,6 +100,7 @@ def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
     eta = float(eta)
     if not eta >= 0.0:  # also rejects NaN
         raise ValueError(f"DDIM eta must be >= 0, got {eta}")
+    v = check_prediction_type(prediction_type) == "v"
     ac = alphas_cumprod.detach().to("cpu", torch.float64)
     taus = [T * (steps - i) // steps - 1 for i in range(steps)]
     coef = torch.full((T, 3), float("nan"), dtype=torch.float64)
@@ -93,15 +110,20 @@ def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0):
         a_t = ac[tau]
         a_p = ac[taus[i + 1]] if i + 1 < steps else one
         sigma = eta * torch.sqrt((1 - a_p) / (1 - a_t)) * torch.sqrt(1 - a_t / a_p)
-        coef[tau, 0] = torch.sqrt(a_p / a_t)
-        coef[tau, 1] = torch.sqrt(torch.clamp(1 - a_p - sigma * sigma, min=0)) - torch.sqrt(a_p) * torch.sqrt(1 - a_t) / torch.sqrt(a_t)
+        c = torch.sqrt(torch.clamp(1 - a_p - sigma * sigma, min=0))
+        if v:
+            coef[tau, 0] = torch.sqrt(a_p) * torch.sqrt(a_t) + c * torch.sqrt(1 - a_t)
+            coef[tau, 1] = c * torch.sqrt(a_t) - torch.sqrt(a_p) * torch.sqrt(1 - a_t)
+        else:
+            coef[tau, 0] = torch.sqrt(a_p / a_t)
+            coef[tau, 1] = c - torch.sqrt(a_p) * torch.sqrt(1 - a_t) / torch.sqrt(a_t)
         coef[tau, 2] = sigma
         if i + 1 < steps:
             next_t[tau] = taus[i + 1]
     return taus, coef.float(), next_t
 
 
-def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
+def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int, prediction_type: str = "eps"):
     """DPM-Solver++(2M) reverse chain (Lu et al., "DPM-Solver++: Fast Solver for Guided Sampling of Diffusion
     Probabilistic Models"), multistep second order in the data-prediction form, over the trained DDPM schedule.
 
@@ -115,6 +137,8 @@ def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
     the ends): the first has K0 = phi, K1 = 0; the last lands on ab = 1 with R = 0, K0 = 1, K1 = 0, i.e. x_0 is the
     x0 prediction.  Both are DDIM eta = 0 steps, so N <= 2 is exactly the DDIM eta = 0 chain.  The chain is
     deterministic after x_T.  The coefficients are computed in float64 from the fp32 alphas_cumprod and stored as fp32.
+    For prediction_type "v" the network output is v and x0 = sqrt(ab_s) x - sqrt(1 - ab_s) v: P = alpha_s, Q = -sigma_s
+    (written directly; P + Q sqrt(1 - ab_s) of the eps rows would subtract two terms of size 1 / alpha_s).
 
     Returns (taus: list of N ints, coef: fp32 [T, 5] rows (P, Q, R, K0, K1), next_t: int64 [T]), both tables on the
     CPU.  Rows off the schedule hold NaN coefficients and next_t = -1; next_t of the last step is -1."""
@@ -124,6 +148,7 @@ def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
     steps = int(steps)
     if not 1 <= steps <= T:
         raise ValueError(f"DPM-Solver steps must be in [1, {T}], got {steps}")
+    v = check_prediction_type(prediction_type) == "v"
     taus, _, next_t = ddim_schedule(alphas_cumprod, steps)
     ac = alphas_cumprod.detach().to("cpu", torch.float64).tolist()
     lam = lambda a: 0.5 * math.log(a / (1.0 - a))  # noqa: E731  log(alpha / sigma)
@@ -131,7 +156,10 @@ def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
     h_prev = None
     for i, s in enumerate(taus):
         a_s = ac[s]
-        P, Q = 1.0 / math.sqrt(a_s), -math.sqrt(1.0 - a_s) / math.sqrt(a_s)
+        if v:
+            P, Q = math.sqrt(a_s), -math.sqrt(1.0 - a_s)
+        else:
+            P, Q = 1.0 / math.sqrt(a_s), -math.sqrt(1.0 - a_s) / math.sqrt(a_s)
         if i + 1 == steps:
             coef[s] = torch.tensor([P, Q, 0.0, 1.0, 0.0], dtype=torch.float64)
             break
@@ -150,10 +178,17 @@ def dpm_schedule(alphas_cumprod: torch.Tensor, steps: int):
 
 
 class Diffusion(nn.Module):
-    """model.py:141-208."""
+    """model.py:141-208.
 
-    def __init__(self, model, img_channels=1, timesteps=1000, beta_schedule="linear"):
+    `prediction_type` (keyword only, an addition beyond the reference) names what the network predicts: "eps", the
+    reference's noise target, or "v" = sqrt(ab) eps - sqrt(1 - ab) x0, from which x0 = sqrt(ab) x_t - sqrt(1 - ab) v
+    carries no 1 / sqrt(ab) amplification (157 at t = 999 on the linear schedule).  A v-model samples with every chain
+    of the eps-model through coefficient tables that fold the conversion in (ddim_schedule, dpm_schedule).  Its
+    tables are non-persistent buffers: state_dict() and checkpoints are the same for both targets."""
+
+    def __init__(self, model, img_channels=1, timesteps=1000, beta_schedule="linear", *, prediction_type="eps"):
         super().__init__()
+        self.prediction_type = check_prediction_type(prediction_type)
         self.model = model
         self.img_channels = img_channels
         self.T = timesteps
@@ -173,6 +208,30 @@ class Diffusion(nn.Module):
         self.register_buffer("sqrt_one_minus_alphas_cumprod", torch.sqrt(1.0 - alphas_cumprod))
         self.register_buffer("sqrt_recip_alphas", torch.sqrt(1.0 / alphas))
         self.register_buffer("posterior_variance", betas * (1.0 - alphas_cumprod_prev) / (1.0 - alphas_cumprod))
+        v_coef = ddpm_coef = None
+        if self.prediction_type == "v":
+            ac = alphas_cumprod.double()
+            # target = c_n noise + c_x x0 (DiffusionLossFn): v = sqrt(ab) eps - sqrt(1 - ab) x0
+            v_coef = torch.stack([ac.sqrt(), -(1 - ac).sqrt()], dim=1).float()
+            # the DDPM chain of a v-model: the folded DDIM table at N = T, eta = 1, which is the posterior step
+            ddpm_coef = ddim_schedule(alphas_cumprod, timesteps, 1.0, "v")[1]
+        self.register_buffer("target_coef", v_coef, persistent=False)
+        self.register_buffer("ddpm_coef", ddpm_coef, persistent=False)
+
+    def min_snr_weights(self, gamma) -> torch.Tensor:
+        """Min-SNR-gamma loss weights (Hang et al., "Efficient Diffusion Training via Min-SNR Weighting Strategy") for
+        this Diffusion's target, SNR = ab / (1 - ab): min(SNR, gamma) / SNR for eps, min(SNR, gamma) / (SNR + 1) for v.
+        Both weight the x0 error by min(SNR, gamma).  gamma is a finite real number > 0 (an int is accepted, a bool
+        is not).  Computed in float64 -> fp32 [T] on the schedule's device."""
+        if isinstance(gamma, bool) or not isinstance(gamma, numbers.Real):
+            raise ValueError(f"min_snr_gamma must be a real number > 0, got {gamma!r}")
+        gamma = float(gamma)
+        if not (math.isfinite(gamma) and gamma > 0):
+            raise ValueError(f"min_snr_gamma must be finite and > 0, got {gamma}")
+        ac = self.alphas_cumprod.double()
+        snr = ac / (1 - ac)
+        w = snr.clamp(max=gamma) / (snr + 1 if self.prediction_type == "v" else snr)
+        return w.float()
 
     # -- sampling ------------------------------------------------------------------------------
     def p_sample(self, x_t, cond, t, noise=None):
@@ -183,6 +242,9 @@ class Diffusion(nn.Module):
         with torch.no_grad():
             eps_theta = self.model(x_t, cond, t)
             z = torch.randn_like(x_t) if noise is None else noise
+            if self.prediction_type == "v":  # eps_theta is v: the posterior step through the folded table
+                return K.ddim_step(x_t.float().contiguous(), eps_theta, z.float().contiguous(), t.contiguous(),
+                                   self.ddpm_coef, self.T)
             return K.p_sample(x_t.float().contiguous(), eps_theta, z.float().contiguous(), t.contiguous(),
                               self.betas, self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
                               self.posterior_variance)
@@ -210,6 +272,10 @@ class Diffusion(nn.Module):
                     x = self.p_sample(x, cond, t_tensor)
                     continue
                 eps_theta = self.model(x, cond, t_tensor)
+                if self.prediction_type == "v":
+                    x = K.ddim_step_seeded(x.float().contiguous(), eps_theta, seed, ids, t_tensor, self.ddpm_coef,
+                                           self.T)
+                    continue
                 x = K.p_sample_seeded(x.float().contiguous(), eps_theta, seed, ids, t_tensor, self.betas,
                                       self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
                                       self.posterior_variance)
@@ -218,7 +284,7 @@ class Diffusion(nn.Module):
     def ddim_sample(self, cond, shape, device, steps=50, eta=0.0, *, seed=None, field_ids=None):
         """Strided DDIM chain of `steps` UNet calls (ddim_schedule), eager; an addition beyond the reference.
         Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T.  `seed` / `field_ids` as in `sample`."""
-        taus, coef, _ = ddim_schedule(self.alphas_cumprod, steps, eta)
+        taus, coef, _ = ddim_schedule(self.alphas_cumprod, steps, eta, self.prediction_type)
         coef = coef.to(device)
         with torch.no_grad():
             B = shape[0]
@@ -237,7 +303,7 @@ class Diffusion(nn.Module):
         """DPM-Solver++(2M) chain of `steps` UNet calls (dpm_schedule), eager; an addition beyond the reference.
         Deterministic after x_T.  `hist` carries the previous step's x0 prediction; the first step does not read it.
         `seed` / `field_ids` as in `sample` (only x_T is random)."""
-        taus, coef, _ = dpm_schedule(self.alphas_cumprod, steps)
+        taus, coef, _ = dpm_schedule(self.alphas_cumprod, steps, self.prediction_type)
         coef = coef.to(device)
         with torch.no_grad():
             B = shape[0]
@@ -258,12 +324,20 @@ class Diffusion(nn.Module):
                                   self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod)
         return x_t, noise
 
-    def loss(self, x0, cond, t=None, noise=None):
+    def loss(self, x0, cond, t=None, noise=None, weights=None):
         """model.py:203-208.  `t` / `noise` default to the reference's draws (randint, then
-        randn_like); passing them makes parity tests deterministic."""
+        randn_like); passing them makes parity tests deterministic.  `weights` (fp32 [T], e.g. `min_snr_weights`)
+        weights each sample's squared error by weights[t]; the loss is sum_b weights[t_b] sum_pixels err^2 / numel.
+        With the eps target and no weights this is the reference's MSE (ops.MseLossFn); otherwise the fused
+        objective (ops.DiffusionLossFn) computes the target and the weighting."""
+        if weights is not None and (not torch.is_tensor(weights) or tuple(weights.shape) != (self.T,)):
+            raise ValueError(f"weights must be a tensor of shape ({self.T},)")
         B = x0.size(0)
         if t is None:
             t = torch.randint(0, self.T, (B,), device=x0.device).long()
         x_t, noise = self.q_sample(x0, t, noise)
         eps_pred = self.model(x_t, cond, t)
-        return ops.MseLossFn.apply(eps_pred, noise.float())
+        if self.prediction_type == "eps" and weights is None:
+            return ops.MseLossFn.apply(eps_pred, noise.float())
+        w = None if weights is None else weights.float().contiguous()
+        return ops.DiffusionLossFn.apply(eps_pred, x0.float(), noise.float(), t.contiguous(), self.target_coef, w)

@@ -1061,6 +1061,33 @@ class MseLossFn(_Fn):
         return deps, dnoise
 
 
+class DiffusionLossFn(_Fn):
+    """sum_b w[t_b] * sum (pred - target)^2 / numel with target = c_n[t] noise + c_x[t] x0 (`tgt_coef` [T, 2], None for
+    the eps target) and per-timestep weights `weight` [T] (None: uniform).  Differentiable in pred, noise and x0 (the
+    target's share; q_sample's share comes through QSampleFn)."""
+
+    @staticmethod
+    def forward(ctx, pred, x0, noise, t, tgt_coef, weight):
+        T = (tgt_coef if tgt_coef is not None else weight).shape[0]
+        loss, diff = K.diffusion_loss_fwd(pred.contiguous(), _c(x0), noise.contiguous(), t.contiguous(), tgt_coef,
+                                          weight, T)
+        ctx.save_for_backward(diff, t, tgt_coef, weight)
+        ctx.T = T
+        return loss
+
+    @staticmethod
+    def backward(ctx, g):
+        diff, t, tgt_coef, weight = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        need_x0 = need[1] and tgt_coef is not None  # the eps target does not depend on x0
+        if not (need[0] or need[2] or need_x0):
+            return None, None, None, None, None, None
+        g = g.reshape(1).float().contiguous()
+        dpred, dnoise, dx0 = K.diffusion_loss_bwd(diff, t, tgt_coef, weight, g, 2.0 / diff.numel(), ctx.T, need[0],
+                                                  need[2], need_x0)
+        return dpred, dx0, dnoise, None, None, None
+
+
 class QSampleFn(_Fn):
     """x_t = sqrt_ac[t] x0 + sqrt_1mac[t] noise (model.py:196-201), differentiable in x0 and noise."""
 

@@ -372,6 +372,21 @@ int cesm_q_sample_bwd(const float* g, const long long* t, const float* sqrt_ac, 
 int cesm_mse_fwd(const float* eps, const float* noise, float* diff, float* loss, long long total, void* stream);
 int cesm_scale_by_scalar(const float* in, const float* gscale, float factor, float* out, long long total,
                          void* stream);
+/* Diffusion objective with a per-timestep target and weight (v-prediction, Min-SNR-gamma).  Per sample b with
+ * tb = t[b]: target = c_n[tb] * noise + c_x[tb] * x0 from the fp32 [T][2] rows (c_n, c_x) of tgt_coef; a NULL
+ * tgt_coef is the eps target (target = noise, x0 not read, may be NULL).  diff = pred - target, and
+ * *loss = sum_b w[tb] * sum diff^2 / (B * per_sample) with w = weight[T] (NULL: 1); *loss is zeroed first.  A t
+ * outside [0, T) makes diff and *loss NaN.  Rejects T, B, per_sample <= 0, B > 65535 and NULL pred, noise, t, diff
+ * or loss with CESM_ERR_INVALID. */
+int cesm_diffusion_loss_fwd(const float* pred, const float* x0, const float* noise, const long long* t,
+                            const float* tgt_coef, const float* weight, float* diff, float* loss, int B,
+                            long long per_sample, int T, void* stream);
+/* Backward of cesm_diffusion_loss_fwd for an incoming gradient *gscale (device scalar): dpred = factor * g * w[tb] *
+ * diff, dnoise = -c_n[tb] * dpred and dx0 = -c_x[tb] * dpred (the target's share of those input gradients).  Any
+ * output may be NULL, not all three.  A t outside [0, T) writes NaN. */
+int cesm_diffusion_loss_bwd(const float* diff, const long long* t, const float* tgt_coef, const float* weight,
+                            const float* gscale, float factor, float* dpred, float* dnoise, float* dx0, int B,
+                            long long per_sample, int T, void* stream);
 int cesm_p_sample(const float* xt, const float* eps, const float* z, const long long* t, const float* betas,
                   const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out, int B,
                   long long per_sample, void* stream);

@@ -27,19 +27,21 @@ import torch.distributed as dist
 from cesm_emulator_b200.engine import SampleEngine
 from cesm_emulator_b200.model import Diffusion
 from cesm_emulator_b200.synthetic import SyntheticEnsemble
-from train import build_model_from_config
+from train import build_model_from_config, prediction_type_from_config
 
 
 def load_diffusion_from_checkpoint(path, device, ema=False):
     """inference.py:47-75.  With `ema=True` the UNet gets the checkpoint's weight EMA (ckpt["ema"], written by a run
-    with train.ema_decay set) instead of its raw weights (ckpt["model"]); a checkpoint without one is an error."""
+    with train.ema_decay set) instead of its raw weights (ckpt["model"]); a checkpoint without one is an error.  The
+    Diffusion predicts the target the run trained (diffusion.prediction_type in ckpt["config"], eps when absent)."""
     ckpt = torch.load(path, map_location=device)
     if ema and "ema" not in ckpt:
         raise KeyError(f'{path} has no "ema" entry: it was not trained with train.ema_decay set '
                        f'(load it without ema=True / --ema to sample from its raw weights)')
     cfg = ckpt["config"]
     diffusion = Diffusion(build_model_from_config(cfg.get("unet", {})),
-                          timesteps=cfg.get("diffusion", {}).get("timesteps", 1000)).to(device)
+                          timesteps=cfg.get("diffusion", {}).get("timesteps", 1000),
+                          prediction_type=prediction_type_from_config(cfg)).to(device)
     missing, unexpected = diffusion.model.load_state_dict(ckpt["ema" if ema else "model"], strict=False)
     if missing or unexpected:
         print(f"[load] missing={list(missing)} unexpected={list(unexpected)}")

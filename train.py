@@ -63,10 +63,20 @@ def save_checkpoint(path, epoch, diffusion, engine, cfg):
     torch.save(ckpt, path)
 
 
+def prediction_type_from_config(cfg: dict) -> str:
+    """diffusion.prediction_type of a run's config (or a checkpoint's "config"); absent means the reference's eps."""
+    return (cfg or {}).get("diffusion", {}).get("prediction_type", "eps")
+
+
 def load_checkpoint(path, diffusion, engine=None, device="cuda"):
     """train.py:915-946 semantics: strict=False on the UNet, buffers merged, start_epoch = epoch + 1.  An engine with a
-    weight EMA loads the checkpoint's "ema", or restarts the EMA from the loaded weights if it has none."""
+    weight EMA loads the checkpoint's "ema", or restarts the EMA from the loaded weights if it has none.  A checkpoint
+    whose config names another prediction_type than `diffusion`'s is an error: its weights predict another target."""
     ckpt = torch.load(path, map_location=device)
+    saved = prediction_type_from_config(ckpt.get("config"))
+    if saved != diffusion.prediction_type:
+        raise ValueError(f"{path} was trained with diffusion.prediction_type={saved!r}; this run uses "
+                         f"{diffusion.prediction_type!r}")
     missing, unexpected = diffusion.model.load_state_dict(ckpt["model"], strict=False)
     if missing or unexpected:
         print(f"[resume] missing={list(missing)} unexpected={list(unexpected)}")
@@ -98,13 +108,14 @@ def main(cfg):
     torch.manual_seed(0)
     diffusion = Diffusion(build_model_from_config(cfg.get("unet", {})),
                           timesteps=cfg.get("diffusion", {}).get("timesteps", 1000),
-                          beta_schedule=cfg.get("diffusion", {}).get("beta_schedule", "linear")).to(dev)
+                          beta_schedule=cfg.get("diffusion", {}).get("beta_schedule", "linear"),
+                          prediction_type=prediction_type_from_config(cfg)).to(dev)
     diffusion.train()
     opt = tcfg.get("optimizer", {})
     engine = TrainEngine(diffusion, (B, 1, h, w), (B, 1, K, h, w), lr=opt.get("lr", 2e-4),
                          betas=tuple(opt.get("betas", (0.9, 0.999))), weight_decay=opt.get("weight_decay", 1e-4),
                          max_grad_norm=tcfg.get("max_grad_norm", 1.0), ema_decay=tcfg.get("ema_decay"),
-                         ema_start=tcfg.get("ema_start", 0))
+                         ema_start=tcfg.get("ema_start", 0), min_snr_gamma=tcfg.get("min_snr_gamma"))
     start = 1
     if tcfg.get("resume") and os.path.exists(tcfg["resume"]):
         start = load_checkpoint(tcfg["resume"], diffusion, engine, dev)

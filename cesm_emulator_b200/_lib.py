@@ -136,10 +136,12 @@ _SIGNATURES: dict[str, list] = {
     "cesm_gather_windows": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P],
     "cesm_qkv_bwd": [_P, _P, _P, _P, _P, _L, _L, _I, _I, _P],
     "cesm_input_patches": [_P, _P, _I, _I, _P, _I, _I, _I, _I, _I, _I, _P],
+    "cesm_input_patches_masked": [_P, _P, _I, _I, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     "cesm_input_weight_pack": [_P, _P, _P, _I, _I, _I, _P],
     "cesm_input_conv_fwd": [_P, _P, _I, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     "cesm_input_conv_wgrad": [_P, _P, _I, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     "cesm_input_conv_dgrad": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _F, _I, _P],
+    "cesm_input_conv_dgrad_masked": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _F, _I, _P],
     "cesm_out_conv_fwd": [_P, _P, _P, _P, _I, _I, _I, _L, _I, _P],
     "cesm_out_conv_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _L, _I, _P],
     "cesm_sinusoidal": [_P, _P, _I, _I, _P],
@@ -157,6 +159,12 @@ _SIGNATURES: dict[str, list] = {
     "cesm_field_normal": [_U, _U, _P, _U, _P, _I, _L, _P],
     "cesm_p_sample_seeded": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
     "cesm_ddim_step_seeded": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _I, _I, _L, _P],
+    "cesm_p_sample_guided": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _F, _P],
+    "cesm_ddim_step_guided": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
+    "cesm_dpm_step_guided": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
+    "cesm_p_sample_seeded_guided": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
+    "cesm_ddim_step_seeded_guided": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
+    "cesm_cond_keep": [_U, _U, _P, _L, _F, _P, _I, _P],
 }
 
 

@@ -76,11 +76,14 @@ colsum_kernel(const h16* __restrict__ x, float* __restrict__ out, long long M, i
 // weight-gradient kernel yields dW (sum of the hi and lo column blocks) and db (the ones column) from
 // the same patch matrix.  A block stages a 16x16 pixel tile's halo once; a warp then writes one pixel's
 // 2*KPAD bytes per trip, each lane a fixed 8-column chunk whose shared-memory offsets it computed once.
+// keep (optional, [B]): batch element b reads its condition plane as zeros where keep[b] == 0 (classifier-free
+// guidance's condition dropout), so the forward GEMM and the weight gradient, which both read these patches, see the
+// null condition without a masked copy of it.
 // ------------------------------------------------------------------------------------------------
 template <int KS, int KPAD>
 __global__ void __launch_bounds__(256)
 input_patches_kernel(const float* __restrict__ in0, const float* __restrict__ in1, int f0, int f1,
-                     h16* __restrict__ out, int F, int H, int W) {
+                     const float* __restrict__ keep, h16* __restrict__ out, int F, int H, int W) {
     pdl_trigger();
     pdl_wait();
     constexpr int T = 16, PAD = KS / 2, PW = T + KS - 1, NT = 2 * KS * KS;
@@ -90,11 +93,12 @@ input_patches_kernel(const float* __restrict__ in0, const float* __restrict__ in
     const int h0 = blockIdx.y * T, w0 = blockIdx.x * T;
     const float* p0 = in0 + ((size_t)b * f0 + (f0 == 1 ? 0 : f)) * H * W;
     const float* p1 = in1 + ((size_t)b * f1 + (f1 == 1 ? 0 : f)) * H * W;
+    const bool drop = keep && keep[b] == 0.f;
     for (int x = threadIdx.x; x < 2 * PW * PW; x += 256) {
         const int ci = x / (PW * PW), rr = (x / PW) % PW, cc = x % PW;
         const int hh = h0 + rr - PAD, ww = w0 + cc - PAD;
         float v = 0.f;
-        if (hh >= 0 && hh < H && ww >= 0 && ww < W) v = (ci ? p1 : p0)[(size_t)hh * W + ww];
+        if (hh >= 0 && hh < H && ww >= 0 && ww < W && !(ci && drop)) v = (ci ? p1 : p0)[(size_t)hh * W + ww];
         const float hi = __half2float(__float2half_rn(v));
         sv[0][ci][rr][cc] = hi;
         sv[1][ci][rr][cc] = __half2float(__float2half_rn(v - hi));
@@ -292,7 +296,8 @@ input_conv_wgrad_kernel(const float* __restrict__ in0, const float* __restrict__
 // the frames (the forward's broadcast) when fp == 1 < F.  Thread = one pixel.  Dynamic shared memory: the weights
 // as float4 {W[co][0][t], W[co][1][t], W[co+1][0][t], W[co+1][1][t]} per (tap, channel pair), then the frame's dy
 // halo tile as half2 words with a pixel stride of COUT/2 + 1 words and a row stride = 16 (mod 32) words, so the 32
-// pixels (2 rows x 16) a warp reads per channel pair fall in 32 different banks.
+// pixels (2 rows x 16) a warp reads per channel pair fall in 32 different banks.  keep (optional, [B]): where
+// keep[b] == 0 the forward read a zero condition, so d_in1 of batch element b is 0 (written, or nothing added).
 template <int KS, int COUT>
 struct InputDgradSmem {
     static constexpr int T = 16, PAD = KS / 2, PW = T + KS - 1, CP = COUT / 2, PS = CP + 1;
@@ -303,8 +308,8 @@ struct InputDgradSmem {
 template <int KS, int COUT, bool DX, bool DC>
 __global__ void __launch_bounds__(256)
 input_conv_dgrad_kernel(const h16* __restrict__ dy, const float* __restrict__ w /* [COUT][2][KS][KS] */,
-                        float* __restrict__ dx, float* __restrict__ dc, int f0, int f1, int F, int H, int W,
-                        float scale, int accumulate) {
+                        float* __restrict__ dx, float* __restrict__ dc, const float* __restrict__ keep, int f0,
+                        int f1, int F, int H, int W, float scale, int accumulate) {
     pdl_trigger();
     pdl_wait();
     using S = InputDgradSmem<KS, COUT>;
@@ -322,6 +327,7 @@ input_conv_dgrad_kernel(const h16* __restrict__ dy, const float* __restrict__ w 
     const int ty = threadIdx.x / T, tx = threadIdx.x % T;
     const int h = h0 + ty, ww = w0 + tx;
     const bool inside = h < H && ww < W;
+    const bool drop = keep && keep[b] == 0.f;  // this batch element read a zero condition
     const size_t HW = (size_t)H * W, pix = (size_t)h * W + ww;
     const auto put = [&](float* p, float v) { *p = accumulate ? fmaf(scale, v, *p) : scale * v; };
     float a0 = 0.f, a1 = 0.f;
@@ -359,12 +365,12 @@ input_conv_dgrad_kernel(const h16* __restrict__ dy, const float* __restrict__ w 
             a0 = 0.f;
         }
         if (DC && f1 == F) {
-            if (inside) put(dc + ((size_t)b * F + f) * HW + pix, a1);
+            if (inside) put(dc + ((size_t)b * F + f) * HW + pix, drop ? 0.f : a1);
             a1 = 0.f;
         }
     }
     if (DX && f0 != F && inside) put(dx + (size_t)b * HW + pix, a0);
-    if (DC && f1 != F && inside) put(dc + (size_t)b * HW + pix, a1);
+    if (DC && f1 != F && inside) put(dc + (size_t)b * HW + pix, drop ? 0.f : a1);
 }
 
 // eps[b][h][w] = bias + sum_c a[(b*F + mid)][h][w][c] * w[c]   ; 8 lanes per pixel (C == 64)
@@ -729,17 +735,29 @@ __device__ __forceinline__ float p_sample_update(float x, float e, float z, long
     const float mean = sqrt_recip_a[tb] * (x - betas[tb] / sqrt_1mac[tb] * e);
     return mean + sqrtf(post_var[tb]) * z;
 }
+// Classifier-free guidance (Ho & Salimans) inside the update kernels: with kGuided the network output holds 2B rows,
+// the B conditional predictions c, then the B null-condition predictions u of the same fields (u of element i at
+// i + half, half = B * per), and the update uses c + w (c - u) = (1 + w) c - w u in the network's own output space.
+// No combined tensor is written.  Without kGuided the kernels read eps[i] as before.
+template <bool kGuided>
+__device__ __forceinline__ float net_out(const float* eps, long long i, long long half, float w) {
+    if (!kGuided) return eps[i];
+    const float c = eps[i];
+    return fmaf(w, c - eps[i + half], c);
+}
+template <bool kGuided>
 __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
                                 const float* __restrict__ z, const long long* __restrict__ t,
                                 const float* __restrict__ betas, const float* __restrict__ sqrt_1mac,
                                 const float* __restrict__ sqrt_recip_a, const float* __restrict__ post_var,
-                                float* __restrict__ out, long long per, long long total) {
+                                float* __restrict__ out, long long per, long long total, float w) {
     pdl_trigger();
     pdl_wait();
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
     const long long tb = t[idx / per];
-    out[idx] = p_sample_update(xt[idx], eps[idx], z[idx], tb, betas, sqrt_1mac, sqrt_recip_a, post_var);
+    out[idx] = p_sample_update(xt[idx], net_out<kGuided>(eps, idx, total, w), z[idx], tb, betas, sqrt_1mac,
+                               sqrt_recip_a, post_var);
 }
 // Strided DDIM step (Song et al.): x_prev = A[t] * x_t + B[t] * eps + S[t] * z, with the three coefficients of each
 // schedule timestep precomputed on the host in float64 (model.ddim_schedule) and stored as coef[T][3] fp32.
@@ -749,10 +767,11 @@ __global__ void p_sample_kernel(const float* __restrict__ xt, const float* __res
 // an out-of-range t is passed through unchanged, so a chain that overruns its schedule keeps producing NaN.
 // The noise term is fmaf(S, z, ddim_mean(...)) in this kernel and in the seeded one.
 __device__ __forceinline__ float ddim_mean(const float* c, float x, float e) { return fmaf(c[0], x, c[1] * e); }
+template <bool kGuided>
 __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps, const float* __restrict__ z,
                                  const long long* __restrict__ t, const float* __restrict__ coef,
                                  const long long* __restrict__ next_t, long long* __restrict__ t_out, float* out,
-                                 int T, long long per, long long total) {
+                                 int T, long long per, long long total, float w) {
     pdl_trigger();
     pdl_wait();
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -766,7 +785,7 @@ __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps,
         return;
     }
     const float* c = coef + 3 * tb;
-    float v = ddim_mean(c, xt[idx], eps[idx]);
+    float v = ddim_mean(c, xt[idx], net_out<kGuided>(eps, idx, total, w));
     if (z) v = fmaf(c[2], z[idx], v);
     out[idx] = v;
 }
@@ -776,10 +795,11 @@ __global__ void ddim_step_kernel(const float* xt, const float* __restrict__ eps,
 // hist is the previous step's x0 prediction.  Where K1 == 0 (the first-order first and last steps) hist is not read,
 // so a stale or NaN history cannot reach the output and a new chain needs no reset.  `out` may alias `xt`; hist
 // aliases nothing.  An out-of-range t writes NaN to out and hist and passes t through to t_out, as ddim_step does.
+template <bool kGuided>
 __global__ void dpm_step_kernel(const float* xt, const float* __restrict__ eps, float* __restrict__ hist,
                                 const long long* __restrict__ t, const float* __restrict__ coef,
                                 const long long* __restrict__ next_t, long long* __restrict__ t_out, float* out,
-                                int T, long long per, long long total) {
+                                int T, long long per, long long total, float w) {
     pdl_trigger();
     pdl_wait();
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -795,7 +815,7 @@ __global__ void dpm_step_kernel(const float* xt, const float* __restrict__ eps, 
     }
     const float* c = coef + 5 * tb;
     const float x = xt[idx];
-    const float x0 = fmaf(c[0], x, c[1] * eps[idx]);
+    const float x0 = fmaf(c[0], x, c[1] * net_out<kGuided>(eps, idx, total, w));
     float v = fmaf(c[2], x, c[3] * x0);
     const float k1 = c[4];
     if (k1 != 0.0f) v = fmaf(k1, hist[idx], v);
@@ -879,13 +899,25 @@ field_normal_kernel(unsigned seed_lo, unsigned seed_hi, const long long* __restr
 
 // p_sample_kernel with z drawn in registers from (seed, field_ids[b], draw t[b]).  `out` may alias `xt` (a thread
 // reads its quad before writing it).  A t outside [0, T) writes NaN instead of reading outside the schedule.
-template <bool kVec>
+// The network output quad of the update: eps's, or with kGuided c + w (c - u) from both halves (net_out).
+template <bool kVec, bool kGuided>
+__device__ __forceinline__ void load_net_quad(const float* eps, long long off, long long half, float w, int n,
+                                              float (&e)[4]) {
+    load_quad<kVec>(eps + off, n, e);
+    if (!kGuided) return;
+    float u[4];
+    load_quad<kVec>(eps + off + half, n, u);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) e[j] = fmaf(w, e[j] - u[j], e[j]);
+}
+
+template <bool kVec, bool kGuided>
 __global__ void __launch_bounds__(256)
 p_sample_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned seed_lo, unsigned seed_hi,
                        const long long* __restrict__ field_ids, const long long* __restrict__ t,
                        const float* __restrict__ betas, const float* __restrict__ sqrt_1mac,
                        const float* __restrict__ sqrt_recip_a, const float* __restrict__ post_var, float* out, int T,
-                       long long per) {
+                       long long per, float w) {
     pdl_trigger();
     pdl_wait();
     const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -904,7 +936,7 @@ p_sample_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned 
     float x[4], e[4], z[4];
     field_normal4(seed_lo, seed_hi, field_ids[b], (unsigned)tb, q, z);
     load_quad<kVec>(xt + off, n, x);
-    load_quad<kVec>(eps + off, n, e);
+    load_net_quad<kVec, kGuided>(eps, off, (long long)gridDim.y * per, w, n, e);
 #pragma unroll
     for (int j = 0; j < 4; ++j)
         v[j] = p_sample_update(x[j], e[j], z[j], tb, betas, sqrt_1mac, sqrt_recip_a, post_var);
@@ -912,12 +944,12 @@ p_sample_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned 
 }
 
 // ddim_step_kernel with z drawn in registers from (seed, field_ids[b], draw t[b]); same t_out / NaN contract.
-template <bool kVec>
+template <bool kVec, bool kGuided>
 __global__ void __launch_bounds__(256)
 ddim_step_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned seed_lo, unsigned seed_hi,
                         const long long* __restrict__ field_ids, const long long* __restrict__ t,
                         const float* __restrict__ coef, const long long* __restrict__ next_t,
-                        long long* __restrict__ t_out, float* out, int T, long long per) {
+                        long long* __restrict__ t_out, float* out, int T, long long per, float w) {
     pdl_trigger();
     pdl_wait();
     const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -938,11 +970,32 @@ ddim_step_seeded_kernel(const float* xt, const float* __restrict__ eps, unsigned
     float x[4], e[4], z[4];
     field_normal4(seed_lo, seed_hi, field_ids[b], (unsigned)tb, q, z);
     load_quad<kVec>(xt + off, n, x);
-    load_quad<kVec>(eps + off, n, e);
+    load_net_quad<kVec, kGuided>(eps, off, (long long)gridDim.y * per, w, n, e);
     const float* c = coef + 3 * tb;
 #pragma unroll
     for (int j = 0; j < 4; ++j) v[j] = fmaf(c[2], z[j], ddim_mean(c, x[j], e[j]));
     store_quad<kVec>(out + off, n, v);
+}
+
+// Condition dropout of a training step: keep[b] = (u >= p) ? 1 : 0 with u the uniform of word 0 of
+//     Philox4x32-10(counter = (g_lo, g_hi, s_lo, s_hi), key = (seed_lo, seed_hi)),   g = first + b, s = *step,
+// then *step += 1.  The draw depends on (seed, step, global sample index g) only, so a global batch split over ranks
+// (first = rank * B) drops the same samples as on one GPU.  One block; the counter is read by every thread before
+// thread 0 advances it.
+__global__ void __launch_bounds__(256)
+cond_keep_kernel(unsigned seed_lo, unsigned seed_hi, long long* __restrict__ step, long long first, float p,
+                 float* __restrict__ keep, int B) {
+    pdl_trigger();
+    pdl_wait();
+    const unsigned long long s = (unsigned long long)*step;
+    for (int b = threadIdx.x; b < B; b += blockDim.x) {
+        const unsigned long long g = (unsigned long long)(first + b);
+        const uint4 w = philox4x32_10(make_uint4((unsigned)g, (unsigned)(g >> 32), (unsigned)s, (unsigned)(s >> 32)),
+                                      seed_lo, seed_hi);
+        keep[b] = philox_uniform(w.x) >= p ? 1.0f : 0.0f;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) *step = (long long)(s + 1);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1028,14 +1081,20 @@ extern "C" int cesm_gather_windows(const float* cond, const float* tgt, const in
     return CESM_OK;
 }
 
-extern "C" int cesm_input_patches(const float* in0, const float* in1, int f0, int f1, void* out, int B, int F, int H,
-                                  int W, int ks, int kpad, void* stream) {
+extern "C" int cesm_input_patches_masked(const float* in0, const float* in1, int f0, int f1, const float* keep, void* out,
+                                         int B, int F, int H, int W, int ks, int kpad, void* stream) {
     CESM_REQUIRE(ks == 7 && kpad == 256, "input patch kernel is specialised for 7x7, 256 columns (ks=%d kpad=%d)", ks, kpad);
     CESM_REQUIRE((f0 == 1 || f0 == F) && (f1 == 1 || f1 == F), "frame counts must be 1 or F");
     dim3 grid(ceil_div(W, 16), ceil_div(H, 16), B * F);
-    launch_pdl(input_patches_kernel<7, 256>, grid, 256, 0, as_stream(stream), in0, in1, f0, f1, (h16*)out, F, H, W);
+    launch_pdl(input_patches_kernel<7, 256>, grid, 256, 0, as_stream(stream), in0, in1, f0, f1, keep, (h16*)out, F, H,
+               W);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
+}
+
+extern "C" int cesm_input_patches(const float* in0, const float* in1, int f0, int f1, void* out, int B, int F, int H,
+                                  int W, int ks, int kpad, void* stream) {
+    return cesm_input_patches_masked(in0, in1, f0, f1, nullptr, out, B, F, H, W, ks, kpad, stream);
 }
 
 extern "C" int cesm_input_weight_pack(const float* w, const float* bias, void* out, int cout, int ks, int kpad,
@@ -1072,8 +1131,8 @@ extern "C" int cesm_input_conv_wgrad(const float* in0, const float* in1, int f0,
 }
 
 template <bool DX, bool DC>
-static int launch_input_conv_dgrad(const void* dy, const float* w, float* dx, float* dc, int f0, int f1, int B, int F,
-                                   int H, int W, float scale, int accumulate, cudaStream_t st) {
+static int launch_input_conv_dgrad(const void* dy, const float* w, float* dx, float* dc, const float* keep, int f0,
+                                   int f1, int B, int F, int H, int W, float scale, int accumulate, cudaStream_t st) {
     auto kern = input_conv_dgrad_kernel<7, 64, DX, DC>;
     constexpr size_t smem = InputDgradSmem<7, 64>::BYTES;
     static bool attr_set = false;
@@ -1082,22 +1141,31 @@ static int launch_input_conv_dgrad(const void* dy, const float* w, float* dx, fl
         attr_set = true;
     }
     dim3 grid(ceil_div(W, 16), ceil_div(H, 16), B);
-    launch_pdl(kern, grid, 256, smem, st, (const h16*)dy, w, dx, dc, f0, f1, F, H, W, scale, accumulate);
+    launch_pdl(kern, grid, 256, smem, st, (const h16*)dy, w, dx, dc, keep, f0, f1, F, H, W, scale, accumulate);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }
 
-extern "C" int cesm_input_conv_dgrad(const void* dy, const float* w, float* d_in0, float* d_in1, int f0, int f1, int B,
-                                     int F, int H, int W, int ks, int cout, float scale, int accumulate, void* stream) {
+extern "C" int cesm_input_conv_dgrad_masked(const void* dy, const float* w, float* d_in0, float* d_in1, const float* keep,
+                                            int f0, int f1, int B, int F, int H, int W, int ks, int cout, float scale,
+                                            int accumulate, void* stream) {
     CESM_REQUIRE(ks == 7 && cout == 64, "input conv kernel is specialised for 7x7, 64 channels (ks=%d cout=%d)", ks, cout);
     CESM_REQUIRE(B > 0 && B <= 65535 && F > 0 && H > 0 && W > 0, "bad input conv dgrad shape (B=%d F=%d H=%d W=%d)", B, F,
                  H, W);
     CESM_REQUIRE((f0 == 1 || f0 == F) && (f1 == 1 || f1 == F), "frame counts must be 1 or F");
     CESM_REQUIRE(dy && w && (d_in0 || d_in1), "input conv dgrad needs dy, w and at least one output");
     cudaStream_t st = as_stream(stream);
-    if (d_in0 && d_in1) return launch_input_conv_dgrad<true, true>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
-    if (d_in0) return launch_input_conv_dgrad<true, false>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
-    return launch_input_conv_dgrad<false, true>(dy, w, d_in0, d_in1, f0, f1, B, F, H, W, scale, accumulate, st);
+    if (d_in0 && d_in1)
+        return launch_input_conv_dgrad<true, true>(dy, w, d_in0, d_in1, keep, f0, f1, B, F, H, W, scale, accumulate, st);
+    if (d_in0)
+        return launch_input_conv_dgrad<true, false>(dy, w, d_in0, d_in1, keep, f0, f1, B, F, H, W, scale, accumulate, st);
+    return launch_input_conv_dgrad<false, true>(dy, w, d_in0, d_in1, keep, f0, f1, B, F, H, W, scale, accumulate, st);
+}
+
+extern "C" int cesm_input_conv_dgrad(const void* dy, const float* w, float* d_in0, float* d_in1, int f0, int f1, int B,
+                                     int F, int H, int W, int ks, int cout, float scale, int accumulate, void* stream) {
+    return cesm_input_conv_dgrad_masked(dy, w, d_in0, d_in1, nullptr, f0, f1, B, F, H, W, ks, cout, scale, accumulate,
+                                        stream);
 }
 
 extern "C" int cesm_out_conv_fwd(const void* a, const float* w, const float* bias, float* eps, int B, int F, int mid,
@@ -1247,8 +1315,43 @@ extern "C" int cesm_p_sample(const float* xt, const float* eps, const float* z, 
                              const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out,
                              int B, long long per_sample, void* stream) {
     const long long total = (long long)B * per_sample;
-    launch_pdl(p_sample_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a,
-                                                                    post_var, out, per_sample, total);
+    launch_pdl(p_sample_kernel<false>, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, betas, sqrt_1mac,
+               sqrt_recip_a, post_var, out, per_sample, total, 0.0f);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+// The guided entries take the 2B-row network output (conditional rows, then null-condition rows) and a finite w > 0.
+#define CESM_REQUIRE_GUIDANCE(what)                                                                              \
+    CESM_REQUIRE(isfinite(guidance) && guidance > 0.0f, what " needs a finite guidance weight > 0 (got %g)",      \
+                 (double)guidance)
+
+extern "C" int cesm_p_sample_guided(const float* xt, const float* eps, const float* z, const long long* t,
+                                    const float* betas, const float* sqrt_1mac, const float* sqrt_recip_a,
+                                    const float* post_var, float* out, int B, long long per_sample, float guidance,
+                                    void* stream) {
+    CESM_REQUIRE(B > 0 && per_sample > 0, "bad guided p_sample sizes (B=%d per_sample=%lld)", B, per_sample);
+    CESM_REQUIRE(xt && eps && z && t && betas && sqrt_1mac && sqrt_recip_a && post_var && out,
+                 "guided p_sample needs xt, eps, z, t, the four schedule tables and out");
+    CESM_REQUIRE_GUIDANCE("guided p_sample");
+    const long long total = (long long)B * per_sample;
+    launch_pdl(p_sample_kernel<true>, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, betas, sqrt_1mac,
+               sqrt_recip_a, post_var, out, per_sample, total, guidance);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+template <bool kGuided>
+static int launch_ddim_step(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
+                            const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                            float w, void* stream) {
+    CESM_REQUIRE(T > 0 && B > 0 && per_sample > 0, "bad DDIM step sizes (T=%d B=%d per_sample=%lld)", T, B, per_sample);
+    CESM_REQUIRE(xt && eps && t && coef && out, "DDIM step needs xt, eps, t, coef and out");
+    CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
+    CESM_REQUIRE(!t_out || (const void*)t_out != (const void*)t, "t_out must not alias t");
+    const long long total = (long long)B * per_sample;
+    launch_pdl(ddim_step_kernel<kGuided>, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, coef, next_t, t_out,
+               out, T, per_sample, total, w);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }
@@ -1256,15 +1359,14 @@ extern "C" int cesm_p_sample(const float* xt, const float* eps, const float* z, 
 extern "C" int cesm_ddim_step(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
                               const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
                               void* stream) {
-    CESM_REQUIRE(T > 0 && B > 0 && per_sample > 0, "bad DDIM step sizes (T=%d B=%d per_sample=%lld)", T, B, per_sample);
-    CESM_REQUIRE(xt && eps && t && coef && out, "DDIM step needs xt, eps, t, coef and out");
-    CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
-    CESM_REQUIRE(!t_out || (const void*)t_out != (const void*)t, "t_out must not alias t");
-    const long long total = (long long)B * per_sample;
-    launch_pdl(ddim_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, z, t, coef, next_t, t_out, out, T,
-               per_sample, total);
-    CESM_CHECK_LAUNCH();
-    return CESM_OK;
+    return launch_ddim_step<false>(xt, eps, z, t, coef, next_t, t_out, out, T, B, per_sample, 0.0f, stream);
+}
+
+extern "C" int cesm_ddim_step_guided(const float* xt, const float* eps, const float* z, const long long* t,
+                                     const float* coef, const long long* next_t, long long* t_out, float* out, int T,
+                                     int B, long long per_sample, float guidance, void* stream) {
+    CESM_REQUIRE_GUIDANCE("guided DDIM step");
+    return launch_ddim_step<true>(xt, eps, z, t, coef, next_t, t_out, out, T, B, per_sample, guidance, stream);
 }
 
 // True when the byte ranges [a, a + na) and [b, b + nb) share a byte (a null b shares none).
@@ -1273,25 +1375,39 @@ static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
     return pb && pa < pb + nb && pb < pa + na;
 }
 
-extern "C" int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
-                             const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
-                             void* stream) {
+template <bool kGuided>
+static int launch_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
+                           const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                           float w, void* stream) {
     CESM_REQUIRE(T > 0 && B > 0 && per_sample > 0, "bad DPM step sizes (T=%d B=%d per_sample=%lld)", T, B, per_sample);
     CESM_REQUIRE(xt && eps && hist && t && coef && out, "DPM step needs xt, eps, hist, t, coef and out");
     CESM_REQUIRE(!t_out || next_t, "t_out needs the next_t table");
     CESM_REQUIRE(!t_out || (const void*)t_out != (const void*)t, "t_out must not alias t");
     const long long total = (long long)B * per_sample;
     const size_t field = (size_t)total * sizeof(float), tb = (size_t)B * sizeof(long long);
-    CESM_REQUIRE(!ranges_overlap(hist, field, xt, field) && !ranges_overlap(hist, field, eps, field) &&
+    CESM_REQUIRE(!ranges_overlap(hist, field, xt, field) && !ranges_overlap(hist, field, eps, (kGuided ? 2 : 1) * field) &&
                      !ranges_overlap(hist, field, out, field) && !ranges_overlap(hist, field, t, tb) &&
                      !ranges_overlap(hist, field, t_out, tb) &&
                      !ranges_overlap(hist, field, coef, (size_t)T * 5 * sizeof(float)) &&
                      !ranges_overlap(hist, field, next_t, (size_t)T * sizeof(long long)),
                  "hist must not overlap xt, eps, out, t, t_out, coef or next_t");
-    launch_pdl(dpm_step_kernel, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, hist, t, coef, next_t, t_out, out,
-               T, per_sample, total);
+    launch_pdl(dpm_step_kernel<kGuided>, nblk(total, 256), 256, 0, as_stream(stream), xt, eps, hist, t, coef, next_t,
+               t_out, out, T, per_sample, total, w);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
+}
+
+extern "C" int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
+                             const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                             void* stream) {
+    return launch_dpm_step<false>(xt, eps, hist, t, coef, next_t, t_out, out, T, B, per_sample, 0.0f, stream);
+}
+
+extern "C" int cesm_dpm_step_guided(const float* xt, const float* eps, float* hist, const long long* t,
+                                    const float* coef, const long long* next_t, long long* t_out, float* out, int T,
+                                    int B, long long per_sample, float guidance, void* stream) {
+    CESM_REQUIRE_GUIDANCE("guided DPM step");
+    return launch_dpm_step<true>(xt, eps, hist, t, coef, next_t, t_out, out, T, B, per_sample, guidance, stream);
 }
 
 // Seeded sampling noise: one thread per quad of a field, grid.y = field row.  The element index inside a field is
@@ -1320,29 +1436,49 @@ extern "C" int cesm_field_normal(unsigned seed_lo, unsigned seed_hi, const long 
     return CESM_OK;
 }
 
-extern "C" int cesm_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
-                                    const long long* field_ids, const long long* t, const float* betas,
-                                    const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var,
-                                    float* out, int T, int B, long long per_sample, void* stream) {
+template <bool kGuided>
+static int launch_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                  const long long* field_ids, const long long* t, const float* betas,
+                                  const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out,
+                                  int T, int B, long long per_sample, float w, void* stream) {
     CESM_REQUIRE_SEEDED_SIZES("seeded p_sample");
     CESM_REQUIRE(T > 0, "seeded p_sample needs T > 0 (T=%d)", T);
     CESM_REQUIRE(xt && eps && field_ids && t && betas && sqrt_1mac && sqrt_recip_a && post_var && out,
                  "seeded p_sample needs xt, eps, field_ids, t, the four schedule tables and out");
     const dim3 grid = quad_grid(B, per_sample);
     if (quads_aligned(per_sample, xt, eps, out))
-        launch_pdl(p_sample_seeded_kernel<true>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi, field_ids,
-                   t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample);
+        launch_pdl(p_sample_seeded_kernel<true, kGuided>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample, w);
     else
-        launch_pdl(p_sample_seeded_kernel<false>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
-                   field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample);
+        launch_pdl(p_sample_seeded_kernel<false, kGuided>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out, T, per_sample, w);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }
 
-extern "C" int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
-                                     const long long* field_ids, const long long* t, const float* coef,
-                                     const long long* next_t, long long* t_out, float* out, int T, int B,
-                                     long long per_sample, void* stream) {
+extern "C" int cesm_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                    const long long* field_ids, const long long* t, const float* betas,
+                                    const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var,
+                                    float* out, int T, int B, long long per_sample, void* stream) {
+    return launch_p_sample_seeded<false>(xt, eps, seed_lo, seed_hi, field_ids, t, betas, sqrt_1mac, sqrt_recip_a,
+                                         post_var, out, T, B, per_sample, 0.0f, stream);
+}
+
+extern "C" int cesm_p_sample_seeded_guided(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                           const long long* field_ids, const long long* t, const float* betas,
+                                           const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var,
+                                           float* out, int T, int B, long long per_sample, float guidance,
+                                           void* stream) {
+    CESM_REQUIRE_GUIDANCE("guided seeded p_sample");
+    return launch_p_sample_seeded<true>(xt, eps, seed_lo, seed_hi, field_ids, t, betas, sqrt_1mac, sqrt_recip_a,
+                                        post_var, out, T, B, per_sample, guidance, stream);
+}
+
+template <bool kGuided>
+static int launch_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                   const long long* field_ids, const long long* t, const float* coef,
+                                   const long long* next_t, long long* t_out, float* out, int T, int B,
+                                   long long per_sample, float w, void* stream) {
     CESM_REQUIRE_SEEDED_SIZES("seeded DDIM step");
     CESM_REQUIRE(T > 0, "seeded DDIM step needs T > 0 (T=%d)", T);
     CESM_REQUIRE(xt && eps && field_ids && t && coef && out, "seeded DDIM step needs xt, eps, field_ids, t, coef and out");
@@ -1351,11 +1487,38 @@ extern "C" int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned
                  "t_out must not alias t or field_ids");
     const dim3 grid = quad_grid(B, per_sample);
     if (quads_aligned(per_sample, xt, eps, out))
-        launch_pdl(ddim_step_seeded_kernel<true>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
-                   field_ids, t, coef, next_t, t_out, out, T, per_sample);
+        launch_pdl(ddim_step_seeded_kernel<true, kGuided>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, coef, next_t, t_out, out, T, per_sample, w);
     else
-        launch_pdl(ddim_step_seeded_kernel<false>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
-                   field_ids, t, coef, next_t, t_out, out, T, per_sample);
+        launch_pdl(ddim_step_seeded_kernel<false, kGuided>, grid, 256, 0, as_stream(stream), xt, eps, seed_lo, seed_hi,
+                   field_ids, t, coef, next_t, t_out, out, T, per_sample, w);
+    CESM_CHECK_LAUNCH();
+    return CESM_OK;
+}
+
+extern "C" int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                     const long long* field_ids, const long long* t, const float* coef,
+                                     const long long* next_t, long long* t_out, float* out, int T, int B,
+                                     long long per_sample, void* stream) {
+    return launch_ddim_step_seeded<false>(xt, eps, seed_lo, seed_hi, field_ids, t, coef, next_t, t_out, out, T, B,
+                                          per_sample, 0.0f, stream);
+}
+
+extern "C" int cesm_ddim_step_seeded_guided(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                            const long long* field_ids, const long long* t, const float* coef,
+                                            const long long* next_t, long long* t_out, float* out, int T, int B,
+                                            long long per_sample, float guidance, void* stream) {
+    CESM_REQUIRE_GUIDANCE("guided seeded DDIM step");
+    return launch_ddim_step_seeded<true>(xt, eps, seed_lo, seed_hi, field_ids, t, coef, next_t, t_out, out, T, B,
+                                         per_sample, guidance, stream);
+}
+
+extern "C" int cesm_cond_keep(unsigned seed_lo, unsigned seed_hi, long long* step, long long first, float p, float* keep,
+                              int B, void* stream) {
+    CESM_REQUIRE(B > 0 && first >= 0, "bad condition-dropout sizes (B=%d first=%lld)", B, first);
+    CESM_REQUIRE(step && keep, "condition dropout needs the step counter and the keep buffer");
+    CESM_REQUIRE(p >= 0.0f && p < 1.0f, "condition dropout probability must be in [0, 1) (got %g)", (double)p);
+    launch_pdl(cond_keep_kernel, 1, 256, 0, as_stream(stream), seed_lo, seed_hi, step, first, p, keep, B);
     CESM_CHECK_LAUNCH();
     return CESM_OK;
 }

@@ -356,21 +356,42 @@ class TrainEngine:
     diffusion's target (`Diffusion.min_snr_weights`), held in a device buffer the captured step reads.  The weights go
     down to 4e-5 (v, t = 999) and scale a sample's whole backward, which runs in fp16: the step divides the loss
     scale's seed by the batch's largest weight (over all ranks), so the fp16 gradient stream carries the magnitudes
-    of an unweighted step, and multiplies the fp32 gradients by it before the optimizer step."""
+    of an unweighted step, and multiplies the fp32 gradients by it before the optimizer step.
+
+    `cond_drop_prob` = p in [0, 1) (CUDA only; 0 is off) trains for classifier-free guidance: each step, each sample
+    sees the null (all-zero) condition with probability p.  The mask is drawn inside the captured step into the device
+    buffer `keep` (fp32 [B], 0 = dropped) by `kernels.cond_keep`, counter-based from (key, step, global sample index
+    rank * B + b): the same global batch drops the same samples on one GPU or split over ranks, and a replay needs no
+    host round trip.  The key comes from torch's default generator when the engine is built (rank 0's under
+    torch.distributed), so `torch.manual_seed` fixes it as it fixes t and the noise.  The input convolution reads the
+    condition through the mask (ops.InputConvFn); no masked copy of it is made."""
 
     def __init__(self, diffusion, batch_shape, cond_shape, lr: float = 2e-4, betas=(0.9, 0.999),
                  weight_decay: float = 1e-4, eps: float = 1e-8, max_grad_norm: Optional[float] = 1.0,
                  n_buckets: int = 4, use_graph: bool = True, process_group=None, ema_decay: Optional[float] = None,
-                 ema_start: int = 0, min_snr_gamma: Optional[float] = None):
+                 ema_start: int = 0, min_snr_gamma: Optional[float] = None, cond_drop_prob: float = 0.0):
+        from .model import check_cond_drop_prob
         ema_decay, ema_start = check_ema_args(ema_decay, ema_start)
+        self.cond_drop_prob = check_cond_drop_prob(cond_drop_prob)
         self.loss_weights = None if min_snr_gamma is None else diffusion.min_snr_weights(min_snr_gamma)
         self.diffusion = diffusion
         dev = next(diffusion.parameters()).device
         if ema_decay is not None and dev.type != "cuda":
             raise RuntimeError("the weight EMA is updated by the CUDA optimizer step; there is none on host tensors")
+        if self.cond_drop_prob > 0 and dev.type != "cuda":
+            raise RuntimeError("the condition-dropout mask is drawn by a CUDA kernel; there is none on host tensors")
         self.device = dev
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.pg = process_group
+        self.keep = None
+        if self.cond_drop_prob > 0:
+            key = torch.randint(0, 1 << 62, (1,), dtype=torch.int64).to(dev)
+            if self.world > 1:
+                dist.broadcast(key, src=0, group=process_group)
+            self.cond_drop_key = int(key.item())
+            self.keep = torch.ones((batch_shape[0],), dtype=torch.float32, device=dev)
+            self.keep_step = torch.zeros((), dtype=torch.int64, device=dev)  # advanced by every executed step
+            self.first_sample = (dist.get_rank(process_group) if self.world > 1 else 0) * batch_shape[0]
         if self.world > 1:
             for t in list(diffusion.parameters()) + list(diffusion.buffers()):
                 dist.broadcast(t.data, src=0, group=process_group)  # what DDP's constructor does
@@ -410,12 +431,16 @@ class TrainEngine:
         ops.set_side_stream(self.side_stream)
         ops.prepack_all()  # one kernel refreshes every fp16 operand copy of the (just updated) weights
         self.buckets.begin_step()
+        drop = {}  # condition dropout off: the call of before
+        if self.keep is not None:
+            drop["keep"] = K.cond_keep(self.cond_drop_key, self.keep_step, self.first_sample, self.cond_drop_prob,
+                                       self.keep)
         if self.loss_weights is None:
-            loss, wmax = self.diffusion.loss(self.x0, self.cond), None
+            loss, wmax = self.diffusion.loss(self.x0, self.cond, **drop), None
         else:
             # the reference's randint draw, made here so that the batch's largest weight is known
             t = torch.randint(0, self.diffusion.T, (self.x0.shape[0],), device=self.x0.device)
-            loss = self.diffusion.loss(self.x0, self.cond, t, weights=self.loss_weights)
+            loss = self.diffusion.loss(self.x0, self.cond, t, weights=self.loss_weights, **drop)
             wmax = self.loss_weights[t].max()
             if self.world > 1:
                 dist.all_reduce(wmax, op=dist.ReduceOp.MAX, group=self.pg)
@@ -553,11 +578,18 @@ class SampleEngine:
 
     A v-prediction diffusion (`diffusion.prediction_type == "v"`) runs every mode through tables with the conversion to
     eps folded in; its DDPM chain is the `ddim_step` (or `ddim_step_seeded`) launch with `diffusion.ddpm_coef`, the
-    N = T, eta = 1 table, in place of `p_sample`."""
+    N = T, eta = 1 table, in place of `p_sample`.
+
+    With `guidance` = w > 0 every mode samples with classifier-free guidance.  `x`, `cond` and `t` are the first halves
+    of static 2B-row buffers whose second halves hold the same fields with the null (all-zero) condition; a replay
+    copies x and t into the second half, makes one UNet call on the 2B rows and one guided update launch that combines
+    the two halves of the output, (1 + w) out_cond - w out_null, while it updates the B fields.  Seeded noise is drawn
+    for the B fields only.  w = 0 is the unguided engine, unchanged."""
 
     def __init__(self, diffusion, shape, use_graph: bool = True, ddim_steps: Optional[int] = None, eta: float = 0.0,
-                 dpm_steps: Optional[int] = None, seed: Optional[int] = None):
-        from .model import ddim_schedule, dpm_schedule
+                 dpm_steps: Optional[int] = None, seed: Optional[int] = None, guidance: float = 0.0):
+        from .model import check_guidance, ddim_schedule, dpm_schedule
+        self.guidance = check_guidance(guidance)
         if seed is not None:
             K.split_seed(seed)
         if dpm_steps is not None and ddim_steps is not None:
@@ -568,14 +600,21 @@ class SampleEngine:
         dev = next(diffusion.parameters()).device
         self.device = dev
         self.shape = tuple(shape)
-        self.x = torch.zeros(self.shape, dtype=torch.float32, device=dev)
-        self.cond = torch.zeros(self.shape, dtype=torch.float32, device=dev)
+        B = self.shape[0]
+        if self.guidance:  # rows [B, 2B): the same fields with the null condition, which stays zero
+            self._x2 = torch.zeros((2 * B, *self.shape[1:]), dtype=torch.float32, device=dev)
+            self._c2 = torch.zeros_like(self._x2)
+            self._t2 = torch.zeros((2 * B,), dtype=torch.long, device=dev)
+            self.x, self.cond, self.t = self._x2[:B], self._c2[:B], self._t2[:B]
+        else:
+            self.x = torch.zeros(self.shape, dtype=torch.float32, device=dev)
+            self.cond = torch.zeros(self.shape, dtype=torch.float32, device=dev)
+            self.t = torch.zeros((B,), dtype=torch.long, device=dev)
         self.seed = None if seed is None else int(seed)
         if seed is None:
             self.z = torch.zeros(self.shape, dtype=torch.float32, device=dev)
         else:
             self.field_ids = torch.arange(self.shape[0], dtype=torch.int64, device=dev)
-        self.t = torch.zeros((self.shape[0],), dtype=torch.long, device=dev)
         self.arena = K.ZeroArena(dev) if dev.type == "cuda" else None
         self.use_graph = use_graph
         self.graph: Optional[torch.cuda.CUDAGraph] = None
@@ -606,44 +645,52 @@ class SampleEngine:
 
     def _body_inner(self):
         d = self.diffusion
+        w = self.guidance or None
         with torch.no_grad():
-            eps = d.model(self.x, self.cond, self.t)
+            if w is None:
+                eps = d.model(self.x, self.cond, self.t)
+            else:
+                B = self.shape[0]
+                self._x2[B:].copy_(self.x)
+                self._t2[B:].copy_(self.t)
+                eps = d.model(self._x2, self._c2, self._t2)
             if self.ddim_steps is not None:
                 z = None
                 if self.seed is not None and self.eta > 0:
                     K.ddim_step_seeded(self.x, eps, self.seed, self.field_ids, self.t, self.ddim_coef, d.T, out=self.x,
-                                       next_t=self.ddim_next_t, t_out=self.t_next)
+                                       next_t=self.ddim_next_t, t_out=self.t_next, guidance=w)
                     self.t.copy_(self.t_next)
                     return
                 if self.eta > 0:
                     self.z.normal_()
                     z = self.z
                 K.ddim_step(self.x, eps, z, self.t, self.ddim_coef, d.T, out=self.x, next_t=self.ddim_next_t,
-                            t_out=self.t_next)
+                            t_out=self.t_next, guidance=w)
                 self.t.copy_(self.t_next)
                 return
             if self.dpm_steps is not None:
                 K.dpm_step(self.x, eps, self.hist, self.t, self.dpm_coef, d.T, out=self.x, next_t=self.dpm_next_t,
-                           t_out=self.t_next)
+                           t_out=self.t_next, guidance=w)
                 self.t.copy_(self.t_next)
                 return
             if self.seed is not None and d.prediction_type == "v":
-                K.ddim_step_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.ddpm_coef, d.T, out=self.x)
+                K.ddim_step_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.ddpm_coef, d.T, out=self.x,
+                                   guidance=w)
                 self.t.sub_(1)
                 return
             if self.seed is not None:
                 K.p_sample_seeded(self.x, eps, self.seed, self.field_ids, self.t, d.betas,
                                   d.sqrt_one_minus_alphas_cumprod, d.sqrt_recip_alphas, d.posterior_variance,
-                                  out=self.x)
+                                  out=self.x, guidance=w)
                 self.t.sub_(1)
                 return
             self.z.normal_()  # model.py:181 randn_like; kept in a static buffer so that a caller can read the draw
             if d.prediction_type == "v":
-                K.ddim_step(self.x, eps, self.z, self.t, d.ddpm_coef, d.T, out=self.x)
+                K.ddim_step(self.x, eps, self.z, self.t, d.ddpm_coef, d.T, out=self.x, guidance=w)
                 self.t.sub_(1)
                 return
             self.x.copy_(K.p_sample(self.x, eps, self.z, self.t, d.betas, d.sqrt_one_minus_alphas_cumprod,
-                                    d.sqrt_recip_alphas, d.posterior_variance))
+                                    d.sqrt_recip_alphas, d.posterior_variance, guidance=w))
             self.t.sub_(1)
 
     def step(self):

@@ -5,6 +5,7 @@ Nothing here computes with PyTorch; torch only owns the memory and the stream.
 from __future__ import annotations
 
 import ctypes
+import math
 import numbers
 from typing import Optional, Sequence, Tuple
 
@@ -499,13 +500,23 @@ def gather_windows(cond, tgt, plan, cond_out, x0_out) -> None:
 INPUT_KPAD = 256  # columns of the input-conv patch matrix: 2 planes x 49 taps x (hi, lo) + 2 ones + padding
 
 
-def input_patches(in0, in1, B: int, F: int, H: int, W: int, ks: int) -> torch.Tensor:
-    """im2col of the two fp32 input planes (frame broadcast folded in) -> fp16 [B*F, H, W, INPUT_KPAD]."""
-    _req_cuda(in0, in1)
+def _keep_vector(keep, B: int) -> None:
+    assert keep.dtype == torch.float32 and tuple(keep.shape) == (B,), (keep.dtype, tuple(keep.shape), B)
+
+
+def input_patches(in0, in1, B: int, F: int, H: int, W: int, ks: int, keep=None) -> torch.Tensor:
+    """im2col of the two fp32 input planes (frame broadcast folded in) -> fp16 [B*F, H, W, INPUT_KPAD].  `keep` (fp32
+    [B] of 0 / 1, optional): batch element b reads a zero condition plane where keep[b] == 0 (condition dropout)."""
+    _req_cuda(in0, in1, keep)
     f0, f1 = in0.numel() // (B * H * W), in1.numel() // (B * H * W)
     out = torch.empty((B * F, H, W, INPUT_KPAD), dtype=H16, device=in0.device)
-    _lib.call("cesm_input_patches", _ptr(in0), _ptr(in1), f0, f1, _ptr(out), B, F, H, W, ks, INPUT_KPAD, _stream(),
-              _meta=_bytes_meta(out))
+    if keep is None:
+        _lib.call("cesm_input_patches", _ptr(in0), _ptr(in1), f0, f1, _ptr(out), B, F, H, W, ks, INPUT_KPAD, _stream(),
+                  _meta=_bytes_meta(out))
+        return out
+    _keep_vector(keep, B)
+    _lib.call("cesm_input_patches_masked", _ptr(in0), _ptr(in1), f0, f1, _ptr(keep), _ptr(out), B, F, H, W, ks,
+              INPUT_KPAD, _stream(), _meta=_bytes_meta(out))
     return out
 
 
@@ -542,12 +553,14 @@ def input_conv_wgrad(in0, in1, dy, B: int, F: int, H: int, W: int, ks: int):
 
 def input_conv_dgrad(dy, w, B: int, F: int, H: int, W: int, ks: int, f0: int, f1: int, *, need_x: bool = True,
                      need_cond: bool = True, dx_out: Optional[torch.Tensor] = None,
-                     dcond_out: Optional[torch.Tensor] = None, scale: float = 1.0, accumulate: bool = False):
+                     dcond_out: Optional[torch.Tensor] = None, scale: float = 1.0, accumulate: bool = False,
+                     keep: Optional[torch.Tensor] = None):
     """Data gradient of the input convolution (cesm_input_conv_dgrad): dy fp16 [B*F, H, W, C] and the fp32 weight
     [C, 2, 1, ks, ks] -> (d_x fp32 [B, 1, f0, H, W] or None, d_cond fp32 [B, 1, f1, H, W] or None).  A side with one
     frame while F > 1 gets the sum over the F frames (the forward's broadcast).  Each result is scale * grad, written
-    into `dx_out` / `dcond_out` when given -- or, with `accumulate`, added to them."""
-    _req_cuda(dy, w, dx_out, dcond_out)
+    into `dx_out` / `dcond_out` when given -- or, with `accumulate`, added to them.  `keep` (the forward's condition
+    dropout mask, fp32 [B]): d_cond of a batch element with keep[b] == 0 is 0 (cesm_input_conv_dgrad_masked)."""
+    _req_cuda(dy, w, dx_out, dcond_out, keep)
     assert dy.dtype == H16 and tuple(dy.shape[:3]) == (B * F, H, W) and w.dtype == torch.float32
     cout = dy.shape[-1]
     assert tuple(w.shape) == (cout, 2, 1, ks, ks), tuple(w.shape)
@@ -566,8 +579,13 @@ def input_conv_dgrad(dy, w, B: int, F: int, H: int, W: int, ks: int, f0: int, f1
     if _lib.PROFILER is not None:
         meta = {"flops": 2.0 * B * F * H * W * cout * ks * ks * (int(need_x) + int(need_cond)),
                 "bytes": float(dy.numel() * 2 + sum(o.numel() * 4 for o in outs if o is not None))}
-    _lib.call("cesm_input_conv_dgrad", _ptr(dy), _ptr(w), _ptr(outs[0]), _ptr(outs[1]), f0, f1, B, F, H, W, ks, cout,
-              float(scale), int(accumulate), _stream(), _meta=meta)
+    if keep is None:
+        _lib.call("cesm_input_conv_dgrad", _ptr(dy), _ptr(w), _ptr(outs[0]), _ptr(outs[1]), f0, f1, B, F, H, W, ks,
+                  cout, float(scale), int(accumulate), _stream(), _meta=meta)
+        return outs[0], outs[1]
+    _keep_vector(keep, B)
+    _lib.call("cesm_input_conv_dgrad_masked", _ptr(dy), _ptr(w), _ptr(outs[0]), _ptr(outs[1]), _ptr(keep), f0, f1, B, F,
+              H, W, ks, cout, float(scale), int(accumulate), _stream(), _meta=meta)
     return outs[0], outs[1]
 
 
@@ -738,49 +756,65 @@ def scale_by_scalar(x, gscale, factor: float):
     return out
 
 
-def p_sample(xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a, post_var):
+def _net_rows(xt, eps, guidance) -> tuple:
+    """(entry-point suffix, trailing guidance argument) of a sampler step.  Without guidance eps has xt's shape; with
+    a weight w > 0 it holds 2B rows: the conditional predictions of the B fields, then their null-condition ones."""
+    if guidance is None:
+        assert eps.shape == xt.shape, (tuple(eps.shape), tuple(xt.shape))
+        return "", ()
+    assert eps.shape == (2 * xt.shape[0], *xt.shape[1:]), (tuple(eps.shape), tuple(xt.shape))
+    assert math.isfinite(guidance) and guidance > 0, guidance
+    return "_guided", (float(guidance),)
+
+
+def p_sample(xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a, post_var, guidance: Optional[float] = None):
+    """The DDPM posterior step.  `guidance` (w > 0, optional): eps holds 2B rows and the step uses (1 + w) c - w u of
+    the conditional rows c and the null-condition rows u (cesm_p_sample_guided)."""
     _req_cuda(xt, eps, z, t, betas, sqrt_1mac, sqrt_recip_a, post_var)
+    suffix, g = _net_rows(xt, eps, guidance)
     out = torch.empty_like(xt)
     B = xt.shape[0]
-    _lib.call("cesm_p_sample", _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(betas), _ptr(sqrt_1mac), _ptr(sqrt_recip_a),
-              _ptr(post_var), _ptr(out), B, xt.numel() // B, _stream())
+    _lib.call("cesm_p_sample" + suffix, _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(betas), _ptr(sqrt_1mac),
+              _ptr(sqrt_recip_a), _ptr(post_var), _ptr(out), B, xt.numel() // B, *g, _stream())
     return out
 
 
-def ddim_step(xt, eps, z, t, coef, T: int, out=None, next_t=None, t_out=None):
+def ddim_step(xt, eps, z, t, coef, T: int, out=None, next_t=None, t_out=None, guidance: Optional[float] = None):
     """out = A[t]*xt + B[t]*eps + S[t]*z per sample from the fp32 [T, 3] table of `model.ddim_schedule`.
     `out` may be `xt` (in place); `z` may be None when every S is 0.  With `t_out`, next_t[t] is written there
-    (a buffer other than `t`)."""
+    (a buffer other than `t`).  `guidance` as in p_sample (cesm_ddim_step_guided)."""
     _req_cuda(xt, eps, z, t, coef, out, next_t, t_out)
     assert coef.dtype == torch.float32 and coef.shape == (T, 3), (coef.dtype, tuple(coef.shape), T)
-    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32
+    suffix, g = _net_rows(xt, eps, guidance)
     assert z is None or (z.dtype == torch.float32 and z.shape == xt.shape)
     assert (t_out is None) == (next_t is None), "next_t and t_out go together"
     assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
     out = torch.empty_like(xt) if out is None else out
     assert out.dtype == torch.float32 and out.shape == xt.shape
     B = xt.shape[0]
-    _lib.call("cesm_ddim_step", _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out), _ptr(out),
-              T, B, xt.numel() // B, _stream())
+    _lib.call("cesm_ddim_step" + suffix, _ptr(xt), _ptr(eps), _ptr(z), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out),
+              _ptr(out), T, B, xt.numel() // B, *g, _stream())
     return out
 
 
-def dpm_step(xt, eps, hist, t, coef, T: int, out=None, next_t=None, t_out=None):
+def dpm_step(xt, eps, hist, t, coef, T: int, out=None, next_t=None, t_out=None, guidance: Optional[float] = None):
     """DPM-Solver++(2M) step per sample from the fp32 [T, 5] table (P, Q, R, K0, K1) of `model.dpm_schedule`:
     x0 = P*xt + Q*eps, out = R*xt + K0*x0 + K1*hist, then hist = x0.  `hist` is read only where K1 != 0 and must
     be a buffer of its own; `out` may be `xt` (in place).  With `t_out`, next_t[t] is written there (a buffer other
-    than `t`)."""
+    than `t`).  `guidance` as in p_sample (cesm_dpm_step_guided)."""
     _req_cuda(xt, eps, hist, t, coef, out, next_t, t_out)
     assert coef.dtype == torch.float32 and coef.shape == (T, 5), (coef.dtype, tuple(coef.shape), T)
-    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32
+    suffix, g = _net_rows(xt, eps, guidance)
     assert hist.dtype == torch.float32 and hist.shape == xt.shape
     assert (t_out is None) == (next_t is None), "next_t and t_out go together"
     assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
     out = torch.empty_like(xt) if out is None else out
     assert out.dtype == torch.float32 and out.shape == xt.shape
     B = xt.shape[0]
-    _lib.call("cesm_dpm_step", _ptr(xt), _ptr(eps), _ptr(hist), _ptr(t), _ptr(coef), _ptr(next_t), _ptr(t_out),
-              _ptr(out), T, B, xt.numel() // B, _stream())
+    _lib.call("cesm_dpm_step" + suffix, _ptr(xt), _ptr(eps), _ptr(hist), _ptr(t), _ptr(coef), _ptr(next_t),
+              _ptr(t_out), _ptr(out), T, B, xt.numel() // B, *g, _stream())
     return out
 
 
@@ -833,35 +867,52 @@ def field_normal(seed: int, field_ids: torch.Tensor, draw: int, shape=None, out:
     return out
 
 
-def p_sample_seeded(xt, eps, seed: int, field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out=None):
+def p_sample_seeded(xt, eps, seed: int, field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out=None,
+                    guidance: Optional[float] = None):
     """p_sample with z = field_normal(seed, field_ids, draw=t[b]) drawn inside the kernel (no z buffer), bit-identical
-    to p_sample fed that draw.  `out` may be `xt` (in place).  A t outside [0, T) gives NaN."""
+    to p_sample fed that draw.  `out` may be `xt` (in place).  A t outside [0, T) gives NaN.  `guidance` as in
+    p_sample: the noise is drawn for the B fields only."""
     lo, hi = split_seed(seed)
     _req_cuda(xt, eps, field_ids, t, betas, sqrt_1mac, sqrt_recip_a, post_var, out)
-    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32
+    suffix, g = _net_rows(xt, eps, guidance)
     out = torch.empty_like(xt) if out is None else out
     assert out.dtype == torch.float32 and out.shape == xt.shape
     B = xt.shape[0]
     _seeded_ids(field_ids, B)
-    _lib.call("cesm_p_sample_seeded", _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(betas),
-              _ptr(sqrt_1mac), _ptr(sqrt_recip_a), _ptr(post_var), _ptr(out), betas.shape[0], B, xt.numel() // B,
+    _lib.call("cesm_p_sample_seeded" + suffix, _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(betas),
+              _ptr(sqrt_1mac), _ptr(sqrt_recip_a), _ptr(post_var), _ptr(out), betas.shape[0], B, xt.numel() // B, *g,
               _stream())
     return out
 
 
-def ddim_step_seeded(xt, eps, seed: int, field_ids, t, coef, T: int, out=None, next_t=None, t_out=None):
+def ddim_step_seeded(xt, eps, seed: int, field_ids, t, coef, T: int, out=None, next_t=None, t_out=None,
+                     guidance: Optional[float] = None):
     """ddim_step with z = field_normal(seed, field_ids, draw=t[b]) drawn inside the kernel (no z buffer),
-    bit-identical to ddim_step fed that draw.  Same `out` / `next_t` / `t_out` contract as ddim_step."""
+    bit-identical to ddim_step fed that draw.  Same `out` / `next_t` / `t_out` contract as ddim_step.  `guidance` as
+    in p_sample: the noise is drawn for the B fields only."""
     lo, hi = split_seed(seed)
     _req_cuda(xt, eps, field_ids, t, coef, out, next_t, t_out)
     assert coef.dtype == torch.float32 and coef.shape == (T, 3), (coef.dtype, tuple(coef.shape), T)
-    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32 and eps.shape == xt.shape
+    assert t.dtype == torch.int64 and xt.dtype == eps.dtype == torch.float32
+    suffix, g = _net_rows(xt, eps, guidance)
     assert (t_out is None) == (next_t is None), "next_t and t_out go together"
     assert next_t is None or (next_t.dtype == torch.int64 and next_t.shape == (T,) and t_out.dtype == torch.int64)
     out = torch.empty_like(xt) if out is None else out
     assert out.dtype == torch.float32 and out.shape == xt.shape
     B = xt.shape[0]
     _seeded_ids(field_ids, B)
-    _lib.call("cesm_ddim_step_seeded", _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(coef),
-              _ptr(next_t), _ptr(t_out), _ptr(out), T, B, xt.numel() // B, _stream())
+    _lib.call("cesm_ddim_step_seeded" + suffix, _ptr(xt), _ptr(eps), lo, hi, _ptr(field_ids), _ptr(t), _ptr(coef),
+              _ptr(next_t), _ptr(t_out), _ptr(out), T, B, xt.numel() // B, *g, _stream())
     return out
+
+
+def cond_keep(seed: int, step: torch.Tensor, first: int, p: float, keep: torch.Tensor) -> torch.Tensor:
+    """Condition-dropout mask of one training step into `keep` (fp32 [B]): keep[b] = 0 with probability p, drawn from
+    (seed, *step, global sample index first + b) by counter-based Philox (cesm_cond_keep), then *step += 1 on the
+    device.  `step` is an int64 device scalar; a replayed CUDA graph advances it."""
+    lo, hi = split_seed(seed)
+    _req_cuda(step, keep)
+    assert step.dtype == torch.int64 and step.numel() == 1 and keep.dtype == torch.float32 and keep.dim() == 1
+    _lib.call("cesm_cond_keep", lo, hi, _ptr(step), int(first), float(p), _ptr(keep), keep.shape[0], _stream())
+    return keep

@@ -36,12 +36,14 @@ class UNet(nn.Module):
             init_kernel_size=init_kernel_size, resnet_groups=groups, use_checkpoint=use_checkpoint,
             use_temp_attn=use_temp_attn, day_cond=day_cond, year_cond=year_cond, cond_map=cond_map)
 
-    def forward(self, x_t, cond, t):
+    def forward(self, x_t, cond, t, cond_keep=None):
         """x_t: [B,1,H,W] or [B,1,F,H,W]; cond: [B,1,H,W] or [B,1,F,H,W]; t: [B] -> [B,1,H,W].
 
         The reference expands the single-frame side to F frames, runs the 3-D net on all frames
         and keeps frame F//2 (model.py:110-130).  Here the broadcast happens inside the input-conv
-        kernel and the 1x1x1 output conv is evaluated for the centre frame only."""
+        kernel and the 1x1x1 output conv is evaluated for the centre frame only.  `cond_keep` (fp32 [B] of 0 / 1,
+        optional, an addition beyond the reference): sample b sees the null (all-zero) condition where
+        cond_keep[b] == 0, without a masked copy of cond."""
         if x_t.ndim == 4:
             x_t = x_t.unsqueeze(2)
         elif x_t.ndim != 5:
@@ -56,7 +58,11 @@ class UNet(nn.Module):
         if Fx != Fc and not (Fx == 1 or Fc == 1):
             raise ValueError(f"Frame mismatch: x_t F={Fx}, cond F={Fc}")
         F = max(Fx, Fc)
-        out = self.net.forward_frames(x_t, t, cond, frames=[F // 2])
+        if cond_keep is not None:
+            if not torch.is_tensor(cond_keep) or tuple(cond_keep.shape) != (x_t.shape[0],):
+                raise ValueError(f"cond_keep must be a tensor of shape ({x_t.shape[0]},)")
+            cond_keep = cond_keep.float().contiguous()
+        out = self.net.forward_frames(x_t, t, cond, frames=[F // 2], cond_keep=cond_keep)
         return out.squeeze(2)
 
 
@@ -69,6 +75,28 @@ def check_prediction_type(prediction_type) -> str:
     if not isinstance(prediction_type, str) or prediction_type not in PREDICTION_TYPES:
         raise ValueError(f"prediction_type must be one of {PREDICTION_TYPES}, got {prediction_type!r}")
     return prediction_type
+
+
+def check_guidance(guidance) -> float:
+    """Classifier-free guidance weight w (Ho & Salimans, "Classifier-Free Diffusion Guidance"): a finite real number
+    >= 0 (an int is accepted, a bool is not).  0 is unguided sampling; w > 0 samples with (1 + w) out_cond - w out_null,
+    which needs a network trained with condition dropout (`TrainEngine(cond_drop_prob=...)`)."""
+    if isinstance(guidance, bool) or not isinstance(guidance, numbers.Real):
+        raise ValueError(f"guidance must be a real number >= 0, got {guidance!r}")
+    guidance = float(guidance)
+    if not (math.isfinite(guidance) and guidance >= 0):
+        raise ValueError(f"guidance must be finite and >= 0, got {guidance}")
+    return guidance
+
+
+def check_cond_drop_prob(p) -> float:
+    """Condition-dropout probability of training for classifier-free guidance: a real number in [0, 1); 0 is off."""
+    if isinstance(p, bool) or not isinstance(p, numbers.Real):
+        raise ValueError(f"cond_drop_prob must be a real number in [0, 1), got {p!r}")
+    p = float(p)
+    if not 0.0 <= p < 1.0:  # also rejects NaN
+        raise ValueError(f"cond_drop_prob must be in [0, 1), got {p}")
+    return p
 
 
 def ddim_schedule(alphas_cumprod: torch.Tensor, steps: int, eta: float = 0.0, prediction_type: str = "eps"):
@@ -184,7 +212,13 @@ class Diffusion(nn.Module):
     reference's noise target, or "v" = sqrt(ab) eps - sqrt(1 - ab) x0, from which x0 = sqrt(ab) x_t - sqrt(1 - ab) v
     carries no 1 / sqrt(ab) amplification (157 at t = 999 on the linear schedule).  A v-model samples with every chain
     of the eps-model through coefficient tables that fold the conversion in (ddim_schedule, dpm_schedule).  Its
-    tables are non-persistent buffers: state_dict() and checkpoints are the same for both targets."""
+    tables are non-persistent buffers: state_dict() and checkpoints are the same for both targets.
+
+    Classifier-free guidance (an addition beyond the reference): `loss(..., keep=)` trains sample b with the null
+    condition where keep[b] == 0, and every sampler takes `guidance=w`.  The null condition is the all-zero window --
+    the dataset-mean emission map in normalised units -- so guidance adds no parameter.  With w > 0 each reverse step
+    makes one UNet call on 2B rows (the fields with their conditions, then with the null condition) and the update
+    kernel combines the two halves (kernels.ddim_step etc. with `guidance`)."""
 
     def __init__(self, model, img_channels=1, timesteps=1000, beta_schedule="linear", *, prediction_type="eps"):
         super().__init__()
@@ -234,20 +268,27 @@ class Diffusion(nn.Module):
         return w.float()
 
     # -- sampling ------------------------------------------------------------------------------
-    def p_sample(self, x_t, cond, t, noise=None):
+    def _net(self, x, cond, t, guidance):
+        """The network output a sampler step consumes: [B] rows, or with guidance w > 0 one call on 2B rows -- x with
+        cond, then x with the null condition -- which the guided update kernels combine.  -> (output, w or None)."""
+        if not guidance:
+            return self.model(x, cond, t), None
+        return self.model(torch.cat([x, x]), torch.cat([cond, torch.zeros_like(cond)]), torch.cat([t, t])), guidance
+
+    def p_sample(self, x_t, cond, t, noise=None, *, guidance=0.0):
         """model.py:168-183.  One reverse step.  posterior_variance[0] == 0, so the reference's
         `(t == 0).all()` branch (a host sync per step) is the same arithmetic as always adding
         sqrt(var_t) * z; the fused kernel does that without the sync.  `noise` may be supplied
-        for deterministic parity tests."""
+        for deterministic parity tests.  `guidance` as in `sample`."""
         with torch.no_grad():
-            eps_theta = self.model(x_t, cond, t)
+            eps_theta, w = self._net(x_t, cond, t, check_guidance(guidance))
             z = torch.randn_like(x_t) if noise is None else noise
             if self.prediction_type == "v":  # eps_theta is v: the posterior step through the folded table
                 return K.ddim_step(x_t.float().contiguous(), eps_theta, z.float().contiguous(), t.contiguous(),
-                                   self.ddpm_coef, self.T)
+                                   self.ddpm_coef, self.T, guidance=w)
             return K.p_sample(x_t.float().contiguous(), eps_theta, z.float().contiguous(), t.contiguous(),
                               self.betas, self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
-                              self.posterior_variance)
+                              self.posterior_variance, guidance=w)
 
     def _x_T(self, shape, device, seed, field_ids):
         """Initial noise: torch's CUDA generator without a seed; with one, the counter-based draw of each field id
@@ -260,30 +301,35 @@ class Diffusion(nn.Module):
         ids = K.field_id_vector(field_ids, shape[0], device)
         return K.field_normal(seed, ids, K.X_T_DRAW, shape), ids
 
-    def sample(self, cond, shape, device, *, seed=None, field_ids=None):
+    def sample(self, cond, shape, device, *, seed=None, field_ids=None, guidance=0.0):
         """model.py:186-194.  With `seed` (an int in [0, 2^64)) every field's noise is drawn from (seed, its id in
-        `field_ids`, default arange(B)) instead of torch's generator, so a field does not depend on its row or batch."""
+        `field_ids`, default arange(B)) instead of torch's generator, so a field does not depend on its row or batch.
+        `guidance` (w >= 0, `check_guidance`): w > 0 samples with classifier-free guidance, (1 + w) out_cond - w
+        out_null in the network's output space, from one UNet call on 2B rows per step; 0 is the unguided chain."""
+        guidance = check_guidance(guidance)
         with torch.no_grad():
             B = shape[0]
             x, ids = self._x_T(shape, device, seed, field_ids)
             for tt in reversed(range(self.T)):
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
                 if ids is None:
-                    x = self.p_sample(x, cond, t_tensor)
+                    x = self.p_sample(x, cond, t_tensor, guidance=guidance)
                     continue
-                eps_theta = self.model(x, cond, t_tensor)
+                eps_theta, w = self._net(x, cond, t_tensor, guidance)
                 if self.prediction_type == "v":
                     x = K.ddim_step_seeded(x.float().contiguous(), eps_theta, seed, ids, t_tensor, self.ddpm_coef,
-                                           self.T)
+                                           self.T, guidance=w)
                     continue
                 x = K.p_sample_seeded(x.float().contiguous(), eps_theta, seed, ids, t_tensor, self.betas,
                                       self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
-                                      self.posterior_variance)
+                                      self.posterior_variance, guidance=w)
             return x
 
-    def ddim_sample(self, cond, shape, device, steps=50, eta=0.0, *, seed=None, field_ids=None):
+    def ddim_sample(self, cond, shape, device, steps=50, eta=0.0, *, seed=None, field_ids=None, guidance=0.0):
         """Strided DDIM chain of `steps` UNet calls (ddim_schedule), eager; an addition beyond the reference.
-        Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T.  `seed` / `field_ids` as in `sample`."""
+        Fewer steps trade fidelity for speed; eta = 0 draws no noise after x_T.  `seed` / `field_ids` / `guidance`
+        as in `sample`."""
+        guidance = check_guidance(guidance)
         taus, coef, _ = ddim_schedule(self.alphas_cumprod, steps, eta, self.prediction_type)
         coef = coef.to(device)
         with torch.no_grad():
@@ -291,18 +337,19 @@ class Diffusion(nn.Module):
             x, ids = self._x_T(shape, device, seed, field_ids)
             for tt in taus:
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
-                eps_theta = self.model(x, cond, t_tensor)
+                eps_theta, w = self._net(x, cond, t_tensor, guidance)
                 if ids is not None and eta > 0:
-                    x = K.ddim_step_seeded(x, eps_theta, seed, ids, t_tensor, coef, self.T)
+                    x = K.ddim_step_seeded(x, eps_theta, seed, ids, t_tensor, coef, self.T, guidance=w)
                     continue
                 z = torch.randn_like(x) if eta > 0 else None
-                x = K.ddim_step(x, eps_theta, z, t_tensor, coef, self.T)
+                x = K.ddim_step(x, eps_theta, z, t_tensor, coef, self.T, guidance=w)
             return x
 
-    def dpm_sample(self, cond, shape, device, steps=20, *, seed=None, field_ids=None):
+    def dpm_sample(self, cond, shape, device, steps=20, *, seed=None, field_ids=None, guidance=0.0):
         """DPM-Solver++(2M) chain of `steps` UNet calls (dpm_schedule), eager; an addition beyond the reference.
         Deterministic after x_T.  `hist` carries the previous step's x0 prediction; the first step does not read it.
-        `seed` / `field_ids` as in `sample` (only x_T is random)."""
+        `seed` / `field_ids` / `guidance` as in `sample` (only x_T is random)."""
+        guidance = check_guidance(guidance)
         taus, coef, _ = dpm_schedule(self.alphas_cumprod, steps, self.prediction_type)
         coef = coef.to(device)
         with torch.no_grad():
@@ -311,8 +358,8 @@ class Diffusion(nn.Module):
             hist = torch.empty_like(x)
             for tt in taus:
                 t_tensor = torch.full((B,), tt, device=device, dtype=torch.long)
-                eps_theta = self.model(x, cond, t_tensor)
-                x = K.dpm_step(x, eps_theta, hist, t_tensor, coef, self.T)
+                eps_theta, w = self._net(x, cond, t_tensor, guidance)
+                x = K.dpm_step(x, eps_theta, hist, t_tensor, coef, self.T, guidance=w)
             return x
 
     # -- training ------------------------------------------------------------------------------
@@ -324,19 +371,20 @@ class Diffusion(nn.Module):
                                   self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod)
         return x_t, noise
 
-    def loss(self, x0, cond, t=None, noise=None, weights=None):
+    def loss(self, x0, cond, t=None, noise=None, weights=None, keep=None):
         """model.py:203-208.  `t` / `noise` default to the reference's draws (randint, then
         randn_like); passing them makes parity tests deterministic.  `weights` (fp32 [T], e.g. `min_snr_weights`)
         weights each sample's squared error by weights[t]; the loss is sum_b weights[t_b] sum_pixels err^2 / numel.
         With the eps target and no weights this is the reference's MSE (ops.MseLossFn); otherwise the fused
-        objective (ops.DiffusionLossFn) computes the target and the weighting."""
+        objective (ops.DiffusionLossFn) computes the target and the weighting.  `keep` (fp32 [B] of 0 / 1, optional):
+        condition dropout -- sample b is trained on the null condition where keep[b] == 0, and its cond gradient is 0."""
         if weights is not None and (not torch.is_tensor(weights) or tuple(weights.shape) != (self.T,)):
             raise ValueError(f"weights must be a tensor of shape ({self.T},)")
         B = x0.size(0)
         if t is None:
             t = torch.randint(0, self.T, (B,), device=x0.device).long()
         x_t, noise = self.q_sample(x0, t, noise)
-        eps_pred = self.model(x_t, cond, t)
+        eps_pred = self.model(x_t, cond, t) if keep is None else self.model(x_t, cond, t, cond_keep=keep)
         if self.prediction_type == "eps" and weights is None:
             return ops.MseLossFn.apply(eps_pred, noise.float())
         w = None if weights is None else weights.float().contiguous()

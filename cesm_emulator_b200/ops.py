@@ -902,28 +902,30 @@ class SpatialAttnBlockFn(_Fn):
 # ------------------------------------------------------------------------------------------------
 class InputConvFn(_Fn):
     """cat([x, cond_map], dim=1) -> Conv3d(2, C, (1,k,k)) with frame broadcast folded in
-    (video_net.py:808-815, model.py:110-121).  x/cond: fp32 [B,1,Fx,H,W]; out: fp16 [B*F,H,W,C]."""
+    (video_net.py:808-815, model.py:110-121).  x/cond: fp32 [B,1,Fx,H,W]; out: fp16 [B*F,H,W,C].  `keep` (fp32 [B]
+    of 0 / 1, or None): batch element b sees the null (all-zero) condition where keep[b] == 0, in the forward, the
+    weight gradient and the condition's gradient (classifier-free guidance's condition dropout)."""
 
     @staticmethod
-    def forward(ctx, x, cond, weight, bias, F: int):
+    def forward(ctx, x, cond, weight, bias, F: int, keep=None):
         """Tensor-core path: fp16 (hi, lo) im2col patches x [w | w | bias] through the tcgen05 implicit GEMM
         (kernels.input_patches / input_weight_pack); the patches are kept for the weight gradient."""
         shapes = (x.shape, cond.shape)
         x, cond = x.contiguous().float(), cond.contiguous().float()
         B, H, W = x.shape[0], x.shape[-2], x.shape[-1]
         ks = weight.shape[-1]
-        patches = K.input_patches(x, cond, B, F, H, W, ks)
+        patches = K.input_patches(x, cond, B, F, H, W, ks, keep=keep)
         out = K.igemm(patches, K.input_weight_pack(weight.detach(), bias.detach()))
         if _train(ctx):
             # the patches serve the weight gradient only
             need_w = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
-            ctx.save_for_backward(patches if need_w else None, weight, bias)
+            ctx.save_for_backward(patches if need_w else None, weight, bias, keep)
             ctx.dims = (B, F, H, W, x.numel() // (B * H * W), cond.numel() // (B * H * W), shapes)
         return out
 
     @staticmethod
     def backward(ctx, dy):
-        patches, weight, bias = ctx.saved_tensors
+        patches, weight, bias, keep = ctx.saved_tensors
         B, F, H, W, f0, f1, shapes = ctx.dims
         ks = weight.shape[-1]
         dy = dy.contiguous()
@@ -932,14 +934,15 @@ class InputConvFn(_Fn):
         sink = _COND_GRAD_SINK[0] if need_c else None
         if sink is not None:  # scale * d cond added into the sink's buffer; autograd gets none
             K.input_conv_dgrad(dy, weight.detach(), B, F, H, W, ks, f0, f1, need_x=False, dcond_out=sink[0],
-                               scale=sink[1], accumulate=True)
+                               scale=sink[1], accumulate=True, keep=keep)
             need_c = False
         if need_x or need_c:
-            dx, dcond = K.input_conv_dgrad(dy, weight.detach(), B, F, H, W, ks, f0, f1, need_x=need_x, need_cond=need_c)
+            dx, dcond = K.input_conv_dgrad(dy, weight.detach(), B, F, H, W, ks, f0, f1, need_x=need_x, need_cond=need_c,
+                                           keep=keep)
             dx = None if dx is None else dx.view(shapes[0])
             dcond = None if dcond is None else dcond.view(shapes[1])
         if not (ctx.needs_input_grad[2] or ctx.needs_input_grad[3]):
-            return dx, dcond, None, None, None
+            return dx, dcond, None, None, None, None
         nt = weight[0].numel()  # 2 * ks * ks
         full = K.wgrad(patches, dy)[:, 0, :]                       # fp32 [cout, KPAD]
         dw = (full[:, :nt] + full[:, nt:2 * nt]).view_as(weight)   # hi and lo column blocks see the same dy
@@ -948,8 +951,8 @@ class InputConvFn(_Fn):
             weight.grad.add_(dw)
             bias.grad.add_(db)
             _ready(weight, bias)
-            return dx, dcond, None, None, None
-        return dx, dcond, dw, db.contiguous(), None
+            return dx, dcond, None, None, None, None
+        return dx, dcond, dw, db.contiguous(), None, None
 
 
 class OutConvFn(_Fn):

@@ -550,11 +550,12 @@ class UNetModel3D(nn.Module):
         return t
 
     def forward_frames(self, x, timesteps, cond_map, days=None, years=None, focus_present_mask=None,
-                       prob_focus_present=0, frames=None):
+                       prob_focus_present=0, frames=None, cond_keep=None):
         """The network pass.  x: fp32 [B, 1, Fx, H, W] and cond_map: [B, 1, Fc, H, W] with
         Fx, Fc in {1, F} (a single frame is broadcast inside the input-conv kernel instead of
         being expanded, model.py:110-118).  Returns fp32 [B, 1, len(frames), H, W] for the
-        requested output frames (default: all F)."""
+        requested output frames (default: all F).  `cond_keep` (fp32 [B] of 0 / 1, optional): sample b's
+        cond_map is read as zeros where cond_keep[b] == 0 (ops.InputConvFn)."""
         if self.n_vars != 1 or cond_map is None:
             raise NotImplementedError("the B200 input/output conv kernels cover n_vars=1 with a cond_map "
                                       "(the only configuration model.UNet builds)")
@@ -574,7 +575,7 @@ class UNetModel3D(nn.Module):
             # prob 0 -> all-False mask -> the mask branches are never taken (video_net.py:405,433)
         akw = dict(pos_bias=pos_bias, focus_present_mask=focus_present_mask)
 
-        x = ops.InputConvFn.apply(x, cond_map, self.input_conv.weight, self.input_conv.bias, F)
+        x = ops.InputConvFn.apply(x, cond_map, self.input_conv.weight, self.input_conv.bias, F, cond_keep)
         x = self.input_temp_op.forward_cl(x, B, F, pos_bias=pos_bias)
         r = x
         t = self._time_embedding(timesteps, days, years)

@@ -333,6 +333,11 @@ int cesm_gather_windows(const float* cond, const float* tgt, const int* plan, fl
  * blocks.  ks = 7, kpad = 256. */
 int cesm_input_patches(const float* in0, const float* in1, int f0, int f1, void* out, int B, int F, int H, int W,
                        int ks, int kpad, void* stream);
+/* cesm_input_patches with condition dropout: keep is an fp32 [B] device vector (NULL: keep all), and batch element b
+ * reads its in1 plane as zeros where keep[b] == 0.  The GEMM and the weight gradient over these patches then see the
+ * null condition; no masked copy of in1 is made. */
+int cesm_input_patches_masked(const float* in0, const float* in1, int f0, int f1, const float* keep, void* out, int B,
+                              int F, int H, int W, int ks, int kpad, void* stream);
 int cesm_input_weight_pack(const float* w, const float* bias, void* out, int cout, int ks, int kpad, void* stream);
 int cesm_input_conv_fwd(const float* in0, const float* in1, int f0, int f1, const float* w, const float* bias,
                         void* out, int B, int F, int H, int W, int ks, int cout, void* stream);
@@ -345,6 +350,11 @@ int cesm_input_conv_wgrad(const float* in0, const float* in1, int f0, int f1, co
  * NULL (not requested), not both.  ks = 7, cout = 64, B <= 65535. */
 int cesm_input_conv_dgrad(const void* dy, const float* w, float* d_in0, float* d_in1, int f0, int f1, int B, int F,
                           int H, int W, int ks, int cout, float scale, int accumulate, void* stream);
+/* cesm_input_conv_dgrad of a forward made with cesm_input_patches_masked: where keep[b] == 0, d_in1 of batch element
+ * b is 0 (written as 0, or nothing added with `accumulate`).  keep NULL: cesm_input_conv_dgrad. */
+int cesm_input_conv_dgrad_masked(const void* dy, const float* w, float* d_in0, float* d_in1, const float* keep, int f0,
+                                 int f1, int B, int F, int H, int W, int ks, int cout, float scale, int accumulate,
+                                 void* stream);
 int cesm_out_conv_fwd(const void* a, const float* w, const float* bias, float* eps, int B, int F, int mid,
                       long long HW, int C, void* stream);
 int cesm_out_conv_bwd(const void* a, const float* w, const float* deps, void* da, float* dw, float* db, int B, int F,
@@ -405,6 +415,20 @@ int cesm_ddim_step(const float* xt, const float* eps, const float* z, const long
 int cesm_dpm_step(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
                   const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
                   void* stream);
+/* Classifier-free guidance.  The *_guided steps take eps with 2B rows of per_sample floats: rows [0, B) are the
+ * network's predictions with the fields' conditions, rows [B, 2B) its predictions for the same fields with the null
+ * (all-zero) condition.  They update the B fields with c + guidance * (c - u) = (1 + w) c - w u, element by element,
+ * in place of eps, in the network's own output space (eps or v); nothing else changes.  guidance must be finite and
+ * > 0 (CESM_ERR_INVALID otherwise); w = 0 is the unguided entry point. */
+int cesm_p_sample_guided(const float* xt, const float* eps, const float* z, const long long* t, const float* betas,
+                         const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out, int B,
+                         long long per_sample, float guidance, void* stream);
+int cesm_ddim_step_guided(const float* xt, const float* eps, const float* z, const long long* t, const float* coef,
+                          const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                          float guidance, void* stream);
+int cesm_dpm_step_guided(const float* xt, const float* eps, float* hist, const long long* t, const float* coef,
+                         const long long* next_t, long long* t_out, float* out, int T, int B, long long per_sample,
+                         float guidance, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Seeded sampling noise.  Element e of field f in draw d is word e & 3 of Philox4x32-10 with counter
@@ -429,6 +453,23 @@ int cesm_p_sample_seeded(const float* xt, const float* eps, unsigned seed_lo, un
 int cesm_ddim_step_seeded(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
                           const long long* field_ids, const long long* t, const float* coef, const long long* next_t,
                           long long* t_out, float* out, int T, int B, long long per_sample, void* stream);
+/* The seeded steps with classifier-free guidance (eps with 2B rows, as cesm_ddim_step_guided).  The noise is drawn for
+ * the B fields only, by field id, so a guided field does not depend on its row or batch either. */
+int cesm_p_sample_seeded_guided(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                const long long* field_ids, const long long* t, const float* betas,
+                                const float* sqrt_1mac, const float* sqrt_recip_a, const float* post_var, float* out,
+                                int T, int B, long long per_sample, float guidance, void* stream);
+int cesm_ddim_step_seeded_guided(const float* xt, const float* eps, unsigned seed_lo, unsigned seed_hi,
+                                 const long long* field_ids, const long long* t, const float* coef,
+                                 const long long* next_t, long long* t_out, float* out, int T, int B,
+                                 long long per_sample, float guidance, void* stream);
+/* Condition dropout of a training step: keep[b] = 1 if u >= p else 0, with u = ((w0 >> 9) + 0.5) * 2^-23 from word 0
+ * of Philox4x32-10 with counter (g_lo, g_hi, s_lo, s_hi) and key (seed_lo, seed_hi), g = first + b the sample's index
+ * in the global batch and s = *step (an int64 device counter); then *step += 1.  The masks depend on (seed, step, g)
+ * only: the same for a global batch on one GPU or split over ranks.  Rejects B < 1, first < 0, p outside [0, 1) and
+ * NULL pointers with CESM_ERR_INVALID. */
+int cesm_cond_keep(unsigned seed_lo, unsigned seed_hi, long long* step, long long first, float p, float* keep, int B,
+                   void* stream);
 
 #ifdef __cplusplus
 }

@@ -6,6 +6,7 @@
     python inference.py --ckpt ... --dpm_steps 15                  # DPM-Solver++(2M) chain: 15 UNet calls per field
     python inference.py --ckpt ... --ema [--dpm_steps 15]          # sample from the weight EMA (ckpt["ema"])
     python inference.py --ckpt ... --seed 7                        # counter-based noise: same fields on any world size
+    python inference.py --ckpt ... --guidance 2 [--dpm_steps 15]   # classifier-free guidance (needs train.cond_drop_prob)
     torchrun --standalone --nproc_per_node=8 inference.py --ckpt ...
 
 `predict_temperature_from_emissions` keeps the reference's flow: rebuild UNet/Diffusion from
@@ -27,7 +28,20 @@ import torch.distributed as dist
 from cesm_emulator_b200.engine import SampleEngine
 from cesm_emulator_b200.model import Diffusion
 from cesm_emulator_b200.synthetic import SyntheticEnsemble
-from train import build_model_from_config, prediction_type_from_config
+from train import build_model_from_config, cond_drop_prob_from_config, prediction_type_from_config
+
+
+def check_guidance_for_config(guidance, cfg) -> float:
+    """Validated guidance weight for a checkpoint with config `cfg`: w >= 0 (model.check_guidance), and w > 0 only if
+    the run trained with condition dropout (train.cond_drop_prob > 0) -- otherwise the network never saw the null
+    condition and its unconditional prediction means nothing."""
+    from cesm_emulator_b200.model import check_guidance
+    w = check_guidance(guidance)
+    p = cond_drop_prob_from_config(cfg)
+    if w > 0 and not (isinstance(p, (int, float)) and not isinstance(p, bool) and p > 0):
+        raise ValueError(f"guidance {w} needs a checkpoint trained with train.cond_drop_prob > 0 (this one has "
+                         f"{p!r}): its network has never seen the null condition")
+    return w
 
 
 def load_diffusion_from_checkpoint(path, device, ema=False):
@@ -53,7 +67,8 @@ def load_diffusion_from_checkpoint(path, device, ema=False):
 
 @torch.no_grad()
 def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_size=16, steps=None, rank=0, world=1,
-                                       device="cuda", ddim_steps=None, eta=0.0, dpm_steps=None, seed=None):
+                                       device="cuda", ddim_steps=None, eta=0.0, dpm_steps=None, seed=None,
+                                       guidance=0.0):
     """cond (T, M, 1, H, W) -> prediction (T, M, H, W); fields are independent and sharded over ranks.
     `ddim_steps=N` generates with the strided DDIM chain (N UNet calls per field, noise scaled by `eta`) instead of
     the full DDPM chain; it cannot be combined with `steps`.  `dpm_steps=N` generates with the deterministic
@@ -62,7 +77,10 @@ def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_
     With `seed` (an int in [0, 2^64)) the noise of (year index t, member m) is drawn from the field id (t << 32) | m,
     so the prediction does not depend on `batch_size`, on the number of ranks or on --times / --members, up to
     run-to-run rounding.  Without it every rank draws from torch's CUDA generator, whose default seed is the same on
-    every process."""
+    every process.
+
+    `guidance` = w > 0 samples every field with classifier-free guidance of weight w (SampleEngine(guidance=w)): each
+    step is one UNet call on twice the batch; seeded fields stay independent of batch size and rank count."""
     if ddim_steps is not None and steps is not None:
         raise ValueError("steps and ddim_steps are mutually exclusive")
     if dpm_steps is not None and (steps is not None or ddim_steps is not None):
@@ -84,7 +102,7 @@ def predict_temperature_from_emissions(diffusion, cond_tm1hw: np.ndarray, batch_
             c = torch.cat([c, c[-1:].expand(batch_size - c.shape[0], -1, -1, -1)], 0)
         if eng is None:
             eng = SampleEngine(diffusion, (batch_size, 1, H, W), ddim_steps=ddim_steps, eta=eta, dpm_steps=dpm_steps,
-                               seed=seed)
+                               seed=seed, guidance=guidance)
         ids = None
         if seed is not None:  # padding rows repeat the last real field
             ids = [((k // M) << 32) | (k % M) for k in sel]
@@ -148,6 +166,9 @@ def _parse_args(argv=None):
     ap.add_argument("--seed", type=int, default=None,
                     help="draw every field's noise from (seed, year, member), in [0, 2**64): the output then does not "
                          "depend on --batch_size or the number of GPUs")
+    ap.add_argument("--guidance", type=float, default=0.0,
+                    help="classifier-free guidance weight w >= 0: sample with (1 + w) out_cond - w out_null (0 = off); "
+                         "needs a checkpoint trained with train.cond_drop_prob > 0")
     ap.add_argument("--members", type=int, default=2)
     ap.add_argument("--times", type=int, default=4)
     ap.add_argument("--out", default="pred.npy")
@@ -160,6 +181,8 @@ def _parse_args(argv=None):
         ap.error("--eta applies to --ddim_steps only; --dpm_steps is deterministic")
     if a.seed is not None and not 0 <= a.seed < 1 << 64:
         ap.error(f"--seed must be in [0, 2**64), got {a.seed}")
+    if not a.guidance >= 0 or a.guidance == float("inf"):  # also rejects NaN
+        ap.error(f"--guidance must be a finite number >= 0, got {a.guidance}")
     return a
 
 
@@ -174,13 +197,15 @@ def _cli():
         dist.init_process_group("nccl", device_id=dev)
     try:
         diffusion, cfg = load_diffusion_from_checkpoint(a.ckpt, dev, ema=a.ema)
-    except KeyError as e:
+        guidance = check_guidance_for_config(a.guidance, cfg)
+    except (KeyError, ValueError) as e:
         raise SystemExit(f"inference.py: error: {e.args[0]}")
     syn = cfg.get("data", {}).get("synthetic", {})
     ds = SyntheticEnsemble(members=a.members, times=a.times, lat=syn.get("lat", 192), lon=syn.get("lon", 288),
                            seed=syn.get("seed", 1234))
     pred = predict_temperature_from_emissions(diffusion, ds.cond, a.batch_size, a.steps, rank, world, dev,
-                                              ddim_steps=a.ddim_steps, eta=a.eta, dpm_steps=a.dpm_steps, seed=a.seed)
+                                              ddim_steps=a.ddim_steps, eta=a.eta, dpm_steps=a.dpm_steps, seed=a.seed,
+                                              guidance=guidance)
     if rank == 0:
         if a.out.endswith(".nc"):
             write_prediction_netcdf(a.out, pred, attrs={"checkpoint": os.path.abspath(a.ckpt), "cond_var": "synthetic"})

@@ -68,6 +68,13 @@ def prediction_type_from_config(cfg: dict) -> str:
     return (cfg or {}).get("diffusion", {}).get("prediction_type", "eps")
 
 
+def cond_drop_prob_from_config(cfg: dict) -> float:
+    """train.cond_drop_prob of a run's config (or a checkpoint's "config"): the condition-dropout probability it trained
+    with for classifier-free guidance; absent means 0 (never trained on the null condition)."""
+    p = (cfg or {}).get("train", {}).get("cond_drop_prob")
+    return 0.0 if p is None else p
+
+
 def load_checkpoint(path, diffusion, engine=None, device="cuda"):
     """train.py:915-946 semantics: strict=False on the UNet, buffers merged, start_epoch = epoch + 1.  An engine with a
     weight EMA loads the checkpoint's "ema", or restarts the EMA from the loaded weights if it has none.  A checkpoint
@@ -115,7 +122,8 @@ def main(cfg):
     engine = TrainEngine(diffusion, (B, 1, h, w), (B, 1, K, h, w), lr=opt.get("lr", 2e-4),
                          betas=tuple(opt.get("betas", (0.9, 0.999))), weight_decay=opt.get("weight_decay", 1e-4),
                          max_grad_norm=tcfg.get("max_grad_norm", 1.0), ema_decay=tcfg.get("ema_decay"),
-                         ema_start=tcfg.get("ema_start", 0), min_snr_gamma=tcfg.get("min_snr_gamma"))
+                         ema_start=tcfg.get("ema_start", 0), min_snr_gamma=tcfg.get("min_snr_gamma"),
+                         cond_drop_prob=cond_drop_prob_from_config(cfg))
     start = 1
     if tcfg.get("resume") and os.path.exists(tcfg["resume"]):
         start = load_checkpoint(tcfg["resume"], diffusion, engine, dev)

@@ -165,6 +165,7 @@ _SIGNATURES: dict[str, list] = {
     "cesm_p_sample_seeded_guided": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
     "cesm_ddim_step_seeded_guided": [_P, _P, _U, _U, _P, _P, _P, _P, _P, _P, _I, _I, _L, _F, _P],
     "cesm_cond_keep": [_U, _U, _P, _L, _F, _P, _I, _P],
+    "cesm_ensemble_scores": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _L, _P],
 }
 
 

@@ -916,3 +916,39 @@ def cond_keep(seed: int, step: torch.Tensor, first: int, p: float, keep: torch.T
     assert step.dtype == torch.int64 and step.numel() == 1 and keep.dtype == torch.float32 and keep.dim() == 1
     _lib.call("cesm_cond_keep", lo, hi, _ptr(step), int(first), float(p), _ptr(keep), keep.shape[0], _stream())
     return keep
+
+
+# ---- ensemble scores ------------------------------------------------------------------------------
+SCORE_MAPS = ("crps", "bias", "sd_pred", "sd_target", "mse_mean")
+SCORE_MAX_MEMBERS = 1024
+
+
+def ensemble_scores(pred: torch.Tensor, target: torch.Tensor) -> dict:
+    """Scores of the generated ensemble `pred` (fp32 [T, n, HW]) against the target ensemble `target` (fp32
+    [T, m, HW]) per (year, pixel) column, in one pass over both (cesm_ensemble_scores, include/cesm_b200.h):
+    -> {"crps", "bias", "sd_pred", "sd_target", "mse_mean": fp32 [T, HW] maps, "rank_hist": int64 [T, n + 1]}.
+    crps is the fair CRPS averaged over the target members; rank_hist bin r counts target values with exactly r
+    predicted values below them (ties are not below).  A column holding a non-finite value is NaN in every map and
+    missing from the histogram.  Bad arguments raise ValueError before anything is launched."""
+    for name, x in (("pred", pred), ("target", target)):
+        if not isinstance(x, torch.Tensor):
+            raise ValueError(f"{name} must be a tensor, got {type(x).__name__}")
+        if not x.is_cuda or x.dtype != torch.float32 or x.dim() != 3 or not x.is_contiguous():
+            raise ValueError(f"{name} must be a contiguous 3-D float32 CUDA tensor [T, members, HW], got "
+                             f"{x.dtype} {tuple(x.shape)} on {x.device}{'' if x.is_contiguous() else ', strided'}")
+    (T, n, HW), m = pred.shape, target.shape[1]
+    if target.shape[0] != T or target.shape[2] != HW:
+        raise ValueError(f"pred {tuple(pred.shape)} and target {tuple(target.shape)} must share T and HW")
+    if pred.device != target.device:
+        raise ValueError(f"pred is on {pred.device} and target on {target.device}")
+    if not (2 <= n <= SCORE_MAX_MEMBERS and 2 <= m <= SCORE_MAX_MEMBERS):
+        raise ValueError(f"ensemble scores need 2..{SCORE_MAX_MEMBERS} members on each side, got n={n} m={m}")
+    if not (1 <= T <= 65535 and HW >= 1):
+        raise ValueError(f"ensemble scores need 1 <= T <= 65535 and HW >= 1, got T={T} HW={HW}")
+    out = {k: torch.empty((T, HW), dtype=torch.float32, device=pred.device) for k in SCORE_MAPS}
+    out["rank_hist"] = torch.empty((T, n + 1), dtype=torch.int64, device=pred.device)
+    meta = _bytes_meta(pred, target, *out.values())
+    with torch.cuda.device(pred.device):
+        _lib.call("cesm_ensemble_scores", _ptr(pred), _ptr(target), *(_ptr(out[k]) for k in SCORE_MAPS),
+                  _ptr(out["rank_hist"]), T, n, m, HW, _stream(), _meta=meta)
+    return out

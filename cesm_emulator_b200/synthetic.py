@@ -47,8 +47,11 @@ class SyntheticEnsemble:
         noise = rng.standard_normal((members, times, lat, lon, 1), dtype=np.float32)
         tgt = resp[None, ..., None] * 4.0 + 0.5 * noise
         # reference layout (T, M, 1, H, W), globally z-scored (train.py:640-646)
-        self.cond = self._z(np.ascontiguousarray(np.transpose(self.cond_mtllc, (1, 0, 4, 2, 3))))
-        self.tgt = self._z(np.ascontiguousarray(np.transpose(tgt, (1, 0, 4, 2, 3))))
+        self.cond, _ = self._z(np.ascontiguousarray(np.transpose(self.cond_mtllc, (1, 0, 4, 2, 3))))
+        self.tgt, (mu, sd) = self._z(np.ascontiguousarray(np.transpose(tgt, (1, 0, 4, 2, 3))))
+        # the known truth in normalised units: member (t, m) is target_mean[t] + target_noise_std * N(0, 1) noise
+        self.target_mean = ((resp.astype(np.float64) * 4.0 - float(mu)) / float(sd)).astype(np.float32)  # (T, H, W)
+        self.target_noise_std = 0.5 / float(sd)
         self.num_units = max(1, self.T - self.K + 1)
 
     @classmethod
@@ -67,15 +70,18 @@ class SyntheticEnsemble:
         self.K, self.crop_hw, self.time_reverse_p = int(K), crop_hw, float(time_reverse_p)
         self._aug = np.random.default_rng(seed + 1)
         self.cond_mtllc = None
+        self.target_mean = self.target_noise_std = None  # unknown for arrays from outside
         self.cond = np.ascontiguousarray(cond, dtype=np.float32)
         self.tgt = np.ascontiguousarray(tgt, dtype=np.float32)
         self.num_units = max(1, self.T - self.K + 1)
         return self
 
     @staticmethod
-    def _z(a: np.ndarray) -> np.ndarray:
+    def _z(a: np.ndarray):
+        """Global z-score -> (z-scored float32 array, (mean, std + 1e-8) it applied)."""
         a = a.astype(np.float32)
-        return (a - a.mean()) / (a.std() + 1e-8)
+        mu, sd = a.mean(), a.std() + 1e-8
+        return (a - mu) / sd, (mu, sd)
 
     def __len__(self) -> int:
         return self.num_units * self.M

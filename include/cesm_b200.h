@@ -471,6 +471,23 @@ int cesm_ddim_step_seeded_guided(const float* xt, const float* eps, unsigned see
 int cesm_cond_keep(unsigned seed_lo, unsigned seed_hi, long long* step, long long first, float p, float* keep, int B,
                    void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Ensemble scores.  pred is fp32 [T][n][HW] (n generated members), target fp32 [T][m][HW] (m target members).  For
+ * each column (year t, pixel p), with X the n predicted and Y the m target values, the fp32 [T][HW] maps get
+ *   crps      = mean_j [ (1/n) sum_i |x_i - y_j| ] - 1/(n(n-1)) sum_{i<k} |x_i - x_k|   (fair CRPS, Ferro 2014)
+ *   bias      = mean(X) - mean(Y)
+ *   sd_pred, sd_target = standard deviations of X and Y with ddof = 1
+ *   mse_mean  = (1/m) sum_j (mean(X) - y_j)^2
+ * and the int64 [T][n+1] rank histogram gets 1 in bin r = #{i : x_i < y_j} for each y_j (a tie is not below).  A
+ * column holding any non-finite value gets NaN in every map and adds nothing to the histogram.  Sums are taken after a
+ * per-column shift, so accuracy does not depend on the data's offset; the maps are bitwise reproducible (no float
+ * atomics).  hist is cleared by one cudaMemsetAsync on the stream, then ONE kernel reads every input value once.
+ * Rejects n or m outside [2, 1024], T outside [1, 65535], HW < 1 and NULL pointers with CESM_ERR_INVALID, before
+ * anything is enqueued. */
+int cesm_ensemble_scores(const float* pred, const float* target, float* crps, float* bias, float* sd_pred,
+                         float* sd_target, float* mse_mean, long long* hist, int T, int n, int m, long long HW,
+                         void* stream);
+
 #ifdef __cplusplus
 }
 #endif

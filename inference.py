@@ -132,12 +132,19 @@ def write_prediction_netcdf(path, pred_tmhw: np.ndarray, stack_coord=None, membe
 def write_netcdf_variable(path, name, data, coords, attrs):
     """One float32 variable `name` over the dimensions `coords` = [(dim name, coordinate values or None for
     arange, length), ...] with its coordinate variables and attributes, as classic NetCDF-3 through scipy."""
+    write_netcdf_variables(path, coords, [(name, data, tuple(dim for dim, _, _ in coords), attrs)])
+
+
+def write_netcdf_variables(path, dims, variables, attrs=None):
+    """Several variables sharing dimensions, as classic NetCDF-3 through scipy.  `dims` = [(dim name, coordinate
+    values or None for arange, length), ...] (each gets a coordinate variable); `variables` = [(name, data, dim names,
+    attributes), ...], written as float32, or int32 when `data` is an integer array; `attrs` are global attributes."""
     from scipy.io import netcdf_file
     d = os.path.dirname(path)
     if d:
         os.makedirs(d, exist_ok=True)
     with netcdf_file(path, "w", version=2) as f:
-        for dim, vals, n in coords:
+        for dim, vals, n in dims:
             f.createDimension(dim, n)
             vals = np.arange(n) if vals is None else np.asarray(vals)
             if vals.shape != (n,):
@@ -145,16 +152,20 @@ def write_netcdf_variable(path, name, data, coords, attrs):
             vals = vals.astype(np.float64 if vals.dtype.kind == "f" else np.int32)
             v = f.createVariable(dim, vals.dtype, (dim,))
             v[:] = vals
-        v = f.createVariable(name, np.float32, tuple(dim for dim, _, _ in coords))
-        v[:] = np.asarray(data, dtype=np.float32)
-        for k, val in attrs.items():
-            setattr(v, k, val)
+        for name, data, vdims, vattrs in variables:
+            data = np.asarray(data)
+            dtype = np.int32 if data.dtype.kind in "iub" else np.float32
+            v = f.createVariable(name, dtype, tuple(vdims))
+            v[:] = data.astype(dtype)
+            for k, val in vattrs.items():
+                setattr(v, k, val)
+        for k, val in (attrs or {}).items():
+            setattr(f, k, val)
 
 
-def _parse_args(argv=None):
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--ckpt", required=True)
-    ap.add_argument("--batch_size", type=int, default=16)
+def add_sampler_args(ap):
+    """The sampler flags shared by the generating CLIs (inference.py, evaluate.py); check them with
+    check_sampler_args."""
     ap.add_argument("--steps", type=int, default=None, help="reverse steps (default: all T)")
     ap.add_argument("--ddim_steps", type=int, default=None,
                     help="generate with a strided DDIM chain of this many UNet calls instead of the T-step DDPM chain")
@@ -169,10 +180,10 @@ def _parse_args(argv=None):
     ap.add_argument("--guidance", type=float, default=0.0,
                     help="classifier-free guidance weight w >= 0: sample with (1 + w) out_cond - w out_null (0 = off); "
                          "needs a checkpoint trained with train.cond_drop_prob > 0")
-    ap.add_argument("--members", type=int, default=2)
-    ap.add_argument("--times", type=int, default=4)
-    ap.add_argument("--out", default="pred.npy")
-    a = ap.parse_args(argv)
+
+
+def check_sampler_args(ap, a):
+    """Reject the sampler-flag combinations add_sampler_args' flags cannot express (ap.error: exit status 2)."""
     if a.steps is not None and a.ddim_steps is not None:
         ap.error("--steps and --ddim_steps are mutually exclusive")
     if a.dpm_steps is not None and (a.steps is not None or a.ddim_steps is not None):
@@ -183,6 +194,18 @@ def _parse_args(argv=None):
         ap.error(f"--seed must be in [0, 2**64), got {a.seed}")
     if not a.guidance >= 0 or a.guidance == float("inf"):  # also rejects NaN
         ap.error(f"--guidance must be a finite number >= 0, got {a.guidance}")
+
+
+def _parse_args(argv=None):
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--ckpt", required=True)
+    ap.add_argument("--batch_size", type=int, default=16)
+    add_sampler_args(ap)
+    ap.add_argument("--members", type=int, default=2)
+    ap.add_argument("--times", type=int, default=4)
+    ap.add_argument("--out", default="pred.npy")
+    a = ap.parse_args(argv)
+    check_sampler_args(ap, a)
     return a
 
 
